@@ -5,7 +5,7 @@ Headline metric (BASELINE.json): ms per updateMap+inflation @4k^2 grid (config C
 static + obstacle layer fed by 8 observations x 360 ray-cast beams, inflation 1.0 m => R = 20 cells, full window);
 the DWA half of the metric (trajectories scored / s, configs C2 and C4) is reported in the same line under "dwa".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 * value   : device time per update cycle with every input already resident in HBM (CUDA events on the costmap's own
             stream, L2 flushed between cycles), max over ranks.  N > 1 runs N independent replicas (a single costmap
@@ -14,12 +14,18 @@ the DWA half of the metric (trajectories scored / s, configs C2 and C4) is repor
             window into pinned memory inside the timed region.
 * roofline: the fused reset+merge+inflation sweep kernel against the measured HBM copy bandwidth.
 * cpu_baseline / --impl reference: the reference's own CPU code (oracle/_ref, else our port) on the host cores.
+* --steps K: the number of timed C3 cycles (value, e2e), C2 calls, C4 sweeps and C5 fleet steps.
+* --dump-outputs DIR: after the timed steps, what the last timed C3 cycle (and, unless --no-dwa, the last timed C2
+            call, C4 sweep and C5 fleet step) handed back to its caller, as DIR/<name>.npy (float32 / float64, under
+            64 MB in all; rank 0's share when N > 1).  The inputs are seeded, so two builds run with the same arguments
+            can be compared array by array.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -144,6 +150,32 @@ def voxel_numbers(api_factory, reps, sync=None, size=None):
 
 def obs_bytes(obs):
     return sum(o["points"].nbytes + 64 for o in obs)
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def master_sample(master):
+    """Half of the master grid's cells, a fixed seeded choice kept in row-major order, as float32: the whole C3 grid
+    in float32 would fill the dump's 64 MB on its own."""
+    flat = master.reshape(-1)
+    idx = np.sort(np.random.default_rng(0).choice(flat.size, flat.size // 2, replace=False))
+    return flat[idx].astype(np.float32)
+
+
+def result_row(r):
+    """A findBestPath result as float64 [cost, xv, yv, thetav, best_index, n_samples, n_scored]."""
+    return np.array([r["cost"], r["xv"], r["yv"], r["thetav"], r["best_index"], r["n_samples"], r["n_scored"]],
+                    np.float64)
+
+
+def write_outputs(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 
@@ -449,10 +481,11 @@ def cpu_baseline_c3():
 
 
 
-def run_native_dwa(api, torch, dist, rank, world, local_rank, steps):
+def run_native_dwa(api, torch, dist, rank, world, local_rank, steps, dump=None):
     """C2 latency (synchronous findBestPath through the C ABI, host pose in / result out) and C4 throughput.
     With world > 1 the C4 sample range is sharded over the ranks: each scores its slice, the per-rank (cost, index)
-    minima are all-gathered over NCCL and every rank finishes with the same winner."""
+    minima are all-gathered over NCCL and every rank finishes with the same winner.  `dump` (dict or None) receives
+    the results of the last timed C2 call and C4 sweep."""
     dev = f"cuda:{local_rank}"
     grid = inflate_local(api, local_map_c2(), device=local_rank)
     out = {}
@@ -462,10 +495,13 @@ def run_native_dwa(api, torch, dist, rank, world, local_rank, steps):
         r2 = call2.find_best_path()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    reps = max(20, steps)
+    reps = steps
     for _ in range(reps):
         r2 = call2.find_best_path()
     out["c2_findBestPath_us"] = 1e6 * (time.perf_counter() - t0) / reps
+    if dump is not None:
+        dump["dwa_c2_result"] = result_row(r2)
+        dump["dwa_c2_points"] = r2["points"].copy()
     out["c2_samples"] = int(r2["n_samples"])
     out["c2_best_index"] = int(r2["best_index"])
     out["c2_traj_per_s"] = r2["n_samples"] / (out["c2_findBestPath_us"] * 1e-6)
@@ -499,7 +535,7 @@ def run_native_dwa(api, torch, dist, rank, world, local_rank, steps):
     if dist is not None:
         dist.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n_sweeps = max(5, steps)
+    n_sweeps = steps
     e0.record(stream)
     t0 = time.perf_counter()
     for _ in range(n_sweeps):
@@ -508,6 +544,9 @@ def run_native_dwa(api, torch, dist, rank, world, local_rank, steps):
     torch.cuda.synchronize()
     wall = (time.perf_counter() - t0) / n_sweeps
     sweep_s = max(wall, 1e-3 * e0.elapsed_time(e1) / n_sweeps)
+    if dump is not None:
+        dump["dwa_c4_result"] = result_row(r4)
+        dump["dwa_c4_points"] = r4["points"].copy()
     if dist is not None:
         t = torch.tensor([sweep_s], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -550,10 +589,11 @@ def fleet_inputs(ids):
             np.array([r["pose"] for r in robots]), np.array([r["vel"] for r in robots]), [r["plan"] for r in robots])
 
 
-def run_native_fleet(api, torch, dist, rank, world, local_rank, steps):
+def run_native_fleet(api, torch, dist, rank, world, local_rank, steps, dump=None):
     """C5: 4096 independent robots per control cycle, partitioned over the ranks (no collective): every robot's raw
     local map is inflated and its 20 x 1 x 20 velocity samples are scored.  Timed through the C ABI with host buffers:
-    `step` = poses/velocities in, results out (maps already resident); `e2e` additionally uploads all raw maps."""
+    `step` = poses/velocities in, results out (maps already resident); `e2e` additionally uploads all raw maps.
+    `dump` (dict or None) receives this rank's per-robot results of the last timed step."""
     from navigation_b200 import sharding
     n_total = C5["n_robots"]
     lo, hi = sharding.split_range(n_total, rank, world)
@@ -565,8 +605,8 @@ def run_native_fleet(api, torch, dist, rank, world, local_rank, steps):
     poses = np.ascontiguousarray(poses)
     vels = np.ascontiguousarray(vels)
     for _ in range(3):
-        fleet.step_raw(poses, vels)
-    reps = max(5, min(steps, 10))
+        results = fleet.step_raw(poses, vels)  # the result array every step writes
+    reps = steps
 
     def timed(fn):
         torch.cuda.synchronize()
@@ -594,6 +634,9 @@ def run_native_fleet(api, torch, dist, rank, world, local_rank, steps):
         fleet.set_maps(raw_pinned, origins)
         fleet.step_raw(poses, vels)
     e2e_s = timed(full)
+    if dump is not None:
+        dump["fleet_c5_results"] = np.array([[r.cost, r.xv, r.yv, r.thetav, r.best_index, r.n_samples, r.n_scored]
+                                             for r in results], np.float64)
     res = fleet.step(poses, vels)
     n_traj = sum(r["n_samples"] for r in res)
     n_valid = sum(r["cost"] >= 0 for r in res)
@@ -680,8 +723,12 @@ def run_native(args, rank, world, local_rank):
     import torch
     import navigation_b200
     from navigation_b200 import build
-    build.build()
-    api = navigation_b200.load()
+    if build.needs_build():
+        # sources newer than the library build() left: compile them, outside the (possibly read-only) tree
+        scratch = tempfile.TemporaryDirectory(prefix="navgpu-bench-")  # removed when the run ends
+        api = navigation_b200.Api(build.build(out=os.path.join(scratch.name, "libnavgpu.so")))
+    else:
+        api = navigation_b200.load()
     if api.device_count() == 0:
         raise SystemExit("bench.py: no CUDA device; libnavgpu has no CPU fallback")
     torch.cuda.set_device(local_rank)
@@ -726,6 +773,7 @@ def run_native(args, rank, world, local_rank):
     launches = api.launch_count() - launches0
     step_ms = [a.elapsed_time(b) for a, b in zip(starts, stops)]
     ms_per_step = float(np.mean(step_ms))
+    dump = {"costmap_c3_master_sample": master_sample(cm.get())} if args.dump_outputs and rank == 0 else None
 
     # ---- the same cycles again with the handle's events ON: durations of the sweep kernels for the roofline
     cm.set_profiling(True)
@@ -794,9 +842,9 @@ def run_native(args, rank, world, local_rank):
     assert np.array_equal(out_np, cm.get()), "host mirror differs from the device master grid"
     e2e_ms, h2d, d2h = e2e["changed_tiles"]
     e2e_full_ms = e2e["full_window"][0]
-    dwa = None if args.no_dwa else run_native_dwa(api, torch, dist, rank, world, local_rank, args.steps)
+    dwa = None if args.no_dwa else run_native_dwa(api, torch, dist, rank, world, local_rank, args.steps, dump)
     if dwa is not None:
-        dwa.update(run_native_fleet(api, torch, dist, rank, world, local_rank, args.steps))
+        dwa.update(run_native_fleet(api, torch, dist, rank, world, local_rank, args.steps, dump))
     launches = api.launch_count() - launches0 if not args.no_dwa else launches
     clocks = sampler.summary()
 
@@ -881,6 +929,8 @@ def run_native(args, rank, world, local_rank):
                 ref_api = pyoracle.load(kind)
                 line["trajectory_planner"]["cpu_baseline"] = dict(
                     tp_numbers(ref_api, inflate_local(ref_api, local_map_c2()), reps=5), kind=kind, cores=1)
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -894,7 +944,14 @@ def main():
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-dwa", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed C3 cycle, C2 call, C4 sweep and C5 step returned as "
+                         "DIR/<name>.npy (bench_outputs/ is git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
         run_reference(args, rank)

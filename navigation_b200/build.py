@@ -29,13 +29,14 @@ def needs_build():
     return any(os.path.getmtime(p) > t for p in deps)
 
 
-def build(force=False, verbose=False):
-    if not force and not needs_build():
+def build(force=False, verbose=False, out=LIB):
+    """Compiles the library to `out` (in-tree by default, where it is only rebuilt when a source is newer)."""
+    if out == LIB and not force and not needs_build():
         return LIB
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", LIB] + sources()
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + sources()
     subprocess.check_call(cmd)
-    return LIB
+    return out
 
 
 if __name__ == "__main__":

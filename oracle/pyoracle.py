@@ -148,9 +148,22 @@ def _declare(lib, prefix):
     return sig
 
 
+def reference_dir():
+    """The checkout of the reference's sources (ROS navigation) that oracle/_ref is compiled from: the directory the
+    NAVIGATION_REFERENCE environment variable names, or None.  Without it the checkers under oracle/_ref are not
+    built and the tests that run them skip."""
+    d = os.environ.get("NAVIGATION_REFERENCE")
+    return d if d and os.path.isdir(d) else None
+
+
+def make(*targets):
+    """oracle/Makefile; the targets under oracle/_ref need reference_dir()."""
+    ref = reference_dir()
+    subprocess.check_call(["make", "-s", "-C", HERE, *targets] + ([f"REF={ref}"] if ref else []))
+
+
 def build(kind="port"):
-    target = {"port": "oracle", "reference": "ref", "reference_hoisted": "ref_hoisted"}[kind]
-    subprocess.check_call(["make", "-s", "-C", HERE, target])
+    make({"port": "oracle", "reference": "ref", "reference_hoisted": "ref_hoisted"}[kind])
 
 
 def lib_path(kind):

@@ -24,10 +24,10 @@ def ref():
     """The reference's own compiled sources (oracle/_ref/libnavref.so); only where it was built."""
     from oracle import pyoracle
     if not pyoracle.available("reference"):
-        if os.path.isdir("/root/reference"):
+        if pyoracle.reference_dir():
             pyoracle.build("reference")
         else:
-            pytest.skip("oracle/_ref/libnavref.so not present (needs /root/reference to build)")
+            pytest.skip("oracle/_ref/libnavref.so not present (needs NAVIGATION_REFERENCE to build)")
     return pyoracle.load("reference")
 
 

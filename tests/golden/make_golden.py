@@ -1,6 +1,6 @@
 """Generates the golden fixtures in this directory from the REFERENCE's own compiled code (oracle/_ref/libnavref.so).
 
-Run in the build container (where /root/reference exists):   python tests/golden/make_golden.py
+Run with NAVIGATION_REFERENCE naming the reference's sources:   python tests/golden/make_golden.py
 Inputs are regenerated from the seed by tests/scenarios.py; only the reference's outputs are stored.
 """
 import os

@@ -1,12 +1,15 @@
 """Drop-in check of the C++ adapters (navigation_b200/plugin) next to the reference's own classes.
 
-oracle/_ref/dropin_harness is built here, where /root/reference exists (`make -C oracle dropin`): the adapters and
-tests/cpp/dropin_harness.cpp are compiled against the reference's headers and linked with the reference's unmodified
-hot-path sources (oracle/_ref/libnavref.so) and libnavgpu.so.  The binary travels to the GPU box with the snapshot."""
+oracle/_ref/dropin_harness is built where NAVIGATION_REFERENCE names the reference's sources (`make -C oracle dropin
+REF=...`): the adapters and tests/cpp/dropin_harness.cpp are compiled against the reference's headers and linked with
+the reference's unmodified hot-path sources (oracle/_ref/libnavref.so) and libnavgpu.so.  A harness built on one
+machine may be run on another that has the library but not the sources."""
 import os
 import subprocess
 
 import pytest
+
+from oracle import pyoracle
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HARNESS = os.path.join(ROOT, "oracle", "_ref", "dropin_harness")
@@ -15,14 +18,14 @@ HARNESS = os.path.join(ROOT, "oracle", "_ref", "dropin_harness")
 def build_harness():
     from navigation_b200 import build
     build.build()
-    subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref", "dropin"])
+    pyoracle.make("ref", "dropin")
 
 
 def test_dropin_harness_builds_against_reference_headers():
     """GpuInflationLayer : costmap_2d::Layer, GpuLayeredCostmap and GpuScoredSamplingPlanner : TrajectorySearch compile
     against the reference's own headers and link with its compiled sources (no GPU needed for that)."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("needs /root/reference")
+    if not pyoracle.reference_dir():
+        pytest.skip("needs NAVIGATION_REFERENCE")
     build_harness()
     assert os.access(HARNESS, os.X_OK)
 
@@ -36,10 +39,10 @@ def test_adapters_match_reference_classes(cuda):
     TrajectoryPlanner through the same public calls; D: GpuLayeredCostmap fed with LaserScans == the checker's stack fed
     with the clouds of the restated ingest path."""
     if not os.path.exists(HARNESS):
-        if os.path.isdir("/root/reference"):
+        if pyoracle.reference_dir():
             build_harness()
         else:
-            pytest.skip("oracle/_ref/dropin_harness was not built (needs /root/reference)")
+            pytest.skip("oracle/_ref/dropin_harness was not built (needs NAVIGATION_REFERENCE)")
     r = subprocess.run([HARNESS], capture_output=True, text=True, timeout=300)
     print(r.stdout)
     assert r.returncode == 0, r.stdout + r.stderr

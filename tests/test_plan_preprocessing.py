@@ -115,13 +115,11 @@ def test_batched_kernels_edge_cases(cuda, port):
 
 def reference_goal_functions():
     from oracle import pyoracle
-    import os
     if not pyoracle.GoalRef.available():
-        if os.path.isdir("/root/reference"):
-            import subprocess
-            subprocess.check_call(["make", "-s", "-C", os.path.dirname(pyoracle.__file__), "goalref"])
+        if pyoracle.reference_dir():
+            pyoracle.make("goalref")
         else:
-            pytest.skip("oracle/_ref/libgoalref.so not present (needs /root/reference to build)")
+            pytest.skip("oracle/_ref/libgoalref.so not present (needs NAVIGATION_REFERENCE to build)")
     return pyoracle.GoalRef()
 
 
