@@ -377,7 +377,7 @@ int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_confi
                         const double* footprint_xy, int n_footprint, int device);
 int navgpu_fleet_destroy(navgpu_fleet* f);
 /* raw (un-inflated) local maps [n][size_y][size_x] and their world origins [n][2], HOST memory */
-int navgpu_fleet_set_maps(navgpu_fleet* f, const uint8_t* raw_maps, const double* origins_xy);
+int navgpu_fleet_set_maps(navgpu_fleet* f, const uint8_t* raw_maps, const double* origins_xy);  /* not on sensing fleets */
 /* DWAPlanner::updatePlanAndLocalCosts for every robot: poses [n][3], concatenated plan points, offsets [n + 1] */
 int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* plan_xy, const int32_t* plan_offsets);
 int navgpu_fleet_reset_oscillation(navgpu_fleet* f);
@@ -386,6 +386,41 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
 /* inflated local costmap of one robot, HOST size_y x size_x */
 int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out);
 int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out);
+/* ---- Fleet mode with sensing: every robot runs move_base's local costmap itself --------------------------------
+ * A second kind of fleet.  Every robot has a rolling size_x x size_y LayeredCostmap (rolling_window: true) with the
+ * plugins [ObstacleLayer, InflationLayer], fed by the robot's own scans, followed by DWAPlanner.  navgpu_fleet_step then
+ * runs, per robot, LayeredCostmap::updateMap(pose) (layered_costmap.cpp:79-150): the rolling origin, ObstacleLayer::
+ * updateBounds (ray-trace clearing of every clearing source before any marking, then marking, then the footprint),
+ * InflationLayer::updateBounds (its own last_* bounds per robot; the whole map on the first step), the cycle's window,
+ * resetMap of the window, ObstacleLayer::updateCosts (footprint polygon to FREE_SPACE, then Overwrite or Max) and
+ * InflationLayer::updateCosts with inflation mode 0 of navgpu_inflation_set_mode -- bit for bit what one
+ * navgpu_costmap with an obstacle and an inflation layer computes -- and then DWAPlanner::findBestPath on the result.
+ * Cells outside a robot's window keep their shifted previous values, as in the reference.  Every robot's maps start at
+ * origin (0, 0) filled with the default value.  One CTA holds a robot's obstacle grid and master grid in shared
+ * memory: maps, inflation radii and footprints beyond what fits it are refused with NAVGPU_ERR_UNSUPPORTED. */
+typedef struct {
+  double inflation_radius, cost_scaling_factor; /* InflationLayer (defaults 0.55, 10) */
+  double max_obstacle_height;                   /* ObstacleLayer (default 2.0) */
+  int32_t combination_method;                   /* 0 updateWithOverwrite, 1 updateWithMax (default) */
+  int32_t footprint_clearing;                   /* default 1 */
+  int32_t track_unknown;                        /* default value NO_INFORMATION (255) instead of FREE_SPACE (0) */
+  int32_t pad_;
+} navgpu_fleet_costmap_config;
+int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                                const double* footprint_xy, int n_footprint, int device);
+/* Robot r's sources are scans[offsets[r] .. offsets[r + 1]) (navgpu_laser_scan records as navgpu_obstacle_set_scans
+ * takes them: LaserScan ranges or is_cloud sensor-frame points).  They replace every robot's previous sources and
+ * persist until the next call, like the observations of navgpu_obstacle_set_scans.  All robots' scans are projected in
+ * one launch.  offsets: n_robots + 1 non-decreasing entries. */
+int navgpu_fleet_set_scans(navgpu_fleet* f, const navgpu_laser_scan* scans, const int32_t* offsets);
+/* per robot, after the last navgpu_fleet_step: the ObstacleLayer's own grid (HOST size_y x size_x) */
+int navgpu_fleet_get_layer(navgpu_fleet* f, int robot, uint8_t* host_out);
+/* per robot, after the last navgpu_fleet_step: the rolled origin and the cycle's window {x0, xn, y0, yn} */
+int navgpu_fleet_get_geometry(navgpu_fleet* f, int robot, double origin_out[2], int32_t window_out[4]);
+/* device time (ms, CUDA events) of the last scan projection (navgpu_fleet_set_scans; 0 when it had no points) and of the
+ * last costmap update of all robots (navgpu_fleet_step); synchronises the fleet's stream */
+int navgpu_fleet_last_timing(navgpu_fleet* f, float* project_ms, float* costmap_ms);
 
 
 /* ---- legacy base_local_planner::TrajectoryPlanner (SURVEY.md 8f-4) ---------------------------------------------

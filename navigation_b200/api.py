@@ -51,6 +51,13 @@ class LaserScan(C.Structure):
                 ("clearing", C.c_int32), ("is_cloud", C.c_int32), ("pad_", C.c_int32)]
 
 
+class FleetCostmapConfig(C.Structure):
+    """navgpu_fleet_costmap_config"""
+    _fields_ = [("inflation_radius", C.c_double), ("cost_scaling_factor", C.c_double),
+                ("max_obstacle_height", C.c_double), ("combination_method", C.c_int32),
+                ("footprint_clearing", C.c_int32), ("track_unknown", C.c_int32), ("pad_", C.c_int32)]
+
+
 class TpConfig(C.Structure):
     """navgpu_tp_config: the legacy base_local_planner::TrajectoryPlanner's parameters."""
     _fields_ = [(n, C.c_double) for n in (
@@ -180,6 +187,12 @@ SIGNATURES = {
     "navgpu_fleet_step": (C.c_int, [C.c_void_p, _f64p, _f64p, C.POINTER(DwaResult)]),
     "navgpu_fleet_get_costmap": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
     "navgpu_fleet_get_oscillation_mask": (C.c_int, [C.c_void_p, C.c_int, _i32p]),
+    "navgpu_fleet_create_sensing": (C.c_int, [_vpp, C.c_int, C.POINTER(DwaConfig), C.c_uint32, C.c_uint32, C.c_double,
+                                              C.POINTER(FleetCostmapConfig), _f64p, C.c_int, C.c_int]),
+    "navgpu_fleet_set_scans": (C.c_int, [C.c_void_p, C.POINTER(LaserScan), _i32p]),
+    "navgpu_fleet_get_layer": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
+    "navgpu_fleet_get_geometry": (C.c_int, [C.c_void_p, C.c_int, _f64p, _i32p]),
+    "navgpu_fleet_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "navgpu_tp_default_config": (None, [C.POINTER(TpConfig)]),
     "navgpu_tp_create": (C.c_int, [_vpp, C.POINTER(TpConfig), C.c_uint32, C.c_uint32, C.c_double, _f64p, C.c_int, C.c_int]),
     "navgpu_tp_destroy": (C.c_int, [C.c_void_p]),
@@ -193,6 +206,34 @@ SIGNATURES = {
     "navgpu_tp_get_grid": (C.c_int, [C.c_void_p, C.c_int, _f64p]),
     "navgpu_tp_last_sample_count": (C.c_int, [C.c_void_p, _i32p]),
 }
+
+
+def pack_scans(scans):
+    """The navgpu_laser_scan array for a list of scan dicts (see Costmap.set_scans), and the arrays it points into."""
+    arr = (LaserScan * max(1, len(scans)))()
+    keep = []
+    for k, sc in enumerate(scans):
+        s = arr[k]
+        if "points" in sc:  # a PointCloud(2) source: (n, 3) float32 in the sensor frame
+            r = np.ascontiguousarray(sc["points"], dtype=np.float32).reshape(-1, 3)
+            s.is_cloud = 1
+        else:
+            r = np.ascontiguousarray(sc["ranges"], dtype=np.float32)
+            s.is_cloud = 0
+            s.angle_min, s.angle_increment = sc["angle_min"], sc["angle_increment"]
+            s.range_min, s.range_max = sc["range_min"], sc["range_max"]
+        keep.append(r)
+        s.ranges = r.ctypes.data_as(C.POINTER(C.c_float))
+        s.n_ranges = len(r)
+        s.inf_is_valid = int(sc.get("inf_is_valid", 0))
+        for j in range(3):
+            s.translation[j] = sc["translation"][j]
+        for j in range(4):
+            s.rotation_xyzw[j] = sc["rotation_xyzw"][j]
+        s.min_obstacle_height, s.max_obstacle_height = sc["min_obstacle_height"], sc["max_obstacle_height"]
+        s.obstacle_range, s.raytrace_range = sc["obstacle_range"], sc["raytrace_range"]
+        s.marking, s.clearing = int(sc.get("marking", True)), int(sc.get("clearing", True))
+    return arr, keep
 
 
 class Costmap:
@@ -296,29 +337,7 @@ class Costmap:
         """On-device observation ingest: scans = list of dicts (ranges, angle_min, angle_increment, range_min,
         range_max, translation, rotation_xyzw, min/max_obstacle_height, obstacle_range, raytrace_range, marking,
         clearing, inf_is_valid)."""
-        arr = (LaserScan * max(1, len(scans)))()
-        keep = []
-        for k, sc in enumerate(scans):
-            s = arr[k]
-            if "points" in sc:  # a PointCloud(2) source: (n, 3) float32 in the sensor frame
-                r = np.ascontiguousarray(sc["points"], dtype=np.float32).reshape(-1, 3)
-                s.is_cloud = 1
-            else:
-                r = np.ascontiguousarray(sc["ranges"], dtype=np.float32)
-                s.is_cloud = 0
-                s.angle_min, s.angle_increment = sc["angle_min"], sc["angle_increment"]
-                s.range_min, s.range_max = sc["range_min"], sc["range_max"]
-            keep.append(r)
-            s.ranges = r.ctypes.data_as(C.POINTER(C.c_float))
-            s.n_ranges = len(r)
-            s.inf_is_valid = int(sc.get("inf_is_valid", 0))
-            for j in range(3):
-                s.translation[j] = sc["translation"][j]
-            for j in range(4):
-                s.rotation_xyzw[j] = sc["rotation_xyzw"][j]
-            s.min_obstacle_height, s.max_obstacle_height = sc["min_obstacle_height"], sc["max_obstacle_height"]
-            s.obstacle_range, s.raytrace_range = sc["obstacle_range"], sc["raytrace_range"]
-            s.marking, s.clearing = int(sc.get("marking", True)), int(sc.get("clearing", True))
+        arr, _keep = pack_scans(scans)
         self.api.check(self.lib.navgpu_obstacle_set_scans(self.h, layer, arr, len(scans)))
 
     def get_cloud(self, layer, index, capacity=1 << 16):
@@ -758,7 +777,9 @@ class Fleet:
     """N independent robots per control cycle (navgpu_fleet_*): local-costmap inflation + DWA scoring, batched."""
 
     def __init__(self, api, n_robots, size_x, size_y, resolution, footprint_xy, inflation_radius=0.55,
-                 cost_scaling_factor=10.0, device=0, **overrides):
+                 cost_scaling_factor=10.0, device=0, sensing=None, **overrides):
+        """sensing: None for a raw-map fleet (set_maps), else a FleetCostmapConfig: every robot then builds its own
+        rolling local costmap from its scans (set_scans; see Api.fleet_sensing)."""
         self.api, self.lib, self.n = api, api.lib, n_robots
         self.size_x, self.size_y = size_x, size_y
         self.cfg = DwaConfig()
@@ -767,8 +788,14 @@ class Fleet:
             setattr(self.cfg, k, v)
         fp = np.ascontiguousarray(footprint_xy, dtype=np.float64).reshape(-1, 2)
         h = C.c_void_p()
-        api.check(self.lib.navgpu_fleet_create(C.byref(h), n_robots, C.byref(self.cfg), size_x, size_y, resolution,
-                                               inflation_radius, cost_scaling_factor, _p(fp, _f64p), fp.shape[0], device))
+        if sensing is None:
+            api.check(self.lib.navgpu_fleet_create(C.byref(h), n_robots, C.byref(self.cfg), size_x, size_y, resolution,
+                                                   inflation_radius, cost_scaling_factor, _p(fp, _f64p), fp.shape[0],
+                                                   device))
+        else:
+            api.check(self.lib.navgpu_fleet_create_sensing(C.byref(h), n_robots, C.byref(self.cfg), size_x, size_y,
+                                                           resolution, C.byref(sensing), _p(fp, _f64p), fp.shape[0],
+                                                           device))
         self.h = h
         self._results = (DwaResult * n_robots)()
 
@@ -818,6 +845,34 @@ class Fleet:
         self.api.check(self.lib.navgpu_fleet_get_oscillation_mask(self.h, robot, C.byref(m)))
         return int(m.value)
 
+    def set_scans(self, scans_per_robot):
+        """Sensing fleets: scans_per_robot[r] = list of robot r's scan dicts (the format of Costmap.set_scans); they
+        replace every robot's previous sources."""
+        assert len(scans_per_robot) == self.n
+        off = np.zeros(self.n + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(s) for s in scans_per_robot])
+        arr, _keep = pack_scans([s for robot in scans_per_robot for s in robot])
+        self.api.check(self.lib.navgpu_fleet_set_scans(self.h, arr, _p(off, _i32p)))
+
+    def layer(self, robot):
+        """Sensing fleets: robot's ObstacleLayer grid after the last step."""
+        out = np.empty((self.size_y, self.size_x), dtype=np.uint8)
+        self.api.check(self.lib.navgpu_fleet_get_layer(self.h, robot, _p(out, _u8p)))
+        return out
+
+    def geometry(self, robot):
+        """Sensing fleets: ((origin_x, origin_y), (x0, xn, y0, yn)) of robot's last step."""
+        o = np.zeros(2)
+        w = np.zeros(4, dtype=np.int32)
+        self.api.check(self.lib.navgpu_fleet_get_geometry(self.h, robot, _p(o, _f64p), _p(w, _i32p)))
+        return (float(o[0]), float(o[1])), tuple(int(v) for v in w)
+
+    def last_timing(self):
+        """Sensing fleets: device ms of the last scan projection and of the last costmap update of all robots."""
+        a, b = C.c_float(), C.c_float()
+        self.api.check(self.lib.navgpu_fleet_last_timing(self.h, C.byref(a), C.byref(b)))
+        return float(a.value), float(b.value)
+
 
 class Api:
     name = "cuda"
@@ -854,6 +909,16 @@ class Api:
 
     def fleet(self, *a, **k):
         return Fleet(self, *a, **k)
+
+    def fleet_sensing(self, n, sx, sy, res, footprint, inflation_radius=0.55, cost_scaling_factor=10.0,
+                      combination_method=1, footprint_clearing=True, max_obstacle_height=2.0, track_unknown=False,
+                      device=0, **dwa_overrides):
+        """A fleet whose robots each run a rolling sx x sy local costmap [ObstacleLayer, InflationLayer] fed by their
+        own scans (Fleet.set_scans), then DWAPlanner (navgpu_fleet_create_sensing)."""
+        cm = FleetCostmapConfig(inflation_radius=inflation_radius, cost_scaling_factor=cost_scaling_factor,
+                                max_obstacle_height=max_obstacle_height, combination_method=combination_method,
+                                footprint_clearing=int(footprint_clearing), track_unknown=int(track_unknown))
+        return Fleet(self, n, sx, sy, res, footprint, device=device, sensing=cm, **dwa_overrides)
 
     def trajectory_planner(self, *a, **k):
         return TrajectoryPlanner(self, *a, **k)

@@ -208,8 +208,13 @@ __global__ void k_project_scans(const ScanRec* __restrict__ recs, int n_scans, c
                                 float* __restrict__ xyz, int total) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= total) return;
-  int k = 0;
-  while (k + 1 < n_scans && recs[k + 1].first_point - recs[0].first_point <= t) ++k;
+  // the last record that starts at or before point t (binary search: a fleet projects thousands of records at once)
+  int k = 0, hi = n_scans - 1;
+  while (k < hi) {
+    const int mid = (k + hi + 1) >> 1;
+    if (recs[mid].first_point - recs[0].first_point <= t) k = mid;
+    else hi = mid - 1;
+  }
   const ScanRec& r = recs[k];
   const int i = t - (r.first_point - recs[0].first_point);
   const float nanf_ = __int_as_float(0x7fc00000);

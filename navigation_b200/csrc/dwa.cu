@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "dwa_kernels.cuh"
+#include "fleet_costmap.cuh"
 #include "tp_kernels.cuh"
 
 using namespace navgpu;
@@ -1030,7 +1031,8 @@ struct navgpu_fleet {
   unsigned sx = 0, sy = 0, stride = 0;  // rows per robot in the stacked grid
   double res = 0;
   navgpu_dwa_config cfg;
-  navgpu_costmap* costmap = nullptr;
+  navgpu_costmap* costmap = nullptr;  // raw-map fleets: the stacked costmap
+  FleetCostmap* sensing = nullptr;    // sensing fleets (navgpu_fleet_create_sensing): the robots' rolling costmaps
   int static_layer = -1;
   cudaStream_t stream = nullptr;  // the costmap's stream
   uint8_t* d_raw = nullptr;       // n x sy x sx: the raw maps as they arrive from the host
@@ -1065,6 +1067,41 @@ struct navgpu_fleet {
   std::vector<size_t> plan_off;  // per robot x 3 plans: offset (in points) into d_plans
 };
 
+// what every fleet holds for its planner side: the DWAPlanner parameters and critic scales ...
+static void init_planner_scalars(navgpu_fleet* f, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                 uint32_t size_y, double resolution, const double* footprint_xy, int n_footprint,
+                                 int device) {
+  f->device = device;
+  f->n = n_robots;
+  f->sx = size_x; f->sy = size_y;
+  f->res = resolution;
+  f->cfg = *cfg;
+  f->footprint.assign(footprint_xy, footprint_xy + 2 * n_footprint);
+  f->path_scale = resolution * cfg->path_distance_bias * 0.5;
+  f->goal_scale = resolution * cfg->goal_distance_bias * 0.5;
+  f->obstacle_scale = resolution * cfg->occdist_scale;
+}
+
+// ... and its per-robot buffers (device and host)
+static int alloc_planner_side(navgpu_fleet* f) {
+  const int n_robots = f->n;
+  NAVGPU_CUDA(cudaSetDevice(f->device));
+  NAVGPU_CUDA(cudaMalloc(&f->d_robots, sizeof(FleetRobot) * n_robots));
+  NAVGPU_CUDA(cudaMalloc(&f->d_dist, size_t(n_robots) * 4 * f->sx * f->sy * sizeof(uint32_t)));
+  NAVGPU_CUDA(cudaMalloc(&f->d_generated, sizeof(unsigned) * n_robots));
+  NAVGPU_CUDA(cudaMemset(f->d_generated, 0, sizeof(unsigned) * n_robots));
+  NAVGPU_CUDA(cudaMalloc(&f->d_results, sizeof(DwaDeviceResult) * n_robots));
+  NAVGPU_CUDA(cudaMallocHost(&f->h_results, sizeof(DwaDeviceResult) * n_robots));
+  f->origins.assign(size_t(2) * n_robots, 0.0);
+  f->plan.resize(n_robots); f->adj_path.resize(n_robots); f->adj_front.resize(n_robots); f->adj_align.resize(n_robots);
+  f->align_is_path.assign(n_robots, 0);
+  f->align_scale.assign(n_robots, 0.0);
+  f->osc.resize(n_robots);
+  f->res_v.assign(size_t(3) * n_robots, 0.0);
+  f->h_robots.resize(n_robots);
+  return NAVGPU_OK;
+}
+
 extern "C" {
 
 int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x, uint32_t size_y,
@@ -1081,15 +1118,8 @@ int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_confi
     return fail(NAVGPU_ERR_UNSUPPORTED, "fleet inflation radius of %.0f cells exceeds the %u rows between stacked maps",
                 std::ceil(inflation_radius / resolution), kFleetPadRows);
   std::unique_ptr<navgpu_fleet> f(new navgpu_fleet);
-  f->device = device;
-  f->n = n_robots;
-  f->sx = size_x; f->sy = size_y; f->stride = size_y + kFleetPadRows;
-  f->res = resolution;
-  f->cfg = *cfg;
-  f->footprint.assign(footprint_xy, footprint_xy + 2 * n_footprint);
-  f->path_scale = resolution * cfg->path_distance_bias * 0.5;
-  f->goal_scale = resolution * cfg->goal_distance_bias * 0.5;
-  f->obstacle_scale = resolution * cfg->occdist_scale;
+  init_planner_scalars(f.get(), n_robots, cfg, size_x, size_y, resolution, footprint_xy, n_footprint, device);
+  f->stride = size_y + kFleetPadRows;
   if ((unsigned long long)f->stride * n_robots > 0x7fffffffull) return fail(NAVGPU_ERR_UNSUPPORTED, "fleet too large");
   // the stacked costmap: every robot's window is "the whole map" each cycle, like a rolling local costmap
   NAVGPU_TRY(navgpu_costmap_create(&f->costmap, size_x, f->stride * n_robots, resolution, 0.0, 0.0, 0, 0, device));
@@ -1106,22 +1136,36 @@ int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_confi
   NAVGPU_CUDA(cudaMalloc(&f->d_stage, stage_bytes));
   NAVGPU_CUDA(cudaMemset(f->d_stage, 0, stage_bytes));
   NAVGPU_CUDA(cudaMalloc(&f->d_raw, size_t(n_robots) * size_y * size_x));
-  NAVGPU_CUDA(cudaMalloc(&f->d_robots, sizeof(FleetRobot) * n_robots));
-  NAVGPU_CUDA(cudaMalloc(&f->d_dist, size_t(n_robots) * 4 * size_x * size_y * sizeof(uint32_t)));
-  NAVGPU_CUDA(cudaMalloc(&f->d_generated, sizeof(unsigned) * n_robots));
-  NAVGPU_CUDA(cudaMemset(f->d_generated, 0, sizeof(unsigned) * n_robots));
-  NAVGPU_CUDA(cudaMalloc(&f->d_results, sizeof(DwaDeviceResult) * n_robots));
-  NAVGPU_CUDA(cudaMallocHost(&f->h_results, sizeof(DwaDeviceResult) * n_robots));
-  f->origins.assign(size_t(2) * n_robots, 0.0);
-  f->plan.resize(n_robots); f->adj_path.resize(n_robots); f->adj_front.resize(n_robots); f->adj_align.resize(n_robots);
-  f->align_is_path.assign(n_robots, 0);
-  f->align_scale.assign(n_robots, 0.0);
-  f->osc.resize(n_robots);
-  f->res_v.assign(size_t(3) * n_robots, 0.0);
-  f->h_robots.resize(n_robots);
+  NAVGPU_TRY(alloc_planner_side(f.get()));
   *out = f.release();
   return NAVGPU_OK;
 }
+
+int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                                const double* footprint_xy, int n_footprint, int device) {
+  if (!out || !cfg || !cm || n_robots <= 0 || size_x == 0 || size_y == 0 || !(resolution > 0) || n_footprint < 0 ||
+      n_footprint > kMaxFootprint || (n_footprint > 0 && !footprint_xy))
+    return fail(NAVGPU_ERR_INVALID, "bad fleet arguments");
+  if (navgpu_device_count() <= device) return fail(NAVGPU_ERR_CUDA, "no CUDA device %d (libnavgpu has no CPU fallback)", device);
+  if (size_x > 32767 || size_y > 32767) return fail(NAVGPU_ERR_UNSUPPORTED, "local costmap too large");
+  std::unique_ptr<navgpu_fleet> f(new navgpu_fleet);
+  init_planner_scalars(f.get(), n_robots, cfg, size_x, size_y, resolution, footprint_xy, n_footprint, device);
+  f->stride = size_y;  // robot r's master grid starts at row r * size_y
+  int rc = fleet_costmap_create(&f->sensing, n_robots, size_x, size_y, resolution, *cm, footprint_xy, n_footprint, device);
+  if (rc == NAVGPU_OK) {
+    f->stream = fleet_costmap_stream(f->sensing);
+    f->d_master = fleet_costmap_master(f->sensing, &f->pitch);
+    rc = alloc_planner_side(f.get());
+  }
+  if (rc != NAVGPU_OK) {  // free what was allocated (the message of the failure stays)
+    navgpu_fleet_destroy(f.release());
+    return rc;
+  }
+  *out = f.release();
+  return NAVGPU_OK;
+}
+
 
 int navgpu_fleet_destroy(navgpu_fleet* f) {
   if (!f) return NAVGPU_OK;
@@ -1131,6 +1175,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
   cudaFree(f->d_block_cost); cudaFree(f->d_block_index); cudaFree(f->d_generated); cudaFree(f->d_results);
   cudaFreeHost(f->h_results);
   navgpu_costmap_destroy(f->costmap);
+  fleet_costmap_destroy(f->sensing);  // (owns the stream of a sensing fleet)
   delete f;
   return NAVGPU_OK;
 }
@@ -1138,6 +1183,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
 // raw (un-inflated) local maps of all robots, [n][size_y][size_x] in HOST memory, and their world origins [n][2]
 int navgpu_fleet_set_maps(navgpu_fleet* f, const uint8_t* raw_maps, const double* origins_xy) {
   if (!f || !raw_maps || !origins_xy) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->sensing) return fail(NAVGPU_ERR_INVALID, "a sensing fleet builds its maps from scans (navgpu_fleet_set_scans)");
   NAVGPU_CUDA(cudaSetDevice(f->device));
   f->origins.assign(origins_xy, origins_xy + size_t(2) * f->n);
   f->grids_dirty = true;  // the robots' map origins changed
@@ -1203,9 +1249,16 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
   NAVGPU_CUDA(cudaSetDevice(f->device));
   const navgpu_dwa_config& c = f->cfg;
   const int n = f->n;
-  // ---- Path A for all robots: one full-window update of the stacked costmap
-  NAVGPU_TRY(navgpu_grid_layer_touch(f->costmap, f->static_layer, 0, 0, f->sx, f->stride * n));
-  NAVGPU_TRY(navgpu_costmap_update_map_async(f->costmap, 0.0, 0.0, 0.0));
+  if (f->sensing) {
+    // ---- sensing fleet: every robot's rolling origin now (host scalars); the costmap kernel follows once the robots'
+    // new geometry is on its way to the device, below
+    NAVGPU_TRY(fleet_costmap_roll(f->sensing, poses, f->origins.data()));
+    f->grids_dirty = true;
+  } else {
+    // ---- Path A for all robots: one full-window update of the stacked costmap
+    NAVGPU_TRY(navgpu_grid_layer_touch(f->costmap, f->static_layer, 0, 0, f->sx, f->stride * n));
+    NAVGPU_TRY(navgpu_costmap_update_map_async(f->costmap, 0.0, 0.0, 0.0));
+  }
 
   // ---- plans (only when they changed)
   if (f->plans_dirty) {
@@ -1257,6 +1310,8 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
     NAVGPU_CUDA(cudaStreamSynchronize(f->stream));  // pageable source, rewritten below
     f->grids_dirty = false;
   }
+  // sensing fleet: LayeredCostmap::updateMap of every robot, before the wavefronts read the master grids
+  if (f->sensing) NAVGPU_TRY(fleet_costmap_enqueue(f->sensing));
   {  // 4 MapGrid wavefronts per robot, one launch
     navgpu_dwa tmp;  // geometry carrier for launch_mapgrid
     tmp.sx = f->sx; tmp.sy = f->sy; tmp.stream = f->stream;
@@ -1355,6 +1410,7 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
 // inflated local costmap of one robot (HOST, size_y x size_x), for parity checks
 int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out) {
   if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->sensing) return fleet_costmap_get(f->sensing, robot, true, host_out);
   return navgpu_costmap_get_window(f->costmap, 0, (int)(robot * f->stride), (int)f->sx, (int)(robot * f->stride + f->sy), host_out);
 }
 
@@ -1362,6 +1418,30 @@ int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out)
   if (!f || robot < 0 || robot >= f->n || !mask_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   *mask_out = f->osc[robot].mask();
   return NAVGPU_OK;
+}
+
+int navgpu_fleet_set_scans(navgpu_fleet* f, const navgpu_laser_scan* scans, const int32_t* offsets) {
+  if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_set_scans(f->sensing, scans, offsets);
+}
+
+int navgpu_fleet_get_layer(navgpu_fleet* f, int robot, uint8_t* host_out) {
+  if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_get(f->sensing, robot, false, host_out);
+}
+
+int navgpu_fleet_get_geometry(navgpu_fleet* f, int robot, double origin_out[2], int32_t window_out[4]) {
+  if (!f || robot < 0 || robot >= f->n || !origin_out || !window_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_geometry(f->sensing, robot, origin_out, window_out);
+}
+
+int navgpu_fleet_last_timing(navgpu_fleet* f, float* project_ms, float* costmap_ms) {
+  if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_last_timing(f->sensing, project_ms, costmap_ms);
 }
 
 }  // extern "C"

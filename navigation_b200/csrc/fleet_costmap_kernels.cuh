@@ -1,0 +1,259 @@
+// fleet_costmap_kernels.cuh -- one LayeredCostmap::updateMap (src/layered_costmap.cpp:79-150) of a rolling local costmap
+// [ObstacleLayer, InflationLayer] for every robot of a sensing fleet, one CTA per robot, both grids in shared memory.
+// Built from the single costmap's device helpers (costmap_kernels.cuh) so a robot's result is bit for bit what
+// navgpu_costmap computes with an obstacle and an inflation layer.
+#pragma once
+
+#include "costmap_kernels.cuh"
+
+namespace navgpu {
+
+// where a robot's sources are in the fleet-wide tables (navgpu_fleet_set_scans)
+struct FleetScanRobot {
+  int clear_first, n_clear, rays;  // clearing DevObs [clear_first, + n_clear) of the fleet's table; total rays
+  int mark_first, n_mark, marks;   // marking DevObs, likewise; total marking points
+  long long mark_base;             // the robot's first entry of the marking scratch
+};
+
+// the host's scalars of one robot and step: Costmap2D::updateOrigin (the new origin and the cell shift that got there)
+// and the pose transformFootprint needs (cos / sin of the yaw from the host libm, like the single costmap)
+struct FleetCmStep {
+  double ox, oy;
+  double rx, ry, cos_th, sin_th;
+  int cell_dx, cell_dy;
+};
+
+constexpr int kFleetCmThreads = 256;
+constexpr int kFleetFootprint = 16;               // = kMaxFootprint of the planner side
+constexpr int kFleetPolyCells = kPolySmallCells;  // footprint rasteriser scratch (entries of each of its two arrays)
+
+struct FleetCostmapArgs {
+  uint8_t* layer;   // n x sy x pitch: every robot's ObstacleLayer grid
+  uint8_t* master;  // n x sy x pitch: every robot's master grid (what the planner side scores against)
+  unsigned sx, sy, pitch;
+  unsigned spitch;  // row pitch of the grids in shared memory
+  double res;
+  uint8_t def;      // default value of both grids (track_unknown ? NO_INFORMATION : FREE_SPACE)
+  int policy;       // NAVGPU_OVERWRITE or NAVGPU_MAX (ObstacleLayer::combination_method_)
+  int footprint_clearing;
+  double max_obstacle_height;
+  int nfp;
+  double fpx[kFleetFootprint], fpy[kFleetFootprint];  // footprint, robot frame
+  const FleetScanRobot* robots;
+  const FleetCmStep* steps;
+  const DevObs* clear;
+  const DevObs* mark;
+  const float* xyz;        // every robot's projected clouds (k_project_scans)
+  long long* mark_cells;   // one entry per marking point
+  DevBox* boxes;           // n x 2: the obstacle layer's touched box (the inflation entry is unused)
+  InflationBoundsState* infl;  // n x 2: InflationLayer::last_* of every robot (entry 1)
+  DevWindow* win;          // n: the cycle's window
+  int reinflate;           // InflationLayer::need_reinflation_ (the first step)
+  double inflation_radius;
+  int R;                   // cell inflation radius; 0: the inflation layer does nothing
+  const uint8_t* cost_d2;  // R * R + 1 entries: cost by squared cell distance
+};
+
+// Dynamic shared memory of k_fleet_costmap: the rasteriser's two arrays, the seed bitmask (one word of 32 cells per
+// row position plus an empty word on either side), the obstacle grid, the master grid, the horizontal seed distances,
+// one "row has a seed" byte per row and the cost table.
+__host__ __device__ inline unsigned fleet_seed_words(unsigned sx) { return (sx + 31) / 32 + 2; }
+__host__ __device__ inline size_t fleet_costmap_smem(unsigned sy, unsigned spitch, unsigned seed_words, int R) {
+  return 2 * kFleetPolyCells * sizeof(uint32_t) + size_t(sy) * seed_words * sizeof(uint32_t) + 3 * size_t(sy) * spitch +
+         sy + size_t(R) * R + 1;
+}
+
+// Per robot (CTA), in the order of the reference:
+//   1. Costmap2D::updateOrigin of both grids: the previous grids shifted by the step's cell offset while they are
+//      loaded, the default value in the new cells (costmap_2d.cpp:264-313)
+//   2. ObstacleLayer::updateBounds (obstacle_layer.cpp:340-413): ray-trace clearing of every clearing source (one warp
+//      per ray, raytrace_ray on the shared grid), a barrier, marking (mark_prepare), the touched bounds of the sensor
+//      origins and the footprint
+//   3. ObstacleLayer::updateCosts' footprint clearing (:427-435) on the obstacle grid
+//   4. the bounds pass (finalize_bounds: InflationLayer::updateBounds with this robot's last_* state, the window)
+//   5. resetMap of the window, the obstacle grid merged with Overwrite or Max, and InflationLayer::updateCosts as the
+//      exact windowed nearest-seed inflation of k_update_costs over the whole robot map (its halo is the map itself)
+//   6. both grids written back
+__global__ void __launch_bounds__(kFleetCmThreads) k_fleet_costmap(FleetCostmapArgs a) {
+  extern __shared__ __align__(16) uint8_t fsm[];
+  __shared__ unsigned long long s_box[kFleetCmThreads / 32][4];
+  __shared__ __align__(8) unsigned char s_ba_bytes[sizeof(BoundsArgs)];  // (BoundsArgs has member initialisers)
+  BoundsArgs& s_ba = *reinterpret_cast<BoundsArgs*>(s_ba_bytes);
+  __shared__ DevWindow s_win;
+  __shared__ PolyArgs s_poly;
+  __shared__ int s_do_poly;
+  const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  constexpr int nt = kFleetCmThreads, n_warps = kFleetCmThreads / 32;
+  const int sx = (int)a.sx, sy = (int)a.sy, sp = (int)a.spitch, R = a.R;
+  const int bw = (int)fleet_seed_words(a.sx);
+  uint32_t* poly_cells = reinterpret_cast<uint32_t*>(fsm);
+  uint32_t* poly_sorted = poly_cells + kFleetPolyCells;
+  uint32_t* bits = poly_sorted + kFleetPolyCells;
+  uint8_t* lay = reinterpret_cast<uint8_t*>(bits + sy * bw);
+  uint8_t* mas = lay + sy * sp;
+  uint8_t* hx = mas + sy * sp;
+  uint8_t* rowany = hx + sy * sp;
+  uint8_t* table = rowany + sy;
+
+  const FleetCmStep st = a.steps[r];
+  const FleetScanRobot rb = a.robots[r];
+  const size_t gbase = (size_t)r * a.sy * a.pitch;
+  const Geom g{a.sx, a.sy, a.spitch, a.res, st.ox, st.oy};
+
+  // 1. both grids, shifted (k_shift_grid's rule)
+  for (int i = tid; i < sy * sx; i += nt) {
+    const int y = i / sx, x = i - y * sx;
+    const long long ox = (long long)x + st.cell_dx, oy = (long long)y + st.cell_dy;
+    uint8_t l = a.def, m = a.def;
+    if (ox >= 0 && ox < sx && oy >= 0 && oy < sy) {
+      const size_t o = gbase + (size_t)oy * a.pitch + (size_t)ox;
+      l = a.layer[o];
+      m = a.master[o];
+    }
+    lay[y * sp + x] = l;
+    mas[y * sp + x] = m;
+  }
+  for (int i = tid; i <= R * R && R > 0; i += nt) table[i] = a.cost_d2[i];
+  BoxAcc acc;
+  if (tid == 0) {
+    // raytraceFreespace touches the origin of every clearing source that lies on the map (:504-521)
+    for (int k = 0; k < rb.n_clear; ++k) {
+      const DevObs& o = a.clear[rb.clear_first + k];
+      unsigned mx, my;
+      if (world_to_map(g, o.ox, o.oy, mx, my)) acc.touch(o.ox, o.oy);
+    }
+    // updateFootprint (:415-425, transformFootprint footprint.cpp:106-120) and the polygon's cells for updateCosts
+    // (worldToMap of every vertex; one off the map: no clearing, costmap_2d.cpp:315-342)
+    int n = 0;
+    bool on_map = true;
+    if (a.footprint_clearing) {
+      for (int k = 0; k < a.nfp; ++k) {
+        const double wx = st.rx + (a.fpx[k] * st.cos_th - a.fpy[k] * st.sin_th);
+        const double wy = st.ry + (a.fpx[k] * st.sin_th + a.fpy[k] * st.cos_th);
+        acc.touch(wx, wy);
+        unsigned mx, my;
+        if (on_map && world_to_map(g, wx, wy, mx, my)) {
+          s_poly.vx[n] = (int)mx;
+          s_poly.vy[n] = (int)my;
+          ++n;
+        } else {
+          on_map = false;
+        }
+      }
+    }
+    s_poly.n = n;
+    s_do_poly = on_map && n >= 3;
+  }
+  __syncthreads();
+
+  // 2. every ray cleared before any point is marked (:362-368)
+  const DevObs* ctab = a.clear + rb.clear_first;
+  for (int ray = warp; ray < rb.rays; ray += n_warps) raytrace_ray(lay, g, ctab, rb.n_clear, a.xyz, rb.rays, acc, ray, lane);
+  __syncthreads();
+  const DevObs* mtab = a.mark + rb.mark_first;
+  long long* cells = a.mark_cells + rb.mark_base;
+  for (int t = tid; t < rb.marks; t += nt) {
+    mark_prepare(g, mtab, rb.n_mark, a.xyz, a.max_obstacle_height, acc, cells, t);
+    const long long c = cells[t];
+    if (c >= 0) lay[c] = kLethal;
+  }
+  __syncthreads();
+
+  // 3. the footprint polygon to FREE_SPACE, after the marks
+  if (s_do_poly) polygon_clear_cta(lay, a.spitch, s_poly, kFree, poly_cells, poly_sorted, kFleetPolyCells);
+
+  // 4. bounds -> window
+  DevBox* box = a.boxes + 2 * (size_t)r;
+  acc.flush_cta(box, s_box);
+  __syncthreads();
+  if (tid == 0) {
+    s_ba.n_layers = 2;
+    s_ba.layer[0] = BoundsLayer{0, 0, 0.0, 0.0, 0.0, 0.0};  // everything the obstacle layer touched is in its box
+    s_ba.layer[1] = BoundsLayer{2, a.reinflate, a.inflation_radius, 0.0, 0.0, 0.0};
+    s_ba.master = g;
+    s_ba.mirror_dirty = nullptr;
+    s_ba.mirror_pad = 0;
+    finalize_bounds(s_ba, box, a.infl + 2 * (size_t)r, &s_win);
+    a.win[r] = s_win;
+  }
+  __syncthreads();
+
+  // 5. reset + merge inside the window, then inflation (k_update_costs' three phases over the whole map)
+  const DevWindow w = s_win;
+  if (w.valid) {
+    const int ww = w.xn - w.x0;
+    for (int i = tid; i < ww * (w.yn - w.y0); i += nt) {
+      const int y = w.y0 + i / ww, x = w.x0 + i % ww;
+      mas[y * sp + x] = apply_policy(a.def, lay[y * sp + x], a.policy);
+    }
+    __syncthreads();
+    if (R > 0) {
+      // seed region: window +- R clamped to the map (inflation_layer.cpp:203-211)
+      const int sx0 = max(0, w.x0 - R), sxn = min(sx, w.xn + R);
+      const int sy0 = max(0, w.y0 - R), syn = min(sy, w.yn + R);
+      for (int i = tid; i < sy * bw; i += nt) {
+        const int y = i / bw, wi = i - y * bw;
+        uint32_t word = 0;
+        if (wi > 0 && wi < bw - 1 && y >= sy0 && y < syn) {
+          const int x0 = (wi - 1) * 32;
+          for (int b = 0; b < 32; ++b) {
+            const int x = x0 + b;
+            if (x >= sx0 && x < sxn && mas[y * sp + x] == kLethal) word |= 1u << b;
+          }
+        }
+        bits[i] = word;
+      }
+      __syncthreads();
+      for (int y = tid; y < sy; y += nt) {
+        uint32_t any = 0;
+        for (int wi = 1; wi < bw - 1; ++wi) any |= bits[y * bw + wi];
+        rowany[y] = any != 0;
+      }
+      // horizontal distance to the nearest seed of the same row, |dx| <= R (255 = none)
+      for (int i = tid; i < sy * sx; i += nt) {
+        const int y = i / sx, x = i - y * sx;
+        const uint32_t* wrow = bits + y * bw;
+        const int p = 32 + x;  // bit position of this cell in the row
+        auto word = [&](int k) -> uint32_t { return (k < 0 || k >= bw) ? 0u : wrow[k]; };
+        auto window32 = [&](int q) -> uint32_t {  // bits q .. q+31
+          const int wi = q >> 5, sh = q & 31;
+          return __funnelshift_r(word(wi), word(wi + 1), sh);
+        };
+        int best = 255;
+        for (int base = 0; base <= R; base += 32) {
+          const uint32_t right = window32(p + base);      // bit k  <-> distance base + k
+          const uint32_t left = window32(p - base - 31);  // bit 31-k <-> distance base + k
+          int d = 255;
+          if (right) d = base + (__ffs(right) - 1);
+          if (left) d = min(d, base + __clz(left));
+          if (d != 255) { best = d; break; }
+        }
+        hx[y * sp + x] = (uint8_t)(best <= R ? best : 255);
+      }
+      __syncthreads();
+      // d^2 = min over dy of dy^2 + hx(y + dy)^2, rows of the map only
+      const int R2 = R * R;
+      for (int i = tid; i < sy * sx; i += nt) {
+        const int y = i / sx, x = i - y * sx;
+        int best = 0x7fffffff;
+        for (int yy = max(0, y - R); yy <= min(sy - 1, y + R); ++yy) {
+          if (!rowany[yy]) continue;
+          const int h = hx[yy * sp + x];
+          if (h != 255) best = min(best, h * h + (yy - y) * (yy - y));
+        }
+        if (best <= R2) mas[y * sp + x] = inflate_combine(mas[y * sp + x], table[best]);
+      }
+    }
+  }
+  __syncthreads();
+
+  // 6. write-back
+  for (int i = tid; i < sy * sx; i += nt) {
+    const int y = i / sx, x = i - y * sx;
+    const size_t o = gbase + (size_t)y * a.pitch + x;
+    a.layer[o] = lay[y * sp + x];
+    a.master[o] = mas[y * sp + x];
+  }
+}
+
+}  // namespace navgpu

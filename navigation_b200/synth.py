@@ -114,3 +114,59 @@ def fleet_robot(robot_id, n=120, res=0.05):
     t = np.linspace(-0.05, 1.2, int(rng.integers(40, 160)))
     plan = np.stack([pose[0] + t * size * 0.75, mid + 0.25 * np.sin(t * rng.uniform(1, 3)) * rng.uniform(0, 1)], 1)
     return dict(raw=raw, origin=(ox, oy), pose=pose, vel=vel, plan=plan)
+
+
+def fleet_sensing_robot(robot_id, n=120, res=0.05, cycles=64):
+    """Config C5 with sensing: one robot's world, seeded by its id -- a 2n x 2n boolean grid with a corridor of thick
+    axis-aligned walls and boxes and a few one-cell posts (point-like obstacles such as table legs), kept clear of the
+    robot's path -- its origin, a pose per cycle driving along the corridor, a velocity and a plan.  The robot senses it
+    through fleet_scan; its local n x n costmap is built from those scans alone."""
+    rng = np.random.default_rng(2_000_003 * 7 + robot_id)
+    wn = 2 * n
+    world = np.zeros((wn, wn), bool)
+    lo, hi = int(wn * rng.uniform(0.3, 0.38)), int(wn * rng.uniform(0.62, 0.7))
+    world[lo - 4:lo, :] = True
+    world[hi:hi + 4, :] = True
+    mid_cell = (lo + hi) // 2
+
+    def off_path(h):  # a row band that keeps an obstacle of height h at least 12 cells from the corridor's middle
+        return int(rng.integers(mid_cell + 12, hi - h - 1)) if rng.random() < 0.5 else int(rng.integers(lo + 1, mid_cell - 12 - h))
+    for _ in range(int(rng.integers(1, 4))):
+        w, h = int(rng.integers(3, 9)), int(rng.integers(3, 9))
+        bx, by = int(rng.integers(0, wn - w)), off_path(h)
+        world[by:by + h, bx:bx + w] = True
+    for _ in range(int(rng.integers(3, 7))):
+        world[off_path(1), int(rng.integers(0, wn))] = True
+    ox, oy = float(rng.uniform(-20, 20)), float(rng.uniform(-20, 20))
+    mid = oy + (mid_cell + 0.5) * res
+    x0 = ox + wn * res * rng.uniform(0.3, 0.4)
+    speed, yaw0, ph = float(rng.uniform(0.01, 0.06)), float(rng.uniform(-0.4, 0.4)), float(rng.uniform(0, 6.28))
+    c = np.arange(cycles)
+    poses = np.stack([x0 + speed * c, mid + 0.1 * np.sin(0.3 * c + ph), yaw0 + 0.05 * np.sin(0.2 * c + ph)], 1)
+    vel = (float(rng.uniform(0.0, 0.5)), 0.0, float(rng.uniform(-0.4, 0.4)))
+    t = np.linspace(-0.05, 1.2, int(rng.integers(40, 160)))
+    plan = np.stack([x0 + t * n * res * 0.75, mid + 0.15 * np.sin(t * rng.uniform(1, 3)) * rng.uniform(0, 1)], 1)
+    return dict(world=world, origin=(ox, oy), resolution=res, poses=poses, vel=vel, plan=plan)
+
+
+def fleet_scan(robot, cycle, cloud=False, n_beams=360, range_max=4.0):
+    """One scan of `robot` (fleet_sensing_robot) at its pose of `cycle`: n_beams rays cast through its world from a
+    sensor 0.3 m above the robot's centre, as a navgpu_laser_scan dict (the format Costmap.set_scans takes).  Beams
+    without a return read +inf with inf_is_valid (laserScanValidInfCallback clears along them).  cloud=True gives the
+    same end points as a PointCloud source (sensor-frame points) instead of ranges."""
+    x, y, yaw = (float(v) for v in robot["poses"][cycle % len(robot["poses"])])
+    phase = 0.001 * cycle
+    pts = raycast_scan(robot["world"], robot["resolution"], robot["origin"], (x, y), n_beams, range_max, phase=phase)
+    dx, dy = pts[:, 0].astype(np.float64) - x, pts[:, 1].astype(np.float64) - y
+    scan = dict(translation=(x, y, 0.3), rotation_xyzw=(0.0, 0.0, float(np.sin(yaw / 2)), float(np.cos(yaw / 2))),
+                min_obstacle_height=0.0, max_obstacle_height=2.0, obstacle_range=2.5, raytrace_range=3.0,
+                marking=True, clearing=True)
+    if cloud:
+        cs, sn = np.cos(yaw), np.sin(yaw)
+        scan["points"] = np.stack([cs * dx + sn * dy, -sn * dx + cs * dy, np.zeros_like(dx)], 1).astype(np.float32)
+        return scan
+    ranges = np.hypot(dx, dy).astype(np.float32)
+    ranges[ranges >= np.float32(range_max - 1e-3)] = np.inf
+    scan.update(ranges=ranges, angle_min=np.float32(phase - yaw), angle_increment=np.float32(2 * np.pi / n_beams),
+                range_min=np.float32(0.05), range_max=np.float32(range_max), inf_is_valid=1)
+    return scan

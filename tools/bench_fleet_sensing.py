@@ -1,0 +1,151 @@
+"""Sensing fleet throughput (navgpu_fleet_create_sensing): 4096 robots, each a rolling 120 x 120 local costmap at 0.05 m
+[ObstacleLayer, InflationLayer] fed one fresh 360-beam LaserScan per step, then DWAPlanner with 20 x 1 x 20 samples and the
+pentagon footprint.  Prints one JSON line:
+  sensing_step_ms   host wall time of set_scans + step (the step ends in a device synchronise), mean over the timed steps
+  project_ms, costmap_ms   device time (CUDA events) of the scan projection (k_project_scans) and of k_fleet_costmap,
+                    means over the timed steps, and their sum
+  raw_step_ms       the raw-map fleet (config C5, navgpu_fleet_create + set_maps) step in the same process, for comparison
+  gpu, power_limit  the card and its power limit, read in the same run
+--check N replays N evenly spaced robots through the CPU checker (rolling LayeredCostmap with the exact windowed
+inflation, then DWAPlanner) over every step and reports how many agree (costmaps bit for bit, results as in
+the tests).  LaserScan projection may differ from glibc's in the last float bit (tests/test_gpu_scan_ingest.py), so a
+disagreement is reported, not fatal.
+
+The scans of K distinct cycles are ray-cast once before timing (ray casting 4096 x 360 beams in numpy takes seconds);
+step k uses cycle k mod K, so every step still uploads and projects a new scan per robot."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+PENTAGON = [(-0.325, -0.325), (-0.325, 0.325), (0.325, 0.325), (0.46, 0.0), (0.325, -0.325)]
+CFG = dict(vx_samples=20, vy_samples=1, vth_samples=20, max_vel_y=0.0, min_vel_y=0.0)
+
+
+def gpu_info():
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        name, limit = [s.strip() for s in out.split(",")]
+        return name, limit
+    except Exception as e:  # the numbers are still reported, without the card's limit
+        return f"unknown ({e})", "unknown"
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--robots", type=int, default=4096)
+    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--cycles", type=int, default=4, help="distinct scan cycles ray-cast before timing")
+    ap.add_argument("--check", type=int, default=0)
+    args = ap.parse_args()
+    if args.steps < 1 or args.robots < 1 or args.cycles < 1:
+        ap.error("--steps, --robots and --cycles must be positive")
+
+    import navigation_b200
+    from navigation_b200 import build, synth
+    build.build()
+    cuda = navigation_b200.load()
+    if cuda.device_count() == 0:
+        sys.exit("bench_fleet_sensing needs a CUDA device (libnavgpu has no CPU path)")
+    n, sx, res = args.robots, 120, 0.05
+
+    t0 = time.perf_counter()
+    robots = [synth.fleet_sensing_robot(i, n=sx, res=res) for i in range(n)]
+    scans = [[[synth.fleet_scan(r, c)] for r in robots] for c in range(args.cycles)]
+    poses = [np.ascontiguousarray([r["poses"][c] for r in robots]) for c in range(args.cycles)]
+    vels = np.ascontiguousarray([r["vel"] for r in robots])
+    prep_s = time.perf_counter() - t0
+
+    fleet = cuda.fleet_sensing(n, sx, sx, res, PENTAGON, **CFG)
+    fleet.set_plans(poses[0], [r["plan"] for r in robots])
+    sample = list(range(0, n, max(1, n // args.check)))[:args.check] if args.check else []
+    history = {i: [] for i in sample}
+    wall, proj, dev = [], [], []
+    for k in range(args.warmup + args.steps):
+        c = k % args.cycles
+        t = time.perf_counter()
+        fleet.set_scans(scans[c])
+        res_arr = fleet.step_raw(poses[c], vels)
+        dt = time.perf_counter() - t
+        for i in sample:
+            g = res_arr[i]
+            history[i].append((g.cost, g.xv, g.yv, g.thetav, g.best_index, g.n_samples, g.n_scored, fleet.oscillation_mask(i)))
+        if k >= args.warmup:
+            wall.append(dt * 1e3)
+            p_ms, c_ms = fleet.last_timing()
+            proj.append(p_ms)
+            dev.append(c_ms)
+    valid = sum(1 for i in range(n) if res_arr[i].cost >= 0)
+
+    # the raw-map fleet (config C5) in the same process
+    raw_robots = [synth.fleet_robot(i) for i in range(n)]
+    raw = cuda.fleet(n, sx, sx, res, PENTAGON, 0.55, 10.0, **CFG)
+    raw.set_maps(np.stack([r["raw"] for r in raw_robots]), np.array([r["origin"] for r in raw_robots]))
+    rposes = np.ascontiguousarray([r["pose"] for r in raw_robots])
+    rvels = np.ascontiguousarray([r["vel"] for r in raw_robots])
+    raw.set_plans(rposes, [r["plan"] for r in raw_robots])
+    raw_ms = []
+    for k in range(args.warmup + args.steps):
+        t = time.perf_counter()
+        raw.step_raw(rposes, rvels)
+        if k >= args.warmup:
+            raw_ms.append((time.perf_counter() - t) * 1e3)
+
+    checked = agree = 0
+    if sample:
+        from oracle import pyoracle
+        port = pyoracle.load("port")
+        final = {i: fleet.costmap(i) for i in sample}
+        for i in sample:
+            cm = port.costmap(sx, sx, res, 0.0, 0.0, rolling=True)
+            o = cm.add_obstacle_layer(1, True, 2.0)
+            il = cm.add_inflation_layer(0.55, 10.0)
+            cm.set_inflation_variant(il, 4)  # exact windowed nearest-seed inflation (inflation mode 0)
+            cm.set_footprint(PENTAGON)
+            d = port.dwa(sx, sx, res, **CFG)
+            ok = True
+            for k in range(args.warmup + args.steps):
+                c = k % args.cycles
+                org, pts = port.project_scan(scans[c][i][0])
+                s_ = scans[c][i][0]
+                cm.set_observations(o, [dict(origin=org, points=pts, obstacle_range=s_["obstacle_range"],
+                                             raytrace_range=s_["raytrace_range"])])
+                cm.update_map(*poses[c][i])
+                d.set_costmap(cm.get(), *cm.origin())
+                if k == 0:
+                    d.set_plan(poses[0][i], robots[i]["plan"])
+                e = d.find_best_path(poses[c][i], vels[i], PENTAGON)
+                got = history[i][k]
+                want = (e["cost"], e["xv"], e["yv"], e["thetav"], e["best_index"], e["n_samples"], e["n_scored"],
+                        d.oscillation_mask())
+                same = got[4:] == want[4:] and (got[0] < 0) == (want[0] < 0) and \
+                    (want[0] < 0 or (np.isclose(got[0], want[0], rtol=1e-5, atol=0) and got[1:4] == want[1:4]))
+                ok = ok and same
+            ok = ok and np.array_equal(final[i], cm.get())
+            checked += 1
+            agree += ok
+
+    name, limit = gpu_info()
+    out = dict(robots=n, map=f"{sx}x{sx}@{res}", samples="20x1x20", steps=args.steps, warmup=args.warmup,
+               scan_cycles=args.cycles, beams=360,
+               sensing_step_ms=float(np.mean(wall)), sensing_step_ms_min=float(np.min(wall)),
+               project_ms=float(np.mean(proj)), costmap_ms=float(np.mean(dev)),
+               project_plus_costmap_ms=float(np.mean(np.add(proj, dev))),
+               raw_step_ms=float(np.mean(raw_ms)), raw_step_ms_min=float(np.min(raw_ms)),
+               valid_robots=valid, checked=checked, checked_agree=agree, input_prep_s=round(prep_s, 1),
+               gpu=name, power_limit=limit)
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
