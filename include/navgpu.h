@@ -152,14 +152,6 @@ int navgpu_costmap_set_profiling(navgpu_costmap* h, int enabled);
 /* test hook: use the generic (any-R) fused sweep kernel even where the R <= 31 two-kernel fast path applies */
 int navgpu_costmap_force_generic_sweep(navgpu_costmap* h, int enabled);
 int navgpu_costmap_last_timing(navgpu_costmap* h, float* cycle_ms, float* sweep_ms);
-/* measurement hook (process started with NAVGPU_TRACE set): first start / last end of the cycle's kernels on the device's
- * global timer in ns -- out[0..1] obstacle kernel, [2..3] k_merge_seed, [4..5] k_inflate, [6] last merge tile in the
- * obstacle box, [7] / [8] first / last inflate tile released by its flags (tools/probe_trace.py) */
-int navgpu_costmap_last_trace(navgpu_costmap* h, uint64_t out[16]);
-/* same hook, per CTA of the last cycle: kernel 0 = k_merge_seed, 1 = k_inflate, 2 = k_obstacle_update; out[8 * cta + 0..6] = start, start of the
- * work proper (after the dependency / flag wait), end (global timer, ns), SM id, k_inflate's stage ends; n_ctas <= 4096
- * (tools/probe_cta_trace.py) */
-int navgpu_costmap_last_cta_trace(navgpu_costmap* h, int kernel, uint64_t* out, int n_ctas);
 /* the sweep's two kernels separately: streaming merge + seed bitmask (k_merge_seed), inflation (k_inflate) */
 int navgpu_costmap_last_timing_split(navgpu_costmap* h, float* merge_ms, float* inflate_ms);
 /* the CUDA stream of this handle (cudaStream_t) so callers can record events on it */

@@ -124,8 +124,6 @@ SIGNATURES = {
     "navgpu_costmap_get": (C.c_int, [C.c_void_p, _u8p]),
     "navgpu_costmap_get_window": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, _u8p]),
     "navgpu_costmap_get_window_into": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, _u8p, C.c_uint32]),
-    "navgpu_costmap_last_trace": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
-    "navgpu_costmap_last_cta_trace": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_uint64), C.c_int]),
     "navgpu_costmap_get_changed": (C.c_int, [C.c_void_p, _u8p, C.c_uint32, _i32p, C.c_int, C.POINTER(C.c_int32),
                                              C.POINTER(C.c_uint64)]),
     "navgpu_costmap_mirror_invalidate": (C.c_int, [C.c_void_p]),
@@ -406,16 +404,6 @@ class Costmap:
         assert host_grid.dtype == np.uint8 and host_grid.flags["C_CONTIGUOUS"]
         self.api.check(self.lib.navgpu_costmap_get_window_into(self.h, x0, y0, xn, yn, _p(host_grid, _u8p),
                                                                host_grid.shape[1]))
-
-    def last_trace(self):
-        out = np.zeros(16, dtype=np.uint64)
-        self.api.check(self.lib.navgpu_costmap_last_trace(self.h, _p(out, C.POINTER(C.c_uint64))))
-        return out
-
-    def last_cta_trace(self, kernel, n_ctas):
-        out = np.zeros((n_ctas, 8), dtype=np.uint64)
-        self.api.check(self.lib.navgpu_costmap_last_cta_trace(self.h, kernel, _p(out, C.POINTER(C.c_uint64)), n_ctas))
-        return out
 
     def get_changed(self, host_grid, max_rects=0):
         """Brings `host_grid` (the full-size host mirror, size_y x size_x uint8, the same array every call) up to date

@@ -208,7 +208,6 @@ struct navgpu_costmap {
   unsigned* d_tile_ready = nullptr;  // early mode: per k_merge_seed tile, the sweep number that last completed it
   unsigned sweep_epoch = 0;
   int sm_count = 0;
-  unsigned long long* d_trace = nullptr;  // NAVGPU_TRACE: kernel start / end stamps of the last cycle (measurement)
   // inflation mode 1 (k_inflate_propagate): per-cell state + two frontier lists, barrier / round control
   uint32_t* d_prop_state = nullptr;
   PropCtl* d_prop_ctl = nullptr;
@@ -372,7 +371,6 @@ int launch_propagate(const UpdateArgs& a, const uint16_t* seeds, const PropBuffe
 struct TileFlags {  // early mode: k_merge_seed -> k_inflate per-tile hand-over (MergeSeedArgs::ready)
   unsigned* ready = nullptr;
   unsigned epoch = 0;
-  unsigned long long* trace = nullptr;
   unsigned* done = nullptr;        // InflateArgs::done
   bool* handed_over = nullptr;     // out: the sweep used the per-tile flags (and published `done`)
 };
@@ -393,9 +391,8 @@ int launch_sweep(const UpdateArgs& a, uint16_t* seeds, cudaStream_t stream, bool
     m.seeds = seeds;
     m.early = a.early; m.ex0 = a.ex0; m.exn = a.exn; m.ey0 = a.ey0; m.eyn = a.eyn;
     m.obst_flag = a.obst_flag; m.obst_epoch = a.obst_epoch;
-    m.trace = flags ? flags->trace : nullptr;
     m.lean = a.ml.n >= 1 && a.ml.n <= 2 && a.ml.policy[0] == NAVGPU_TRUE_OVERWRITE &&
-             (a.ml.n == 1 || a.ml.policy[1] == NAVGPU_MAX || a.ml.policy[1] == NAVGPU_OVERWRITE) && !getenv("NAVGPU_NO_LEAN_MERGE");
+             (a.ml.n == 1 || a.ml.policy[1] == NAVGPU_MAX || a.ml.policy[1] == NAVGPU_OVERWRITE);
     if (R > 0 && !seeds) return fail(NAVGPU_ERR_INVALID, "seed bitmask missing");
     dim3 block(kMSGroupsX, kMSRowsY);
     dim3 grid((a.pitch + kMSGroupsX * 16 - 1) / (kMSGroupsX * 16), (a.sy + kMSTileH - 1) / kMSTileH);
@@ -421,7 +418,6 @@ int launch_sweep(const UpdateArgs& a, uint16_t* seeds, cudaStream_t stream, bool
         ia.done = flags->done;
         if (flags->handed_over) *flags->handed_over = flags->done != nullptr;
       }
-      ia.trace = flags ? flags->trace : nullptr;
       dim3 igrid((a.sx + kITX - 1) / kITX, (a.sy + kITY - 1) / kITY);
       // the instantiation whose unrolled row walk just covers the effective reach (what k_inflate calls R)
       const int reach = (int)sqrtf((float)a.reach2 + 0.5f);
@@ -497,7 +493,6 @@ int launch_update(navgpu_costmap* h, const MergeLayers& ml, int do_reset, int R,
   if (R > 0 && (R <= 31 || propagate)) NAVGPU_TRY(ensure_seeds(&h->d_seeds, &h->seeds_capacity, h->pitch, h->sy, h->stream));
   if (h->profile && R > 0) cudaEventRecord(h->ev_sweep[0], h->stream);
   TileFlags tf;
-  tf.trace = h->d_trace;
   if (a.early && R > 0 && R <= 31 && !propagate) {
     const size_t n_tiles = size_t((a.pitch + kMSGroupsX * 16 - 1) / (kMSGroupsX * 16)) * ((a.sy + kMSTileH - 1) / kMSTileH);
     if (!h->d_tile_ready) {
@@ -560,15 +555,6 @@ int footprint_polygon(navgpu_costmap* h, const Layer& L, PolyArgs& pa, int* mode
 // One LayeredCostmap::updateMap cycle (layered_costmap.cpp:79-150), enqueued on the handle's stream.
 int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
   NAVGPU_TRY(use_device(h));
-  static const bool tracing = getenv("NAVGPU_TRACE") != nullptr;
-  if (tracing) {
-    if (!h->d_trace) {
-      NAVGPU_CUDA(cudaMalloc(&h->d_trace, (16 + 24 * (size_t)kCtaTraceMax) * sizeof(unsigned long long)));
-      NAVGPU_CUDA(cudaMemsetAsync(h->d_trace, 0, (16 + 24 * (size_t)kCtaTraceMax) * sizeof(unsigned long long), h->stream));
-    }
-    static const unsigned long long init[16] = {~0ull, 0, ~0ull, 0, ~0ull, 0, 0, ~0ull, 0, 0, 0, 0, 0, 0, ~0ull, 0};
-    NAVGPU_CUDA(cudaMemcpyAsync(h->d_trace, init, sizeof(init), cudaMemcpyHostToDevice, h->stream));
-  }
   // rolling window: master origin follows the robot (:86-91)
   if (h->rolling)
     NAVGPU_TRY(roll_grid(h, h->master, h->cur, h->ox, h->oy, h->def, rx - h->size_m_x() / 2, ry - h->size_m_y() / 2));
@@ -665,8 +651,7 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
   }
 
   EarlyBox early;
-  static const bool no_early = getenv("NAVGPU_NO_EARLY_MERGE") != nullptr;  // measurement switch (tools/probe_overlap.py)
-  if (whole_map && box_known && !no_early) {
+  if (whole_map && box_known) {
     early.on = 1;
     if (ebx1 >= ebx0 && eby1 >= eby0) {  // cells, two to spare on every side, clamped to the map
       auto cell = [&](double w, double origin, int size, int pad) {
@@ -732,7 +717,6 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
     oa.do_poly = mode == 1;
     oa.do_finalize = (int)li == last_obstacle;
     if (oa.do_finalize) oa.ba = ba;
-    oa.trace = h->d_trace;
     oa.tile_used = L.d_tile_used;
     if (mode == 2) standalone_polygon = true;
     if (early.on && (int)li == last_obstacle && !standalone_polygon) {
@@ -859,8 +843,7 @@ int navgpu_costmap_create(navgpu_costmap** out, uint32_t size_x, uint32_t size_y
     // empty -- also on the SMs that hold the merge CTAs waiting for the obstacle kernel, or that kernel's last CTA.
     // (k_merge_seed streams and k_obstacle_update scatters single bytes: neither misses the L1 it gives up.)
     static bool done_for_device[64] = {};
-    static const bool separate = getenv("NAVGPU_SEPARATE_CARVEOUTS") != nullptr;  // measurement switch
-    if (!separate && h->device >= 0 && h->device < 64 && !done_for_device[h->device]) {
+    if (h->device >= 0 && h->device < 64 && !done_for_device[h->device]) {
       done_for_device[h->device] = true;
       const int c = cudaSharedmemCarveoutMaxShared;
       NAVGPU_CUDA(cudaFuncSetAttribute(k_obstacle_update, cudaFuncAttributePreferredSharedMemoryCarveout, c));
@@ -905,7 +888,7 @@ int navgpu_costmap_destroy(navgpu_costmap* h) {
   cudaFree(h->master[0]); cudaFree(h->master[1]);
   cudaFree(h->d_boxes); cudaFree(h->d_infl); cudaFree(h->d_win); cudaFree(h->d_seeds); cudaFree(h->d_ticket); cudaFree(h->d_obst_done); cudaFree(h->d_inflate_done); cudaFree(h->d_occupancy);
   cudaFree(h->d_prop_state); cudaFree(h->d_prop_ctl);
-  cudaFree(h->d_shadow); cudaFree(h->d_mirror_counters); cudaFree(h->d_mirror_dirty); cudaFree(h->d_tile_ready); cudaFree(h->d_trace);
+  cudaFree(h->d_shadow); cudaFree(h->d_mirror_counters); cudaFree(h->d_mirror_dirty); cudaFree(h->d_tile_ready);
   if (h->h_mirror_stage) cudaFreeHost(h->h_mirror_stage);
   if (h->h_mirror_tiles) cudaFreeHost(h->h_mirror_tiles);
   if (h->h_mirror_ctl) cudaFreeHost(h->h_mirror_ctl);
@@ -951,8 +934,7 @@ int navgpu_costmap_add_obstacle_layer(navgpu_costmap* h, int combination_method,
   NAVGPU_TRY(add_cost_layer(h, L));
   // The only writers of such a layer's grid are its own kernel's clears (FREE_SPACE) and marks: the tiles without a mark
   // are known to hold the default value.  Not for rolling maps (the grid shifts) or NO_INFORMATION defaults.
-  static const bool no_summary = getenv("NAVGPU_NO_LAYER_SUMMARY") != nullptr;  // measurement switch
-  if (!h->rolling && L.def == kFree && !no_summary) {
+  if (!h->rolling && L.def == kFree) {
     const size_t n_tiles = size_t((h->pitch + kMarkTileW - 1) / kMarkTileW) * ((h->sy + kMarkTileH - 1) / kMarkTileH);
     NAVGPU_CUDA(cudaMalloc(&L.d_tile_used, n_tiles));
     NAVGPU_CUDA(cudaMemsetAsync(L.d_tile_used, 0, n_tiles, h->stream));
@@ -1422,25 +1404,6 @@ int navgpu_costmap_update_map(navgpu_costmap* h, double rx, double ry, double ry
   return NAVGPU_OK;
 }
 
-int navgpu_costmap_last_trace(navgpu_costmap* h, uint64_t out[16]) {
-  if (!h || !out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
-  if (!h->d_trace) return fail(NAVGPU_ERR_INVALID, "tracing is off (set NAVGPU_TRACE before the first update)");
-  NAVGPU_TRY(use_device(h));
-  NAVGPU_CUDA(cudaStreamSynchronize(h->stream));
-  NAVGPU_CUDA(cudaMemcpy(out, h->d_trace, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
-  return NAVGPU_OK;
-}
-
-int navgpu_costmap_last_cta_trace(navgpu_costmap* h, int kernel, uint64_t* out, int n_ctas) {
-  if (!h || !out || kernel < 0 || kernel > 2 || n_ctas < 0 || n_ctas > kCtaTraceMax) return fail(NAVGPU_ERR_INVALID, "bad arguments");
-  if (!h->d_trace) return fail(NAVGPU_ERR_INVALID, "tracing is off (set NAVGPU_TRACE before the first update)");
-  NAVGPU_TRY(use_device(h));
-  NAVGPU_CUDA(cudaStreamSynchronize(h->stream));
-  NAVGPU_CUDA(cudaMemcpy(out, h->d_trace + 16 + 8 * (size_t)kernel * kCtaTraceMax, 8 * (size_t)n_ctas * sizeof(uint64_t),
-                         cudaMemcpyDeviceToHost));
-  return NAVGPU_OK;
-}
-
 int navgpu_costmap_last_timing_split(navgpu_costmap* h, float* merge_ms, float* inflate_ms) {
   if (!h || !h->profile) return fail(NAVGPU_ERR_INVALID, "profiling is not enabled on this handle");
   NAVGPU_TRY(use_device(h));
@@ -1580,8 +1543,7 @@ int navgpu_costmap_get_changed(navgpu_costmap* h, uint8_t* host_grid, uint32_t h
   h->refine_valid = true;  // from here on: until a cycle that is not of the refinable kind
   h->refine[0] = h->refine[1] = h->refine[2] = h->refine[3] = 0;
   const unsigned launched_tiles = std::max(1u, a.tw * a.th);  // (one CTA at least: it publishes the counts and the window)
-  static const bool no_tile_wait = getenv("NAVGPU_NO_MIRROR_TILE_WAIT") != nullptr;
-  if (mirror_refinable && h->inflate_done_epoch != 0 && !no_tile_wait) {
+  if (mirror_refinable && h->inflate_done_epoch != 0) {
     a.inflate_done = h->d_inflate_done;
     a.inflate_epoch = h->inflate_done_epoch;
     a.inflate_pitch = h->inflate_done_pitch;
@@ -1592,20 +1554,17 @@ int navgpu_costmap_get_changed(navgpu_costmap* h, uint8_t* host_grid, uint32_t h
   NAVGPU_LAUNCHED(1);
   NAVGPU_CUDA(cudaGetLastError());
   {  // wait for the kernel's last word in mapped memory; a stream synchronisation backs the poll up (errors, hangs)
-    static const bool no_poll = getenv("NAVGPU_NO_MIRROR_POLL") != nullptr;
     const volatile unsigned* seq = &h->h_mirror_ctl->seq;
     bool seen = false;
-    if (!no_poll) {
-      const auto t0 = std::chrono::steady_clock::now();
-      for (unsigned spin = 0;; ++spin) {
-        if (*seq == a.seq) { seen = true; break; }
-        if ((spin & 1023u) == 1023u && std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(2)) break;
+    const auto t0 = std::chrono::steady_clock::now();
+    for (unsigned spin = 0;; ++spin) {
+      if (*seq == a.seq) { seen = true; break; }
+      if ((spin & 1023u) == 1023u && std::chrono::steady_clock::now() - t0 > std::chrono::milliseconds(2)) break;
 #if defined(__x86_64__)
-        __builtin_ia32_pause();
+      __builtin_ia32_pause();
 #endif
-      }
-      std::atomic_thread_fence(std::memory_order_acquire);
     }
+    std::atomic_thread_fence(std::memory_order_acquire);
     if (!seen) NAVGPU_CUDA(cudaStreamSynchronize(h->stream));
   }
   const MirrorCtl& ctl = *h->h_mirror_ctl;

@@ -8,37 +8,6 @@
 
 namespace navgpu {
 
-// measurement only (NAVGPU_TRACE, tools/probe_trace.py): first start / last end of every kernel of a cycle on the
-// device's global timer, so that the overlap of the three kernels can be read off.  [2k] = min start, [2k + 1] = max end
-// for k = 0 obstacle, 1 merge, 2 inflate; [6] = last end of a merge tile in the obstacle box, [7] = first start of
-// actual work (after the flag wait) of an inflate tile, [8] = last flag wait end of an inflate tile.
-__device__ __forceinline__ unsigned long long trace_now() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ void trace_start(unsigned long long* tr, int k) {
-  if (tr && (threadIdx.x | threadIdx.y) == 0) atomicMin(&tr[2 * k], trace_now());
-}
-__device__ __forceinline__ void trace_end(unsigned long long* tr, int k) {
-  if (tr && (threadIdx.x | threadIdx.y) == 0) atomicMax(&tr[2 * k + 1], trace_now());
-}
-// per-CTA records behind the 16 summary words (tools/probe_cta_trace.py): 8 words per CTA -- start, start of the
-// actual work (after the flag / dependency wait), end, SM id, and for k_inflate the ends of its seed-word, pruning and
-// phase-2 stages -- k_merge_seed's CTAs first, k_inflate's from kCtaTraceMax
-constexpr int kCtaTraceMax = 4096;
-__device__ __forceinline__ void trace_cta(unsigned long long* tr, int kernel, int cta, int slot) {
-  if (tr && (threadIdx.x | threadIdx.y) == 0 && cta < kCtaTraceMax) {
-    unsigned long long* rec = tr + 16 + 8 * ((size_t)kernel * kCtaTraceMax + cta);
-    rec[slot] = trace_now();
-    if (slot == 0) {
-      unsigned smid;
-      asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-      rec[3] = smid;
-    }
-  }
-}
-
 struct Geom {
   unsigned sx, sy, pitch;
   double res, ox, oy;
@@ -681,7 +650,6 @@ struct ObstacleArgs {
   DevBox* boxes;
   InflationBoundsState* infl;
   DevWindow* win;
-  unsigned long long* trace = nullptr;
   uint8_t* tile_used = nullptr;  // MergeLayers::used of this layer (nullable)
   // set to done_epoch (release, gpu scope) by the last CTA as soon as the layer grid is complete (rays cleared, marks
   // stored, footprint cleared), before the bounds pass: early-mode k_merge_seed tiles in the rays' box wait for this
@@ -700,16 +668,13 @@ __global__ void __maxnreg__(48) k_obstacle_update(ObstacleArgs a) {
   __shared__ bool s_last;
   const int lane = threadIdx.x & 31, cta_warp = threadIdx.x >> 5;
   cudaTriggerProgrammaticLaunchCompletion();  // k_merge_seed may be scheduled behind us; it waits for our completion
-  if (a.trace && threadIdx.x == 0) atomicMin(&a.trace[0], trace_now());
   // the observation tables travel in the kernel parameters when they fit (no dependent global loads to find a ray's
   // observation), else they are read from device memory
   const DevObs* clear_tab = a.n_clear <= kInlineObs ? a.clear_inline : a.clear;
   const DevObs* mark_tab = a.n_mark <= kInlineObs ? a.mark_inline : a.mark;
   BoxAcc acc;
-  trace_cta(a.trace, 2, blockIdx.x, 0);
   if (cta_warp < kObstacleRayWarps) {
     raytrace_ray(a.grid, a.g, clear_tab, a.n_clear, a.xyz, a.total_rays, acc, blockIdx.x * kObstacleRayWarps + cta_warp, lane);
-    trace_cta(a.trace, 2, blockIdx.x, 4);
     // (a ray touches its end point from lane 0 only: nothing to reduce within the warp)
     if (lane == 0) { s_box[cta_warp][0] = acc.minx; s_box[cta_warp][1] = acc.miny; s_box[cta_warp][2] = acc.maxx; s_box[cta_warp][3] = acc.maxy; }
   } else {  // this CTA's share of the marking tests
@@ -719,22 +684,15 @@ __global__ void __maxnreg__(48) k_obstacle_update(ObstacleArgs a) {
       if (t < a.total_marks)
         mark_prepare(a.g, mark_tab, a.n_mark, a.xyz, a.max_obstacle_height, acc, a.mark_cells, t);
     }
-    if (a.trace && lane == 0 && blockIdx.x < kCtaTraceMax) a.trace[16 + 8 * (2 * (size_t)kCtaTraceMax + blockIdx.x) + 5] = trace_now();
     acc.reduce_warp();
     if (lane == 0) { s_box[cta_warp][0] = acc.minx; s_box[cta_warp][1] = acc.miny; s_box[cta_warp][2] = acc.maxx; s_box[cta_warp][3] = acc.maxy; }
   }
   __syncthreads();
   BoxAcc::flush_rows(a.box, s_box, kObstacleRayWarps + 1);
   __syncthreads();
-  trace_cta(a.trace, 2, blockIdx.x, 6);
   if (threadIdx.x == 0) {
     __threadfence();
     s_last = atomicAdd(a.ticket, 1u) == gridDim.x - 1;
-    trace_cta(a.trace, 2, blockIdx.x, 2);
-    if (a.trace) {  // [14] first / [9] last CTA through with its rays; [10] marks stored, [11] polygon cleared
-      atomicMin(&a.trace[14], trace_now());
-      atomicMax(&a.trace[9], trace_now());
-    }
   }
   __syncthreads();
   if (!s_last) return;
@@ -746,10 +704,7 @@ __global__ void __maxnreg__(48) k_obstacle_update(ObstacleArgs a) {
   constexpr int kTailThreads = 32 * kObstacleRayWarps;  // warps 0..6 and 8
   __shared__ bool s_regular;
   if (cta_warp == kObstacleRayWarps - 1) {
-    if (lane == 0) {
-      if (a.do_finalize) finalize_bounds(a.ba, a.boxes, a.infl, a.win);
-      if (a.trace) atomicMax(&a.trace[1], trace_now());
-    }
+    if (lane == 0 && a.do_finalize) finalize_bounds(a.ba, a.boxes, a.infl, a.win);
     return;
   }
   const int ttid = cta_warp < kObstacleRayWarps ? (int)threadIdx.x : (int)threadIdx.x - 32;  // 0 .. kTailThreads - 1
@@ -760,12 +715,10 @@ __global__ void __maxnreg__(48) k_obstacle_update(ObstacleArgs a) {
     if (lane == 0) s_regular = regular;
   }
   asm volatile("bar.sync 1, %0;" ::"n"(kTailThreads) : "memory");
-  if (a.trace && threadIdx.x == 0) a.trace[10] = trace_now();
   if (a.do_poly) {
     if (s_regular) polygon_fill_regular(a.grid, a.g.pitch, a.poly, kFree, poly_cells, poly_sorted, ttid, kTailThreads);
     else polygon_fill_irregular(a.grid, a.g.pitch, a.poly, kFree, poly_cells, poly_sorted, kPolySmallCells, ttid, kTailThreads);
   }
-  if (a.trace && threadIdx.x == 0) a.trace[11] = trace_now();
   if (a.done_flag) {
     asm volatile("bar.sync 1, %0;" ::"n"(kTailThreads) : "memory");  // every mark / polygon store before the release
     if (threadIdx.x == 0) {
@@ -774,7 +727,6 @@ __global__ void __maxnreg__(48) k_obstacle_update(ObstacleArgs a) {
     }
   }
   if (threadIdx.x == 0) *a.ticket = 0;  // re-armed for the next cycle
-  if (a.trace && threadIdx.x == 0) atomicMax(&a.trace[1], trace_now());
 }
 
 // Costmap2DPublisher's cost -> occupancy translation (src/costmap_2d_publisher.cpp:56-71, applied per cell in
@@ -1288,7 +1240,7 @@ __global__ void __launch_bounds__(kUpdateThreads) k_update_costs(UpdateArgs a) {
 //                  inflation reaches.  A tile whose seed words are all zero exits after the load.
 // k_merge_seed: a CTA walks kMSSubTiles sub-tiles of 256 columns x 32 rows (what MergeLayers::used summarises) top to
 // bottom: 256 x 128 cells per CTA.  (CTAs of one sub-tile live ~1.7 us and a freed slot stays empty for about a
-// microsecond before its next CTA runs -- tools/probe_cta_trace.py --; four times the work per CTA makes the 4000^2 pass
+// microsecond before its next CTA runs -- DESIGN.md "Known limits" --; four times the work per CTA makes the 4000^2 pass
 // a single wave of 500 CTAs.)
 constexpr int kMSGroupsX = 16, kMSRowsY = 16, kMSRowIters = 2, kMSSubTiles = 2;
 constexpr int kMSTileH = kMSRowsY * kMSRowIters * kMSSubTiles;
@@ -1318,7 +1270,6 @@ struct MergeSeedArgs {
   // its tile (master cells and seed bits) is written, and k_inflate's tiles wait for just the tiles they read
   unsigned* ready = nullptr;
   unsigned epoch = 0;
-  unsigned long long* trace = nullptr;
   int lean = 0;  // the stack is "TrueOverwrite, then at most one Max / Overwrite layer": interior tiles take merge_seed_lean
 };
 
@@ -1540,8 +1491,6 @@ __global__ void __launch_bounds__(kMSGroupsX * kMSRowsY, 5) k_merge_seed(MergeSe
   // launched with programmatic stream serialization: let k_inflate be scheduled as soon as every CTA of this grid
   // is resident, and wait for the kernel before us (window, obstacle grid) before reading anything
   cudaTriggerProgrammaticLaunchCompletion();
-  trace_start(a.trace, 1);
-  trace_cta(a.trace, 0, blockIdx.y * gridDim.x + blockIdx.x, 0);
   constexpr int kW = kMSGroupsX * 16, kH = kMSTileH;
   const int bx0 = blockIdx.x * kW, by0 = blockIdx.y * kH;
   DevWindow w;
@@ -1570,12 +1519,8 @@ __global__ void __launch_bounds__(kMSGroupsX * kMSRowsY, 5) k_merge_seed(MergeSe
       __syncthreads();
     }
     if (a.lean) {  // every tile: the window is the whole map
-      trace_cta(a.trace, 0, blockIdx.y * gridDim.x + blockIdx.x, 1);
       if (bx0 + kW <= (int)a.sx && by0 + kH <= (int)a.sy) merge_seed_lean<false>(a, bx0 + threadIdx.x * 16, by0);
       else merge_seed_lean<true>(a, bx0 + threadIdx.x * 16, by0);
-      trace_end(a.trace, 1);
-      trace_cta(a.trace, 0, blockIdx.y * gridDim.x + blockIdx.x, 2);
-      if (a.trace && touched && (threadIdx.x | threadIdx.y) == 0) atomicMax(&a.trace[6], trace_now());
       if (a.ready) {
         __syncthreads();
         if ((threadIdx.x | threadIdx.y) == 0)
@@ -1588,7 +1533,6 @@ __global__ void __launch_bounds__(kMSGroupsX * kMSRowsY, 5) k_merge_seed(MergeSe
     cudaGridDependencySynchronize();
     w = *a.win;
   }
-  trace_cta(a.trace, 0, blockIdx.y * gridDim.x + blockIdx.x, 1);
   if (!w.valid) return;
   const int R = a.R;
   // everything k_inflate can read: its tiles intersect window +- 2R, extend up to a tile further, and look R rows /
@@ -1619,10 +1563,6 @@ __global__ void __launch_bounds__(kMSGroupsX * kMSRowsY, 5) k_merge_seed(MergeSe
       }
     }
   }
-  trace_end(a.trace, 1);
-  trace_cta(a.trace, 0, blockIdx.y * gridDim.x + blockIdx.x, 2);
-  if (a.trace && a.early && bx0 < a.exn && bx0 + kW > a.ex0 && by0 < a.eyn && by0 + kH > a.ey0 && (threadIdx.x | threadIdx.y) == 0)
-    atomicMax(&a.trace[6], trace_now());
   if (a.ready) {  // (early mode: the window is the whole map, no CTA left above)
     __syncthreads();
     if ((threadIdx.x | threadIdx.y) == 0)  // (release at gpu scope: cumulative over what the barrier made visible here)
@@ -1675,7 +1615,6 @@ struct InflateArgs {
   unsigned epoch = 0;
   int ready_pitch = 0;  // k_merge_seed's gridDim.x
   unsigned* done = nullptr;  // nullable: one word per tile of this grid, set to `epoch` when the tile's cells are final
-  unsigned long long* trace = nullptr;
 };
 
 // RMAX bounds the effective reach (in cells) this instantiation can handle: the phase-3 walk is unrolled over
@@ -1706,8 +1645,6 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
   const unsigned* my_flag = nullptr;
   unsigned flag_seen = 0;
   cudaTriggerProgrammaticLaunchCompletion();  // (a k_mirror_diff behind us may become resident; it waits for our end)
-  trace_start(a.trace, 2);
-  trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 0);
   if (a.ready) {
     constexpr int kMW = kMSGroupsX * 16, kMH = kMSTileH;
     const int mx0 = max(0, tx0 - 32) / kMW, mx1 = min((int)a.pitch - 1, tx0 + kITX + 31) / kMW;
@@ -1737,15 +1674,9 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
       }
     }
     __syncthreads();  // (the window is the whole map: every tile of the grid is in it)
-    if (a.trace && threadIdx.x == 0) {
-      atomicMin(&a.trace[7], trace_now());
-      atomicMax(&a.trace[8], trace_now());
-    }
-    trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 1);
   } else {
     cudaGridDependencySynchronize();
     const DevWindow w = *a.win;
-    trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 1);
     if (!w.valid) return;
     const int R = a.R;
     if (tx0 >= w.xn + 2 * R || tx0 + kITX <= w.x0 - 2 * R || ty0 >= w.yn + 2 * R || ty0 + kITY <= w.y0 - 2 * R) return;
@@ -1778,12 +1709,7 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
       any |= v[k] != 0;
     }
   }
-  if (!__syncthreads_or(any)) {
-    trace_end(a.trace, 2);
-    trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 2);
-    return;
-  }
-  trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 4);
+  if (!__syncthreads_or(any)) return;
 
   // ---- interior seeds cannot be the nearest seed of any other cell: a seed whose four neighbours are seeds too has,
   // for every non-seed cell p, a neighbouring seed strictly closer to p (step along the larger coordinate difference),
@@ -1833,7 +1759,6 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
     if (seeded && !dup) rowlist[base + __popc(lm & ((1u << lane) - 1u))] = (uint8_t)r;
   }
   __syncthreads();
-  trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 5);
 
   // ---- phase 2: squared horizontal distances for the listed rows (one warp per row); before that every row learns
   // canon[r], the nearest row at or above it that does not repeat its predecessor
@@ -1865,7 +1790,6 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
     }
   }
   __syncthreads();
-  trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 6);
 
   // ---- phase 3 + epilogue: a warp takes 64 columns x 8 rows at a time
   const uint32_t R2x2 = (uint32_t)a.reach2 * 0x10001u;
@@ -2011,8 +1935,6 @@ __device__ __forceinline__ void inflate_tile(const InflateArgs& a) {
       }
     }
   }
-  trace_end(a.trace, 2);
-  trace_cta(a.trace, 1, blockIdx.y * gridDim.x + blockIdx.x, 2);
 }
 
 template <int RMAX>

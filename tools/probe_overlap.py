@@ -1,5 +1,5 @@
-"""Measurement helper: where the C3 cycle's time goes -- obstacle layer on / off / without observations, with and
-without the early merge (run twice: NAVGPU_NO_EARLY_MERGE=1 disables it), flushed and hot L2."""
+"""Measurement helper: where the C3 cycle's time goes -- obstacle layer on / off / without observations, flushed and
+hot L2."""
 import os
 import sys
 
@@ -42,8 +42,7 @@ def measure(label):
         cm.update_map_async(*robot)
     b.record(stream)
     torch.cuda.synchronize()
-    print(f"{label:34s} early={'off' if os.environ.get('NAVGPU_NO_EARLY_MERGE') else 'on '} "
-          f"flushed_us={1e3 * cold:.1f} hot_us={1e3 * a.elapsed_time(b) / n:.1f}", flush=True)
+    print(f"{label:34s} flushed_us={1e3 * cold:.1f} hot_us={1e3 * a.elapsed_time(b) / n:.1f}", flush=True)
 
 
 cm.set_observations(o, obs)

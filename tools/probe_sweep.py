@@ -1,5 +1,4 @@
-"""Measurement helper (not part of the product): times the fused sweep kernel of the C3 cycle with CUDA events.
-NAVGPU_DEBUG_SKIP=1|2|3 disables phases of the fast kernel (wrong results) to attribute its time."""
+"""Measurement helper (not part of the product): times the fused sweep kernel of the C3 cycle with CUDA events."""
 import os
 import sys
 
