@@ -413,6 +413,30 @@ int navgpu_fleet_get_geometry(navgpu_fleet* f, int robot, double origin_out[2], 
 /* device time (ms, CUDA events) of the last scan projection (navgpu_fleet_set_scans; 0 when it had no points) and of the
  * last costmap update of all robots (navgpu_fleet_step); synchronises the fleet's stream */
 int navgpu_fleet_last_timing(navgpu_fleet* f, float* project_ms, float* costmap_ms);
+/* ---- Sensing fleet with a VoxelLayer (map_type: voxel) -----------------------------------------------------------
+ * A third kind of fleet: every robot's rolling local costmap is [VoxelLayer, InflationLayer], the VoxelLayer of
+ * navgpu_costmap_add_voxel_layer (3-D ray-trace clearing on columns of up to 16 voxels, so a ray that passes over a low
+ * obstacle does not clear it; marking; the columns move with the rolling origin).  cm keeps its meaning
+ * (max_obstacle_height, combination_method, footprint_clearing, track_unknown and the inflation parameters); voxel
+ * gives the VoxelLayer's own parameters, checked like navgpu_costmap_add_voxel_layer's (same error codes; mark_threshold
+ * must be 0).  Every robot's columns start unknown, as VoxelGrid does.  set_scans, set_plans, step, get_costmap,
+ * get_geometry and last_timing work as on a sensing fleet; navgpu_fleet_get_layer returns the VoxelLayer's 2-D grid.
+ * One CTA holds a robot's grids and its columns (4 B per cell) in shared memory: larger maps are refused with
+ * NAVGPU_ERR_UNSUPPORTED (on a B200 with the default inflation at 0.05 m, up to about 188 x 188 cells). */
+typedef struct {
+  double origin_z, z_resolution; /* VoxelLayer (defaults 0.0, 0.2) */
+  int32_t z_voxels;              /* defaults 10; same range as navgpu_costmap_add_voxel_layer */
+  int32_t unknown_threshold;     /* default 15 (VoxelPlugin.cfg), before reconfigureCB's + (16 - z_voxels) */
+  int32_t mark_threshold;        /* default 0 */
+  int32_t pad_;
+} navgpu_fleet_voxel_config;
+int navgpu_fleet_create_sensing_voxel(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                      uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                                      const navgpu_fleet_voxel_config* voxel, const double* footprint_xy,
+                                      int n_footprint, int device);
+/* per robot, after the last navgpu_fleet_step: the VoxelLayer's columns (HOST size_y x size_x uint32, the layout of
+ * navgpu_layer_get_voxels); NAVGPU_ERR_INVALID on fleets without a VoxelLayer */
+int navgpu_fleet_get_voxels(navgpu_fleet* f, int robot, uint32_t* host_out);
 
 
 /* ---- legacy base_local_planner::TrajectoryPlanner (SURVEY.md 8f-4) ---------------------------------------------

@@ -58,6 +58,16 @@ class FleetCostmapConfig(C.Structure):
                 ("footprint_clearing", C.c_int32), ("track_unknown", C.c_int32), ("pad_", C.c_int32)]
 
 
+class FleetVoxelConfig(C.Structure):
+    """navgpu_fleet_voxel_config (the VoxelLayer of navgpu_fleet_create_sensing_voxel)"""
+    _fields_ = [("origin_z", C.c_double), ("z_resolution", C.c_double), ("z_voxels", C.c_int32),
+                ("unknown_threshold", C.c_int32), ("mark_threshold", C.c_int32), ("pad_", C.c_int32)]
+
+
+# cfg/VoxelPlugin.cfg
+VOXEL_DEFAULTS = dict(origin_z=0.0, z_resolution=0.2, z_voxels=10, unknown_threshold=15, mark_threshold=0)
+
+
 class TpConfig(C.Structure):
     """navgpu_tp_config: the legacy base_local_planner::TrajectoryPlanner's parameters."""
     _fields_ = [(n, C.c_double) for n in (
@@ -191,6 +201,10 @@ SIGNATURES = {
     "navgpu_fleet_get_layer": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
     "navgpu_fleet_get_geometry": (C.c_int, [C.c_void_p, C.c_int, _f64p, _i32p]),
     "navgpu_fleet_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
+    "navgpu_fleet_create_sensing_voxel": (C.c_int, [_vpp, C.c_int, C.POINTER(DwaConfig), C.c_uint32, C.c_uint32,
+                                                    C.c_double, C.POINTER(FleetCostmapConfig),
+                                                    C.POINTER(FleetVoxelConfig), _f64p, C.c_int, C.c_int]),
+    "navgpu_fleet_get_voxels": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_uint32)]),
     "navgpu_tp_default_config": (None, [C.POINTER(TpConfig)]),
     "navgpu_tp_create": (C.c_int, [_vpp, C.POINTER(TpConfig), C.c_uint32, C.c_uint32, C.c_double, _f64p, C.c_int, C.c_int]),
     "navgpu_tp_destroy": (C.c_int, [C.c_void_p]),
@@ -765,9 +779,10 @@ class Fleet:
     """N independent robots per control cycle (navgpu_fleet_*): local-costmap inflation + DWA scoring, batched."""
 
     def __init__(self, api, n_robots, size_x, size_y, resolution, footprint_xy, inflation_radius=0.55,
-                 cost_scaling_factor=10.0, device=0, sensing=None, **overrides):
+                 cost_scaling_factor=10.0, device=0, sensing=None, voxel=None, **overrides):
         """sensing: None for a raw-map fleet (set_maps), else a FleetCostmapConfig: every robot then builds its own
-        rolling local costmap from its scans (set_scans; see Api.fleet_sensing)."""
+        rolling local costmap from its scans (set_scans; see Api.fleet_sensing).  voxel: with sensing, a
+        FleetVoxelConfig makes that costmap's obstacle layer a VoxelLayer."""
         self.api, self.lib, self.n = api, api.lib, n_robots
         self.size_x, self.size_y = size_x, size_y
         self.cfg = DwaConfig()
@@ -780,10 +795,14 @@ class Fleet:
             api.check(self.lib.navgpu_fleet_create(C.byref(h), n_robots, C.byref(self.cfg), size_x, size_y, resolution,
                                                    inflation_radius, cost_scaling_factor, _p(fp, _f64p), fp.shape[0],
                                                    device))
-        else:
+        elif voxel is None:
             api.check(self.lib.navgpu_fleet_create_sensing(C.byref(h), n_robots, C.byref(self.cfg), size_x, size_y,
                                                            resolution, C.byref(sensing), _p(fp, _f64p), fp.shape[0],
                                                            device))
+        else:
+            api.check(self.lib.navgpu_fleet_create_sensing_voxel(C.byref(h), n_robots, C.byref(self.cfg), size_x,
+                                                                 size_y, resolution, C.byref(sensing), C.byref(voxel),
+                                                                 _p(fp, _f64p), fp.shape[0], device))
         self.h = h
         self._results = (DwaResult * n_robots)()
 
@@ -843,9 +862,16 @@ class Fleet:
         self.api.check(self.lib.navgpu_fleet_set_scans(self.h, arr, _p(off, _i32p)))
 
     def layer(self, robot):
-        """Sensing fleets: robot's ObstacleLayer grid after the last step."""
+        """Sensing fleets: robot's ObstacleLayer (or VoxelLayer) grid after the last step."""
         out = np.empty((self.size_y, self.size_x), dtype=np.uint8)
         self.api.check(self.lib.navgpu_fleet_get_layer(self.h, robot, _p(out, _u8p)))
+        return out
+
+    def voxels(self, robot):
+        """Voxel fleets: robot's VoxelLayer columns after the last step (size_y x size_x uint32: bit z = unknown or
+        marked, bit z + 16 = marked)."""
+        out = np.empty((self.size_y, self.size_x), dtype=np.uint32)
+        self.api.check(self.lib.navgpu_fleet_get_voxels(self.h, robot, out.ctypes.data_as(C.POINTER(C.c_uint32))))
         return out
 
     def geometry(self, robot):
@@ -900,13 +926,17 @@ class Api:
 
     def fleet_sensing(self, n, sx, sy, res, footprint, inflation_radius=0.55, cost_scaling_factor=10.0,
                       combination_method=1, footprint_clearing=True, max_obstacle_height=2.0, track_unknown=False,
-                      device=0, **dwa_overrides):
+                      device=0, voxel=None, **dwa_overrides):
         """A fleet whose robots each run a rolling sx x sy local costmap [ObstacleLayer, InflationLayer] fed by their
-        own scans (Fleet.set_scans), then DWAPlanner (navgpu_fleet_create_sensing)."""
+        own scans (Fleet.set_scans), then DWAPlanner (navgpu_fleet_create_sensing).  voxel: a FleetVoxelConfig or a
+        dict of its fields (origin_z, z_resolution, z_voxels, unknown_threshold, mark_threshold; missing ones take
+        VoxelPlugin.cfg's defaults) makes it [VoxelLayer, InflationLayer] (navgpu_fleet_create_sensing_voxel)."""
         cm = FleetCostmapConfig(inflation_radius=inflation_radius, cost_scaling_factor=cost_scaling_factor,
                                 max_obstacle_height=max_obstacle_height, combination_method=combination_method,
                                 footprint_clearing=int(footprint_clearing), track_unknown=int(track_unknown))
-        return Fleet(self, n, sx, sy, res, footprint, device=device, sensing=cm, **dwa_overrides)
+        if isinstance(voxel, dict):
+            voxel = FleetVoxelConfig(**{**VOXEL_DEFAULTS, **voxel})
+        return Fleet(self, n, sx, sy, res, footprint, device=device, sensing=cm, voxel=voxel, **dwa_overrides)
 
     def trajectory_planner(self, *a, **k):
         return TrajectoryPlanner(self, *a, **k)

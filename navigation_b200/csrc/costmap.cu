@@ -1846,7 +1846,8 @@ int navgpu_merge_host(uint8_t* master, const uint8_t* layer, uint32_t size_x, ui
 
 // ==================================================================================================================
 // Sensing fleet (navgpu_fleet_create_sensing, fleet_costmap.cuh): n rolling local costmaps [ObstacleLayer,
-// InflationLayer] updated by k_fleet_costmap, one CTA per robot.  The host keeps per robot what navgpu_costmap keeps for
+// InflationLayer], or [VoxelLayer, InflationLayer] (navgpu_fleet_create_sensing_voxel), updated by k_fleet_costmap, one
+// CTA per robot.  The host keeps per robot what navgpu_costmap keeps for
 // one: the origin and the observation tables; the cost table is shared.
 // ==================================================================================================================
 namespace navgpu {
@@ -1863,6 +1864,9 @@ struct FleetCostmap {
   cudaStream_t stream = nullptr;
   uint8_t* d_layer = nullptr;   // n x sy x pitch
   uint8_t* d_master = nullptr;  // n x sy x pitch
+  bool voxel = false;           // the obstacle layer is a VoxelLayer
+  VoxelGeom vg{};
+  uint32_t* d_vox = nullptr;    // voxel fleets: n x sy x pitch columns
   uint8_t* d_cost_d2 = nullptr;
   DevBox* d_boxes = nullptr;
   InflationBoundsState* d_infl = nullptr;
@@ -1892,7 +1896,7 @@ struct FleetCostmap {
   ~FleetCostmap() {  // (also what a failed fleet_costmap_create leaves behind)
     cudaSetDevice(device);
     if (stream) cudaStreamSynchronize(stream);
-    cudaFree(d_layer); cudaFree(d_master); cudaFree(d_cost_d2); cudaFree(d_boxes); cudaFree(d_infl); cudaFree(d_win);
+    cudaFree(d_layer); cudaFree(d_master); cudaFree(d_vox); cudaFree(d_cost_d2); cudaFree(d_boxes); cudaFree(d_infl); cudaFree(d_win);
     cudaFree(d_steps); cudaFree(d_robots); cudaFree(d_obs); cudaFree(d_xyz); cudaFree(d_mark_cells); cudaFree(d_scan);
     if (h_steps) cudaFreeHost(h_steps);
     for (cudaEvent_t e : ev)
@@ -1913,9 +1917,17 @@ static int ensure_device(T** p, size_t* cap, size_t n) {
 }
 
 int fleet_costmap_create(FleetCostmap** out, int n, unsigned sx, unsigned sy, double resolution,
-                         const navgpu_fleet_costmap_config& cm, const double* footprint_xy, int n_footprint, int device) {
+                         const navgpu_fleet_costmap_config& cm, const navgpu_fleet_voxel_config* voxel,
+                         const double* footprint_xy, int n_footprint, int device) {
   if (cm.combination_method != 0 && cm.combination_method != 1)
     return fail(NAVGPU_ERR_INVALID, "combination_method %d: 0 (Overwrite) or 1 (Max)", cm.combination_method);
+  if (voxel) {  // navgpu_costmap_add_voxel_layer's checks
+    const navgpu_fleet_voxel_config& v = *voxel;
+    if (v.z_voxels < 0 || v.z_voxels > 16 || !(v.z_resolution > 0) || v.unknown_threshold < 0 || v.mark_threshold < 0)
+      return fail(NAVGPU_ERR_INVALID, "bad voxel layer arguments");
+    if (v.mark_threshold != 0)
+      return fail(NAVGPU_ERR_UNSUPPORTED, "mark_threshold %d: only the reference's default 0 is implemented", v.mark_threshold);
+  }
   if (n_footprint > kFleetFootprint) return fail(NAVGPU_ERR_INVALID, "more than %d footprint vertices", kFleetFootprint);
   std::unique_ptr<FleetCostmap> fc(new FleetCostmap);
   FleetCostmap& F = *fc;
@@ -1926,6 +1938,10 @@ int fleet_costmap_create(FleetCostmap** out, int n, unsigned sx, unsigned sy, do
   F.cm = cm;
   F.fp.assign(footprint_xy, footprint_xy + 2 * n_footprint);
   F.def = cm.track_unknown ? kNoInfo : kFree;  // layered_costmap.cpp:53-56, costmap_layer.cpp:14-19
+  F.voxel = voxel != nullptr;
+  if (voxel)  // VoxelLayer::reconfigureCB (voxel_layer.cpp:84-95): unknown_threshold_ = unknown_threshold + (16 - z_voxels)
+    F.vg = VoxelGeom{voxel->origin_z, voxel->z_resolution, (unsigned)voxel->z_voxels,
+                     (unsigned)(voxel->unknown_threshold + (16 - voxel->z_voxels)), (unsigned)voxel->mark_threshold};
   std::vector<Pt> fp;
   for (int i = 0; i < n_footprint; ++i) fp.push_back(Pt{footprint_xy[2 * i], footprint_xy[2 * i + 1]});
   double inscribed = 0, circumscribed = 0;
@@ -1941,8 +1957,8 @@ int fleet_costmap_create(FleetCostmap** out, int n, unsigned sx, unsigned sy, do
   int smem_optin = 0;
   NAVGPU_CUDA(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
   cudaFuncAttributes fa;
-  NAVGPU_CUDA(cudaFuncGetAttributes(&fa, k_fleet_costmap));
-  F.smem = fleet_costmap_smem(sy, F.spitch, fleet_seed_words(sx), (int)R);
+  NAVGPU_CUDA(cudaFuncGetAttributes(&fa, F.voxel ? k_fleet_costmap_voxel : k_fleet_costmap));
+  F.smem = fleet_costmap_smem(sy, F.spitch, fleet_seed_words(sx), (int)R, F.voxel);
   if (F.smem + fa.sharedSizeBytes > (size_t)smem_optin)
     return fail(NAVGPU_ERR_UNSUPPORTED,
                 "a %u x %u map with a cell inflation radius of %u needs %zu B of shared memory per robot; the device allows %d",
@@ -1969,6 +1985,13 @@ int fleet_costmap_create(FleetCostmap** out, int n, unsigned sx, unsigned sy, do
   NAVGPU_CUDA(cudaMalloc(&F.d_master, grid_bytes));
   NAVGPU_CUDA(cudaMemset(F.d_layer, F.def, grid_bytes));
   NAVGPU_CUDA(cudaMemset(F.d_master, F.def, grid_bytes));
+  if (F.voxel) {  // VoxelGrid starts with all-unknown columns (voxel_grid.cpp:41-59)
+    NAVGPU_CUDA(cudaMalloc(&F.d_vox, grid_bytes * sizeof(uint32_t)));
+    std::vector<uint32_t> unknown(size_t(sy) * F.pitch, 0x0000ffffu);
+    for (int r = 0; r < n; ++r)
+      NAVGPU_CUDA(cudaMemcpy(F.d_vox + size_t(r) * sy * F.pitch, unknown.data(), unknown.size() * sizeof(uint32_t),
+                             cudaMemcpyHostToDevice));
+  }
   NAVGPU_CUDA(cudaMalloc(&F.d_cost_d2, F.tables.by_d2.size()));
   NAVGPU_CUDA(cudaMemcpy(F.d_cost_d2, F.tables.by_d2.data(), F.tables.by_d2.size(), cudaMemcpyHostToDevice));
   NAVGPU_CUDA(cudaMalloc(&F.d_boxes, sizeof(DevBox) * 2 * n));
@@ -2091,6 +2114,8 @@ int fleet_costmap_enqueue(FleetCostmap* fc) {
   NAVGPU_CUDA(cudaMemcpyAsync(fc->d_steps, fc->h_steps, sizeof(FleetCmStep) * fc->n, cudaMemcpyHostToDevice, fc->stream));
   FleetCostmapArgs a;
   a.layer = fc->d_layer;
+  a.vox = fc->d_vox;
+  a.v = fc->vg;
   a.master = fc->d_master;
   a.sx = fc->sx; a.sy = fc->sy; a.pitch = fc->pitch; a.spitch = fc->spitch;
   a.res = fc->res;
@@ -2117,9 +2142,10 @@ int fleet_costmap_enqueue(FleetCostmap* fc) {
   a.R = (int)fc->tables.R;
   a.cost_d2 = fc->d_cost_d2;
   // the limit belongs to the kernel, not to this fleet: another fleet (other map size, other radius) may have set its own
-  NAVGPU_CUDA(cudaFuncSetAttribute(k_fleet_costmap, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fc->smem));
+  auto* kernel = fc->voxel ? k_fleet_costmap_voxel : k_fleet_costmap;
+  NAVGPU_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fc->smem));
   NAVGPU_CUDA(cudaEventRecord(fc->ev[2], fc->stream));
-  k_fleet_costmap<<<fc->n, kFleetCmThreads, fc->smem, fc->stream>>>(a);
+  kernel<<<fc->n, kFleetCmThreads, fc->smem, fc->stream>>>(a);
   NAVGPU_LAUNCHED(1);
   NAVGPU_CUDA(cudaGetLastError());
   NAVGPU_CUDA(cudaEventRecord(fc->ev[3], fc->stream));
@@ -2133,6 +2159,16 @@ int fleet_costmap_get(FleetCostmap* fc, int robot, bool master, uint8_t* host_ou
   NAVGPU_CUDA(cudaSetDevice(fc->device));
   const uint8_t* src = (master ? fc->d_master : fc->d_layer) + size_t(robot) * fc->sy * fc->pitch;
   NAVGPU_CUDA(cudaMemcpy2DAsync(host_out, fc->sx, src, fc->pitch, fc->sx, fc->sy, cudaMemcpyDeviceToHost, fc->stream));
+  NAVGPU_CUDA(cudaStreamSynchronize(fc->stream));
+  return NAVGPU_OK;
+}
+
+int fleet_costmap_get_voxels(FleetCostmap* fc, int robot, uint32_t* host_out) {
+  if (!fc->voxel) return fail(NAVGPU_ERR_INVALID, "not a voxel fleet (navgpu_fleet_create_sensing_voxel)");
+  NAVGPU_CUDA(cudaSetDevice(fc->device));
+  const uint32_t* src = fc->d_vox + size_t(robot) * fc->sy * fc->pitch;
+  NAVGPU_CUDA(cudaMemcpy2DAsync(host_out, fc->sx * sizeof(uint32_t), src, fc->pitch * sizeof(uint32_t),
+                                fc->sx * sizeof(uint32_t), fc->sy, cudaMemcpyDeviceToHost, fc->stream));
   NAVGPU_CUDA(cudaStreamSynchronize(fc->stream));
   return NAVGPU_OK;
 }

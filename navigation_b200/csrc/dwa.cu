@@ -1141,9 +1141,11 @@ int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_confi
   return NAVGPU_OK;
 }
 
-int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
-                                uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
-                                const double* footprint_xy, int n_footprint, int device) {
+// navgpu_fleet_create_sensing and navgpu_fleet_create_sensing_voxel (voxel non-null)
+static int create_sensing(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                          uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                          const navgpu_fleet_voxel_config* voxel, const double* footprint_xy, int n_footprint,
+                          int device) {
   if (!out || !cfg || !cm || n_robots <= 0 || size_x == 0 || size_y == 0 || !(resolution > 0) || n_footprint < 0 ||
       n_footprint > kMaxFootprint || (n_footprint > 0 && !footprint_xy))
     return fail(NAVGPU_ERR_INVALID, "bad fleet arguments");
@@ -1152,7 +1154,8 @@ int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_d
   std::unique_ptr<navgpu_fleet> f(new navgpu_fleet);
   init_planner_scalars(f.get(), n_robots, cfg, size_x, size_y, resolution, footprint_xy, n_footprint, device);
   f->stride = size_y;  // robot r's master grid starts at row r * size_y
-  int rc = fleet_costmap_create(&f->sensing, n_robots, size_x, size_y, resolution, *cm, footprint_xy, n_footprint, device);
+  int rc = fleet_costmap_create(&f->sensing, n_robots, size_x, size_y, resolution, *cm, voxel, footprint_xy, n_footprint,
+                                device);
   if (rc == NAVGPU_OK) {
     f->stream = fleet_costmap_stream(f->sensing);
     f->d_master = fleet_costmap_master(f->sensing, &f->pitch);
@@ -1164,6 +1167,20 @@ int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_d
   }
   *out = f.release();
   return NAVGPU_OK;
+}
+
+int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                                const double* footprint_xy, int n_footprint, int device) {
+  return create_sensing(out, n_robots, cfg, size_x, size_y, resolution, cm, nullptr, footprint_xy, n_footprint, device);
+}
+
+int navgpu_fleet_create_sensing_voxel(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
+                                      uint32_t size_y, double resolution, const navgpu_fleet_costmap_config* cm,
+                                      const navgpu_fleet_voxel_config* voxel, const double* footprint_xy,
+                                      int n_footprint, int device) {
+  if (!voxel) return fail(NAVGPU_ERR_INVALID, "null voxel config");
+  return create_sensing(out, n_robots, cfg, size_x, size_y, resolution, cm, voxel, footprint_xy, n_footprint, device);
 }
 
 
@@ -1430,6 +1447,12 @@ int navgpu_fleet_get_layer(navgpu_fleet* f, int robot, uint8_t* host_out) {
   if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
   return fleet_costmap_get(f->sensing, robot, false, host_out);
+}
+
+int navgpu_fleet_get_voxels(navgpu_fleet* f, int robot, uint32_t* host_out) {
+  if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing_voxel)");
+  return fleet_costmap_get_voxels(f->sensing, robot, host_out);
 }
 
 int navgpu_fleet_get_geometry(navgpu_fleet* f, int robot, double origin_out[2], int32_t window_out[4]) {

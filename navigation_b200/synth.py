@@ -170,3 +170,83 @@ def fleet_scan(robot, cycle, cloud=False, n_beams=360, range_max=4.0):
     scan.update(ranges=ranges, angle_min=np.float32(phase - yaw), angle_increment=np.float32(2 * np.pi / n_beams),
                 range_min=np.float32(0.05), range_max=np.float32(range_max), inf_is_valid=1)
     return scan
+
+
+# elevation rows of fleet_cloud_3d, degrees: straight down (floor returns under the robot: z-dominant rays), a shallow
+# downward row (low obstacles; its floor return is beyond obstacle_range, so the floor only clears), the scan plane,
+# two upward rows (tall obstacles, overhangs) and a steep upward one (z-dominant, ends above max_obstacle_height)
+VOXEL_ELEVATIONS = (-80.0, -6.0, 0.0, 4.0, 25.0, 80.0)
+
+
+def fleet_voxel_robot(robot_id, n=120, res=0.05, cycles=64):
+    """fleet_sensing_robot's world with heights, for VoxelLayer fleets: every occupied cell gets a column [bottom, top]
+    in metres -- the corridor walls 2.5 m (above the default max_obstacle_height), boxes and posts 0.12 .. 1.2 m in 8 x 8
+    cell patches -- plus, next to the start of the path (off it by 14 cells or more), a 0.15 m high box below the scan
+    plane and a tabletop from 0.7 to 0.75 m above it (an overhang the scan plane passes under).  Adds `bottom`, `top`
+    (float32, top = -inf where free) and `seed` to fleet_sensing_robot's dict."""
+    r = fleet_sensing_robot(robot_id, n=n, res=res, cycles=cycles)
+    rng = np.random.default_rng(3_000_017 * 7 + robot_id)
+    world = r["world"]
+    wn = world.shape[0]
+    patch = rng.uniform(0.12, 1.2, (wn // 8 + 1, wn // 8 + 1)).astype(np.float32)
+    ys, xs = np.mgrid[0:wn, 0:wn]
+    top = np.where(world, patch[ys // 8, xs // 8], -np.inf).astype(np.float32)
+    top[world.all(axis=1), :] = 2.5
+    bottom = np.zeros((wn, wn), np.float32)
+    (ox, oy), poses = r["origin"], r["poses"]
+    cx = int((poses[0, 0] - ox) / res)
+    mc = int(round((poses[:, 1].mean() - oy) / res - 0.5))  # the corridor's middle row, to a cell or two
+    low_y, low_x = mc + 14 + int(rng.integers(0, 3)), cx + int(rng.integers(30, 40))
+    top[low_y:low_y + 4, low_x:low_x + 4] = 0.15
+    tab_y, tab_x = mc - 24 + int(rng.integers(0, 3)), cx + int(rng.integers(8, 16))
+    top[tab_y:tab_y + 8, tab_x:tab_x + 8] = 0.75
+    bottom[tab_y:tab_y + 8, tab_x:tab_x + 8] = 0.7
+    r.update(bottom=bottom, top=top, seed=robot_id)
+    return r
+
+
+def fleet_cloud_3d(robot, cycle, n_az=180, range_max=4.0, sensor_z=0.3):
+    """One 3-D cloud of `robot` (fleet_voxel_robot) at its pose of `cycle`: len(VOXEL_ELEVATIONS) rows of n_az beams
+    from a sensor sensor_z above the robot's centre, as an is_cloud navgpu_laser_scan dict (sensor-frame points, the
+    format Costmap.set_scans takes).  A beam ends where it first enters an occupied column, on the floor (z = 0 with
+    seeded noise of -3 .. +2 cm, so some returns lie below origin_z = 0) or, without a return, at range_max (the steep
+    upward row then ends far above max_obstacle_height).  The projection keeps every point (heights -0.5 .. 5 m); the
+    layer applies its own max_obstacle_height.  Vectorised over beams: the horizontal march is shared by the rows."""
+    x, y, yaw = (float(v) for v in robot["poses"][cycle % len(robot["poses"])])
+    res, (ox, oy) = robot["resolution"], robot["origin"]
+    top, bottom = robot["top"], robot["bottom"]
+    wn_y, wn_x = top.shape
+    az = 0.001 * cycle + np.arange(n_az) * (2 * np.pi / n_az)
+    step = 0.5 * res
+    t = np.arange(1, int(range_max / step) + 1) * step  # horizontal distance of every march step
+    px = x + np.cos(az)[:, None] * t
+    py = y + np.sin(az)[:, None] * t
+    mx = np.floor((px - ox) / res).astype(np.int64)
+    my = np.floor((py - oy) / res).astype(np.int64)
+    inside = (mx >= 0) & (mx < wn_x) & (my >= 0) & (my < wn_y)
+    col_top = np.full(px.shape, -np.inf, np.float32)
+    col_bot = np.zeros(px.shape, np.float32)
+    col_top[inside] = top[my[inside], mx[inside]]
+    col_bot[inside] = bottom[my[inside], mx[inside]]
+    el = np.radians(np.asarray(VOXEL_ELEVATIONS))
+    z = sensor_z + np.tan(el)[:, None] * t  # (rows, steps): the same for every azimuth
+    hit = (z[:, None, :] <= col_top[None]) & (z[:, None, :] >= col_bot[None])
+    floor = np.broadcast_to((z <= 0.0)[:, None, :], hit.shape)
+    far = np.broadcast_to((t[None, :] / np.cos(el)[:, None] > range_max)[:, None, :] | ~inside[None], hit.shape)
+    stop = hit | floor | far
+    first = np.where(stop.any(axis=2), stop.argmax(axis=2), len(t) - 1)  # (rows, azimuths)
+    took = lambda a: np.take_along_axis(a, first[..., None], axis=2)[..., 0]
+    was_hit, was_floor = took(hit), took(floor) & ~took(hit)
+    r3 = np.where(was_hit, t[first] / np.cos(el)[:, None], range_max)  # 3-D range along the beam
+    tf = sensor_z / -np.tan(np.minimum(el, -1e-9))  # horizontal distance to the floor (downward rows)
+    rng = np.random.default_rng((robot.get("seed", 0), cycle))
+    floor_z = rng.uniform(-0.03, 0.02, first.shape)
+    h = np.where(was_floor, np.broadcast_to(tf[:, None], first.shape), r3 * np.cos(el)[:, None])
+    ez = np.where(was_floor, floor_z, sensor_z + r3 * np.sin(el)[:, None])
+    dx, dy = (np.cos(az)[None, :] * h).ravel(), (np.sin(az)[None, :] * h).ravel()
+    cs, sn = np.cos(yaw), np.sin(yaw)
+    pts = np.stack([cs * dx + sn * dy, -sn * dx + cs * dy, ez.ravel() - sensor_z], 1).astype(np.float32)
+    return dict(points=pts, translation=(x, y, sensor_z),
+                rotation_xyzw=(0.0, 0.0, float(np.sin(yaw / 2)), float(np.cos(yaw / 2))),
+                min_obstacle_height=-0.5, max_obstacle_height=5.0, obstacle_range=2.5, raytrace_range=3.0,
+                marking=True, clearing=True)

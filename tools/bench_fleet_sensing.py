@@ -12,7 +12,12 @@ the tests).  LaserScan projection may differ from glibc's in the last float bit 
 disagreement is reported, not fatal.
 
 The scans of K distinct cycles are ray-cast once before timing (ray casting 4096 x 360 beams in numpy takes seconds);
-step k uses cycle k mod K, so every step still uploads and projects a new scan per robot."""
+step k uses cycle k mod K, so every step still uploads and projects a new scan per robot.
+
+--voxel benches the same fleet with map_type: voxel -- every robot's costmap is [VoxelLayer, InflationLayer]
+(cfg/VoxelPlugin.cfg's defaults: 10 voxels of 0.2 m from z = 0) fed one fresh 3-D cloud per step instead of the scan
+(synth.fleet_cloud_3d: 6 rows of 180 beams through a world with heights, 1080 points per robot) -- and adds
+"voxel": true to the JSON line.  costmap_ms is then the device time of k_fleet_costmap_voxel."""
 import argparse
 import json
 import os
@@ -28,6 +33,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 PENTAGON = [(-0.325, -0.325), (-0.325, 0.325), (0.325, 0.325), (0.46, 0.0), (0.325, -0.325)]
 CFG = dict(vx_samples=20, vy_samples=1, vth_samples=20, max_vel_y=0.0, min_vel_y=0.0)
+VOXEL = dict(origin_z=0.0, z_resolution=0.2, z_voxels=10, unknown_threshold=15, mark_threshold=0)
 
 
 def gpu_info():
@@ -47,6 +53,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--cycles", type=int, default=4, help="distinct scan cycles ray-cast before timing")
     ap.add_argument("--check", type=int, default=0)
+    ap.add_argument("--voxel", action="store_true", help="[VoxelLayer, InflationLayer] fed 3-D clouds")
     args = ap.parse_args()
     if args.steps < 1 or args.robots < 1 or args.cycles < 1:
         ap.error("--steps, --robots and --cycles must be positive")
@@ -60,13 +67,17 @@ def main():
     n, sx, res = args.robots, 120, 0.05
 
     t0 = time.perf_counter()
-    robots = [synth.fleet_sensing_robot(i, n=sx, res=res) for i in range(n)]
-    scans = [[[synth.fleet_scan(r, c)] for r in robots] for c in range(args.cycles)]
+    if args.voxel:
+        robots = [synth.fleet_voxel_robot(i, n=sx, res=res) for i in range(n)]
+        scans = [[[synth.fleet_cloud_3d(r, c)] for r in robots] for c in range(args.cycles)]
+    else:
+        robots = [synth.fleet_sensing_robot(i, n=sx, res=res) for i in range(n)]
+        scans = [[[synth.fleet_scan(r, c)] for r in robots] for c in range(args.cycles)]
     poses = [np.ascontiguousarray([r["poses"][c] for r in robots]) for c in range(args.cycles)]
     vels = np.ascontiguousarray([r["vel"] for r in robots])
     prep_s = time.perf_counter() - t0
 
-    fleet = cuda.fleet_sensing(n, sx, sx, res, PENTAGON, **CFG)
+    fleet = cuda.fleet_sensing(n, sx, sx, res, PENTAGON, voxel=VOXEL if args.voxel else None, **CFG)
     fleet.set_plans(poses[0], [r["plan"] for r in robots])
     sample = list(range(0, n, max(1, n // args.check)))[:args.check] if args.check else []
     history = {i: [] for i in sample}
@@ -108,7 +119,7 @@ def main():
         final = {i: fleet.costmap(i) for i in sample}
         for i in sample:
             cm = port.costmap(sx, sx, res, 0.0, 0.0, rolling=True)
-            o = cm.add_obstacle_layer(1, True, 2.0)
+            o = cm.add_voxel_layer(1, True, 2.0, **VOXEL) if args.voxel else cm.add_obstacle_layer(1, True, 2.0)
             il = cm.add_inflation_layer(0.55, 10.0)
             cm.set_inflation_variant(il, 4)  # exact windowed nearest-seed inflation (inflation mode 0)
             cm.set_footprint(PENTAGON)
@@ -144,6 +155,8 @@ def main():
                raw_step_ms=float(np.mean(raw_ms)), raw_step_ms_min=float(np.min(raw_ms)),
                valid_robots=valid, checked=checked, checked_agree=agree, input_prep_s=round(prep_s, 1),
                gpu=name, power_limit=limit)
+    if args.voxel:
+        out.update(voxel=True, beams=len(synth.VOXEL_ELEVATIONS) * 180)
     print(json.dumps(out))
 
 
