@@ -837,7 +837,7 @@ int navgpu_costmap_create(navgpu_costmap** out, uint32_t size_x, uint32_t size_y
   NAVGPU_CUDA(cudaMalloc(&h->d_ticket, sizeof(unsigned)));
   NAVGPU_CUDA(cudaMemset(h->d_ticket, 0, sizeof(unsigned)));
   {
-    // One L1 / shared-memory split (the largest shared-memory carve-out, which k_inflate's 8 x 26 KB need anyway) for the
+    // One L1 / shared-memory split (the largest shared-memory carve-out, which k_inflate's 8 x 27 KB need anyway) for the
     // three kernels of a cycle: CTAs of two kernels share an SM only if its split suits both, and an SM must drain to
     // change it.  With the same split k_inflate's CTAs move in as k_merge_seed's leave instead of waiting for the SM to
     // empty -- also on the SMs that hold the merge CTAs waiting for the obstacle kernel, or that kernel's last CTA.

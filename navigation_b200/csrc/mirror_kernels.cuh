@@ -55,13 +55,15 @@ struct MirrorArgs {
   unsigned host_pitch;
   unsigned seq;  // MirrorCtl::seq of this call
   // non-null: the sweep in front of this kernel was a whole-map cycle whose k_inflate publishes `inflate_epoch` per
-  // 64 x 128 tile (inflate_pitch tiles per row) when the tile's cells are final: a tile is compared as soon as the
-  // (at most two) inflate tiles that write it are done, while the rest of that kernel is still running
+  // 128 x 64 tile (inflate_pitch tiles per row) when the tile's cells are final: a tile is compared as soon as the
+  // inflate tile that writes it is done, while the rest of that kernel is still running
   const unsigned* inflate_done = nullptr;
   unsigned inflate_epoch = 0;
   int inflate_pitch = 0;
 };
-constexpr int kMirrorInflateTileW = 64, kMirrorInflateTileH = 128;  // = k_inflate's tile (static_assert in costmap.cu)
+constexpr int kMirrorInflateTileW = 128, kMirrorInflateTileH = 64;  // = k_inflate's tile (static_assert in costmap.cu)
+static_assert(kMirrorTileW % kMirrorInflateTileW == 0 && kMirrorInflateTileH % kMirrorTileH == 0,
+              "a mirror tile lies inside one row of inflate tiles");
 
 __device__ __forceinline__ void mirror_wait_word(const unsigned* p, unsigned want) {
   unsigned seen;
@@ -117,7 +119,7 @@ __global__ void __launch_bounds__(kMirrorWarps * 32) k_mirror_diff(MirrorArgs a)
                          (int)(ty_ * kMirrorTileH) < ryn && (int)((ty_ + 1) * kMirrorTileH) > ry0;
   if (tile < n_tiles && in_region) {
     const unsigned tx = tx_, ty = ty_;
-    if (a.inflate_done) {  // the two inflate tiles that cover this 128 x 16 tile
+    if (a.inflate_done) {  // the inflate tile that covers this 128 x 16 tile
       if (lane < kMirrorTileW / kMirrorInflateTileW) {
         const int ix = (int)(tx * kMirrorTileW) / kMirrorInflateTileW + lane, iy = (int)(ty * kMirrorTileH) / kMirrorInflateTileH;
         if (ix < a.inflate_pitch) mirror_wait_word(a.inflate_done + iy * a.inflate_pitch + ix, a.inflate_epoch);
