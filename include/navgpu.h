@@ -362,7 +362,8 @@ int navgpu_plans_prune(int n_plans, const int32_t* offsets, const double* plan_x
  * Every robot has its own local costmap (raw obstacles in, inflated on the device exactly like a layered costmap
  * with a static-style layer + InflationLayer), plan, pose, velocity and oscillation state; one navgpu_fleet_step is
  * LayeredCostmap::updateMap + DWAPlanner::findBestPath for all of them in a handful of launches.  Robots are
- * independent, so a multi-GPU job gives each rank its own fleet with its share of the robots (no collective). */
+ * independent, so a multi-GPU job gives each rank its own fleet with its share of the robots (no collective).  Every
+ * fleet kind can plan with the legacy TrajectoryPlanner instead (navgpu_fleet_use_trajectory_planner, below). */
 typedef struct navgpu_fleet navgpu_fleet;
 int navgpu_fleet_create(navgpu_fleet** out, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
                         uint32_t size_y, double resolution, double inflation_radius, double cost_scaling_factor,
@@ -495,6 +496,32 @@ int navgpu_tp_score_trajectory(navgpu_tp* h, const double pose[3], const double 
 int navgpu_tp_get_grid(navgpu_tp* h, int which, double* host_out);
 /* number of velocity samples the last findBestPath scored on the device */
 int navgpu_tp_last_sample_count(navgpu_tp* h, int* n_out);
+
+/* ---- Fleets of legacy TrajectoryPlanners (TrajectoryPlannerROS, move_base's default base_local_planner) ---------
+ * Any of the three fleet kinds can run base_local_planner::TrajectoryPlanner instead of DWAPlanner.  Its costmap side is
+ * unchanged (set_maps / set_scans, get_costmap, get_layer, get_voxels, get_geometry and last_timing work as before).
+ * navgpu_fleet_set_plans is then TrajectoryPlanner::updatePlan per robot (final goal, resolution-adjusted plan; empty
+ * plans are accepted, as navgpu_tp_update_plan accepts them; the poses argument is not used), and each robot keeps its
+ * own oscillation / escape state.  Per step, every robot's footprint cells, both wavefronts (path_map_, goal_map_) and
+ * every robot's velocity samples run in one launch each; the samples are enumerated and the reference's selection is
+ * made on the host, per robot, as navgpu_tp_find_best_path does.  One config for the whole fleet; the footprint is the
+ * fleet's.  navgpu_fleet_step, navgpu_fleet_reset_oscillation and navgpu_fleet_get_oscillation_mask return
+ * NAVGPU_ERR_INVALID on such a fleet, the calls below NAVGPU_ERR_INVALID on a DWA fleet. */
+/* Makes f's planner base_local_planner::TrajectoryPlanner (trajectory_planner.cpp, TrajectoryPlannerROS's planner)
+ * instead of DWAPlanner; cfg as for navgpu_tp_create (refused with its codes).  Any fleet kind; only between creation
+ * and the first set_plans / step (NAVGPU_ERR_INVALID otherwise, and for a second call).  Footprints whose filled cells
+ * could exceed the per-robot buffer (12000 cells, bounded from the circumscribed radius and the edge lengths) are
+ * refused with NAVGPU_ERR_UNSUPPORTED. */
+int navgpu_fleet_use_trajectory_planner(navgpu_fleet* f, const navgpu_tp_config* cfg);
+/* one control cycle: every robot's costmap update (as navgpu_fleet_step), then TrajectoryPlanner::findBestPath per
+ * robot; poses, vels [n][3]; results[r] as navgpu_tp_find_best_path returns it (points are not materialised, n_points
+ * is their count) */
+int navgpu_fleet_step_tp(navgpu_fleet* f, const double* poses, const double* vels, navgpu_tp_result* results);
+/* path_map_ (which = 0) / goal_map_ (1) of robot after the last step, fp64 HOST size_y x size_x (as navgpu_tp_get_grid) */
+int navgpu_fleet_tp_get_grid(navgpu_fleet* f, int robot, int which, double* host_out);
+/* device time (ms, CUDA events) of the last step's footprint-cell, wavefront and scoring launches (0 before the first
+ * step); synchronises the fleet's stream */
+int navgpu_fleet_tp_last_timing(navgpu_fleet* f, float* footprint_ms, float* wavefront_ms, float* score_ms);
 
 #ifdef __cplusplus
 }

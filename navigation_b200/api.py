@@ -217,6 +217,11 @@ SIGNATURES = {
     "navgpu_tp_score_trajectory": (C.c_int, [C.c_void_p, _f64p, _f64p, _f64p, _f64p]),
     "navgpu_tp_get_grid": (C.c_int, [C.c_void_p, C.c_int, _f64p]),
     "navgpu_tp_last_sample_count": (C.c_int, [C.c_void_p, _i32p]),
+    "navgpu_fleet_use_trajectory_planner": (C.c_int, [C.c_void_p, C.POINTER(TpConfig)]),
+    "navgpu_fleet_step_tp": (C.c_int, [C.c_void_p, _f64p, _f64p, C.POINTER(TpResult)]),
+    "navgpu_fleet_tp_get_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _f64p]),
+    "navgpu_fleet_tp_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float),
+                                              C.POINTER(C.c_float)]),
 }
 
 
@@ -682,21 +687,28 @@ class Dwa:
         return out
 
 
+def tp_config(lib, overrides):
+    """TrajectoryPlannerROS's defaults (navgpu_tp_default_config) with `overrides` (TpConfig field names; y_vels as a
+    list) applied."""
+    cfg = TpConfig()
+    lib.navgpu_tp_default_config(C.byref(cfg))
+    for k, v in overrides.items():
+        if k == "y_vels":
+            for j, y in enumerate(v):
+                cfg.y_vels[j] = y
+            cfg.n_y_vels = len(v)
+        else:
+            setattr(cfg, k, v)
+    return cfg
+
+
 class TrajectoryPlanner:
     """The legacy base_local_planner::TrajectoryPlanner (navgpu_tp_*)."""
 
     def __init__(self, api, size_x, size_y, resolution, footprint_xy, device=0, **overrides):
         self.api, self.lib = api, api.lib
         self.size_x, self.size_y = size_x, size_y
-        self.cfg = TpConfig()
-        self.lib.navgpu_tp_default_config(C.byref(self.cfg))
-        for k, v in overrides.items():
-            if k == "y_vels":
-                for j, y in enumerate(v):
-                    self.cfg.y_vels[j] = y
-                self.cfg.n_y_vels = len(v)
-            else:
-                setattr(self.cfg, k, v)
+        self.cfg = tp_config(self.lib, overrides)
         f = np.ascontiguousarray(footprint_xy, dtype=np.float64).reshape(-1, 2)
         h = C.c_void_p()
         api.check(self.lib.navgpu_tp_create(C.byref(h), C.byref(self.cfg), size_x, size_y, resolution, _p(f, _f64p),
@@ -779,10 +791,13 @@ class Fleet:
     """N independent robots per control cycle (navgpu_fleet_*): local-costmap inflation + DWA scoring, batched."""
 
     def __init__(self, api, n_robots, size_x, size_y, resolution, footprint_xy, inflation_radius=0.55,
-                 cost_scaling_factor=10.0, device=0, sensing=None, voxel=None, **overrides):
+                 cost_scaling_factor=10.0, device=0, sensing=None, voxel=None, trajectory_planner=None, **overrides):
         """sensing: None for a raw-map fleet (set_maps), else a FleetCostmapConfig: every robot then builds its own
         rolling local costmap from its scans (set_scans; see Api.fleet_sensing).  voxel: with sensing, a
-        FleetVoxelConfig makes that costmap's obstacle layer a VoxelLayer."""
+        FleetVoxelConfig makes that costmap's obstacle layer a VoxelLayer.  trajectory_planner: None for DWAPlanner
+        (`overrides` are then DwaConfig fields), else a dict of TpConfig overrides, possibly empty: the robots run the
+        legacy base_local_planner::TrajectoryPlanner (navgpu_fleet_use_trajectory_planner) and step() returns its
+        results."""
         self.api, self.lib, self.n = api, api.lib, n_robots
         self.size_x, self.size_y = size_x, size_y
         self.cfg = DwaConfig()
@@ -804,7 +819,13 @@ class Fleet:
                                                                  size_y, resolution, C.byref(sensing), C.byref(voxel),
                                                                  _p(fp, _f64p), fp.shape[0], device))
         self.h = h
-        self._results = (DwaResult * n_robots)()
+        self.tp_cfg = None
+        if trajectory_planner is None:
+            self._results = (DwaResult * n_robots)()
+        else:
+            self.tp_cfg = tp_config(self.lib, trajectory_planner)
+            api.check(self.lib.navgpu_fleet_use_trajectory_planner(self.h, C.byref(self.tp_cfg)))
+            self._results = (TpResult * n_robots)()
 
     def __del__(self):
         if getattr(self, "h", None):
@@ -829,18 +850,35 @@ class Fleet:
         self.api.check(self.lib.navgpu_fleet_reset_oscillation(self.h))
 
     def step(self, poses, vels):
+        """One control cycle.  Per robot: cost, xv, yv, thetav, best_index, n_samples, n_scored with DWAPlanner;
+        cost, xv, yv, thetav, flags, n_points with the TrajectoryPlanner (navgpu_tp_result)."""
         p = np.ascontiguousarray(poses, dtype=np.float64)
         v = np.ascontiguousarray(vels, dtype=np.float64)
         assert p.shape == (self.n, 3) and v.shape == (self.n, 3)
-        self.api.check(self.lib.navgpu_fleet_step(self.h, _p(p, _f64p), _p(v, _f64p), self._results))
-        r = self._results
+        r = self.step_raw(p, v)
+        if self.tp_cfg is not None:
+            return [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, flags=r[i].flags,
+                         n_points=r[i].n_points) for i in range(self.n)]
         return [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, best_index=r[i].best_index,
                      n_samples=r[i].n_samples, n_scored=r[i].n_scored) for i in range(self.n)]
 
     def step_raw(self, poses, vels):
         """step() without building Python dicts (benchmarks); returns the ctypes result array."""
-        self.api.check(self.lib.navgpu_fleet_step(self.h, _p(poses, _f64p), _p(vels, _f64p), self._results))
+        step = self.lib.navgpu_fleet_step if self.tp_cfg is None else self.lib.navgpu_fleet_step_tp
+        self.api.check(step(self.h, _p(poses, _f64p), _p(vels, _f64p), self._results))
         return self._results
+
+    def tp_grid(self, robot, which):
+        """TrajectoryPlanner fleets: path_map_ (which = 0) or goal_map_ (1) of robot after the last step."""
+        out = np.empty((self.size_y, self.size_x), dtype=np.float64)
+        self.api.check(self.lib.navgpu_fleet_tp_get_grid(self.h, robot, which, _p(out, _f64p)))
+        return out
+
+    def tp_timing(self):
+        """TrajectoryPlanner fleets: device ms of the last step's footprint-cell, wavefront and scoring launches."""
+        a, b, c = C.c_float(), C.c_float(), C.c_float()
+        self.api.check(self.lib.navgpu_fleet_tp_last_timing(self.h, C.byref(a), C.byref(b), C.byref(c)))
+        return float(a.value), float(b.value), float(c.value)
 
     def costmap(self, robot):
         out = np.empty((self.size_y, self.size_x), dtype=np.uint8)
@@ -922,21 +960,25 @@ class Api:
         self.check(self.lib.navgpu_dwa_shard_connect_local(arr, len(dwas)))
 
     def fleet(self, *a, **k):
+        """A raw-map fleet (see Fleet); trajectory_planner={...} runs the legacy TrajectoryPlanner instead of DWAPlanner."""
         return Fleet(self, *a, **k)
 
     def fleet_sensing(self, n, sx, sy, res, footprint, inflation_radius=0.55, cost_scaling_factor=10.0,
                       combination_method=1, footprint_clearing=True, max_obstacle_height=2.0, track_unknown=False,
-                      device=0, voxel=None, **dwa_overrides):
+                      device=0, voxel=None, trajectory_planner=None, **dwa_overrides):
         """A fleet whose robots each run a rolling sx x sy local costmap [ObstacleLayer, InflationLayer] fed by their
         own scans (Fleet.set_scans), then DWAPlanner (navgpu_fleet_create_sensing).  voxel: a FleetVoxelConfig or a
         dict of its fields (origin_z, z_resolution, z_voxels, unknown_threshold, mark_threshold; missing ones take
-        VoxelPlugin.cfg's defaults) makes it [VoxelLayer, InflationLayer] (navgpu_fleet_create_sensing_voxel)."""
+        VoxelPlugin.cfg's defaults) makes it [VoxelLayer, InflationLayer] (navgpu_fleet_create_sensing_voxel).
+        trajectory_planner: a dict of TpConfig overrides, possibly empty, runs the legacy TrajectoryPlanner instead of
+        DWAPlanner (see Fleet)."""
         cm = FleetCostmapConfig(inflation_radius=inflation_radius, cost_scaling_factor=cost_scaling_factor,
                                 max_obstacle_height=max_obstacle_height, combination_method=combination_method,
                                 footprint_clearing=int(footprint_clearing), track_unknown=int(track_unknown))
         if isinstance(voxel, dict):
             voxel = FleetVoxelConfig(**{**VOXEL_DEFAULTS, **voxel})
-        return Fleet(self, n, sx, sy, res, footprint, device=device, sensing=cm, voxel=voxel, **dwa_overrides)
+        return Fleet(self, n, sx, sy, res, footprint, device=device, sensing=cm, voxel=voxel,
+                     trajectory_planner=trajectory_planner, **dwa_overrides)
 
     def trajectory_planner(self, *a, **k):
         return TrajectoryPlanner(self, *a, **k)

@@ -1025,6 +1025,11 @@ namespace {
 constexpr unsigned kFleetPadRows = 64;  // >= 2 * the largest cell inflation radius the fast sweep supports (31)
 }
 
+// the planner side of fleets of legacy TrajectoryPlanners (navgpu_fleet_use_trajectory_planner, tp_host.inc)
+struct FleetTp;
+static void fleet_tp_free(FleetTp* t);
+static int fleet_tp_set_plans(navgpu_fleet* f, const double* plan_xy, const int32_t* plan_offsets);
+
 struct navgpu_fleet {
   int device = 0;
   int n = 0;
@@ -1065,6 +1070,8 @@ struct navgpu_fleet {
   bool plans_dirty = true;
   std::vector<FleetRobot> h_robots;
   std::vector<size_t> plan_off;  // per robot x 3 plans: offset (in points) into d_plans
+  bool started = false;          // set_plans or a step has run
+  FleetTp* tp = nullptr;         // non-null: the robots run base_local_planner::TrajectoryPlanner instead of DWAPlanner
 };
 
 // what every fleet holds for its planner side: the DWAPlanner parameters and critic scales ...
@@ -1191,6 +1198,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
   cudaFree(f->d_stage); cudaFree(f->d_raw); cudaFree(f->d_robots); cudaFree(f->d_plans); cudaFree(f->d_samples); cudaFree(f->d_dist);
   cudaFree(f->d_block_cost); cudaFree(f->d_block_index); cudaFree(f->d_generated); cudaFree(f->d_results);
   cudaFreeHost(f->h_results);
+  fleet_tp_free(f->tp);
   navgpu_costmap_destroy(f->costmap);
   fleet_costmap_destroy(f->sensing);  // (owns the stream of a sensing fleet)
   delete f;
@@ -1223,6 +1231,8 @@ int navgpu_fleet_set_maps(navgpu_fleet* f, const uint8_t* raw_maps, const double
 // points, poses [n][3]
 int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* plan_xy, const int32_t* plan_offsets) {
   if (!f || !poses || !plan_xy || !plan_offsets) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  f->started = true;
+  if (f->tp) return fleet_tp_set_plans(f, plan_xy, plan_offsets);
   const navgpu_dwa_config& c = f->cfg;
   for (int r = 0; r < f->n; ++r) {
     const int b = plan_offsets[r], e = plan_offsets[r + 1];
@@ -1255,6 +1265,7 @@ int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* p
 
 int navgpu_fleet_reset_oscillation(navgpu_fleet* f) {
   if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (f->tp) return fail(NAVGPU_ERR_INVALID, "a TrajectoryPlanner fleet has no DWA oscillation flags (see navgpu_fleet_step_tp's flags)");
   for (Oscillation& o : f->osc) o.reset();
   return NAVGPU_OK;
 }
@@ -1263,6 +1274,8 @@ int navgpu_fleet_reset_oscillation(navgpu_fleet* f) {
 // poses, vels: [n][3]; results: n entries (n_points is always 0: the winners' points are not materialised).
 int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, navgpu_dwa_result* results) {
   if (!f || !poses || !vels || !results) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->tp) return fail(NAVGPU_ERR_INVALID, "a TrajectoryPlanner fleet steps with navgpu_fleet_step_tp");
+  f->started = true;
   NAVGPU_CUDA(cudaSetDevice(f->device));
   const navgpu_dwa_config& c = f->cfg;
   const int n = f->n;
@@ -1433,6 +1446,7 @@ int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out) {
 
 int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out) {
   if (!f || robot < 0 || robot >= f->n || !mask_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->tp) return fail(NAVGPU_ERR_INVALID, "a TrajectoryPlanner fleet has no DWA oscillation flags (see navgpu_fleet_step_tp's flags)");
   *mask_out = f->osc[robot].mask();
   return NAVGPU_OK;
 }

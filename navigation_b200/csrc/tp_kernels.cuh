@@ -273,4 +273,214 @@ __global__ void __launch_bounds__(kDwaWarpsPerBlock * 32) k_tp_score(TpScoreArgs
   tp_score_sample(a, sample, lane, scratch[warp]);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// FootprintHelper::getFootprintCells(pos, footprint_spec_, costmap_, fill = true), footprint_helper.cpp:180-246, for
+// the host (the single planner) and the device (fleets) alike.  Cells are packed y << 16 | x (maps are at most 32767
+// cells a side) into a caller-provided buffer of `cap` cells; cos / sin of the heading come from the caller, so both
+// sides see the host's libm values.  Returns the number of cells, or -1 when they would not fit (tp_footprint_capacity
+// bounds them).  Multiplications are rounded one by one, as the reference's x86-64 code rounds them.
+__host__ __device__ __forceinline__ double tp_mul(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __dmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+
+struct TpCellBuffer {
+  uint32_t* cell;
+  int n, cap;
+  __host__ __device__ bool push(unsigned x, unsigned y) {
+    if (n >= cap) return false;
+    cell[n++] = (y << 16) | x;
+    return true;
+  }
+};
+
+// Costmap2D::worldToMap (costmap_2d.cpp:208-220)
+__host__ __device__ __forceinline__ bool tp_world_to_map(double wx, double wy, double ox, double oy, double res,
+                                                         unsigned sx, unsigned sy, unsigned& mx, unsigned& my) {
+  if (wx < ox || wy < oy) return false;
+  mx = (int)((wx - ox) / res);
+  my = (int)((wy - oy) / res);
+  return mx < sx && my < sy;
+}
+
+// FootprintHelper::getLineCells, footprint_helper.cpp:51-120
+__host__ __device__ inline bool tp_line_cells(int x0, int x1, int y0, int y1, TpCellBuffer& out) {
+  const int dx = abs(x1 - x0), dy = abs(y1 - y0);
+  const int sxi = x1 >= x0 ? 1 : -1, syi = y1 >= y0 ? 1 : -1;
+  const bool xmajor = dx >= dy;
+  const int den = xmajor ? dx : dy, numadd = xmajor ? dy : dx;
+  int num = den / 2, x = x0, y = y0;
+  for (int k = 0; k <= den; ++k) {
+    if (!out.push((unsigned)x, (unsigned)y)) return false;
+    num += numadd;
+    if (num >= den) {
+      num -= den;
+      if (xmajor) y += syi; else x += sxi;
+    }
+    if (xmajor) x += sxi; else y += syi;
+  }
+  return true;
+}
+
+// FootprintHelper::getFillCells, footprint_helper.cpp:123-178: the outline sorted by x (stable for equal x, as the
+// adjacent-swap sort is), then one [min_y, max_y) run per column, appended to the list the walk itself is reading
+__host__ __device__ inline bool tp_fill_cells(TpCellBuffer& fp) {
+  uint32_t* c = fp.cell;
+  for (int k = 1; k < fp.n; ++k) {  // insertion sort by x: stable
+    const uint32_t key = c[k];
+    int j = k - 1;
+    while (j >= 0 && (c[j] & 0xffffu) > (key & 0xffffu)) {
+      c[j + 1] = c[j];
+      --j;
+    }
+    c[j + 1] = key;
+  }
+  int i = 0;
+  const unsigned min_x = c[0] & 0xffffu, max_x = c[fp.n - 1] & 0xffffu;
+  for (unsigned x = min_x; x <= max_x; ++x) {
+    if (i >= fp.n - 1) break;
+    uint32_t lo, hi;
+    if ((c[i] >> 16) < (c[i + 1] >> 16)) { lo = c[i]; hi = c[i + 1]; }
+    else { lo = c[i + 1]; hi = c[i]; }
+    i += 2;
+    while (i < fp.n && (c[i] & 0xffffu) == x) {
+      if ((c[i] >> 16) < (lo >> 16)) lo = c[i];
+      else if ((c[i] >> 16) > (hi >> 16)) hi = c[i];
+      ++i;
+    }
+    for (unsigned y = lo >> 16; y < (hi >> 16); ++y)
+      if (!fp.push(x, y)) return false;
+  }
+  return true;
+}
+
+__host__ __device__ inline int tp_footprint_cells(const double* fpx, const double* fpy, int nfp, double x_i, double y_i,
+                                                  double cos_th, double sin_th, double ox, double oy, double res,
+                                                  unsigned sx, unsigned sy, uint32_t* cells, int cap) {
+  TpCellBuffer b{cells, 0, cap};
+  if (nfp <= 1) {
+    unsigned mx, my;
+    if (tp_world_to_map(x_i, y_i, ox, oy, res, sx, sy, mx, my) && !b.push(mx, my)) return -1;
+    return b.n;
+  }
+  for (int i = 0; i < nfp; ++i) {  // edges (i, i + 1), the closing edge last
+    const int j = i + 1 < nfp ? i + 1 : 0;
+    unsigned x0, y0, x1, y1;
+    // a vertex off the map: the outline cells gathered so far, unfilled
+    if (!tp_world_to_map(x_i + (tp_mul(fpx[i], cos_th) - tp_mul(fpy[i], sin_th)),
+                         y_i + (tp_mul(fpx[i], sin_th) + tp_mul(fpy[i], cos_th)), ox, oy, res, sx, sy, x0, y0))
+      return b.n;
+    if (!tp_world_to_map(x_i + (tp_mul(fpx[j], cos_th) - tp_mul(fpy[j], sin_th)),
+                         y_i + (tp_mul(fpx[j], sin_th) + tp_mul(fpy[j], cos_th)), ox, oy, res, sx, sy, x1, y1))
+      return b.n;
+    if (!tp_line_cells((int)x0, (int)x1, (int)y0, (int)y1, b)) return -1;
+  }
+  if (!tp_fill_cells(b)) return -1;
+  return b.n;
+}
+
+// An upper bound of tp_footprint_cells' count for a footprint at any pose and resolution: every edge's line (at most
+// its length in cells + 2), plus one run per column of the outline's bounding box, both at most the circumscribed
+// diameter + 2 cells long
+inline long long tp_footprint_capacity(const double* fpx, const double* fpy, int nfp, double res) {
+  if (nfp <= 1) return 1;
+  double r = 0.0;
+  long long outline = 0;
+  for (int i = 0; i < nfp; ++i) {
+    const int j = i + 1 < nfp ? i + 1 : 0;
+    r = fmax(r, hypot(fpx[i], fpy[i]));
+    outline += (long long)(hypot(fpx[j] - fpx[i], fpy[j] - fpy[i]) / res) + 3;
+  }
+  const long long side = (long long)(2.0 * r / res) + 3;
+  return outline + side * side;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Fleets of legacy TrajectoryPlanners (navgpu_fleet_use_trajectory_planner): what changes per robot and step
+struct TpFleetRobot {
+  double x, y, theta, vx, vy, vtheta;  // through (float), as navgpu_tp_find_best_path rounds them
+  double cos_th, sin_th;               // the host's cos / sin of theta, for the footprint cells
+  double ox, oy;                       // the robot's map origin
+  double goal_x, goal_y;               // last pose of its plan (0, 0 without one)
+  int plan_offset, n_plan;             // its raw plan in the fleet's plan array (n_plan is 0 without heading scoring)
+  int sample_offset, n_samples;        // its slice of the step's samples and results
+};
+
+struct TpFleetLayout {
+  const uint8_t* cost;       // robot r's local costmap at cost + r * cost_stride, row pitch g.pitch
+  size_t cost_stride;
+  uint32_t* dist;            // robot r: path_map_ at dist + 2r * sx*sy, goal_map_ right after it
+  uint32_t* within;          // robot r: MapCell::within_robot bits at within + r * within_words
+  int within_words;
+  const double* plans_raw;   // every robot's raw plan, (x, y) pairs
+  const double* samples;     // n_total x 3
+  TpSampleResult* out;       // n_total
+  const double* fpx;         // the footprint (device copy), nfp vertices
+  const double* fpy;
+  int cells_cap;             // tp_footprint_capacity of the footprint
+};
+
+// TrajectoryPlanner::findBestPath's path_map_ cells under the robot (trajectory_planner.cpp:918-930) for every robot:
+// one warp per robot clears its bit mask while lane 0 gathers the cells in shared memory; the warp then sets them
+__global__ void __launch_bounds__(32) k_tp_fleet_footprint(TpFleetLayout L, const TpFleetRobot* robots, unsigned sx,
+                                                           unsigned sy, double res, int nfp) {
+  extern __shared__ uint32_t s_cells[];
+  __shared__ int s_n;
+  const int robot = blockIdx.x, lane = threadIdx.x;
+  uint32_t* within = L.within + (size_t)robot * L.within_words;
+  for (int w = lane; w < L.within_words; w += 32) within[w] = 0u;
+  if (lane == 0) {
+    const TpFleetRobot& r = robots[robot];
+    s_n = tp_footprint_cells(L.fpx, L.fpy, nfp, r.x, r.y, r.cos_th, r.sin_th, r.ox, r.oy, res, sx, sy, s_cells, L.cells_cap);
+  }
+  __syncwarp();
+  const int W = (int)(sx + 31) / 32;
+  for (int k = lane; k < s_n; k += 32) {
+    const unsigned x = s_cells[k] & 0xffffu, y = s_cells[k] >> 16;
+    if (x < sx && y < sy) atomicOr(&within[y * W + (x >> 5)], 1u << (x & 31));
+  }
+}
+
+// generateTrajectory of every robot's velocity samples in one launch: robot-major CTAs, blocks_per_robot per robot, one
+// warp per sample, each CTA scoring against its robot's view of the arguments (no points are stored)
+__global__ void __launch_bounds__(kDwaWarpsPerBlock * 32) k_tp_fleet_score(TpScoreArgs base, TpFleetLayout L,
+                                                                         const TpFleetRobot* robots, int blocks_per_robot) {
+  __shared__ TpScoreArgs s_a;
+  __shared__ double scratch[kDwaWarpsPerBlock][kWarpScratchDoubles];
+  const int robot = blockIdx.x / blocks_per_robot, local = blockIdx.x % blocks_per_robot;
+  const TpFleetRobot& r = robots[robot];
+  const int n = r.n_samples;
+  if (local * kDwaWarpsPerBlock >= n) return;  // no samples for this CTA
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(&base);
+  uint32_t* dst = reinterpret_cast<uint32_t*>(&s_a);
+  for (int i = threadIdx.x; i < (int)(sizeof(TpScoreArgs) / 4); i += blockDim.x) dst[i] = src[i];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const size_t cells = (size_t)base.g.sx * base.g.sy;
+    s_a.g.cost = L.cost + (size_t)robot * L.cost_stride;
+    s_a.g.ox = r.ox;
+    s_a.g.oy = r.oy;
+    s_a.path_dist = L.dist + 2 * (size_t)robot * cells;
+    s_a.goal_dist = s_a.path_dist + cells;
+    s_a.samples = L.samples + 3 * (size_t)r.sample_offset;
+    s_a.n = n;
+    s_a.x = r.x; s_a.y = r.y; s_a.theta = r.theta;
+    s_a.vx = r.vx; s_a.vy = r.vy; s_a.vtheta = r.vtheta;
+    s_a.goal_x = r.goal_x;
+    s_a.goal_y = r.goal_y;
+    s_a.plan_xy = L.plans_raw + 2 * (size_t)r.plan_offset;
+    s_a.n_plan = r.n_plan;
+    s_a.out = L.out + r.sample_offset;
+    s_a.points = nullptr;
+  }
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int sample = local * kDwaWarpsPerBlock + warp;
+  if (sample >= n) return;
+  tp_score_sample(s_a, sample, lane, scratch[warp]);
+}
+
 }  // namespace navgpu
