@@ -407,6 +407,37 @@ int navgpu_fleet_create_sensing(navgpu_fleet** out, int n_robots, const navgpu_d
  * persist until the next call, like the observations of navgpu_obstacle_set_scans.  All robots' scans are projected in
  * one launch.  offsets: n_robots + 1 non-decreasing entries. */
 int navgpu_fleet_set_scans(navgpu_fleet* f, const navgpu_laser_scan* scans, const int32_t* offsets);
+/* Batched ingest for fleets whose robots all carry the same sensors: one source of every robot as dense arrays.  The
+ * fields have navgpu_laser_scan's meaning; row r of data and of sensor_to_global belong to robot r. */
+typedef struct {
+  const float* data;              /* [n_robots][n_points] LaserScan ranges, or [n_robots][n_points][3] sensor-frame points (is_cloud) */
+  const double* sensor_to_global; /* [n_robots][7]: translation x, y, z, then rotation x, y, z, w (tf order) */
+  int32_t n_points;               /* per robot, >= 0 */
+  int32_t is_cloud, inf_is_valid, marking, clearing;
+  float angle_min, angle_increment, range_min, range_max;
+  double min_obstacle_height, max_obstacle_height, obstacle_range, raytrace_range;
+} navgpu_fleet_scan_source;
+/* Equivalent to navgpu_fleet_set_scans with robot r's list [source 0, ..., source n_sources - 1], each entry built from
+ * the source's shared fields, row r of data and row r of sensor_to_global: the same grids, columns, windows, origins
+ * and planner results bit for bit.  The sources replace the previous ones and persist.  One kernel builds every
+ * robot's observation records and projects every point; nothing per robot is built on the host.  n_sources = 0
+ * empties every robot's list.  Sensing fleets of either kind, with either planner; NAVGPU_ERR_INVALID on a raw-map
+ * fleet.  Refused, with the fleet's sources left as they were: a null handle or sources, n_sources < 0, a null
+ * sensor_to_global, a null data with n_points > 0, n_points < 0 or is_cloud / marking / clearing outside {0, 1}
+ * (NAVGPU_ERR_INVALID); more than 32 sources, or n_robots x the points of all sources beyond 2^31 - 1
+ * (NAVGPU_ERR_UNSUPPORTED).
+ * navgpu_fleet_set_scan_batch: the arrays are HOST memory, pageable or registered (navgpu_host_register); each is copied
+ * to the device with its own copy, and the call returns once they were read.
+ * navgpu_fleet_set_scan_batch_device: the arrays are device (or managed) memory of the fleet's device, anything else is
+ * refused with NAVGPU_ERR_INVALID; the descriptors themselves are host memory.  The arrays are read in place on the
+ * fleet's stream (navgpu_fleet_stream) and the call returns without waiting for it.  The caller orders its writes of
+ * the arrays before that stream (for example cudaEventRecord on the writing stream, then cudaStreamWaitEvent on
+ * navgpu_fleet_stream(f)), and must not change them until the fleet's stream has read them: the return of the next
+ * navgpu_fleet_step / navgpu_fleet_step_tp is enough. */
+int navgpu_fleet_set_scan_batch(navgpu_fleet* f, const navgpu_fleet_scan_source* sources, int n_sources);
+int navgpu_fleet_set_scan_batch_device(navgpu_fleet* f, const navgpu_fleet_scan_source* sources, int n_sources);
+/* the CUDA stream every kernel of this fleet runs on (cudaStream_t), like navgpu_costmap_stream / navgpu_dwa_stream */
+void* navgpu_fleet_stream(navgpu_fleet* f);
 /* per robot, after the last navgpu_fleet_step: the ObstacleLayer's own grid (HOST size_y x size_x) */
 int navgpu_fleet_get_layer(navgpu_fleet* f, int robot, uint8_t* host_out);
 /* per robot, after the last navgpu_fleet_step: the rolled origin and the cycle's window {x0, xn, y0, yn} */

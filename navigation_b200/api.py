@@ -5,6 +5,7 @@ this module never imports or loads anything from oracle/.
 """
 import ctypes as C
 import os
+import sys
 
 import numpy as np
 
@@ -49,6 +50,15 @@ class LaserScan(C.Structure):
                 ("min_obstacle_height", C.c_double), ("max_obstacle_height", C.c_double),
                 ("obstacle_range", C.c_double), ("raytrace_range", C.c_double), ("marking", C.c_int32),
                 ("clearing", C.c_int32), ("is_cloud", C.c_int32), ("pad_", C.c_int32)]
+
+
+class FleetScanSource(C.Structure):
+    """navgpu_fleet_scan_source: one sensor of every robot of a sensing fleet, as dense arrays"""
+    _fields_ = [("data", C.c_void_p), ("sensor_to_global", C.c_void_p), ("n_points", C.c_int32),
+                ("is_cloud", C.c_int32), ("inf_is_valid", C.c_int32), ("marking", C.c_int32), ("clearing", C.c_int32),
+                ("angle_min", C.c_float), ("angle_increment", C.c_float), ("range_min", C.c_float),
+                ("range_max", C.c_float), ("min_obstacle_height", C.c_double), ("max_obstacle_height", C.c_double),
+                ("obstacle_range", C.c_double), ("raytrace_range", C.c_double)]
 
 
 class FleetCostmapConfig(C.Structure):
@@ -198,6 +208,9 @@ SIGNATURES = {
     "navgpu_fleet_create_sensing": (C.c_int, [_vpp, C.c_int, C.POINTER(DwaConfig), C.c_uint32, C.c_uint32, C.c_double,
                                               C.POINTER(FleetCostmapConfig), _f64p, C.c_int, C.c_int]),
     "navgpu_fleet_set_scans": (C.c_int, [C.c_void_p, C.POINTER(LaserScan), _i32p]),
+    "navgpu_fleet_set_scan_batch": (C.c_int, [C.c_void_p, C.POINTER(FleetScanSource), C.c_int]),
+    "navgpu_fleet_set_scan_batch_device": (C.c_int, [C.c_void_p, C.POINTER(FleetScanSource), C.c_int]),
+    "navgpu_fleet_stream": (C.c_void_p, [C.c_void_p]),
     "navgpu_fleet_get_layer": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
     "navgpu_fleet_get_geometry": (C.c_int, [C.c_void_p, C.c_int, _f64p, _i32p]),
     "navgpu_fleet_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
@@ -800,6 +813,8 @@ class Fleet:
         results."""
         self.api, self.lib, self.n = api, api.lib, n_robots
         self.size_x, self.size_y = size_x, size_y
+        self.device = device
+        self._batch_keep = None  # the device arrays of the last set_scan_batch, alive until the next one
         self.cfg = DwaConfig()
         self.lib.navgpu_dwa_default_config(C.byref(self.cfg))
         for k, v in overrides.items():
@@ -898,6 +913,76 @@ class Fleet:
         off[1:] = np.cumsum([len(s) for s in scans_per_robot])
         arr, _keep = pack_scans([s for robot in scans_per_robot for s in robot])
         self.api.check(self.lib.navgpu_fleet_set_scans(self.h, arr, _p(off, _i32p)))
+
+    def set_scan_batch(self, sources):
+        """Sensing fleets whose robots carry the same sensors: robot r's sources become [source 0, source 1, ...],
+        each built from the source's shared fields and row r of its arrays -- set_scans with those lists, bit for bit.
+        A source is a dict with the scan-dict fields (angle_min, angle_increment, range_min, range_max, inf_is_valid,
+        min_obstacle_height, max_obstacle_height, obstacle_range, raytrace_range, marking, clearing), either `ranges`
+        [n, B] float32 (LaserScan) or `points` [n, B, 3] float32 (sensor-frame cloud), and `sensor_to_global` [n, 7]
+        float64 (translation x, y, z, rotation x, y, z, w).
+        numpy arrays and CPU torch tensors are copied to the device and read before the call returns
+        (navgpu_fleet_set_scan_batch).  Contiguous CUDA torch tensors on the fleet's device are read in place on the
+        fleet's stream, after the work already queued on torch's current stream (navgpu_fleet_set_scan_batch_device):
+        leave them unchanged until the next step returns.  Mixed host and device arrays, wrong shapes and wrong dtypes
+        raise ValueError."""
+        torch = sys.modules.get("torch")  # a torch tensor can only come from a caller that imported torch
+        arr = (FleetScanSource * max(1, len(sources)))()
+        keep, where = [], set()
+
+        def take(x, what, dtype, shape):
+            if torch is not None and isinstance(x, torch.Tensor):
+                if x.dtype != getattr(torch, dtype) or x.dim() != len(shape) or \
+                        any(s is not None and x.shape[i] != s for i, s in enumerate(shape)):
+                    raise ValueError(f"{what}: a {dtype} tensor of shape {shape}, not {x.dtype} {tuple(x.shape)}")
+                if x.is_cuda:
+                    if x.device.index != self.device or not x.is_contiguous():
+                        raise ValueError(f"{what}: a contiguous tensor on cuda:{self.device}")
+                    where.add("device")
+                    keep.append(x)
+                    return x.data_ptr(), x.shape
+                x = x.detach().numpy()
+            if not isinstance(x, np.ndarray):
+                raise ValueError(f"{what}: a numpy array or a torch tensor, not {type(x).__name__}")
+            if x.dtype != np.dtype(dtype) or x.ndim != len(shape) or \
+                    any(s is not None and x.shape[i] != s for i, s in enumerate(shape)):
+                raise ValueError(f"{what}: a {dtype} array of shape {shape}, not {x.dtype} {x.shape}")
+            x = np.ascontiguousarray(x)
+            where.add("host")
+            keep.append(x)
+            return x.ctypes.data, x.shape
+
+        for k, src in enumerate(sources):
+            cloud = "points" in src
+            if cloud == ("ranges" in src):
+                raise ValueError(f"source {k}: give either ranges or points")
+            s = arr[k]
+            if cloud:
+                s.data, shape = take(src["points"], f"source {k} points", "float32", (self.n, None, 3))
+            else:
+                s.data, shape = take(src["ranges"], f"source {k} ranges", "float32", (self.n, None))
+                s.angle_min, s.angle_increment = src["angle_min"], src["angle_increment"]
+                s.range_min, s.range_max = src["range_min"], src["range_max"]
+            s.sensor_to_global, _ = take(src["sensor_to_global"], f"source {k} sensor_to_global", "float64", (self.n, 7))
+            s.n_points, s.is_cloud = int(shape[1]), int(cloud)
+            s.inf_is_valid = int(src.get("inf_is_valid", 0))
+            s.min_obstacle_height, s.max_obstacle_height = src["min_obstacle_height"], src["max_obstacle_height"]
+            s.obstacle_range, s.raytrace_range = src["obstacle_range"], src["raytrace_range"]
+            s.marking, s.clearing = int(src.get("marking", True)), int(src.get("clearing", True))
+        if len(where) > 1:
+            raise ValueError("a batch is either host arrays or device arrays, not both")
+        if where == {"device"}:
+            dev = torch.device("cuda", self.device)
+            torch.cuda.ExternalStream(self.stream(), device=dev).wait_stream(torch.cuda.current_stream(dev))
+            self.api.check(self.lib.navgpu_fleet_set_scan_batch_device(self.h, arr, len(sources)))
+            self._batch_keep = keep
+        else:
+            self.api.check(self.lib.navgpu_fleet_set_scan_batch(self.h, arr, len(sources)))
+            self._batch_keep = None
+
+    def stream(self):
+        """The CUDA stream (cudaStream_t as an int) every kernel of this fleet runs on."""
+        return self.lib.navgpu_fleet_stream(self.h)
 
     def layer(self, robot):
         """Sensing fleets: robot's ObstacleLayer (or VoxelLayer) grid after the last step."""

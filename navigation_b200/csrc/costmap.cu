@@ -1213,17 +1213,7 @@ static void scan_record(const navgpu_laser_scan& sc, int first_point, int first_
   r.angle_increment = sc.angle_increment;
   r.range_min = sc.range_min;
   r.range_max = sc.range_max;
-  // pcl_ros::transformPointCloud: Eigen::Quaternionf(w, x, y, z) -> float rotation matrix (Eigen's
-  // QuaternionBase::toRotationMatrix), Eigen::Vector3f origin; all arithmetic in float
-  const float qx = (float)sc.sensor_to_global_rotation_xyzw[0], qy = (float)sc.sensor_to_global_rotation_xyzw[1],
-              qz = (float)sc.sensor_to_global_rotation_xyzw[2], qw = (float)sc.sensor_to_global_rotation_xyzw[3];
-  const float tx = 2.0f * qx, ty = 2.0f * qy, tz = 2.0f * qz;
-  const float twx = tx * qw, twy = ty * qw, twz = tz * qw, txx = tx * qx, txy = ty * qx, txz = tz * qx, tyy = ty * qy,
-              tyz = tz * qy, tzz = tz * qz;
-  r.m[0] = 1.0f - (tyy + tzz); r.m[1] = txy - twz; r.m[2] = txz + twy;
-  r.m[3] = txy + twz; r.m[4] = 1.0f - (txx + tzz); r.m[5] = tyz - twx;
-  r.m[6] = txz - twy; r.m[7] = tyz + twx; r.m[8] = 1.0f - (txx + tyy);
-  for (int k = 0; k < 3; ++k) r.t[k] = (float)sc.sensor_to_global_translation[k];
+  sensor_affine(sc.sensor_to_global_rotation_xyzw, sc.sensor_to_global_translation, r.m, r.t);
   r.min_obstacle_height = sc.min_obstacle_height;
   r.max_obstacle_height = sc.max_obstacle_height;
   r.inf_is_valid = sc.inf_is_valid;
@@ -2086,6 +2076,106 @@ int fleet_costmap_set_scans(FleetCostmap* fc, const navgpu_laser_scan* scans, co
     NAVGPU_CUDA(cudaGetLastError());
   }
   NAVGPU_CUDA(cudaStreamSynchronize(fc->stream));  // the staging vectors above are pageable
+  return NAVGPU_OK;
+}
+
+// device or managed memory of `device`
+static bool on_device(const void* p, int device) {
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();  // not a CUDA pointer at all: clear the error, it is the caller's
+    return false;
+  }
+  return (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && at.device == device;
+}
+
+int fleet_costmap_set_scan_batch(FleetCostmap* fc, const navgpu_fleet_scan_source* sources, int n_sources, bool device) {
+  // every check before anything changes: a refused call leaves the previous sources in place
+  if (n_sources < 0 || !sources) return fail(NAVGPU_ERR_INVALID, "bad sources");
+  if (n_sources > kScanBatchSources)
+    return fail(NAVGPU_ERR_UNSUPPORTED, "%d sources: a batch holds up to %d", n_sources, kScanBatchSources);
+  const auto bit = [](int32_t v) { return v == 0 || v == 1; };
+  long long per_robot = 0;
+  for (int s = 0; s < n_sources; ++s) {
+    const navgpu_fleet_scan_source& c = sources[s];
+    if (!c.sensor_to_global || c.n_points < 0 || (c.n_points > 0 && !c.data) || !bit(c.is_cloud) || !bit(c.marking) ||
+        !bit(c.clearing))
+      return fail(NAVGPU_ERR_INVALID, "bad source %d", s);
+    per_robot += c.n_points;
+  }
+  if (per_robot * fc->n > 0x7fffffffll) return fail(NAVGPU_ERR_UNSUPPORTED, "more than 2^31 scan points");
+  if (device)
+    for (int s = 0; s < n_sources; ++s)
+      if (!on_device(sources[s].sensor_to_global, fc->device) || (sources[s].n_points > 0 && !on_device(sources[s].data, fc->device)))
+        return fail(NAVGPU_ERR_INVALID, "source %d: not device memory of device %d", s, fc->device);
+  NAVGPU_CUDA(cudaSetDevice(fc->device));
+
+  // the regular layout of k_fleet_scan_batch, and set_scans' listing rules: a clearing source is listed even without
+  // points (raytraceFreespace still touches its origin), a marking source only with points
+  ScanBatchArgs a;
+  a.n_sources = n_sources;
+  a.n = fc->n;
+  a.points = a.n_clear = a.n_mark = a.rays = a.marks = 0;
+  size_t stage_bytes = 0;  // host variant: every array behind the previous one (transforms 8-byte aligned, first)
+  for (int s = 0; s < n_sources; ++s) {
+    const navgpu_fleet_scan_source& c = sources[s];
+    ScanBatchSource& b = a.src[s];
+    b.data = c.data;
+    b.stg = c.sensor_to_global;
+    b.angle_min = c.angle_min;
+    b.angle_increment = c.angle_increment;
+    b.min_obstacle_height = c.min_obstacle_height;
+    b.max_obstacle_height = c.max_obstacle_height;
+    b.obstacle_range = c.obstacle_range;
+    b.raytrace_range = c.raytrace_range;
+    b.range_min = c.range_min;
+    b.range_max = c.range_max;
+    b.n_points = c.n_points;
+    b.is_cloud = c.is_cloud;
+    b.inf_is_valid = c.inf_is_valid;
+    b.flags = (c.marking ? 1 : 0) | (c.clearing ? 2 : 0);
+    b.point_first = a.points;
+    b.clear_slot = b.mark_slot = -1;
+    b.clear_ray = b.mark_ray = 0;
+    if (c.clearing) { b.clear_slot = a.n_clear++; b.clear_ray = a.rays; a.rays += c.n_points; }
+    if (c.marking && c.n_points > 0) { b.mark_slot = a.n_mark++; b.mark_ray = a.marks; a.marks += c.n_points; }
+    a.points += c.n_points;
+    stage_bytes += size_t(fc->n) * (7 * sizeof(double) + size_t(c.n_points) * (c.is_cloud ? 3 : 1) * sizeof(float));
+  }
+  const size_t n = size_t(fc->n);
+  NAVGPU_TRY(ensure_device(&fc->d_obs, &fc->obs_capacity, n * (a.n_clear + a.n_mark)));
+  NAVGPU_TRY(ensure_device(&fc->d_xyz, &fc->xyz_capacity, n * a.points * 3));
+  NAVGPU_TRY(ensure_device(&fc->d_mark_cells, &fc->mark_capacity, n * a.marks));
+  if (!device) {  // one plain copy per array into the staging buffer, then the device path on the copies
+    NAVGPU_TRY(ensure_device(&fc->d_scan, &fc->scan_capacity, stage_bytes));
+    char* p = fc->d_scan;
+    for (int s = 0; s < n_sources; ++s) {
+      const size_t bytes = n * 7 * sizeof(double);
+      NAVGPU_CUDA(cudaMemcpyAsync(p, sources[s].sensor_to_global, bytes, cudaMemcpyHostToDevice, fc->stream));
+      a.src[s].stg = reinterpret_cast<const double*>(p);
+      p += bytes;
+    }
+    for (int s = 0; s < n_sources; ++s) {
+      const size_t bytes = n * sources[s].n_points * (sources[s].is_cloud ? 3 : 1) * sizeof(float);
+      if (bytes) NAVGPU_CUDA(cudaMemcpyAsync(p, sources[s].data, bytes, cudaMemcpyHostToDevice, fc->stream));
+      a.src[s].data = reinterpret_cast<const float*>(p);
+      p += bytes;
+    }
+  }
+  a.xyz = fc->d_xyz;
+  a.obs = fc->d_obs;
+  a.robots = fc->d_robots;
+  long long threads = fc->n;
+  for (int s = 0; s < n_sources; ++s) threads = std::max(threads, (long long)fc->n * sources[s].n_points);
+  const dim3 grid((unsigned)((threads + kScanBatchThreads - 1) / kScanBatchThreads), (unsigned)std::max(1, n_sources));
+  NAVGPU_CUDA(cudaEventRecord(fc->ev[0], fc->stream));
+  k_fleet_scan_batch<<<grid, kScanBatchThreads, 0, fc->stream>>>(a);
+  NAVGPU_LAUNCHED(1);
+  NAVGPU_CUDA(cudaGetLastError());
+  NAVGPU_CUDA(cudaEventRecord(fc->ev[1], fc->stream));
+  fc->n_clear = fc->n * a.n_clear;
+  fc->projected = a.points > 0;
+  if (!device) NAVGPU_CUDA(cudaStreamSynchronize(fc->stream));  // the host arrays may be pageable
   return NAVGPU_OK;
 }
 

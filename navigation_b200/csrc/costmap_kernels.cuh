@@ -173,6 +173,62 @@ struct ScanRec {
   int is_cloud;     // 0: LaserScan ranges; 1: a PointCloud / PointCloud2 source, n_points x (x, y, z) in the sensor frame
 };
 
+// pcl_ros::transformPointCloud's Affine3f of a tf transform: Eigen::Quaternionf(w, x, y, z) -> float rotation matrix
+// (Eigen's QuaternionBase::toRotationMatrix, row-major into m), Eigen::Vector3f translation into t; all arithmetic in
+// float.  Shared by the host's record builder and k_fleet_scan_batch: x86-64 g++ does not contract and the device
+// build has -fmad=false, so both round every operation alike.
+__host__ __device__ inline void sensor_affine(const double q[4], const double tr[3], float m[9], float t[3]) {
+  const float qx = (float)q[0], qy = (float)q[1], qz = (float)q[2], qw = (float)q[3];
+  const float tx = 2.0f * qx, ty = 2.0f * qy, tz = 2.0f * qz;
+  const float twx = tx * qw, twy = ty * qw, twz = tz * qw, txx = tx * qx, txy = ty * qx, txz = tz * qx, tyy = ty * qy,
+              tyz = tz * qy, tzz = tz * qz;
+  m[0] = 1.0f - (tyy + tzz); m[1] = txy - twz; m[2] = txz + twy;
+  m[3] = txy + twz; m[4] = 1.0f - (txx + tzz); m[5] = tyz - twx;
+  m[6] = txz - twy; m[7] = tyz + twx; m[8] = 1.0f - (txx + tyy);
+  for (int k = 0; k < 3; ++k) t[k] = (float)tr[k];
+}
+
+// Point i of the scan described by r (first_point / first_range are not read): its world-frame (x, y, z) into out, or
+// NaN when the ray is dropped.  src: the scan's ranges, or its sensor-frame points for a cloud.  affine(m, t) yields
+// the record's rotation and translation (r.m / r.t are not read); it is called after the sensor-frame point exists, so
+// a caller that computes them does not hold them across sincos.
+template <class Affine>
+__device__ __forceinline__ void project_point(const ScanRec& r, const float* __restrict__ src, int i,
+                                              float* __restrict__ out, Affine affine) {
+  const float nanf_ = __int_as_float(0x7fc00000);
+  float ox = nanf_, oy = nanf_, oz = nanf_;
+  float x = 0.0f, y = 0.0f, z = 0.0f;
+  bool keep;
+  if (r.is_cloud) {  // pointCloudCallback / pointCloud2Callback (obstacle_layer.cpp:313-339): the points as they are
+    x = src[3 * i];
+    y = src[3 * i + 1];
+    z = src[3 * i + 2];
+    keep = true;
+  } else {
+    float range = src[i];
+    if (r.inf_is_valid && !isfinite(range) && range > 0) range = r.range_max - 0.0001f;
+    keep = range < r.range_max && range >= r.range_min;
+    if (keep) {
+      const double ang = r.angle_min + (double)i * r.angle_increment;
+      double sn, cs;
+      sincos(ang, &sn, &cs);
+      x = (float)((double)range * cs);
+      y = (float)((double)range * sn);
+    }
+  }
+  if (keep) {
+    float m[9], t[3];
+    affine(m, t);
+    const float gx = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z)), t[0]);
+    const float gy = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[3], x), __fmul_rn(m[4], y)), __fmul_rn(m[5], z)), t[1]);
+    const float gz = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[6], x), __fmul_rn(m[7], y)), __fmul_rn(m[8], z)), t[2]);
+    if ((double)gz <= r.max_obstacle_height && (double)gz >= r.min_obstacle_height) {
+      ox = gx; oy = gy; oz = gz;
+    }
+  }
+  out[0] = ox; out[1] = oy; out[2] = oz;
+}
+
 __global__ void k_project_scans(const ScanRec* __restrict__ recs, int n_scans, const float* __restrict__ ranges,
                                 float* __restrict__ xyz, int total) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -186,37 +242,10 @@ __global__ void k_project_scans(const ScanRec* __restrict__ recs, int n_scans, c
   }
   const ScanRec& r = recs[k];
   const int i = t - (r.first_point - recs[0].first_point);
-  const float nanf_ = __int_as_float(0x7fc00000);
-  float ox = nanf_, oy = nanf_, oz = nanf_;
-  float x = 0.0f, y = 0.0f, z = 0.0f;
-  bool keep;
-  if (r.is_cloud) {  // pointCloudCallback / pointCloud2Callback (obstacle_layer.cpp:313-339): the points as they are
-    x = ranges[r.first_range + 3 * i];
-    y = ranges[r.first_range + 3 * i + 1];
-    z = ranges[r.first_range + 3 * i + 2];
-    keep = true;
-  } else {
-    float range = ranges[r.first_range + i];
-    if (r.inf_is_valid && !isfinite(range) && range > 0) range = r.range_max - 0.0001f;
-    keep = range < r.range_max && range >= r.range_min;
-    if (keep) {
-      const double ang = r.angle_min + (double)i * r.angle_increment;
-      double sn, cs;
-      sincos(ang, &sn, &cs);
-      x = (float)((double)range * cs);
-      y = (float)((double)range * sn);
-    }
-  }
-  if (keep) {
-    const float gx = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(r.m[0], x), __fmul_rn(r.m[1], y)), __fmul_rn(r.m[2], z)), r.t[0]);
-    const float gy = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(r.m[3], x), __fmul_rn(r.m[4], y)), __fmul_rn(r.m[5], z)), r.t[1]);
-    const float gz = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(r.m[6], x), __fmul_rn(r.m[7], y)), __fmul_rn(r.m[8], z)), r.t[2]);
-    if ((double)gz <= r.max_obstacle_height && (double)gz >= r.min_obstacle_height) {
-      ox = gx; oy = gy; oz = gz;
-    }
-  }
-  float* out = xyz + 3 * (size_t)(r.first_point + i);
-  out[0] = ox; out[1] = oy; out[2] = oz;
+  project_point(r, ranges + r.first_range, i, xyz + 3 * (size_t)(r.first_point + i), [&](float m[9], float tr[3]) {
+    for (int k = 0; k < 9; ++k) m[k] = r.m[k];
+    for (int k = 0; k < 3; ++k) tr[k] = r.t[k];
+  });
 }
 
 // ObstacleLayer::raytraceFreespace (plugins/obstacle_layer.cpp:498-576) + Costmap2D::raytraceLine / bresenham2D

@@ -1448,6 +1448,20 @@ int navgpu_fleet_set_scans(navgpu_fleet* f, const navgpu_laser_scan* scans, cons
   return fleet_costmap_set_scans(f->sensing, scans, offsets);
 }
 
+int navgpu_fleet_set_scan_batch(navgpu_fleet* f, const navgpu_fleet_scan_source* sources, int n_sources) {
+  if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_set_scan_batch(f->sensing, sources, n_sources, false);
+}
+
+int navgpu_fleet_set_scan_batch_device(navgpu_fleet* f, const navgpu_fleet_scan_source* sources, int n_sources) {
+  if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");
+  return fleet_costmap_set_scan_batch(f->sensing, sources, n_sources, true);
+}
+
+void* navgpu_fleet_stream(navgpu_fleet* f) { return f ? (void*)f->stream : nullptr; }
+
 int navgpu_fleet_get_layer(navgpu_fleet* f, int robot, uint8_t* host_out) {
   if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   if (!f->sensing) return fail(NAVGPU_ERR_INVALID, "not a sensing fleet (navgpu_fleet_create_sensing)");

@@ -19,6 +19,8 @@ cudaStream_t fleet_costmap_stream(const FleetCostmap* fc);
 // the robots' master grids: robot r's is sy rows of `pitch` bytes at master + r * sy * pitch
 const uint8_t* fleet_costmap_master(const FleetCostmap* fc, unsigned* pitch);
 int fleet_costmap_set_scans(FleetCostmap* fc, const navgpu_laser_scan* scans, const int32_t* offsets);
+// navgpu_fleet_set_scan_batch (device false: host arrays, staged and waited for) and _device (device true)
+int fleet_costmap_set_scan_batch(FleetCostmap* fc, const navgpu_fleet_scan_source* sources, int n_sources, bool device);
 // host part of one updateMap for every robot: the rolled origins (Costmap2D::updateOrigin's scalars) into origins_xy
 // [n][2]; must be followed by fleet_costmap_enqueue before the next roll
 int fleet_costmap_roll(FleetCostmap* fc, const double* poses, double* origins_xy);

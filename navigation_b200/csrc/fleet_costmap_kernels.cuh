@@ -305,4 +305,85 @@ __global__ void __launch_bounds__(kFleetCmThreads) k_fleet_costmap(FleetCostmapA
 // registers (a single-argument bound settles on 64 registers and spills)
 __global__ void __launch_bounds__(kFleetCmThreads, 2) k_fleet_costmap_voxel(FleetCostmapArgs a) { fleet_costmap_cta<true>(a); }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Batched scan ingest (navgpu_fleet_set_scan_batch): every robot carries the same sources, source s of robot r is row r
+// of the source's arrays.  The tables k_fleet_costmap reads are then regular, and what navgpu_fleet_set_scans lists
+// robot by robot is one index computation away:
+//   points     robot-major: point i of source s of robot r is r * points + point_first(s) + i
+//   d_obs      n * n_clear clearing entries (robot-major, a robot's clearing sources in order, listed even without
+//              points), then n * n_mark marking entries (sources with points only)
+//   mark_base  r * marks
+constexpr int kScanBatchSources = 32;  // sources per batch: they travel as kernel parameters
+constexpr int kScanBatchThreads = 256;
+
+struct ScanBatchSource {
+  const float* data;      // [n][n_points] ranges or [n][n_points][3] sensor-frame points
+  const double* stg;      // [n][7]: translation x, y, z, rotation x, y, z, w
+  double angle_min, angle_increment;  // the float fields, widened exactly (ScanRec)
+  double min_obstacle_height, max_obstacle_height, obstacle_range, raytrace_range;
+  float range_min, range_max;
+  int n_points, is_cloud, inf_is_valid, flags;  // flags: bit0 marking, bit1 clearing (DevObs)
+  int point_first;             // the source's first point within its robot
+  int clear_slot, mark_slot;   // its entry among the robot's clearing / marking entries; -1: not listed
+  int clear_ray, mark_ray;     // DevObs::first_ray of those entries
+};
+
+struct ScanBatchArgs {
+  ScanBatchSource src[kScanBatchSources];
+  int n_sources, n;
+  int points, n_clear, n_mark, rays, marks;  // per robot
+  float* xyz;
+  DevObs* obs;
+  FleetScanRobot* robots;
+};
+
+// grid (x, max(1, n_sources)): blockIdx.y is the source; x covers max(n, n * n_points) threads.  Thread t < n of source
+// s writes robot t's DevObs of s (and, on source 0, robot t's FleetScanRobot); thread t < n * n_points projects point
+// t % n_points of robot t / n_points through project_point, the per-point body of k_project_scans.
+__global__ void __launch_bounds__(kScanBatchThreads) k_fleet_scan_batch(const ScanBatchArgs a) {
+  const int t = blockIdx.x * kScanBatchThreads + threadIdx.x, s = blockIdx.y;
+  if (s == 0 && t < a.n) {
+    FleetScanRobot rb;
+    rb.clear_first = t * a.n_clear; rb.n_clear = a.n_clear; rb.rays = a.rays;
+    rb.mark_first = a.n * a.n_clear + t * a.n_mark; rb.n_mark = a.n_mark; rb.marks = a.marks;
+    rb.mark_base = (long long)t * a.marks;
+    a.robots[t] = rb;
+  }
+  if (s >= a.n_sources) return;
+  const ScanBatchSource& src = a.src[s];
+  if (t < a.n && (src.clear_slot >= 0 || src.mark_slot >= 0)) {
+    const double* tr = src.stg + 7 * (size_t)t;
+    DevObs d;
+    d.ox = tr[0]; d.oy = tr[1]; d.oz = tr[2];  // the sensor origin (observation_buffer.cpp:143-151)
+    d.obstacle_range = src.obstacle_range;
+    d.raytrace_range = src.raytrace_range;
+    d.first_point = t * a.points + src.point_first;
+    d.n_points = src.n_points;
+    d.flags = src.flags;
+    if (src.clear_slot >= 0) {
+      d.first_ray = src.clear_ray;
+      a.obs[t * a.n_clear + src.clear_slot] = d;
+    }
+    if (src.mark_slot >= 0) {
+      d.first_ray = src.mark_ray;
+      a.obs[a.n * a.n_clear + t * a.n_mark + src.mark_slot] = d;
+    }
+  }
+  if (t >= a.n * src.n_points) return;
+  const int r = t / src.n_points, i = t - r * src.n_points;
+  const double* tr = src.stg + 7 * (size_t)r;
+  ScanRec rec;  // the projection record of (robot r, source s); its transform is built after the sensor-frame point
+  rec.angle_min = src.angle_min;
+  rec.angle_increment = src.angle_increment;
+  rec.range_min = src.range_min;
+  rec.range_max = src.range_max;
+  rec.min_obstacle_height = src.min_obstacle_height;
+  rec.max_obstacle_height = src.max_obstacle_height;
+  rec.inf_is_valid = src.inf_is_valid;
+  rec.is_cloud = src.is_cloud;
+  const float* row = src.data + (size_t)r * src.n_points * (src.is_cloud ? 3 : 1);
+  project_point(rec, row, i, a.xyz + 3 * ((size_t)r * a.points + src.point_first + i),
+                [&](float m[9], float t3[3]) { sensor_affine(tr + 3, tr, m, t3); });
+}
+
 }  // namespace navgpu

@@ -172,6 +172,68 @@ def fleet_scan(robot, cycle, cloud=False, n_beams=360, range_max=4.0):
     return scan
 
 
+def _sensor_to_global(poses, z):
+    """[n][7] tf transforms (translation, rotation xyzw) of sensors z above robots at poses [n][3]."""
+    poses = np.asarray(poses, dtype=np.float64)
+    yaw = poses[:, 2]
+    zeros = np.zeros(len(poses))
+    return np.ascontiguousarray(np.stack([poses[:, 0], poses[:, 1], np.full(len(poses), z), zeros, zeros,
+                                          np.sin(yaw / 2), np.cos(yaw / 2)], 1))
+
+
+def fleet_scan_batch(robots, cycle, cloud=False, n_beams=360, range_max=4.0):
+    """One scan of every robot (fleet_sensing_robot) at its pose of `cycle`, as one source of Fleet.set_scan_batch:
+    dense [n, n_beams] ranges (or [n, n_beams, 3] sensor-frame points with cloud=True) and [n, 7] sensor transforms.
+    Unlike fleet_scan, every robot's scan shares one sensor-frame angle_min, so the rays are cast at world angle
+    yaw + angle_min + i * angle_increment; the other fields are fleet_scan's."""
+    angle_min, inc = np.float32(0.001 * cycle), np.float32(2 * np.pi / n_beams)
+    poses = np.array([r["poses"][cycle % len(r["poses"])] for r in robots], dtype=np.float64)
+    out = dict(sensor_to_global=_sensor_to_global(poses, 0.3), min_obstacle_height=0.0, max_obstacle_height=2.0,
+               obstacle_range=2.5, raytrace_range=3.0, marking=True, clearing=True)
+    rows = []
+    for r, (x, y, yaw) in zip(robots, poses):
+        pts = raycast_scan(r["world"], r["resolution"], r["origin"], (x, y), n_beams, range_max,
+                           phase=yaw + float(angle_min))
+        dx, dy = pts[:, 0].astype(np.float64) - x, pts[:, 1].astype(np.float64) - y
+        if cloud:
+            cs, sn = np.cos(yaw), np.sin(yaw)
+            rows.append(np.stack([cs * dx + sn * dy, -sn * dx + cs * dy, np.zeros_like(dx)], 1).astype(np.float32))
+        else:
+            ranges = np.hypot(dx, dy).astype(np.float32)
+            ranges[ranges >= np.float32(range_max - 1e-3)] = np.inf
+            rows.append(ranges)
+    if cloud:
+        out["points"] = np.ascontiguousarray(np.stack(rows))
+    else:
+        out.update(ranges=np.ascontiguousarray(np.stack(rows)), angle_min=angle_min, angle_increment=inc,
+                   range_min=np.float32(0.05), range_max=np.float32(range_max), inf_is_valid=1)
+    return out
+
+
+def fleet_cloud_3d_batch(robots, cycle, **kw):
+    """fleet_cloud_3d of every robot (fleet_voxel_robot) as one source of Fleet.set_scan_batch: the clouds are in the
+    sensor frame with shared fields, so the batch is their stack ([n, points, 3]) and the robots' [n, 7] transforms."""
+    clouds = [fleet_cloud_3d(r, cycle, **kw) for r in robots]
+    out = {k: v for k, v in clouds[0].items() if k not in ("points", "translation", "rotation_xyzw")}
+    out["points"] = np.ascontiguousarray(np.stack([c["points"] for c in clouds]))
+    out["sensor_to_global"] = np.ascontiguousarray([list(c["translation"]) + list(c["rotation_xyzw"]) for c in clouds],
+                                                   dtype=np.float64)
+    return out
+
+
+def batch_scans(sources, n):
+    """The per-robot scan-dict lists (Fleet.set_scans) that a batch of sources (Fleet.set_scan_batch) stands for:
+    robot r's list holds, per source, its shared fields with row r of its arrays."""
+    out = [[] for _ in range(n)]
+    for src in sources:
+        shared = {k: v for k, v in src.items() if k not in ("ranges", "points", "sensor_to_global")}
+        key = "points" if "points" in src else "ranges"
+        data, stg = np.asarray(src[key]), np.asarray(src["sensor_to_global"], dtype=np.float64)
+        for r in range(n):
+            out[r].append(dict(shared, **{key: data[r]}, translation=tuple(stg[r, :3]), rotation_xyzw=tuple(stg[r, 3:])))
+    return out
+
+
 # elevation rows of fleet_cloud_3d, degrees: straight down (floor returns under the robot: z-dominant rays), a shallow
 # downward row (low obstacles; its floor return is beyond obstacle_range, so the floor only clears), the scan plane,
 # two upward rows (tall obstacles, overhangs) and a steep upward one (z-dominant, ends above max_obstacle_height)
