@@ -554,6 +554,34 @@ int navgpu_fleet_tp_get_grid(navgpu_fleet* f, int robot, int which, double* host
  * step); synchronises the fleet's stream */
 int navgpu_fleet_tp_last_timing(navgpu_fleet* f, float* footprint_ms, float* wavefront_ms, float* score_ms);
 
+/* ---- Goal handling for fleets: robots that stop and rotate ----------------------------------------------------
+ * At the goal, DWAPlannerROS and TrajectoryPlannerROS stop searching: LatchedStopRotateController / rotateToGoal
+ * propose one stop or rotate command and accept it if checkTrajectory scores it >= 0.  The two calls below let a
+ * fleet do the same per robot; the goal tolerance and latch logic stay with the caller, as for single handles.
+ * Both work on every fleet kind, with either planner. */
+/* Which robots the following steps plan for: active[n_robots] bytes, 0 or 1; null means every robot.  The mask persists
+ * until the next call; a new fleet starts with every robot active.  A robot with active[r] == 0 still gets its costmap
+ * update in navgpu_fleet_step / navgpu_fleet_step_tp, but nothing of its planner runs: no MapGrid wavefronts (its
+ * distance grids stay as its last planning step left them), no sample enumeration or scoring, no footprint cells
+ * (TrajectoryPlanner), no change to its oscillation, result or escape state, and results[r] is not written.
+ * navgpu_fleet_set_plans still applies every robot's plan.  NAVGPU_ERR_INVALID for any byte other than 0 or 1, and the
+ * previous mask stays. */
+int navgpu_fleet_set_active(navgpu_fleet* f, const uint8_t* active);
+/* checkTrajectory of each robot's candidate commands: robot r's are vel_samples[offsets[r] .. offsets[r + 1]), 3 doubles
+ * (vx, vy, vtheta) each; offsets has n_robots + 1 non-decreasing entries starting at 0; poses, vels [n][3]; costs_out
+ * gets one cost per candidate (>= 0: legal).
+ * DWAPlanner fleets: what navgpu_dwa_check_trajectory returns on a handle holding the robot's current costmap and
+ * origin, its plans of the last set_plans (alignment scale included), the distance grids of its last planning step and
+ * the fleet's footprint; a robot with candidates has its oscillation flags reset (dwa_planner.cpp:217), so the call
+ * equals that handle's check of each candidate in order.
+ * TrajectoryPlanner fleets: what navgpu_tp_score_trajectory returns (pose and velocity as given, not rounded through
+ * float); no state changes.
+ * Robots without candidates are untouched.  NAVGPU_ERR_INVALID, with no state changed, for null pointers, offsets that
+ * decrease or do not start at 0, and candidates for a robot that was never active in a step.  One kernel launch
+ * whatever the robots and candidates; returns once the costs are in costs_out. */
+int navgpu_fleet_check_trajectories(navgpu_fleet* f, const double* poses, const double* vels, const int32_t* offsets,
+                                    const double* vel_samples, double* costs_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -235,6 +235,8 @@ SIGNATURES = {
     "navgpu_fleet_tp_get_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _f64p]),
     "navgpu_fleet_tp_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                               C.POINTER(C.c_float)]),
+    "navgpu_fleet_set_active": (C.c_int, [C.c_void_p, _u8p]),
+    "navgpu_fleet_check_trajectories": (C.c_int, [C.c_void_p, _f64p, _f64p, _i32p, _f64p, _f64p]),
 }
 
 
@@ -815,6 +817,7 @@ class Fleet:
         self.size_x, self.size_y = size_x, size_y
         self.device = device
         self._batch_keep = None  # the device arrays of the last set_scan_batch, alive until the next one
+        self._active = None      # the set_active mask (None: every robot)
         self.cfg = DwaConfig()
         self.lib.navgpu_dwa_default_config(C.byref(self.cfg))
         for k, v in overrides.items():
@@ -866,16 +869,49 @@ class Fleet:
 
     def step(self, poses, vels):
         """One control cycle.  Per robot: cost, xv, yv, thetav, best_index, n_samples, n_scored with DWAPlanner;
-        cost, xv, yv, thetav, flags, n_points with the TrajectoryPlanner (navgpu_tp_result)."""
+        cost, xv, yv, thetav, flags, n_points with the TrajectoryPlanner (navgpu_tp_result); None for a robot that
+        set_active left out."""
         p = np.ascontiguousarray(poses, dtype=np.float64)
         v = np.ascontiguousarray(vels, dtype=np.float64)
         assert p.shape == (self.n, 3) and v.shape == (self.n, 3)
         r = self.step_raw(p, v)
+        act = self._active
         if self.tp_cfg is not None:
-            return [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, flags=r[i].flags,
-                         n_points=r[i].n_points) for i in range(self.n)]
-        return [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, best_index=r[i].best_index,
-                     n_samples=r[i].n_samples, n_scored=r[i].n_scored) for i in range(self.n)]
+            out = [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, flags=r[i].flags,
+                        n_points=r[i].n_points) for i in range(self.n)]
+        else:
+            out = [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, best_index=r[i].best_index,
+                        n_samples=r[i].n_samples, n_scored=r[i].n_scored) for i in range(self.n)]
+        return out if act is None else [g if a else None for g, a in zip(out, act)]
+
+    def set_active(self, mask):
+        """Which robots the following steps plan for (navgpu_fleet_set_active): n_robots booleans or 0 / 1 values, or
+        None for every robot.  A left-out robot keeps its costmap updates but none of its planner runs, and step()
+        returns None for it; check_trajectories still checks commands against its last planning step."""
+        if mask is None:
+            self.api.check(self.lib.navgpu_fleet_set_active(self.h, None))
+            self._active = None
+            return
+        m = np.asarray(mask)
+        assert m.shape == (self.n,)
+        u = np.ascontiguousarray(np.where((m == 0) | (m == 1), m, 2), dtype=np.uint8)  # (other values are refused)
+        self.api.check(self.lib.navgpu_fleet_set_active(self.h, _p(u, _u8p)))
+        self._active = u.astype(bool)
+
+    def check_trajectories(self, poses, vels, candidates):
+        """checkTrajectory of each robot's candidate commands (navgpu_fleet_check_trajectories): candidates[r] is a
+        (k_r, 3) array of (vx, vy, vtheta), possibly empty; returns one array of k_r costs per robot (>= 0: legal)."""
+        p = np.ascontiguousarray(poses, dtype=np.float64)
+        v = np.ascontiguousarray(vels, dtype=np.float64)
+        assert p.shape == (self.n, 3) and v.shape == (self.n, 3) and len(candidates) == self.n
+        cand = [np.asarray(c, dtype=np.float64).reshape(-1, 3) for c in candidates]
+        off = np.zeros(self.n + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(c) for c in cand])
+        s = np.ascontiguousarray(np.concatenate(cand) if off[-1] else np.zeros((1, 3)))
+        costs = np.zeros(max(int(off[-1]), 1))
+        self.api.check(self.lib.navgpu_fleet_check_trajectories(self.h, _p(p, _f64p), _p(v, _f64p), _p(off, _i32p),
+                                                                _p(s, _f64p), _p(costs, _f64p)))
+        return [costs[off[r]:off[r + 1]].copy() for r in range(self.n)]
 
     def step_raw(self, poses, vels):
         """step() without building Python dicts (benchmarks); returns the ctypes result array."""

@@ -1036,6 +1036,8 @@ constexpr unsigned kFleetPadRows = 64;  // >= 2 * the largest cell inflation rad
 struct FleetTp;
 static void fleet_tp_free(FleetTp* t);
 static int fleet_tp_set_plans(navgpu_fleet* f, const double* plan_xy, const int32_t* plan_offsets);
+static int fleet_tp_check(navgpu_fleet* f, const double* poses, const double* vels, const int32_t* offsets,
+                          const double* vel_samples, double* costs_out);
 
 struct navgpu_fleet {
   int device = 0;
@@ -1077,6 +1079,13 @@ struct navgpu_fleet {
   std::vector<size_t> plan_off;  // per robot x 3 plans: offset (in points) into d_plans
   bool started = false;          // set_plans or a step has run
   FleetTp* tp = nullptr;         // non-null: the robots run base_local_planner::TrajectoryPlanner instead of DWAPlanner
+  // per robot: 1 = planned by the steps (navgpu_fleet_set_active); planned = was active in a step, so its distance
+  // grids hold that step's wavefronts; aliased = in that step its alignment grid was its path grid (DWAPlanner)
+  std::vector<uint8_t> active, planned, aliased;
+  // navgpu_fleet_check_trajectories (DWAPlanner): per robot a one-sample record, per candidate its robot, velocity, cost
+  std::vector<FleetRobot> h_check;
+  char* d_check = nullptr;
+  size_t check_capacity = 0;
 };
 
 // what every fleet holds for its planner side: the DWAPlanner parameters and critic scales ...
@@ -1107,6 +1116,9 @@ static int alloc_planner_side(navgpu_fleet* f) {
   f->osc.resize(n_robots);
   f->res_v.assign(size_t(3) * n_robots, 0.0);
   f->h_robots.resize(n_robots);
+  f->active.assign(n_robots, 1);
+  f->planned.assign(n_robots, 0);
+  f->aliased.assign(n_robots, 0);
   return NAVGPU_OK;
 }
 
@@ -1173,6 +1185,13 @@ static int fleet_upload_grids(navgpu_fleet* f, SetJobs set_jobs) {
   NAVGPU_CUDA(cudaStreamSynchronize(f->stream));  // pageable source, rewritten by the step
   f->grids_dirty = false;
   return NAVGPU_OK;
+}
+
+// the scoring arguments every robot of a DWAPlanner fleet shares (fleet_patch_args adds each robot's own)
+static void fleet_dwa_base_args(const navgpu_fleet* f, DwaScoreArgs& base) {
+  memset(&base, 0, sizeof(base));
+  base.g = DwaGeom{nullptr, f->sx, f->sy, f->pitch, f->res, 0.0, 0.0, 1.0 / f->res};
+  dwa_config_args(f->cfg, f->scales, f->footprint.data(), (int)(f->footprint.size() / 2), base);  // (scale_alignment: per robot)
 }
 
 // the MapGrid wavefronts of every robot, jobs_per_robot each, in one launch (each CTA reads its robot's record)
@@ -1266,6 +1285,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
   if (f->stream) cudaStreamSynchronize(f->stream);
   cudaFree(f->d_stage); cudaFree(f->d_raw); cudaFree(f->d_robots); cudaFree(f->d_plans); cudaFree(f->d_samples); cudaFree(f->d_dist);
   cudaFree(f->d_block_cost); cudaFree(f->d_block_index); cudaFree(f->d_generated); cudaFree(f->d_results);
+  cudaFree(f->d_check);
   cudaFreeHost(f->h_results);
   fleet_tp_free(f->tp);
   navgpu_costmap_destroy(f->costmap);
@@ -1357,6 +1377,8 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
       job[3].dist = dist;
       job[3].skip = 1;
     }
+    if (!f->active[r])  // left out of the search: its grids stay as its last planning step left them
+      for (int k = 0; k < 4; ++k) job[k].skip = 1;
   };
   NAVGPU_TRY(fleet_upload_grids(f, jobs));
   // sensing fleet: LayeredCostmap::updateMap of every robot, before the wavefronts read the master grids
@@ -1368,6 +1390,12 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
   samples.clear();
   int max_samples = 0;
   for (int r = 0; r < n; ++r) {
+    FleetRobot& R = f->h_robots[r];
+    if (!f->active[r]) {  // no samples: its scoring CTAs exit at once
+      R.nx = R.ny = R.nth = 0;
+      R.samples_offset = (int)samples.size();
+      continue;
+    }
     const float pos[3] = {(float)poses[3 * r], (float)poses[3 * r + 1], (float)poses[3 * r + 2]};
     const float vel[3] = {(float)vels[3 * r], (float)vels[3 * r + 1], (float)vels[3 * r + 2]};
     const float goal[2] = {(float)f->plans[r].plan.back().x, (float)f->plans[r].plan.back().y};
@@ -1376,7 +1404,6 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
       cudaStreamSynchronize(f->stream);
       return fail(NAVGPU_ERR_UNSUPPORTED, "more than %d per-axis samples per robot", kInlineSamples);
     }
-    FleetRobot& R = f->h_robots[r];
     for (int k = 0; k < 3; ++k) { R.pos[k] = pos[k]; R.vel[k] = vel[k]; }
     R.osc_mask = f->osc[r].mask();
     R.scale_alignment = f->plans[r].alignment_scale;
@@ -1391,9 +1418,10 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
     NAVGPU_CUDA(cudaMalloc(&f->d_samples, samples.size() * 2 * sizeof(float)));
     f->samples_capacity = samples.size() * 2;
   }
-  NAVGPU_CUDA(cudaMemcpyAsync(f->d_samples, samples.data(), samples.size() * sizeof(float), cudaMemcpyHostToDevice, f->stream));
+  if (!samples.empty())
+    NAVGPU_CUDA(cudaMemcpyAsync(f->d_samples, samples.data(), samples.size() * sizeof(float), cudaMemcpyHostToDevice, f->stream));
   NAVGPU_CUDA(cudaMemcpyAsync(f->d_robots, f->h_robots.data(), sizeof(FleetRobot) * n, cudaMemcpyHostToDevice, f->stream));
-  const int bpr = (max_samples + kDwaWarpsPerBlock - 1) / kDwaWarpsPerBlock;
+  const int bpr = (max_samples + kDwaWarpsPerBlock - 1) / kDwaWarpsPerBlock;  // (0: no robot is active)
   const size_t blocks = size_t(bpr) * n;
   if (blocks > f->blocks_capacity) {
     if (f->d_block_cost) cudaFree(f->d_block_cost);
@@ -1407,23 +1435,26 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
 
   // ---- rollouts + critics + per-robot argmin
   DwaScoreArgs base;
-  memset(&base, 0, sizeof(base));
-  base.g = DwaGeom{nullptr, f->sx, f->sy, f->pitch, f->res, 0.0, 0.0, 1.0 / f->res};
-  dwa_config_args(c, f->scales, f->footprint.data(), (int)(f->footprint.size() / 2), base);  // (scale_alignment: per robot)
-  k_fleet_score<<<(unsigned)blocks, kDwaWarpsPerBlock * 32, 0, f->stream>>>(base, f->d_robots, f->d_samples, bpr, f->d_block_cost,
-                                                                          f->d_block_index, f->d_generated);
-  k_fleet_finish<<<n, 32, 0, f->stream>>>(base, f->d_robots, f->d_samples, bpr, f->d_block_cost, f->d_block_index,
-                                          f->d_generated, f->d_results);
-  NAVGPU_LAUNCHED(2);
-  NAVGPU_CUDA(cudaGetLastError());
-  NAVGPU_CUDA(cudaMemcpyAsync(f->h_results, f->d_results, sizeof(DwaDeviceResult) * n, cudaMemcpyDeviceToHost, f->stream));
+  fleet_dwa_base_args(f, base);
+  if (bpr > 0) {
+    k_fleet_score<<<(unsigned)blocks, kDwaWarpsPerBlock * 32, 0, f->stream>>>(base, f->d_robots, f->d_samples, bpr,
+                                                                            f->d_block_cost, f->d_block_index, f->d_generated);
+    k_fleet_finish<<<n, 32, 0, f->stream>>>(base, f->d_robots, f->d_samples, bpr, f->d_block_cost, f->d_block_index,
+                                            f->d_generated, f->d_results);
+    NAVGPU_LAUNCHED(2);
+    NAVGPU_CUDA(cudaGetLastError());
+    NAVGPU_CUDA(cudaMemcpyAsync(f->h_results, f->d_results, sizeof(DwaDeviceResult) * n, cudaMemcpyDeviceToHost, f->stream));
+  }
   NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
 
-  // ---- host epilogue per robot: result_traj_ bookkeeping + oscillation flags
+  // ---- host epilogue per active robot: result_traj_ bookkeeping + oscillation flags
   for (int r = 0; r < n; ++r) {
+    if (!f->active[r]) continue;
     const FleetRobot& R = f->h_robots[r];
     apply_dwa_result(f->h_results[r], c, poses + 3 * r, R.nx * R.ny * R.nth, &f->res_v[3 * r], f->osc[r], &results[r]);
     results[r].n_points = 0;
+    f->planned[r] = 1;
+    f->aliased[r] = f->plans[r].align_is_path;
   }
   return NAVGPU_OK;
 }
@@ -1439,6 +1470,87 @@ int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out)
   if (!f || robot < 0 || robot >= f->n || !mask_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   if (f->tp) return fail(NAVGPU_ERR_INVALID, "a TrajectoryPlanner fleet has no DWA oscillation flags (see navgpu_fleet_step_tp's flags)");
   *mask_out = f->osc[robot].mask();
+  return NAVGPU_OK;
+}
+
+int navgpu_fleet_set_active(navgpu_fleet* f, const uint8_t* active) {
+  if (!f) return fail(NAVGPU_ERR_INVALID, "null handle");
+  if (active)
+    for (int r = 0; r < f->n; ++r)
+      if (active[r] > 1) return fail(NAVGPU_ERR_INVALID, "active[%d] is %d, not 0 or 1", r, (int)active[r]);
+  for (int r = 0; r < f->n; ++r) {
+    const uint8_t a = active ? active[r] : 1;
+    if (a != f->active[r]) f->grids_dirty = true;  // the robot's MapGrid jobs change (skip)
+    f->active[r] = a;
+  }
+  return NAVGPU_OK;
+}
+
+// DWAPlanner::checkTrajectory (dwa_planner.cpp:213-237) of every candidate, as navgpu_dwa_check_trajectory computes it
+// on a handle holding the robot's current costmap and plans and the distance grids of its last planning step
+int navgpu_fleet_check_trajectories(navgpu_fleet* f, const double* poses, const double* vels, const int32_t* offsets,
+                                    const double* vel_samples, double* costs_out) {
+  if (!f || !poses || !vels || !offsets || !vel_samples || !costs_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (offsets[0] != 0) return fail(NAVGPU_ERR_INVALID, "candidate offsets must start at 0");
+  for (int r = 0; r < f->n; ++r)
+    if (offsets[r + 1] < offsets[r]) return fail(NAVGPU_ERR_INVALID, "candidate offsets decrease at robot %d", r);
+  for (int r = 0; r < f->n; ++r)
+    if (offsets[r + 1] > offsets[r] && !f->planned[r])
+      return fail(NAVGPU_ERR_INVALID, "robot %d has candidates but was never active in a step", r);
+  NAVGPU_CUDA(cudaSetDevice(f->device));
+  if (f->tp) return fleet_tp_check(f, poses, vels, offsets, vel_samples, costs_out);
+  const int n = f->n, total = offsets[n];
+  if (total == 0) return NAVGPU_OK;
+  const size_t cells = size_t(f->sx) * f->sy;
+  // device copies: [one record per robot | robot of each candidate | candidates (float) | costs]
+  auto up16 = [](size_t b) { return (b + 15) & ~size_t(15); };
+  const size_t b_rob = up16(sizeof(FleetRobot) * n), b_of = up16(sizeof(int32_t) * total),
+               b_vel = up16(sizeof(float) * 3 * total), b_cost = sizeof(double) * total;
+  const size_t need = b_rob + b_of + b_vel + b_cost;
+  if (need > f->check_capacity) {
+    cudaFree(f->d_check);
+    f->d_check = nullptr;
+    f->check_capacity = 0;
+    NAVGPU_CUDA(cudaMalloc(&f->d_check, 2 * need));
+    f->check_capacity = 2 * need;
+  }
+  FleetRobot* d_rob = reinterpret_cast<FleetRobot*>(f->d_check);
+  int32_t* d_of = reinterpret_cast<int32_t*>(f->d_check + b_rob);
+  float* d_vel = reinterpret_cast<float*>(f->d_check + b_rob + b_of);
+  double* d_cost = reinterpret_cast<double*>(f->d_check + b_rob + b_of + b_vel);
+  std::vector<int32_t> robot_of(total);
+  std::vector<float> vel_f(size_t(3) * total);
+  f->h_check.resize(n);
+  for (int r = 0; r < n; ++r) {
+    const int b = offsets[r], e = offsets[r + 1];
+    if (e == b) continue;
+    f->osc[r].reset();  // dwa_planner.cpp:217
+    FleetRobot& R = f->h_check[r];
+    R.grids.g = DwaGeom{f->d_master + size_t(r) * f->stride * f->pitch, f->sx, f->sy, f->pitch, f->res, f->origins[2 * r],
+                        f->origins[2 * r + 1], 1.0 / f->res};
+    uint32_t* dist = f->d_dist + size_t(r) * 4 * cells;
+    for (int k = 0; k < 4; ++k) R.grids.job[k].dist = dist + k * cells;
+    if (f->aliased[r]) R.grids.job[3].dist = dist;
+    for (int k = 0; k < 3; ++k) { R.pos[k] = (float)poses[3 * r + k]; R.vel[k] = (float)vels[3 * r + k]; }
+    R.osc_mask = 0;
+    R.scale_alignment = f->plans[r].alignment_scale;
+    R.nx = R.ny = R.nth = 1;
+    R.samples_offset = 0;  // k_fleet_check hands each CTA its own candidate as the sample array
+    for (int i = b; i < e; ++i) {
+      robot_of[i] = r;
+      for (int k = 0; k < 3; ++k) vel_f[3 * size_t(i) + k] = (float)vel_samples[3 * size_t(i) + k];  // Eigen::Vector3f
+    }
+  }
+  NAVGPU_CUDA(cudaMemcpyAsync(d_rob, f->h_check.data(), sizeof(FleetRobot) * n, cudaMemcpyHostToDevice, f->stream));
+  NAVGPU_CUDA(cudaMemcpyAsync(d_of, robot_of.data(), sizeof(int32_t) * total, cudaMemcpyHostToDevice, f->stream));
+  NAVGPU_CUDA(cudaMemcpyAsync(d_vel, vel_f.data(), sizeof(float) * 3 * total, cudaMemcpyHostToDevice, f->stream));
+  DwaScoreArgs base;
+  fleet_dwa_base_args(f, base);
+  k_fleet_check<<<(unsigned)total, 32, 0, f->stream>>>(base, d_rob, d_of, d_vel, d_cost);
+  NAVGPU_LAUNCHED(1);
+  NAVGPU_CUDA(cudaGetLastError());
+  NAVGPU_CUDA(cudaMemcpyAsync(costs_out, d_cost, b_cost, cudaMemcpyDeviceToHost, f->stream));
+  NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
   return NAVGPU_OK;
 }
 

@@ -1593,4 +1593,19 @@ __global__ void __launch_bounds__(32) k_fleet_finish(DwaScoreArgs base, const Fl
   finish_winner(s_a, bi, bc, results + robot, nullptr, 0, s_scratch, generated + robot);
 }
 
+// DWAPlanner::checkTrajectory of any robots' candidates in one launch (navgpu_fleet_check_trajectories): one warp (= one
+// CTA) per candidate.  Each robot's record is a one-sample block (nx = ny = nth = 1, samples_offset 0), so passing the
+// candidate's own 3 floats as the sample array makes it sample 0 -- k_dwa_check's way, with its cost rule.  (A minimum
+// of one CTA per SM lets ptxas keep the values live across the sincos slow path in registers instead of spilling them.)
+__global__ void __launch_bounds__(32, 1) k_fleet_check(DwaScoreArgs base, const FleetRobot* robots,
+                                                    const int* __restrict__ robot_of, const float* __restrict__ candidates,
+                                                    double* __restrict__ costs) {
+  __shared__ DwaScoreArgs s_a;
+  __shared__ double s_scratch[kWarpScratchDoubles];
+  const int c = blockIdx.x;
+  fleet_patch_args(s_a, base, robots[robot_of[c]], candidates + 3 * (size_t)c);
+  const TrajResult r = score_sample<true>(s_a, 0, threadIdx.x & 31, nullptr, nullptr, 0, s_scratch, s_a.g.cost);
+  if (threadIdx.x == 0) costs[c] = r.generated ? r.cost : ((s_a.nfp == 0 && s_a.scale_obstacle != 0.0) ? -9.0 : 0.0);
+}
+
 }  // namespace navgpu

@@ -424,12 +424,15 @@ struct TpFleetLayout {
 };
 
 // TrajectoryPlanner::findBestPath's path_map_ cells under the robot (trajectory_planner.cpp:918-930) for every robot:
-// one warp per robot clears its bit mask while lane 0 gathers the cells in shared memory; the warp then sets them
+// one warp per robot clears its bit mask while lane 0 gathers the cells in shared memory; the warp then sets them.
+// A robot without samples is left out of the step (navgpu_fleet_set_active; an active robot always has the backup
+// sample): its bits stay as they are.
 __global__ void __launch_bounds__(32) k_tp_fleet_footprint(TpFleetLayout L, const TpFleetRobot* robots, unsigned sx,
                                                            unsigned sy, double res, int nfp) {
   extern __shared__ uint32_t s_cells[];
   __shared__ int s_n;
   const int robot = blockIdx.x, lane = threadIdx.x;
+  if (robots[robot].n_samples == 0) return;
   uint32_t* within = L.within + (size_t)robot * L.within_words;
   for (int w = lane; w < L.within_words; w += 32) within[w] = 0u;
   if (lane == 0) {
