@@ -376,6 +376,22 @@ int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* p
 int navgpu_fleet_reset_oscillation(navgpu_fleet* f);
 /* one control cycle; poses, vels [n][3]; results: n entries (n_points = 0, winners' points are not materialised) */
 int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, navgpu_dwa_result* results);
+/* navgpu_fleet_step with device memory of the fleet's device: poses [n][3] and vels [n][3] (double) are read and
+ * results [n] written on the fleet's stream (navgpu_fleet_stream); the call returns without waiting for the device.
+ * After the stream has run, results, every costmap, layer, voxel column, window and origin, every oscillation mask and
+ * distance grid, and all later behaviour are those of navgpu_fleet_step with the same poses and velocities.  One
+ * exception by construction: a sensing fleet's footprint clearing takes cos / sin of each yaw from CUDA's sincos
+ * instead of the host libm (as the scan projection does).  Robots navgpu_fleet_set_active left out keep their results
+ * entry untouched; n_points is 0.  The caller orders its writes of poses and vels before the fleet's stream and reads
+ * results after work ordered behind it.  Host and device steps, and every other call, may be mixed on one fleet: a
+ * host call that reads the planner state (navgpu_fleet_step, _reset_oscillation, _get_oscillation_mask,
+ * _check_trajectories, _get_geometry) first waits for the fleet's stream.  A device step that follows a device step,
+ * with no set_plans, set_active, set_maps or reset_oscillation in between, neither waits for the host, allocates nor
+ * copies from pageable memory, so it can be captured in a CUDA graph.  The scoring grid is sized from the
+ * configuration: at most max(2, n) + 1 samples per axis configured with n.  Refused, with the fleet unchanged: null
+ * or non-device pointers (NAVGPU_ERR_INVALID), TrajectoryPlanner fleets, use_dwa = 0 and more than 640 per-axis
+ * samples by that bound (NAVGPU_ERR_UNSUPPORTED). */
+int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double* vels, navgpu_dwa_result* results);
 /* inflated local costmap of one robot, HOST size_y x size_x */
 int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out);
 int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out);

@@ -203,6 +203,7 @@ SIGNATURES = {
     "navgpu_fleet_set_plans": (C.c_int, [C.c_void_p, _f64p, _f64p, _i32p]),
     "navgpu_fleet_reset_oscillation": (C.c_int, [C.c_void_p]),
     "navgpu_fleet_step": (C.c_int, [C.c_void_p, _f64p, _f64p, C.POINTER(DwaResult)]),
+    "navgpu_fleet_step_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "navgpu_fleet_get_costmap": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
     "navgpu_fleet_get_oscillation_mask": (C.c_int, [C.c_void_p, C.c_int, _i32p]),
     "navgpu_fleet_create_sensing": (C.c_int, [_vpp, C.c_int, C.POINTER(DwaConfig), C.c_uint32, C.c_uint32, C.c_double,
@@ -883,6 +884,38 @@ class Fleet:
             out = [dict(cost=r[i].cost, xv=r[i].xv, yv=r[i].yv, thetav=r[i].thetav, best_index=r[i].best_index,
                         n_samples=r[i].n_samples, n_scored=r[i].n_scored) for i in range(self.n)]
         return out if act is None else [g if a else None for g, a in zip(out, act)]
+
+    def step_device(self, poses, vels, out=None):
+        """step() on the device (navgpu_fleet_step_device), for a simulator that keeps its robots on the GPU: poses and
+        vels are contiguous float64 CUDA tensors [n, 3] on the fleet's device.  The fleet's stream first waits for
+        torch's current stream, and torch's current stream then waits for the fleet's, so torch work queued after
+        this call sees the results; nothing waits on the host.  Returns views of one CUDA buffer of n result records:
+        cost, xv, yv, thetav (float64), best_index, n_samples, n_scored (int32), and the buffer itself as `records`
+        (uint8), which `out` may pass back to be written again.  A robot that set_active left out keeps its record as
+        it was.  Wrong devices, dtypes or shapes raise ValueError."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        for what, x in (("poses", poses), ("vels", vels)):
+            if not isinstance(x, torch.Tensor) or x.dtype != torch.float64 or tuple(x.shape) != (self.n, 3) or \
+                    not x.is_cuda or x.device.index != self.device or not x.is_contiguous():
+                raise ValueError(f"{what}: a contiguous float64 tensor of shape ({self.n}, 3) on cuda:{self.device}")
+        nbytes = self.n * C.sizeof(DwaResult)
+        if out is None:
+            out = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        elif not isinstance(out, torch.Tensor) or out.dtype != torch.uint8 or tuple(out.shape) != (nbytes,) or \
+                not out.is_cuda or out.device.index != self.device or not out.is_contiguous():
+            raise ValueError(f"out: a contiguous uint8 tensor of {nbytes} bytes on cuda:{self.device}")
+        fleet_stream = torch.cuda.ExternalStream(self.stream(), device=dev)
+        fleet_stream.wait_stream(torch.cuda.current_stream(dev))
+        # (no record_stream on the fleet's stream, which may be destroyed before the tensors are freed: torch's current
+        # stream waits for the fleet's below, so memory torch reuses there is only written after the step read it)
+        self.api.check(self.lib.navgpu_fleet_step_device(self.h, poses.data_ptr(), vels.data_ptr(), out.data_ptr()))
+        torch.cuda.current_stream(dev).wait_stream(fleet_stream)
+        words = C.sizeof(DwaResult) // 8
+        f64 = out.view(torch.float64).view(self.n, words)
+        i32 = out.view(torch.int32).view(self.n, 2 * words)
+        return dict(cost=f64[:, 0], xv=f64[:, 1], yv=f64[:, 2], thetav=f64[:, 3], best_index=i32[:, 8],
+                    n_samples=i32[:, 9], n_scored=i32[:, 10], records=out)
 
     def set_active(self, mask):
         """Which robots the following steps plan for (navgpu_fleet_set_active): n_robots booleans or 0 / 1 values, or

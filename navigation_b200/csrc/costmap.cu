@@ -2079,8 +2079,7 @@ int fleet_costmap_set_scans(FleetCostmap* fc, const navgpu_laser_scan* scans, co
   return NAVGPU_OK;
 }
 
-// device or managed memory of `device`
-static bool on_device(const void* p, int device) {
+bool on_device(const void* p, int device) {
   cudaPointerAttributes at;
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
     cudaGetLastError();  // not a CUDA pointer at all: clear the error, it is the caller's
@@ -2180,28 +2179,29 @@ int fleet_costmap_set_scan_batch(FleetCostmap* fc, const navgpu_fleet_scan_sourc
 }
 
 int fleet_costmap_roll(FleetCostmap* fc, const double* poses, double* origins_xy) {
-  // LayeredCostmap::updateMap's rolling origin (:86-91) and Costmap2D::updateOrigin's scalars, as roll_grid computes
-  // them; master and obstacle layer move together, so one origin serves both.  Nothing is committed here: a step that
-  // fails before its kernel is enqueued leaves the fleet as it was.
-  const double size_m_x = (fc->sx - 1 + 0.5) * fc->res, size_m_y = (fc->sy - 1 + 0.5) * fc->res;
+  // nothing is committed here: a step that fails before its kernel is enqueued leaves the fleet as it was
   for (int r = 0; r < fc->n; ++r) {
-    const double rx = poses[3 * r], ry = poses[3 * r + 1], ryaw = poses[3 * r + 2];
-    const double gox0 = fc->origins[2 * r], goy0 = fc->origins[2 * r + 1];
-    const double new_ox = rx - size_m_x / 2, new_oy = ry - size_m_y / 2;
-    const int cell_ox = int((new_ox - gox0) / fc->res), cell_oy = int((new_oy - goy0) / fc->res);
-    const double gox = gox0 + cell_ox * fc->res, goy = goy0 + cell_oy * fc->res;
-    fc->rolled[2 * r] = gox;
-    fc->rolled[2 * r + 1] = goy;
-    fc->h_steps[r] = FleetCmStep{gox, goy, rx, ry, cos(ryaw), sin(ryaw), cell_ox, cell_oy};
-    origins_xy[2 * r] = gox;
-    origins_xy[2 * r + 1] = goy;
+    const FleetCmStep st = fleet_roll_step(poses + 3 * r, fc->origins[2 * r], fc->origins[2 * r + 1], fc->sx, fc->sy, fc->res);
+    fc->rolled[2 * r] = st.ox;
+    fc->rolled[2 * r + 1] = st.oy;
+    fc->h_steps[r] = st;
+    origins_xy[2 * r] = st.ox;
+    origins_xy[2 * r + 1] = st.oy;
   }
   return NAVGPU_OK;
 }
 
-int fleet_costmap_enqueue(FleetCostmap* fc) {
+FleetCmStep* fleet_costmap_device_steps(FleetCostmap* fc) { return fc->d_steps; }
+
+void fleet_costmap_set_origins(FleetCostmap* fc, const double* origins_xy) {
+  fc->origins.assign(origins_xy, origins_xy + size_t(2) * fc->n);
+  fc->rolled = fc->origins;
+}
+
+int fleet_costmap_enqueue(FleetCostmap* fc, bool device_steps) {
   NAVGPU_CUDA(cudaSetDevice(fc->device));
-  NAVGPU_CUDA(cudaMemcpyAsync(fc->d_steps, fc->h_steps, sizeof(FleetCmStep) * fc->n, cudaMemcpyHostToDevice, fc->stream));
+  if (!device_steps)
+    NAVGPU_CUDA(cudaMemcpyAsync(fc->d_steps, fc->h_steps, sizeof(FleetCmStep) * fc->n, cudaMemcpyHostToDevice, fc->stream));
   FleetCostmapArgs a;
   a.layer = fc->d_layer;
   a.vox = fc->d_vox;
@@ -2239,7 +2239,7 @@ int fleet_costmap_enqueue(FleetCostmap* fc) {
   NAVGPU_LAUNCHED(1);
   NAVGPU_CUDA(cudaGetLastError());
   NAVGPU_CUDA(cudaEventRecord(fc->ev[3], fc->stream));
-  fc->origins = fc->rolled;  // the grids on the device now follow the rolled origins
+  if (!device_steps) fc->origins = fc->rolled;  // the grids on the device now follow the rolled origins
   fc->reinflate = false;
   fc->stepped = true;
   return NAVGPU_OK;

@@ -7,6 +7,7 @@
 #include <cstddef>
 
 #include "common.cuh"
+#include "fleet_costmap.cuh"
 
 namespace navgpu {
 
@@ -736,6 +737,150 @@ struct DwaDeviceResult {
   double cost, xv, yv, thetav;
   long long best_index;
   int n_points, n_scored;
+};
+
+// ---------------------------------------------------------------------------------------------------------------
+// A planner's per-cycle scalar arithmetic, shared by the host (navgpu_dwa_*, navgpu_fleet_step) and the device fleet
+// step (k_fleet_prepare, k_fleet_apply): IEEE operations without a libm call, compiled with -fmad=false on both sides,
+// so both give the same bits.  (std::min / std::max restated: a < b picks as they do, for device code.)
+__host__ __device__ inline double dwa_min(double a, double b) { return b < a ? b : a; }
+__host__ __device__ inline double dwa_max(double a, double b) { return a < b ? b : a; }
+
+// the most samples VelocityIterator gives an axis configured with n (>= 1) samples: max(2, n) - 1 steps, the zero it
+// inserts once when the range crosses it, and the maximum
+__host__ __device__ inline int dwa_axis_bound(int n) { return (n < 2 ? 2 : n) + 1; }
+
+// VelocityIterator, base_local_planner/include/base_local_planner/velocity_iterator.h:49-74: the samples of [mn, mx]
+// as floats into out (room for dwa_axis_bound(n)); returns how many
+__host__ __device__ inline int velocity_samples(double mn, double mx, int n, float* out) {
+  if (mn == mx) {
+    out[0] = (float)mn;
+    return 1;
+  }
+  n = n < 2 ? 2 : n;
+  const double step = (mx - mn) / double(n - 1 < 1 ? 1 : n - 1);
+  double cur, next = mn;
+  int k = 0;
+  for (int j = 0; j < n - 1; ++j) {
+    cur = next;
+    next += step;
+    out[k++] = (float)cur;
+    if (cur < 0 && next > 0) out[k++] = 0.0f;
+  }
+  out[k++] = (float)mx;
+  return k;
+}
+
+// the per-axis sample counts of the configuration (dwa_planner.cpp:86-109) and their bounds
+__host__ __device__ inline void dwa_axis_samples(const navgpu_dwa_config& cfg, int n[3]) {
+  n[0] = cfg.vx_samples <= 0 ? 1 : cfg.vx_samples;
+  n[1] = cfg.vy_samples <= 0 ? 1 : cfg.vy_samples;
+  n[2] = cfg.vth_samples <= 0 ? 1 : cfg.vth_samples;
+}
+
+// SimpleTrajectoryGenerator::initialise, simple_trajectory_generator.cpp:60-135: xs | ys | ths into out (room for the
+// three dwa_axis_bound), their counts into counts.  The use_dwa = 0 window takes hypot, which only the host may call
+// for bit-exact results: the device fleet step refuses such configurations.
+__host__ __device__ inline void enumerate_samples(const navgpu_dwa_config& cfg, const float pos[3], const float vel[3],
+                                                  const float goal[2], float* out, int counts[3]) {
+  const double max_vel_th = cfg.max_rot_vel, min_vel_th = -1.0 * max_vel_th;
+  const float acc[3] = {float(cfg.acc_lim_x), float(cfg.acc_lim_y), float(cfg.acc_lim_theta)};
+  double min_vel_x = cfg.min_vel_x, max_vel_x = cfg.max_vel_x, min_vel_y = cfg.min_vel_y, max_vel_y = cfg.max_vel_y;
+  int n[3];
+  dwa_axis_samples(cfg, n);
+  float mx[3], mn[3];
+  if (!cfg.use_dwa) {
+    const double dist = hypot(goal[0] - pos[0], goal[1] - pos[1]);
+    max_vel_x = dwa_max(dwa_min(max_vel_x, dist / cfg.sim_time), min_vel_x);
+    max_vel_y = dwa_max(dwa_min(max_vel_y, dist / cfg.sim_time), min_vel_y);
+    mx[0] = dwa_min(max_vel_x, vel[0] + acc[0] * cfg.sim_time);
+    mx[1] = dwa_min(max_vel_y, vel[1] + acc[1] * cfg.sim_time);
+    mx[2] = dwa_min(max_vel_th, vel[2] + acc[2] * cfg.sim_time);
+    mn[0] = dwa_max(min_vel_x, vel[0] - acc[0] * cfg.sim_time);
+    mn[1] = dwa_max(min_vel_y, vel[1] - acc[1] * cfg.sim_time);
+    mn[2] = dwa_max(min_vel_th, vel[2] - acc[2] * cfg.sim_time);
+  } else {
+    mx[0] = dwa_min(max_vel_x, vel[0] + acc[0] * cfg.sim_period);
+    mx[1] = dwa_min(max_vel_y, vel[1] + acc[1] * cfg.sim_period);
+    mx[2] = dwa_min(max_vel_th, vel[2] + acc[2] * cfg.sim_period);
+    mn[0] = dwa_max(min_vel_x, vel[0] - acc[0] * cfg.sim_period);
+    mn[1] = dwa_max(min_vel_y, vel[1] - acc[1] * cfg.sim_period);
+    mn[2] = dwa_max(min_vel_th, vel[2] - acc[2] * cfg.sim_period);
+  }
+  int k = 0;
+  for (int a = 0; a < 3; ++a) {
+    counts[a] = velocity_samples(mn[a], mx[a], n[a], out + k);
+    k += counts[a];
+  }
+}
+
+// OscillationCostFunction's latched state (oscillation_cost_function.h:78-83, .cpp:56-164)
+struct Oscillation {
+  bool strafe_pos_only = false, strafe_neg_only = false, strafing_pos = false, strafing_neg = false;
+  bool rot_pos_only = false, rot_neg_only = false, rotating_pos = false, rotating_neg = false;
+  bool forward_pos_only = false, forward_neg_only = false, forward_pos = false, forward_neg = false;
+  float prev[3] = {0.f, 0.f, 0.f};
+  __host__ __device__ void reset() {
+    strafe_pos_only = strafe_neg_only = strafing_pos = strafing_neg = false;
+    rot_pos_only = rot_neg_only = rotating_pos = rotating_neg = false;
+    forward_pos_only = forward_neg_only = forward_pos = forward_neg = false;
+  }
+  __host__ __device__ int mask() const {
+    return int(forward_pos_only) | int(forward_neg_only) << 1 | int(strafe_pos_only) << 2 | int(strafe_neg_only) << 3 |
+           int(rot_pos_only) << 4 | int(rot_neg_only) << 5;
+  }
+  __host__ __device__ bool set_flags(double xv, double yv, double thv, double min_vel_trans) {
+    bool flag_set = false;
+    if (xv < 0.0) { if (forward_pos) { forward_neg_only = true; flag_set = true; } forward_pos = false; forward_neg = true; }
+    if (xv > 0.0) { if (forward_neg) { forward_pos_only = true; flag_set = true; } forward_neg = false; forward_pos = true; }
+    if (fabs(xv) <= min_vel_trans) {
+      if (yv < 0) { if (strafing_pos) { strafe_neg_only = true; flag_set = true; } strafing_pos = false; strafing_neg = true; }
+      if (yv > 0) { if (strafing_neg) { strafe_pos_only = true; flag_set = true; } strafing_neg = false; strafing_pos = true; }
+      if (thv < 0) { if (rotating_pos) { rot_neg_only = true; flag_set = true; } rotating_pos = false; rotating_neg = true; }
+      if (thv > 0) { if (rotating_neg) { rot_pos_only = true; flag_set = true; } rotating_neg = false; rotating_pos = true; }
+    }
+    return flag_set;
+  }
+  __host__ __device__ void update(const float pos[3], double cost, double xv, double yv, double thv, double min_vel_trans,
+                                  double reset_dist, double reset_angle) {
+    if (cost < 0) return;
+    if (set_flags(xv, yv, thv, min_vel_trans)) { prev[0] = pos[0]; prev[1] = pos[1]; prev[2] = pos[2]; }
+    if (forward_pos_only || forward_neg_only || strafe_pos_only || strafe_neg_only || rot_pos_only || rot_neg_only) {
+      const double x_diff = pos[0] - prev[0], y_diff = pos[1] - prev[1];
+      const double sq_dist = x_diff * x_diff + y_diff * y_diff;
+      const double th_diff = pos[2] - prev[2];
+      if (sq_dist > reset_dist * reset_dist || fabs(th_diff) > reset_angle) reset();
+    }
+  }
+};
+
+// what findBestPath does on the host with the winner d of a search (dwa_planner.cpp:316-357): result_traj_'s
+// velocities persist across cycles (res_v), then the oscillation flags; fills *out (when given) but its n_points
+__host__ __device__ inline void apply_dwa_result(const DwaDeviceResult& d, const navgpu_dwa_config& c, const double pose[3],
+                                                 int32_t n_samples, double res_v[3], Oscillation& osc,
+                                                 navgpu_dwa_result* out) {
+  if (d.cost >= 0) { res_v[0] = d.xv; res_v[1] = d.yv; res_v[2] = d.thetav; }
+  const float pos[3] = {(float)pose[0], (float)pose[1], (float)pose[2]};
+  // oscillation_costs_.updateOscillationFlags(pos, &result_traj_, min_trans_vel), dwa_planner.cpp:357
+  osc.update(pos, d.cost, res_v[0], res_v[1], res_v[2], c.min_trans_vel, c.oscillation_reset_dist,
+             c.oscillation_reset_angle);
+  if (!out) return;
+  out->cost = d.cost;
+  out->xv = res_v[0]; out->yv = res_v[1]; out->thetav = res_v[2];
+  out->best_index = (int32_t)d.best_index;
+  out->n_samples = n_samples;
+  out->n_scored = d.n_scored;
+}
+
+// What a DWAPlanner fleet keeps per robot from one step to the next: the oscillation flags, result_traj_'s
+// velocities, whether a step planned the robot (its distance grids hold that step's wavefronts) and whether its
+// alignment grid was its path grid then, and a sensing fleet's rolled origin.  The fleet holds a host and a device
+// copy of the array and knows which one is current.
+struct FleetDwaState {
+  Oscillation osc;
+  double res_v[3];
+  double origin[2];
+  uint8_t planned, aliased;
 };
 
 // Multi-GPU sample sweep (config C4): one record per rank and sweep parity in every rank's exchange buffer.  The last
@@ -1606,6 +1751,78 @@ __global__ void __launch_bounds__(32, 1) k_fleet_check(DwaScoreArgs base, const 
   fleet_patch_args(s_a, base, robots[robot_of[c]], candidates + 3 * (size_t)c);
   const TrajResult r = score_sample<true>(s_a, 0, threadIdx.x & 31, nullptr, nullptr, 0, s_scratch, s_a.g.cost);
   if (threadIdx.x == 0) costs[c] = r.generated ? r.cost : ((s_a.nfp == 0 && s_a.scale_obstacle != 0.0) ? -9.0 : 0.0);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// The device fleet step (navgpu_fleet_step_device): what navgpu_fleet_step does per robot on the host, one thread per
+// robot, with the host step's own functions (fleet_roll_step, enumerate_samples, Oscillation, apply_dwa_result).
+constexpr int kFleetRobotThreads = 128;
+constexpr uint8_t kFleetActive = 1, kFleetAligned = 2;  // per-robot flags: planned by the steps; alignment grid = path grid
+
+struct FleetPrepareArgs {
+  const double* poses;  // [n][3], device memory
+  const double* vels;
+  FleetRobot* robots;
+  FleetDwaState* state;
+  const uint8_t* flags;
+  float* samples;  // robot r's per-axis samples at r * slot
+  int slot, n;
+  navgpu_dwa_config cfg;
+  FleetCmStep* steps;  // sensing fleets: the costmap update's step records; null on raw-map fleets
+  unsigned sx, sy;
+  double res;
+};
+
+// Before the costmap update: a sensing fleet's roll of every robot (fleet_costmap_roll), whose origin also goes into
+// the robot's MapGrid record; then, for robots the steps plan, the record's per-step fields and velocity samples
+// (navgpu_fleet_step's per-robot loop).  A left-out robot gets no samples, so its scoring CTAs exit at once.
+__global__ void __launch_bounds__(kFleetRobotThreads) k_fleet_prepare(FleetPrepareArgs a) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= a.n) return;
+  const double pose[3] = {a.poses[3 * r], a.poses[3 * r + 1], a.poses[3 * r + 2]};
+  FleetRobot& R = a.robots[r];
+  FleetDwaState& S = a.state[r];
+  if (a.steps) {
+    const FleetCmStep st = fleet_roll_step(pose, S.origin[0], S.origin[1], a.sx, a.sy, a.res);
+    a.steps[r] = st;
+    S.origin[0] = st.ox;
+    S.origin[1] = st.oy;
+    R.grids.g.ox = st.ox;
+    R.grids.g.oy = st.oy;
+  }
+  R.samples_offset = r * a.slot;
+  if (!(a.flags[r] & kFleetActive)) {
+    R.nx = R.ny = R.nth = 0;
+    return;
+  }
+  const float pos[3] = {(float)pose[0], (float)pose[1], (float)pose[2]};
+  const float vel[3] = {(float)a.vels[3 * r], (float)a.vels[3 * r + 1], (float)a.vels[3 * r + 2]};
+  const float goal[2] = {0.f, 0.f};  // (use_dwa = 0 only, which device steps refuse)
+  int counts[3];
+  enumerate_samples(a.cfg, pos, vel, goal, a.samples + (size_t)r * a.slot, counts);
+  for (int k = 0; k < 3; ++k) { R.pos[k] = pos[k]; R.vel[k] = vel[k]; }
+  R.osc_mask = S.osc.mask();
+  R.nx = counts[0]; R.ny = counts[1]; R.nth = counts[2];
+}
+
+// After k_fleet_finish: the host step's epilogue per planned robot (apply_dwa_result: result_traj_'s velocities, the
+// oscillation flags, the result record), the record written to the caller's device buffer; left-out robots' records
+// and state stay as they are
+__global__ void __launch_bounds__(kFleetRobotThreads) k_fleet_apply(navgpu_dwa_config cfg, const double* poses,
+                                                                    const FleetRobot* robots, const uint8_t* flags,
+                                                                    const DwaDeviceResult* found, FleetDwaState* state,
+                                                                    navgpu_dwa_result* results, int n) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n || !(flags[r] & kFleetActive)) return;
+  const FleetRobot& R = robots[r];
+  FleetDwaState S = state[r];
+  navgpu_dwa_result out;
+  apply_dwa_result(found[r], cfg, poses + 3 * r, R.nx * R.ny * R.nth, S.res_v, S.osc, &out);
+  out.n_points = 0;
+  S.planned = 1;
+  S.aliased = (flags[r] & kFleetAligned) ? 1 : 0;
+  state[r] = S;
+  results[r] = out;
 }
 
 }  // namespace navgpu

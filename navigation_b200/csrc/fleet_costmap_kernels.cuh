@@ -5,6 +5,7 @@
 #pragma once
 
 #include "costmap_kernels.cuh"
+#include "fleet_costmap.cuh"
 
 namespace navgpu {
 
@@ -13,14 +14,6 @@ struct FleetScanRobot {
   int clear_first, n_clear, rays;  // clearing DevObs [clear_first, + n_clear) of the fleet's table; total rays
   int mark_first, n_mark, marks;   // marking DevObs, likewise; total marking points
   long long mark_base;             // the robot's first entry of the marking scratch
-};
-
-// the host's scalars of one robot and step: Costmap2D::updateOrigin (the new origin and the cell shift that got there)
-// and the pose transformFootprint needs (cos / sin of the yaw from the host libm, like the single costmap)
-struct FleetCmStep {
-  double ox, oy;
-  double rx, ry, cos_th, sin_th;
-  int cell_dx, cell_dy;
 };
 
 constexpr int kFleetCmThreads = 256;
