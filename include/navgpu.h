@@ -523,7 +523,9 @@ void navgpu_tp_default_config(navgpu_tp_config* cfg);
 int navgpu_tp_create(navgpu_tp** out, const navgpu_tp_config* cfg, uint32_t size_x, uint32_t size_y, double resolution,
                      const double* footprint_xy, int n_footprint, int device);
 int navgpu_tp_destroy(navgpu_tp* h);
-/* TrajectoryPlanner::reconfigure (trajectory_planner.cpp:59-133); the oscillation / escape state is kept */
+/* TrajectoryPlanner::reconfigure (trajectory_planner.cpp:59-133); the oscillation / escape state is kept.  Validated
+ * as navgpu_tp_create validates (a refused configuration leaves the handle unchanged); trajectories may grow longer
+ * than at creation, and findBestPath still returns all of their points. */
 int navgpu_tp_reconfigure(navgpu_tp* h, const navgpu_tp_config* cfg);
 /* TrajectoryPlanner::setFootprint (trajectory_planner.h:195) */
 int navgpu_tp_set_footprint(navgpu_tp* h, const double* footprint_xy, int n_footprint);

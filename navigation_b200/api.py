@@ -528,6 +528,15 @@ class Dwa:
         api.check(self.lib.navgpu_dwa_create(C.byref(h), C.byref(self.cfg), size_x, size_y, resolution, device))
         self.h = h
 
+    def reconfigure(self, **overrides):
+        """DWAPlanner::reconfigure (navgpu_dwa_reconfigure) with the current configuration and `overrides`; plans,
+        oscillation flags and the last result are kept."""
+        cfg = DwaConfig.from_buffer_copy(self.cfg)
+        for k, v in overrides.items():
+            setattr(cfg, k, v)
+        self.api.check(self.lib.navgpu_dwa_reconfigure(self.h, C.byref(cfg)))
+        self.cfg = cfg
+
     def __del__(self):
         if getattr(self, "h", None):
             self.lib.navgpu_dwa_destroy(self.h)
@@ -703,11 +712,14 @@ class Dwa:
         return out
 
 
-def tp_config(lib, overrides):
-    """TrajectoryPlannerROS's defaults (navgpu_tp_default_config) with `overrides` (TpConfig field names; y_vels as a
-    list) applied."""
-    cfg = TpConfig()
-    lib.navgpu_tp_default_config(C.byref(cfg))
+def tp_config(lib, overrides, base=None):
+    """TrajectoryPlannerROS's defaults (navgpu_tp_default_config), or a copy of `base`, with `overrides` (TpConfig field
+    names; y_vels as a list) applied."""
+    if base is None:
+        cfg = TpConfig()
+        lib.navgpu_tp_default_config(C.byref(cfg))
+    else:
+        cfg = TpConfig.from_buffer_copy(base)
     for k, v in overrides.items():
         if k == "y_vels":
             for j, y in enumerate(v):
@@ -730,6 +742,19 @@ class TrajectoryPlanner:
         api.check(self.lib.navgpu_tp_create(C.byref(h), C.byref(self.cfg), size_x, size_y, resolution, _p(f, _f64p),
                                             f.shape[0], device))
         self.h = h
+
+    def reconfigure(self, **overrides):
+        """TrajectoryPlanner::reconfigure (navgpu_tp_reconfigure) with the current configuration and `overrides`
+        (y_vels as a list); the oscillation and escape state is kept.  A refused configuration raises and changes
+        nothing."""
+        cfg = tp_config(self.lib, overrides, base=self.cfg)
+        self.api.check(self.lib.navgpu_tp_reconfigure(self.h, C.byref(cfg)))
+        self.cfg = cfg
+
+    def set_footprint(self, xy):
+        """TrajectoryPlanner::setFootprint (navgpu_tp_set_footprint): (x, y) vertices in the robot frame."""
+        f = np.ascontiguousarray(xy, dtype=np.float64).reshape(-1, 2)
+        self.api.check(self.lib.navgpu_tp_set_footprint(self.h, _p(f, _f64p), f.shape[0]))
 
     def __del__(self):
         if getattr(self, "h", None):

@@ -25,7 +25,8 @@ def needs_build():
     if not os.path.exists(LIB):
         return True
     t = os.path.getmtime(LIB)
-    deps = sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(HERE, "..", "include", "*.h"))
+    deps = (sources() + glob.glob(os.path.join(CSRC, "*.cuh")) + glob.glob(os.path.join(CSRC, "*.inc")) +
+            glob.glob(os.path.join(HERE, "..", "include", "*.h")))
     return any(os.path.getmtime(p) > t for p in deps)
 
 

@@ -1608,6 +1608,15 @@ void* navo_tp_create(const navo_tp_config* cfg, uint32_t size_x, uint32_t size_y
   return t;
 }
 void navo_tp_destroy(void* h) { delete static_cast<Tp*>(h); }
+void navo_tp_reconfigure(void* h, const navo_tp_config* cfg) {  // trajectory_planner.cpp:59-133
+  Tp* t = static_cast<Tp*>(h);
+  t->cfg = *cfg;
+  if (t->cfg.vx_samples <= 0) t->cfg.vx_samples = 1;
+  if (t->cfg.vtheta_samples <= 0) t->cfg.vtheta_samples = 1;
+}
+void navo_tp_set_footprint(void* h, const double* xy, int n) {  // trajectory_planner.h:195
+  static_cast<Tp*>(h)->footprint = to_pts(xy, n);
+}
 void navo_tp_set_costmap(void* h, const uint8_t* grid, double origin_x, double origin_y) {
   Tp* t = static_cast<Tp*>(h);
   t->cm.ox = origin_x;
@@ -1852,6 +1861,11 @@ void* navo_dwa_create(const navo_dwa_config* cfg, uint32_t size_x, uint32_t size
   return d;
 }
 void navo_dwa_destroy(void* h) { delete static_cast<Dwa*>(h); }
+void navo_dwa_reconfigure(void* h, const navo_dwa_config* cfg) {  // dwa_planner.cpp:52-112
+  Dwa* d = static_cast<Dwa*>(h);
+  d->cfg = *cfg;
+  d->reconfigure();
+}
 void navo_dwa_set_costmap(void* h, const uint8_t* grid, double origin_x, double origin_y) {
   Dwa* d = static_cast<Dwa*>(h);
   d->cm.ox = origin_x;

@@ -140,6 +140,10 @@ typedef struct {
 void navo_dwa_default_config(navo_dwa_config* cfg);
 void* navo_dwa_create(const navo_dwa_config* cfg, uint32_t size_x, uint32_t size_y, double resolution);
 void navo_dwa_destroy(void* h);
+/* DWAPlanner::reconfigure (dwa_planner.cpp:52-112) of a live handle: plans, oscillation flags and result_traj_ are
+ * kept.  cheat_factor and sum_scores, which the reference reads only at construction, are taken from cfg as well,
+ * as navgpu_dwa_reconfigure takes them. */
+void navo_dwa_reconfigure(void* h, const navo_dwa_config* cfg);
 void navo_dwa_set_costmap(void* h, const uint8_t* grid, double origin_x, double origin_y);
 /* DWAPlanner::updatePlanAndLocalCosts (dwa_planner.cpp:240-286); plan_xy = n (x,y) pairs */
 void navo_dwa_set_plan(void* h, const double pose[3], const double* plan_xy, int n);
@@ -195,6 +199,13 @@ void navo_tp_default_config(navo_tp_config* cfg); /* trajectory_planner_ros.cpp:
 void* navo_tp_create(const navo_tp_config* cfg, uint32_t size_x, uint32_t size_y, double resolution,
                      const double* footprint_xy, int n_footprint);
 void navo_tp_destroy(void* h);
+/* TrajectoryPlanner::reconfigure (trajectory_planner.cpp:59-133) of a live handle, which clamps vx_samples and
+ * vtheta_samples to at least 1; the oscillation and escape state, the plan and the distance maps are kept.  sim_period,
+ * which the reference reads only at construction, is taken from cfg as well, as navgpu_tp_reconfigure takes it
+ * (stop_time_buffer, the other such parameter, is read by neither findBestPath nor scoreTrajectory). */
+void navo_tp_reconfigure(void* h, const navo_tp_config* cfg);
+/* TrajectoryPlanner::setFootprint (trajectory_planner.h:195): xy = n (x,y) pairs in the robot frame */
+void navo_tp_set_footprint(void* h, const double* xy, int n);
 void navo_tp_set_costmap(void* h, const uint8_t* grid, double origin_x, double origin_y);
 /* TrajectoryPlanner::updatePlan(plan, compute_dists = false), trajectory_planner.cpp:477-502 */
 void navo_tp_update_plan(void* h, const double* plan_xy, int n);

@@ -123,7 +123,8 @@ def _declare(lib, prefix):
         "impl_name": (C.c_char_p, []),
         "project_scan": (i, [C.POINTER(LaserScan), C.POINTER(C.c_float), i, _f64p]),
     }
-    # the legacy TrajectoryPlanner (both checkers export it; tolerated as missing for an older prebuilt library)
+    # the legacy TrajectoryPlanner and the reconfigure entry points (both checkers export them; tolerated as missing for
+    # an older prebuilt library)
     optional = {
         "tp_default_config": (None, [C.POINTER(TpConfig)]),
         "tp_create": (vp, [C.POINTER(TpConfig), u, u, d, _f64p, i]),
@@ -132,6 +133,9 @@ def _declare(lib, prefix):
         "tp_update_plan": (None, [vp, _f64p, i]),
         "tp_find_best_path": (i, [vp, _f64p, _f64p, C.POINTER(TpResult), _f64p, i]),
         "tp_score_trajectory": (d, [vp, _f64p, _f64p, _f64p]),
+        "tp_reconfigure": (None, [vp, C.POINTER(TpConfig)]),
+        "tp_set_footprint": (None, [vp, _f64p, i]),
+        "dwa_reconfigure": (None, [vp, C.POINTER(DwaConfig)]),
         "tp_get_grid": (None, [vp, i, _f64p]),
         "plan_transform": (i, [_f64p, i, _f64p, _f64p, _f64p, d, _i32p, _f64p]),
         "plan_prune": (i, [_f64p, i, _f64p]),
@@ -301,6 +305,15 @@ class Dwa:
             setattr(self.cfg, k, v)
         self.h = C.c_void_p(self.lib.navo_dwa_create(C.byref(self.cfg), size_x, size_y, resolution))
 
+    def reconfigure(self, **overrides):
+        """DWAPlanner::reconfigure with the current configuration and `overrides` (same signature as
+        navigation_b200.api.Dwa.reconfigure)."""
+        cfg = DwaConfig.from_buffer_copy(self.cfg)
+        for k, v in overrides.items():
+            setattr(cfg, k, v)
+        self.lib.navo_dwa_reconfigure(self.h, C.byref(cfg))
+        self.cfg = cfg
+
     def __del__(self):
         if getattr(self, "h", None):
             self.lib.navo_dwa_destroy(self.h)
@@ -353,6 +366,16 @@ class Dwa:
         self.lib.navo_dwa_prepare_only(self.h)
 
 
+def _tp_override(cfg, overrides):
+    for k, v in overrides.items():
+        if k == "y_vels":
+            for j, y in enumerate(v):
+                cfg.y_vels[j] = y
+            cfg.n_y_vels = len(v)
+        else:
+            setattr(cfg, k, v)
+
+
 class TrajectoryPlanner:
     """The legacy base_local_planner::TrajectoryPlanner."""
 
@@ -361,16 +384,22 @@ class TrajectoryPlanner:
         self.size_x, self.size_y = size_x, size_y
         self.cfg = TpConfig()
         self.lib.navo_tp_default_config(C.byref(self.cfg))
-        for k, v in overrides.items():
-            if k == "y_vels":
-                for j, y in enumerate(v):
-                    self.cfg.y_vels[j] = y
-                self.cfg.n_y_vels = len(v)
-            else:
-                setattr(self.cfg, k, v)
+        _tp_override(self.cfg, overrides)
         f = np.ascontiguousarray(footprint_xy, dtype=np.float64).reshape(-1, 2)
         self.h = C.c_void_p(self.lib.navo_tp_create(C.byref(self.cfg), size_x, size_y, resolution, _p(f, _f64p),
                                                     f.shape[0]))
+
+    def reconfigure(self, **overrides):
+        """TrajectoryPlanner::reconfigure with the current configuration and `overrides` (y_vels as a list; same
+        signature as navigation_b200.api.TrajectoryPlanner.reconfigure)."""
+        cfg = TpConfig.from_buffer_copy(self.cfg)
+        _tp_override(cfg, overrides)
+        self.lib.navo_tp_reconfigure(self.h, C.byref(cfg))
+        self.cfg = cfg
+
+    def set_footprint(self, xy):
+        f = np.ascontiguousarray(xy, dtype=np.float64).reshape(-1, 2)
+        self.lib.navo_tp_set_footprint(self.h, _p(f, _f64p), f.shape[0])
 
     def __del__(self):
         if getattr(self, "h", None):

@@ -41,9 +41,11 @@
 #undef private
 
 #include <cmath>
+#include <cstdio>
 #include <limits>
 #include <memory>
 #include <queue>
+#include <string>
 #include <vector>
 
 #include "oracle_api.h"
@@ -739,6 +741,14 @@ void* navo_dwa_create(const navo_dwa_config* cfg, uint32_t size_x, uint32_t size
   return new DwaHandle(*cfg, size_x, size_y, resolution);
 }
 void navo_dwa_destroy(void* hv) { delete static_cast<DwaHandle*>(hv); }
+void navo_dwa_reconfigure(void* hv, const navo_dwa_config* cfg) {
+  DwaHandle* h = static_cast<DwaHandle*>(hv);
+  h->cfg = *cfg;
+  // the two construction parameters that navo_dwa_config carries (dwa_planner.cpp:116-182) follow cfg too
+  h->cheat_factor_ = cfg->cheat_factor;
+  h->obstacle_costs_.setSumScores(cfg->sum_scores != 0);
+  h->reconfigure();
+}
 void navo_dwa_set_costmap(void* hv, const uint8_t* grid, double ox, double oy) {
   setCostmap(static_cast<DwaHandle*>(hv)->costmap, grid, ox, oy);
 }
@@ -958,6 +968,39 @@ void* navo_tp_create(const navo_tp_config* cfg, uint32_t size_x, uint32_t size_y
   return new TpHandle(*cfg, size_x, size_y, resolution, footprint_xy, n_footprint);
 }
 void navo_tp_destroy(void* hv) { delete static_cast<TpHandle*>(hv); }
+void navo_tp_reconfigure(void* hv, const navo_tp_config* c) {
+  TpHandle* h = static_cast<TpHandle*>(hv);
+  base_local_planner::BaseLocalPlannerConfig config;  // what TrajectoryPlannerROS::reconfigureCB hands over (trajectory_planner_ros.cpp)
+  config.acc_lim_x = c->acc_lim_x; config.acc_lim_y = c->acc_lim_y; config.acc_lim_theta = c->acc_lim_theta;
+  config.max_vel_x = c->max_vel_x; config.min_vel_x = c->min_vel_x;
+  config.max_vel_theta = c->max_vel_th; config.min_vel_theta = c->min_vel_th;
+  config.min_in_place_vel_theta = c->min_in_place_vel_th;
+  config.sim_time = c->sim_time; config.sim_granularity = c->sim_granularity;
+  config.angular_sim_granularity = c->angular_sim_granularity;
+  config.pdist_scale = c->pdist_scale; config.gdist_scale = c->gdist_scale; config.occdist_scale = c->occdist_scale;
+  config.oscillation_reset_dist = c->oscillation_reset_dist; config.escape_reset_dist = c->escape_reset_dist;
+  config.escape_reset_theta = c->escape_reset_theta;
+  config.vx_samples = c->vx_samples; config.vtheta_samples = c->vtheta_samples;
+  config.heading_lookahead = c->heading_lookahead;
+  config.holonomic_robot = c->holonomic_robot != 0;
+  config.escape_vel = c->backup_vel;
+  config.dwa = c->dwa != 0;
+  config.heading_scoring = c->heading_scoring != 0;
+  config.heading_scoring_timestep = c->heading_scoring_timestep;
+  config.simple_attractor = c->simple_attractor != 0;
+  std::string y;  // parsed back by reconfigure; %.17g round-trips every double
+  for (int i = 0; i < c->n_y_vels; ++i) {
+    char buf[32];
+    snprintf(buf, sizeof(buf), "%s%.17g", i ? "," : "", c->y_vels[i]);
+    y += buf;
+  }
+  config.y_vels = y;
+  h->tp->sim_period_ = c->sim_period;  // a construction parameter (trajectory_planner.cpp:135-187) navo_tp_config carries
+  h->tp->reconfigure(config);
+}
+void navo_tp_set_footprint(void* hv, const double* xy, int n) {
+  static_cast<TpHandle*>(hv)->tp->setFootprint(toPoints(xy, n));
+}
 void navo_tp_set_costmap(void* hv, const uint8_t* grid, double ox, double oy) {
   setCostmap(static_cast<TpHandle*>(hv)->costmap, grid, ox, oy);
 }

@@ -339,11 +339,12 @@ def tp_results_equal(a, b, rtol=0.0):
                 np.allclose(a["scores"], b["scores"], rtol=rtol, atol=0))
 
 
-def run_tp_boxed_scenario(api, cycles=9):
+def run_tp_boxed_scenario(api, cycles=9, reconfigure=None):
     """The legacy TrajectoryPlanner in a slot just wider than the robot, open along y: driving forward and rotating in
     place collide, so createTrajectories falls through to strafing (trajectory_planner.cpp:752-797); the plan is then
     reversed (the other strafing direction wins and the first one is latched as stuck), and finally the slot is closed
-    on both sides, which leaves backing up and escape mode (:851-903)."""
+    on both sides, which leaves backing up and escape mode (:851-903).  `reconfigure`: {cycle: overrides} applied
+    before that cycle's findBestPath."""
     n, res = 120, 0.05
     grid = np.zeros((n, n), np.uint8)
     grid[:, 50:52] = 254   # wall behind the robot: x in [2.50, 2.60)
@@ -363,6 +364,8 @@ def run_tp_boxed_scenario(api, cycles=9):
             closed[49:51, :] = 254
             closed[70:72, :] = 254
             tp.set_costmap(closed, 0.0, 0.0)
+        if reconfigure and cyc in reconfigure:
+            tp.reconfigure(**reconfigure[cyc])
         r = tp.find_best_path(pose, vel)
         r["grids"] = [tp.grid(0), tp.grid(1)]
         r["scores"] = np.array([tp.score_trajectory(pose, vel, (0.0, 0.1, 0.0)), tp.score_trajectory(pose, vel, (0.1, 0.0, 0.0))])
@@ -423,3 +426,206 @@ def run_tp_edge_cases(api, grid_api):
             r["scores"] = np.array([tp.score_trajectory(c["pose"], s["vel"], (0.2, 0.0, 0.1))])
             out.append(r)
     return out
+
+
+def run_dwa_sequence(api, grid, origin, pose, plan, vel, ops, **create):
+    """A DWAPlanner handle driven through `ops` on one local costmap.  Ops: ("reconfigure", overrides), ("plan",) =
+    updatePlanAndLocalCosts at the current pose, ("plan_at", pose, plan), ("find",), ("check", [vel_samples, ...]),
+    ("follow",) = take the last result as the next velocity, alternating forward and backward so that the oscillation
+    flags latch (as run_dwa_scenario does), ("costmap", grid).  Returns one record per "find" / "check"."""
+    d = api.dwa(120, 120, 0.05, **create)
+    d.set_costmap(grid, *origin)
+    pose, vel = np.array(pose, dtype=np.float64), np.array(vel, dtype=np.float64)
+    out, last, n_find = [], None, 0
+    for op in ops:
+        if op[0] == "reconfigure":
+            d.reconfigure(**op[1])
+        elif op[0] == "plan":
+            d.set_plan(pose, plan)
+        elif op[0] == "plan_at":
+            d.set_plan(op[1], op[2])
+        elif op[0] == "costmap":
+            d.set_costmap(op[1], *origin)
+        elif op[0] == "find":
+            last = d.find_best_path(pose, vel, PENTAGON)
+            last["mask"] = d.oscillation_mask()
+            last["grids"] = [d.grid(k) for k in range(4)]
+            last["cfg"] = bytes(d.cfg)
+            last["pose"], last["vel"] = pose.copy(), vel.copy()
+            out.append(last)
+            n_find += 1
+        elif op[0] == "check":
+            out.append(dict(checks=[d.check_trajectory(pose, vel, v, PENTAGON) for v in op[1]], mask=d.oscillation_mask()))
+        elif op[0] == "follow":
+            vel = (np.array([last["xv"] * (-1 if n_find % 2 == 0 else 1), last["yv"], -last["thetav"]]) if last["ok"]
+                   else vel * 0)
+            pose = pose + np.array([0.01 * vel[0], 0, 0.01 * vel[2]])
+    return out
+
+
+def run_tp_sequence(api, grid, origin, pose, plan, vel, ops, footprint=PENTAGON, **create):
+    """A legacy TrajectoryPlanner handle driven through `ops`: ("reconfigure", overrides), ("footprint", xy),
+    ("plan", plan), ("find",) = findBestPath + both distance maps + two scoreTrajectory probes, ("follow", step) = take
+    the last result as the next velocity and move by step x velocity.  Returns one record per "find"."""
+    tp = api.trajectory_planner(120, 120, 0.05, footprint, **create)
+    tp.set_costmap(grid, *origin)
+    if plan is not None:
+        tp.update_plan(plan)
+    pose, vel = np.array(pose, dtype=np.float64), np.array(vel, dtype=np.float64)
+    out = []
+    for op in ops:
+        if op[0] == "reconfigure":
+            tp.reconfigure(**op[1])
+        elif op[0] == "footprint":
+            tp.set_footprint(op[1])
+        elif op[0] == "plan":
+            tp.update_plan(op[1])
+        elif op[0] == "find":
+            r = tp.find_best_path(pose, vel)
+            r["grids"] = [tp.grid(0), tp.grid(1)]
+            r["scores"] = np.array([tp.score_trajectory(pose, vel, p) for p in ((0.3, 0.0, 0.2), (0.0, 0.1, -0.6))])
+            out.append(r)
+        elif op[0] == "follow":
+            vel = np.array([out[-1]["xv"], out[-1]["yv"], out[-1]["thetav"]]) if out[-1]["cost"] >= 0 else vel * 0
+            pose = pose + np.array([op[1] * vel[0] * np.cos(pose[2]), op[1] * vel[0] * np.sin(pose[2]), op[1] * vel[2]])
+    return out
+
+
+def reconfigure_world(seed=3, style="corridor", unknown=False):
+    """A local costmap, pose, velocity and plan of dwa_scenario for the reconfigure sequences; `unknown` marks a band of
+    NO_INFORMATION cells across the robot's way."""
+    from oracle import pyoracle
+    rng = np.random.default_rng(seed)
+    s = dwa_scenario(rng, style=style)
+    grid = local_costmap(pyoracle.load("port"), np.random.default_rng(seed + 1000), ox=s["origin"][0],
+                         oy=s["origin"][1], style=style)
+    if unknown:
+        cx = int((s["pose"][0] - s["origin"][0]) / 0.05)
+        grid[:, cx + 8:cx + 11] = 255
+    return dict(grid=grid, origin=s["origin"], pose=s["pose"], plan=s["plan"], vel=s["vel"])
+
+
+def dwa_reconfigure_cases():
+    """name -> (world, create overrides, ops) of the DWAPlanner reconfigure sequences."""
+    find = [("plan",), ("find",), ("check", [(0.3, 0.0, 0.2), (0.0, 0.0, 0.0), (0.5, 0.1, -0.7)]), ("follow",)]
+    cases = {}
+    # per-axis sample counts across the 640 values carried inline in the kernel parameters, and back, at one velocity:
+    # the staged set of the second and the fourth search is the same
+    xy0 = dict(max_vel_y=0.0, min_vel_y=0.0)
+    cases["samples_inline_staged"] = (dict(seed=3), dict(vx_samples=20, vy_samples=1, vth_samples=20, **xy0), [
+        ("plan",), ("find",), ("reconfigure", dict(vx_samples=400, vth_samples=400)), ("plan",), ("find",),
+        ("reconfigure", dict(vx_samples=3, vy_samples=10, vth_samples=20, max_vel_y=0.1, min_vel_y=-0.1)), ("plan",),
+        ("find",), ("reconfigure", dict(vx_samples=400, vy_samples=1, vth_samples=400, **xy0)), ("plan",), ("find",)])
+    # the goal-front target and the alignment scale come from the configuration of set_plan; the reconfigure between
+    # set_plan and findBestPath restores the alignment scale, which set_plan zeroed near the goal
+    crit = dict(forward_point_distance=0.6, cheat_factor=2.0, path_distance_bias=20.0, goal_distance_bias=40.0)
+    crit2 = dict(forward_point_distance=0.1, cheat_factor=0.5, path_distance_bias=32.0, goal_distance_bias=24.0)
+    for where in ("near", "far", "far_then_near"):
+        ops = []
+        for k in range(3):
+            near = where == "near" or (where == "far_then_near" and k > 0)
+            ops += [("plan_at", None, near), ("reconfigure", crit if k % 2 == 0 else crit2), ("find",),
+                    ("check", [(0.3, 0.0, 0.2), (0.1, 0.0, -0.5)])]
+        cases[f"critics_{where}"] = (dict(seed=5, style="empty"), dict(vx_samples=6, vy_samples=1, vth_samples=9), ops)
+    # oscillation flags latched by alternating commands, then new reset distance / angle, then further cycles
+    # (without checkTrajectory, which resets the flags)
+    step = [("plan",), ("find",), ("follow",)]
+    cases["oscillation_reset"] = (dict(seed=11), dict(vx_samples=5, vy_samples=3, vth_samples=7, min_vel_x=-0.2),
+                                  step * 4 + [("reconfigure", dict(oscillation_reset_dist=0.001,
+                                                                   oscillation_reset_angle=0.01))] + step * 3)
+    cases["use_dwa_sum_scores"] = (dict(seed=7), dict(vx_samples=5, vy_samples=2, vth_samples=8), find + [
+        ("reconfigure", dict(use_dwa=0))] + find + [("reconfigure", dict(use_dwa=1, sum_scores=1))] + find + [
+        ("reconfigure", dict(sum_scores=0))] + find)
+    cases["allow_unknown"] = (dict(seed=7, unknown=True), dict(vx_samples=5, vy_samples=1, vth_samples=8), find + [
+        ("reconfigure", dict(allow_unknown=1))] + find + [("reconfigure", dict(allow_unknown=0))] + find)
+    cases["limits_and_horizon"] = (dict(seed=13), dict(vx_samples=6, vy_samples=3, vth_samples=9), find + [
+        ("reconfigure", dict(max_vel_x=0.3, max_trans_vel=0.35, min_rot_vel=0.2, max_rot_vel=0.6, acc_lim_x=1.0,
+                             acc_lim_theta=6.0))] + find + [
+        ("reconfigure", dict(sim_time=3.0, sim_granularity=0.01, angular_sim_granularity=0.05, sim_period=0.2))] + find + [
+        ("reconfigure", dict(sim_time=0.8, sim_granularity=0.05, angular_sim_granularity=0.2))] + find)
+    cases["zero_samples"] = (dict(seed=13), dict(vx_samples=4, vy_samples=2, vth_samples=6), find + [
+        ("reconfigure", dict(vx_samples=0, vy_samples=0, vth_samples=0))] + find + [
+        ("reconfigure", dict(vx_samples=-3, vy_samples=1, vth_samples=5))] + find + [
+        ("reconfigure", dict(vx_samples=4, vy_samples=2, vth_samples=6))] + find)
+    return cases
+
+
+def dwa_case_world(case):
+    world, create, ops = dwa_reconfigure_cases()[case]
+    w = reconfigure_world(**world)
+    resolved = []
+    for op in ops:
+        if op[0] == "plan_at":  # near: a plan that ends 0.3 m ahead of the robot; far: the scenario's plan
+            if op[2]:
+                p = np.array(w["pose"][:2])
+                resolved.append(("plan_at", w["pose"], np.stack([np.linspace(p[0] - 0.5, p[0] + 0.3, 17),
+                                                                  np.full(17, p[1])], 1)))
+            else:
+                resolved.append(("plan_at", w["pose"], w["plan"]))
+        else:
+            resolved.append(op)
+    return w, create, resolved
+
+
+def run_dwa_reconfigure_case(api, case):
+    w, create, ops = dwa_case_world(case)
+    return run_dwa_sequence(api, w["grid"], w["origin"], w["pose"], w["plan"], w["vel"], ops, **create)
+
+
+def tp_points_stride(cfg):
+    """The points per sample a TrajectoryPlanner handle sizes for `cfg` (tp_check_config of tp_host.inc)."""
+    vmax = max(abs(cfg.max_vel_x), abs(cfg.min_vel_x), abs(cfg.backup_vel))
+    vymax = max([0.1] + [abs(cfg.y_vels[i]) for i in range(cfg.n_y_vels)])
+    wmax = max(abs(cfg.max_vel_th), abs(cfg.min_vel_th), abs(cfg.min_in_place_vel_th))
+    return int(max(max(np.hypot(vmax, vymax) * cfg.sim_time, cfg.sim_time) / cfg.sim_granularity,
+                   wmax / cfg.angular_sim_granularity) + 2.0)
+
+
+def tp_open_world():
+    """An empty 6 m x 6 m map, the robot at (1, 3) heading along the plan (+x) at 0.5 m/s."""
+    plan = np.stack([np.arange(1.0, 5.9, 0.05), np.full(98, 3.0)], 1)
+    return dict(grid=np.zeros((120, 120), np.uint8), origin=(0.0, 0.0), pose=(1.0, 3.0, 0.0), plan=plan,
+                vel=(0.5, 0.0, 0.0))
+
+
+def tp_reconfigure_cases():
+    """name -> (world, create overrides, ops, lengthening) of the TrajectoryPlanner reconfigure sequences; a
+    lengthening case returns trajectories longer than the handle's creation configuration allows."""
+    f = [("find",), ("follow", 0.02)]
+    turn = dict(pose=(1.0, 3.0, 1.2), vel=(0.3, 0.0, -0.8))  # heading away from the plan: the winner turns
+    cases = {
+        "longer_sim_time": (dict(), dict(), f + [("reconfigure", dict(sim_time=3.0))] + f * 2, True),
+        "finer_angular_granularity": (turn, dict(dwa=0), f + [("reconfigure", dict(angular_sim_granularity=0.005))] + f * 2,
+                                      True),
+        "finer_granularity": (dict(), dict(), f + [("reconfigure", dict(sim_granularity=0.01))] + f * 2, True),
+        "faster_max_vel_x": (dict(vel=(1.4, 0.0, 0.0)), dict(), f + [("reconfigure", dict(max_vel_x=1.5))] + f * 2, True),
+        "faster_max_vel_th": (turn, dict(dwa=0), f + [("reconfigure", dict(max_vel_th=4.0, min_vel_th=-4.0,
+                                                                          acc_lim_theta=8.0))] + f * 2, True),
+        "shorter": (dict(), dict(sim_time=2.0, sim_granularity=0.01), f + [
+            ("reconfigure", dict(sim_time=0.5, sim_granularity=0.05, angular_sim_granularity=0.1))] + f * 2, False),
+        # 30 x 40 forward samples: past the 256 samples the buffers start with, regrown together with the stride
+        "sample_capacity": (dict(), dict(), f + [("reconfigure", dict(vx_samples=30, vtheta_samples=40, sim_time=2.5))] +
+                            f + [("reconfigure", dict(vx_samples=3, vtheta_samples=20, sim_time=1.0))] + f + [
+                                ("reconfigure", dict(vx_samples=30, vtheta_samples=40, sim_time=2.5))] + f, True),
+        "zero_samples": (dict(), dict(), f + [("reconfigure", dict(vx_samples=0, vtheta_samples=0))] + f + [
+            ("reconfigure", dict(vx_samples=3, vtheta_samples=20))] + f, False),
+        "modes": (dict(seed=21), dict(), f + [("reconfigure", dict(heading_scoring=1, heading_scoring_timestep=0.45))] + f + [
+            ("plan", None)] + f + [("reconfigure", dict(heading_scoring=0, dwa=0))] + f + [
+            ("reconfigure", dict(holonomic_robot=0, dwa=1, y_vels=[-0.2, 0.2]))] + f + [
+            ("reconfigure", dict(holonomic_robot=1, heading_scoring=1, heading_scoring_timestep=0.1))] + f, False),
+        "footprints": (dict(seed=21), dict(), f + [("footprint", square_footprint(0.4))] + f + [
+            ("footprint", square_footprint(0.15))] + f + [
+            ("footprint", [(0.3 * np.cos(a), 0.3 * np.sin(a)) for a in np.linspace(0, 2 * np.pi, 16, endpoint=False)])] +
+            f + [("footprint", PENTAGON)] + f, False),
+    }
+    return cases
+
+
+def run_tp_reconfigure_case(api, case):
+    world, create, ops, _ = tp_reconfigure_cases()[case]
+    if "seed" in world:  # a corridor of dwa_scenario; ("plan", None) halves its plan
+        w = reconfigure_world(seed=world["seed"])
+        ops = [("plan", w["plan"][:len(w["plan"]) // 2]) if op == ("plan", None) else op for op in ops]
+    else:
+        w = dict(tp_open_world(), **world)
+    return run_tp_sequence(api, w["grid"], w["origin"], w["pose"], w["plan"], w["vel"], ops, **create)
