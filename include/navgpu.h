@@ -566,10 +566,31 @@ int navgpu_fleet_use_trajectory_planner(navgpu_fleet* f, const navgpu_tp_config*
  * robot; poses, vels [n][3]; results[r] as navgpu_tp_find_best_path returns it (points are not materialised, n_points
  * is their count) */
 int navgpu_fleet_step_tp(navgpu_fleet* f, const double* poses, const double* vels, navgpu_tp_result* results);
+/* navgpu_fleet_step_tp with device memory of the fleet's device, for any fleet kind: poses [n][3] and vels [n][3]
+ * (double) are read and results [n] written on the fleet's stream (navgpu_fleet_stream); the call returns without
+ * waiting for the device.  Per robot, the rounding through float, the samples of createTrajectories and the selection
+ * with its oscillation / escape state run on the device too.  After the stream has run, results (n_points: the chosen
+ * trajectory's point count), every costmap, layer, voxel column, window and origin, both distance grids of every robot
+ * and all later behaviour are those of navgpu_fleet_step_tp with the same poses and velocities.  One exception by
+ * construction: cos / sin of each robot's yaw (its footprint cells, a sensing fleet's footprint clearing) come from
+ * CUDA's sincos instead of the host libm.  hypot is computed as glibc 2.35+ computes it (which is not correctly
+ * rounded); where the process's libm hypot gives other bits on a fixed list of pairs, checked once per process, the
+ * call is refused.  Robots navgpu_fleet_set_active left out keep their results entry untouched.  The caller orders its
+ * writes of poses and vels before the fleet's stream and reads results after work ordered behind it.  Host and device
+ * steps, and every other call, may be mixed on one fleet: a host call that reads or changes the planner state
+ * (navgpu_fleet_step_tp, _set_plans, _check_trajectories, _get_geometry) first waits for the fleet's stream.  A device
+ * step that follows a device step, with no set_plans, set_active or set_maps in between, neither waits for the host,
+ * allocates nor copies from pageable memory, so it can be captured in a CUDA graph.  Each robot's samples sit in a slot
+ * sized from the configuration: vx_samples * vtheta_samples + vtheta_samples + 1, plus 2 + n_y_vels when holonomic (87
+ * with TrajectoryPlannerROS's defaults).  Refused, with the fleet unchanged: null or non-device pointers and fleets
+ * that are not TrajectoryPlanner fleets (NAVGPU_ERR_INVALID), slots of more than 4096 samples and a libm whose hypot
+ * differs (NAVGPU_ERR_UNSUPPORTED). */
+int navgpu_fleet_step_tp_device(navgpu_fleet* f, const double* poses, const double* vels, navgpu_tp_result* results);
 /* path_map_ (which = 0) / goal_map_ (1) of robot after the last step, fp64 HOST size_y x size_x (as navgpu_tp_get_grid) */
 int navgpu_fleet_tp_get_grid(navgpu_fleet* f, int robot, int which, double* host_out);
-/* device time (ms, CUDA events) of the last step's footprint-cell, wavefront and scoring launches (0 before the first
- * step); synchronises the fleet's stream */
+/* device time (ms, CUDA events) of the last host step's (navgpu_fleet_step_tp) footprint-cell, wavefront and scoring
+ * launches (0 before the first one); synchronises the fleet's stream.  Device steps (navgpu_fleet_step_tp_device)
+ * record no events and leave these times as they were: time them with events of your own on navgpu_fleet_stream. */
 int navgpu_fleet_tp_last_timing(navgpu_fleet* f, float* footprint_ms, float* wavefront_ms, float* score_ms);
 
 /* ---- Goal handling for fleets: robots that stop and rotate ----------------------------------------------------

@@ -233,6 +233,7 @@ SIGNATURES = {
     "navgpu_tp_last_sample_count": (C.c_int, [C.c_void_p, _i32p]),
     "navgpu_fleet_use_trajectory_planner": (C.c_int, [C.c_void_p, C.POINTER(TpConfig)]),
     "navgpu_fleet_step_tp": (C.c_int, [C.c_void_p, _f64p, _f64p, C.POINTER(TpResult)]),
+    "navgpu_fleet_step_tp_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "navgpu_fleet_tp_get_grid": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _f64p]),
     "navgpu_fleet_tp_last_timing": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_float),
                                               C.POINTER(C.c_float)]),
@@ -918,13 +919,31 @@ class Fleet:
         cost, xv, yv, thetav (float64), best_index, n_samples, n_scored (int32), and the buffer itself as `records`
         (uint8), which `out` may pass back to be written again.  A robot that set_active left out keeps its record as
         it was.  Wrong devices, dtypes or shapes raise ValueError."""
+        out = self._device_step(self.lib.navgpu_fleet_step_device, DwaResult, poses, vels, out)
+        f64, i32 = out["f64"], out["i32"]
+        return dict(cost=f64[:, 0], xv=f64[:, 1], yv=f64[:, 2], thetav=f64[:, 3], best_index=i32[:, 8],
+                    n_samples=i32[:, 9], n_scored=i32[:, 10], records=out["records"])
+
+    def step_tp_device(self, poses, vels, out=None):
+        """step() of a TrajectoryPlanner fleet on the device (navgpu_fleet_step_tp_device), as step_device is for
+        DWAPlanner fleets: the same arguments, stream ordering and ValueErrors.  Returns views of one CUDA buffer of n
+        navgpu_tp_result records: cost, xv, yv, thetav (float64), n_points, flags (int32), and the buffer itself as
+        `records` (uint8), which `out` may pass back to be written again."""
+        out = self._device_step(self.lib.navgpu_fleet_step_tp_device, TpResult, poses, vels, out)
+        f64, i32 = out["f64"], out["i32"]
+        return dict(cost=f64[:, 0], xv=f64[:, 1], yv=f64[:, 2], thetav=f64[:, 3], n_points=i32[:, 8], flags=i32[:, 9],
+                    records=out["records"])
+
+    def _device_step(self, call, record, poses, vels, out):
+        """Checks the tensors, runs call(handle, poses, vels, out) between the stream waits of step_device, and returns
+        the result buffer with its float64 and int32 views, one row per robot."""
         import torch
         dev = torch.device("cuda", self.device)
         for what, x in (("poses", poses), ("vels", vels)):
             if not isinstance(x, torch.Tensor) or x.dtype != torch.float64 or tuple(x.shape) != (self.n, 3) or \
                     not x.is_cuda or x.device.index != self.device or not x.is_contiguous():
                 raise ValueError(f"{what}: a contiguous float64 tensor of shape ({self.n}, 3) on cuda:{self.device}")
-        nbytes = self.n * C.sizeof(DwaResult)
+        nbytes = self.n * C.sizeof(record)
         if out is None:
             out = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         elif not isinstance(out, torch.Tensor) or out.dtype != torch.uint8 or tuple(out.shape) != (nbytes,) or \
@@ -934,13 +953,11 @@ class Fleet:
         fleet_stream.wait_stream(torch.cuda.current_stream(dev))
         # (no record_stream on the fleet's stream, which may be destroyed before the tensors are freed: torch's current
         # stream waits for the fleet's below, so memory torch reuses there is only written after the step read it)
-        self.api.check(self.lib.navgpu_fleet_step_device(self.h, poses.data_ptr(), vels.data_ptr(), out.data_ptr()))
+        self.api.check(call(self.h, poses.data_ptr(), vels.data_ptr(), out.data_ptr()))
         torch.cuda.current_stream(dev).wait_stream(fleet_stream)
-        words = C.sizeof(DwaResult) // 8
-        f64 = out.view(torch.float64).view(self.n, words)
-        i32 = out.view(torch.int32).view(self.n, 2 * words)
-        return dict(cost=f64[:, 0], xv=f64[:, 1], yv=f64[:, 2], thetav=f64[:, 3], best_index=i32[:, 8],
-                    n_samples=i32[:, 9], n_scored=i32[:, 10], records=out)
+        words = C.sizeof(record) // 8
+        return dict(f64=out.view(torch.float64).view(self.n, words), i32=out.view(torch.int32).view(self.n, 2 * words),
+                    records=out)
 
     def set_active(self, mask):
         """Which robots the following steps plan for (navgpu_fleet_set_active): n_robots booleans or 0 / 1 values, or
@@ -984,7 +1001,8 @@ class Fleet:
         return out
 
     def tp_timing(self):
-        """TrajectoryPlanner fleets: device ms of the last step's footprint-cell, wavefront and scoring launches."""
+        """TrajectoryPlanner fleets: device ms of the last host step's (step()) footprint-cell, wavefront and scoring
+        launches; step_tp_device does not time them."""
         a, b, c = C.c_float(), C.c_float(), C.c_float()
         self.api.check(self.lib.navgpu_fleet_tp_last_timing(self.h, C.byref(a), C.byref(b), C.byref(c)))
         return float(a.value), float(b.value), float(c.value)

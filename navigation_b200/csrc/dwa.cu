@@ -937,6 +937,7 @@ static void fleet_tp_free(FleetTp* t);
 static int fleet_tp_set_plans(navgpu_fleet* f, const double* plan_xy, const int32_t* plan_offsets);
 static int fleet_tp_check(navgpu_fleet* f, const double* poses, const double* vels, const int32_t* offsets,
                           const double* vel_samples, double* costs_out);
+static int fleet_tp_state_download(navgpu_fleet* f);
 
 struct navgpu_fleet {
   int device = 0;
@@ -1118,6 +1119,7 @@ static int fleet_state_to_host(navgpu_fleet* f) {
   if (!f->state_on_device) return NAVGPU_OK;
   NAVGPU_CUDA(cudaSetDevice(f->device));
   NAVGPU_CUDA(cudaMemcpyAsync(f->h_state, f->d_state, sizeof(FleetDwaState) * f->n, cudaMemcpyDeviceToHost, f->stream));
+  if (f->tp) NAVGPU_TRY(fleet_tp_state_download(f));  // the robots' TrajectoryPlanner state
   NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
   f->state_on_device = false;
   if (f->sensing) {  // the device rolled the origins
@@ -1405,7 +1407,7 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
 int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double* vels, navgpu_dwa_result* results) {
   // every check before anything changes: a refused call leaves the fleet as it was
   if (!f || !poses || !vels || !results) return fail(NAVGPU_ERR_INVALID, "bad arguments");
-  if (f->tp) return fail(NAVGPU_ERR_UNSUPPORTED, "a TrajectoryPlanner fleet steps on the host (navgpu_fleet_step_tp)");
+  if (f->tp) return fail(NAVGPU_ERR_UNSUPPORTED, "a TrajectoryPlanner fleet steps with navgpu_fleet_step_tp or navgpu_fleet_step_tp_device");
   const navgpu_dwa_config& c = f->cfg;
   if (!c.use_dwa) return fail(NAVGPU_ERR_UNSUPPORTED, "use_dwa = 0: its velocity window takes glibc's hypot, which the device does not reproduce");
   if (!on_device(poses, f->device) || !on_device(vels, f->device) || !on_device(results, f->device))

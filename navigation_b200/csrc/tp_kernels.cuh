@@ -11,6 +11,7 @@
 #pragma once
 
 #include "dwa_kernels.cuh"
+#include "glibc_hypot.cuh"
 
 namespace navgpu {
 
@@ -399,6 +400,227 @@ inline long long tp_footprint_capacity(const double* fpx, const double* fpy, int
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// createTrajectories' scalar side (trajectory_planner.cpp:537-905): the velocity samples in their order, and the
+// sequential selection among the scored ones with the state it keeps across cycles.  One implementation for the planner
+// handle and host fleet steps (on the host) and device fleet steps (k_tp_fleet_prepare, k_tp_fleet_select): IEEE
+// operations without a libm call but fmod (exact) and hypot, compiled with -fmad=false on both sides.  hypot is the
+// host libm's on the host and glibc_hypot on the device, which gives glibc 2.35+'s bits; device fleet steps run only
+// where the running libm agrees with it (glibc_hypot_matches_libm).
+__host__ __device__ inline double tp_hypot(double x, double y) {
+#ifdef __CUDA_ARCH__
+  return glibc_hypot(x, y);
+#else
+  return hypot(x, y);
+#endif
+}
+
+// angles::shortest_angular_distance (ros/angles, angles.h): normalize_angle(to - from)
+__host__ __device__ inline double tp_shortest_angular_distance(double from, double to) {
+  double a = fmod(fmod(to - from, 2.0 * M_PI) + 2.0 * M_PI, 2.0 * M_PI);
+  if (a > M_PI) a -= 2.0 * M_PI;
+  return a;
+}
+
+// TrajectoryPlanner's state across cycles (trajectory_planner.h:283-305): one per planner handle, one per fleet robot
+struct TpState {
+  bool stuck_left = false, stuck_right = false, stuck_left_strafe = false, stuck_right_strafe = false;
+  bool rotating_left = false, rotating_right = false, strafe_left = false, strafe_right = false;
+  bool escaping = false, final_goal_valid = false;
+  double prev_x = 0, prev_y = 0, escape_x = 0, escape_y = 0, escape_theta = 0, final_goal_x = 0, final_goal_y = 0;
+};
+
+// The most samples createTrajectories gives one robot of configuration c: vx_samples x vtheta_samples forward ones and
+// two diagonal ones (holonomic), vtheta_samples in-place rotations, n_y_vels strafing ones (holonomic) and backing up
+__host__ __device__ inline long long tp_max_samples(const navgpu_tp_config& c) {
+  const long long vx = c.vx_samples <= 0 ? 1 : c.vx_samples, vth = c.vtheta_samples <= 0 ? 1 : c.vtheta_samples;
+  const long long holonomic = c.holonomic_robot ? 1 : 0;
+  return vx * vth + 2 * holonomic + vth + c.n_y_vels * holonomic + 1;
+}
+
+// Where createTrajectories' groups of samples are among the n samples of one enumeration (n x 3 doubles, in the
+// caller's storage of tp_max_samples entries)
+struct TpSamples {
+  int n;
+  int a_begin, a_end;  // forward samples (absent while escaping)
+  int b_begin, n_b;    // in-place rotations
+  int c_begin, n_c;    // strafing (holonomic)
+  int d_index;         // backing up
+  double dvtheta;
+  double b_vtheta0;    // the first rotation's un-clamped vtheta_samp; the others follow by += dvtheta, as enumerated
+};
+
+// the samples of TrajectoryPlanner::createTrajectories (:537-905) with its own fp64 accumulations, into v and s
+__host__ __device__ inline void tp_enumerate(const navgpu_tp_config& c, const TpState& st, double x, double y, double vx,
+                                             double vtheta, double* v, TpSamples& s) {
+  const int vx_samples = c.vx_samples <= 0 ? 1 : c.vx_samples, vth_samples = c.vtheta_samples <= 0 ? 1 : c.vtheta_samples;
+  double max_vel_x = c.max_vel_x, max_vel_theta, min_vel_x, min_vel_theta;
+  if (st.final_goal_valid) {
+    const double final_goal_dist = tp_hypot(st.final_goal_x - x, st.final_goal_y - y);
+    max_vel_x = dwa_min(max_vel_x, final_goal_dist / c.sim_time);
+  }
+  const double horizon = c.dwa ? c.sim_period : c.sim_time;
+  max_vel_x = dwa_max(dwa_min(max_vel_x, vx + c.acc_lim_x * horizon), c.min_vel_x);
+  min_vel_x = dwa_max(c.min_vel_x, vx - c.acc_lim_x * horizon);
+  max_vel_theta = dwa_min(c.max_vel_th, vtheta + c.acc_lim_theta * horizon);
+  min_vel_theta = dwa_max(c.min_vel_th, vtheta - c.acc_lim_theta * horizon);
+  const double dvx = (max_vel_x - min_vel_x) / (vx_samples - 1);
+  const double dvtheta = (max_vel_theta - min_vel_theta) / (vth_samples - 1);
+  int n = 0;
+  auto push = [&](double a, double b, double t) {
+    v[3 * n] = a;
+    v[3 * n + 1] = b;
+    v[3 * n + 2] = t;
+    ++n;
+  };
+  s.n_c = 0;
+  s.dvtheta = dvtheta;
+  double vx_samp = min_vel_x, vtheta_samp;
+  s.a_begin = 0;
+  if (!st.escaping) {
+    for (int i = 0; i < vx_samples; ++i) {
+      push(vx_samp, 0.0, 0.0);  // the straight trajectory first
+      vtheta_samp = min_vel_theta;
+      for (int j = 0; j < vth_samples - 1; ++j) {
+        push(vx_samp, 0.0, vtheta_samp);
+        vtheta_samp += dvtheta;
+      }
+      vx_samp += dvx;
+    }
+    if (c.holonomic_robot) {
+      push(0.1, 0.1, 0.0);
+      push(0.1, -0.1, 0.0);
+    }
+  }
+  s.a_end = n;
+  s.b_begin = n;
+  s.n_b = vth_samples;
+  s.b_vtheta0 = min_vel_theta;
+  vtheta_samp = min_vel_theta;
+  for (int i = 0; i < vth_samples; ++i) {
+    const double limited = vtheta_samp > 0 ? dwa_max(vtheta_samp, c.min_in_place_vel_th)
+                                           : dwa_min(vtheta_samp, -1.0 * c.min_in_place_vel_th);
+    push(0.0, 0.0, limited);
+    vtheta_samp += dvtheta;
+  }
+  s.c_begin = n;
+  if (c.holonomic_robot) {
+    s.n_c = c.n_y_vels;
+    for (int i = 0; i < c.n_y_vels; ++i) push(0.0, c.y_vels[i], 0.0);
+  }
+  s.d_index = n;
+  push(c.backup_vel, 0.0, 0.0);
+  s.n = n;
+}
+
+// The selection of createTrajectories (:575-905) on the scored samples r of the enumeration (s, v), in their order,
+// with the state st it reads and updates; fills result (n_points: the chosen trajectory's, at most points_stride) and
+// returns the chosen sample.  The planner handle and every fleet robot, on the host or the device, go through it.
+__host__ __device__ inline int tp_select(const navgpu_tp_config& c, const TpSamples& s, const double* v,
+                                         const TpSampleResult* r, TpState& st, double x, double y, double theta,
+                                         int points_stride, navgpu_tp_result* result) {
+  int best = -1;
+  double best_cost = -1.0;
+  auto best_xv = [&]() { return best < 0 ? 0.0 : v[3 * best]; };
+  auto best_yv = [&]() { return best < 0 ? 0.0 : v[3 * best + 1]; };
+  auto best_thv = [&]() { return best < 0 ? 0.0 : v[3 * best + 2]; };
+  auto take = [&](int k) { best = k; best_cost = r[k].cost; };
+  for (int k = s.a_begin; k < s.a_end; ++k)
+    if (r[k].cost >= 0 && (r[k].cost < best_cost || best_cost < 0)) take(k);
+  double heading_dist = 1.7976931348623157e308;  // DBL_MAX
+  double vtheta_samp = s.b_vtheta0;
+  for (int i = 0; i < s.n_b; ++i) {  // rotating in place, towards open space (:650-697)
+    const int k = s.b_begin + i;
+    if (r[k].cost >= 0 && (r[k].cost <= best_cost || best_cost < 0 || best_yv() != 0.0) &&
+        (vtheta_samp > s.dvtheta || vtheta_samp < -1 * s.dvtheta)) {
+      if (r[k].ahead_gdist >= 0) {
+        const double ahead_gdist = r[k].ahead_gdist;
+        if (ahead_gdist < heading_dist) {
+          if (vtheta_samp < 0 && !st.stuck_left) { take(k); heading_dist = ahead_gdist; }
+          else if (vtheta_samp > 0 && !st.stuck_right) { take(k); heading_dist = ahead_gdist; }
+        }
+      }
+    }
+    vtheta_samp += s.dvtheta;
+  }
+  auto reset_oscillation_if_moved = [&]() {  // (:731-741)
+    if (tp_hypot(x - st.prev_x, y - st.prev_y) > c.oscillation_reset_dist) {
+      st.rotating_left = st.rotating_right = st.strafe_left = st.strafe_right = false;
+      st.stuck_left = st.stuck_right = st.stuck_left_strafe = st.stuck_right_strafe = false;
+    }
+  };
+  auto leave_escape_if_moved = [&]() {  // (:743-747)
+    if (tp_hypot(x - st.escape_x, y - st.escape_y) > c.escape_reset_dist ||
+        fabs(tp_shortest_angular_distance(st.escape_theta, theta)) > c.escape_reset_theta)
+      st.escaping = false;
+  };
+  bool decided = false;
+  if (best_cost >= 0) {  // (:700-749)
+    if (!(best_xv() > 0)) {
+      if (best_thv() < 0) { if (st.rotating_right) st.stuck_right = true; st.rotating_right = true; }
+      else if (best_thv() > 0) { if (st.rotating_left) st.stuck_left = true; st.rotating_left = true; }
+      else if (best_yv() > 0) { if (st.strafe_right) st.stuck_right_strafe = true; st.strafe_right = true; }
+      else if (best_yv() < 0) { if (st.strafe_left) st.stuck_left_strafe = true; st.strafe_left = true; }
+      st.prev_x = x;
+      st.prev_y = y;
+    }
+    reset_oscillation_if_moved();
+    leave_escape_if_moved();
+    decided = true;
+  }
+  if (!decided && c.holonomic_robot) {  // strafing (:752-797)
+    for (int i = 0; i < s.n_c; ++i) {
+      const int k = s.c_begin + i;
+      const double vy_samp = v[3 * k + 1];
+      if (r[k].cost >= 0 && (r[k].cost <= best_cost || best_cost < 0)) {
+        if (r[k].ahead_gdist >= 0) {
+          const double ahead_gdist = r[k].ahead_gdist;
+          if (ahead_gdist < heading_dist) {
+            if (vy_samp > 0 && !st.stuck_left_strafe) { take(k); heading_dist = ahead_gdist; }
+            else if (vy_samp < 0 && !st.stuck_right_strafe) { take(k); heading_dist = ahead_gdist; }
+          }
+        }
+      }
+    }
+  }
+  if (!decided && best_cost >= 0) {  // (:800-848; note the flags it sets differ from the block above)
+    if (!(best_xv() > 0)) {
+      if (best_thv() < 0) { if (st.rotating_right) st.stuck_right = true; st.rotating_left = true; }
+      else if (best_thv() > 0) { if (st.rotating_left) st.stuck_left = true; st.rotating_right = true; }
+      else if (best_yv() > 0) { if (st.strafe_right) st.stuck_right_strafe = true; st.strafe_left = true; }
+      else if (best_yv() < 0) { if (st.strafe_left) st.stuck_left_strafe = true; st.strafe_right = true; }
+      st.prev_x = x;
+      st.prev_y = y;
+    }
+    reset_oscillation_if_moved();
+    leave_escape_if_moved();
+    decided = true;
+  }
+  if (!decided) {  // back up slowly, whatever the map says (:851-903)
+    take(s.d_index);
+    reset_oscillation_if_moved();
+    if (!st.escaping && best_cost > -2.0) {
+      st.escape_x = x;
+      st.escape_y = y;
+      st.escape_theta = theta;
+      st.escaping = true;
+    }
+    leave_escape_if_moved();
+    if (best_cost == -1.0) best_cost = 1.0;
+  }
+
+  result->cost = best_cost;
+  result->xv = best_xv();
+  result->yv = best_yv();
+  result->thetav = best_thv();
+  // (the device keeps points_stride points per sample)
+  result->n_points = r[best].n_points < points_stride ? r[best].n_points : points_stride;
+  result->flags = (st.stuck_left ? 1 : 0) | (st.stuck_right ? 2 : 0) | (st.stuck_left_strafe ? 4 : 0) |
+                  (st.stuck_right_strafe ? 8 : 0) | (st.rotating_left ? 16 : 0) | (st.rotating_right ? 32 : 0) |
+                  (st.strafe_left ? 64 : 0) | (st.strafe_right ? 128 : 0) | (st.escaping ? 256 : 0);
+  return best;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // Fleets of legacy TrajectoryPlanners (navgpu_fleet_use_trajectory_planner): what changes per robot and step
 struct TpFleetRobot {
   double x, y, theta, vx, vy, vtheta;  // through (float), as navgpu_tp_find_best_path rounds them
@@ -484,6 +706,85 @@ __global__ void __launch_bounds__(kDwaWarpsPerBlock * 32) k_tp_fleet_score(TpSco
   const int sample = local * kDwaWarpsPerBlock + warp;
   if (sample >= n) return;
   tp_score_sample(s_a, sample, lane, scratch[warp]);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// The device fleet step of TrajectoryPlanner fleets (navgpu_fleet_step_tp_device): what navgpu_fleet_step_tp does per
+// robot on the host, one thread per robot, with the host step's own functions (fleet_roll_step, tp_enumerate,
+// tp_select).  Every robot's samples and their scores sit in a slot of tp_max_samples entries at robot * slot.
+struct TpFleetPrepareArgs {
+  const double* poses;  // [n][3], device memory
+  const double* vels;
+  FleetRobot* grids;    // the MapGrid records: a sensing fleet's rolled origin
+  TpFleetRobot* robots;
+  TpSamples* sets;      // per robot: its enumeration
+  double* samples;      // robot r's at 3 * r * slot
+  const TpState* st;
+  FleetDwaState* state; // a sensing fleet's origin
+  const uint8_t* flags; // kFleetActive
+  FleetCmStep* steps;   // sensing fleets: the costmap update's step records; null on raw-map fleets
+  navgpu_tp_config cfg;
+  int slot, n, nfp;
+  unsigned sx, sy;
+  double res;
+};
+
+// Before the costmap update: a sensing fleet's roll of every robot (fleet_costmap_roll), whose origin also goes into the
+// robot's MapGrid and scoring records; then, for robots the steps plan, the scoring record's per-step fields and the
+// samples of createTrajectories (navgpu_fleet_step_tp's per-robot loop).  The heading's cos / sin for the footprint
+// cells come from CUDA's sincos.  A left-out robot gets no samples: no footprint cells, its scoring CTAs exit at once.
+__global__ void __launch_bounds__(kFleetRobotThreads) k_tp_fleet_prepare(TpFleetPrepareArgs a) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= a.n) return;
+  const double pose[3] = {a.poses[3 * r], a.poses[3 * r + 1], a.poses[3 * r + 2]};
+  TpFleetRobot& R = a.robots[r];
+  if (a.steps) {
+    FleetDwaState& S = a.state[r];
+    const FleetCmStep st = fleet_roll_step(pose, S.origin[0], S.origin[1], a.sx, a.sy, a.res);
+    a.steps[r] = st;
+    S.origin[0] = st.ox;
+    S.origin[1] = st.oy;
+    a.grids[r].grids.g.ox = st.ox;
+    a.grids[r].grids.g.oy = st.oy;
+    R.ox = st.ox;
+    R.oy = st.oy;
+  }
+  R.sample_offset = r * a.slot;
+  if (!(a.flags[r] & kFleetActive)) {
+    R.n_samples = 0;
+    return;
+  }
+  // Eigen::Vector3f pos / vel (:911-912)
+  R.x = (float)pose[0]; R.y = (float)pose[1]; R.theta = (float)pose[2];
+  R.vx = (float)a.vels[3 * r]; R.vy = (float)a.vels[3 * r + 1]; R.vtheta = (float)a.vels[3 * r + 2];
+  double s = 0.0, c = 0.0;
+  if (a.nfp > 1) sincos(R.theta, &s, &c);
+  R.cos_th = c;
+  R.sin_th = s;
+  TpSamples set;
+  tp_enumerate(a.cfg, a.st[r], R.x, R.y, R.vx, R.vtheta, a.samples + 3 * (size_t)r * a.slot, set);
+  a.sets[r] = set;
+  R.n_samples = set.n;
+}
+
+// After k_tp_fleet_score: the selection of every planned robot on its scored slot (tp_select), its state, and its
+// result record written to the caller's device buffer; left-out robots' records and state stay as they are
+__global__ void __launch_bounds__(kFleetRobotThreads) k_tp_fleet_select(navgpu_tp_config cfg, const TpFleetRobot* robots,
+                                                                        const TpSamples* sets, const double* samples,
+                                                                        const TpSampleResult* scored, TpState* st,
+                                                                        FleetDwaState* state, const uint8_t* flags,
+                                                                        navgpu_tp_result* results, int slot,
+                                                                        int points_stride, int n) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n || !(flags[r] & kFleetActive)) return;
+  const TpFleetRobot& R = robots[r];
+  TpState S = st[r];
+  navgpu_tp_result out;
+  tp_select(cfg, sets[r], samples + 3 * (size_t)r * slot, scored + (size_t)r * slot, S, R.x, R.y, R.theta, points_stride,
+            &out);
+  st[r] = S;
+  state[r].planned = 1;
+  results[r] = out;
 }
 
 }  // namespace navgpu
