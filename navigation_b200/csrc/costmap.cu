@@ -555,6 +555,11 @@ int footprint_polygon(navgpu_costmap* h, const Layer& L, PolyArgs& pa, int* mode
 // One LayeredCostmap::updateMap cycle (layered_costmap.cpp:79-150), enqueued on the handle's stream.
 int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
   NAVGPU_TRY(use_device(h));
+  // The inflation tables first: a radius the sweeps cannot run is refused before the cycle changes anything, so the
+  // handle stays as it was -- grid layer updates and reinflation requests still pending, layer grids and the host
+  // mirror's bookkeeping untouched -- and the next accepted configuration picks up where it left off.
+  for (Layer& L : h->layers)
+    if (L.kind == 2 && L.enabled) NAVGPU_TRY(upload_tables(h, L));
   // rolling window: master origin follows the robot (:86-91)
   if (h->rolling)
     NAVGPU_TRY(roll_grid(h, h->master, h->cur, h->ox, h->oy, h->def, rx - h->size_m_x() / 2, ry - h->size_m_y() / 2));
@@ -783,8 +788,7 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
       ++ml.n;
       pending = true;
     } else {
-      if (!L.enabled) continue;
-      NAVGPU_TRY(upload_tables(h, L));
+      if (!L.enabled) continue;  // (its tables were uploaded at the start of the cycle)
       if (L.tables.R == 0) continue;  // the reference dereferences NULL tables here; we make it a no-op
       if (!do_reset && ml.n > 0) {    // merges that read what a previous inflation wrote: keep them a separate pass
         NAVGPU_TRY(launch_update(h, ml, 0, 0, nullptr));

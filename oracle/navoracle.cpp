@@ -617,6 +617,9 @@ struct InflationLayer : LayerBase {  // inflation_layer.cpp
 
   void update_costs(Costmap& cm, int min_i, int min_j, int max_i, int max_j) override {  // :172-266
     if (!enabled) return;
+    // R == 0: compute_caches left the tables empty, and the reference would index them (undefined behaviour); an
+    // inflation radius below one cell inflates nothing instead, as the CUDA library does
+    if (R == 0) return;
     Grid& m = cm.master;
     unsigned size_x = m.sx, size_y = m.sy;
     if (seen.size() != size_t(size_x) * size_y) seen.resize(size_t(size_x) * size_y);
@@ -782,6 +785,7 @@ struct InflationLayer : LayerBase {  // inflation_layer.cpp
       return;
     }
     for (unsigned index : popped) write_cell(m, index, costs[0]);
+    last_rounds = 1;  // the seeds pop in the first round (distance 0), as the CUDA library counts rounds
     struct Best { double d; int32_t src; };
     auto best_entry = [&](unsigned idx) {
       int x = idx % size_x, y = idx / size_x;
@@ -1757,7 +1761,13 @@ void navo_grid_layer_touch(void* h, int layer, uint32_t x, uint32_t y, uint32_t 
   g->x = x; g->y = y; g->w = w; g->h = hgt;
   g->updated = true;
 }
-void navo_layer_set_enabled(void* h, int layer, int enabled) { static_cast<Costmap*>(h)->layers[layer]->enabled = enabled != 0; }
+void navo_layer_set_enabled(void* h, int layer, int enabled) {
+  LayerBase* l = static_cast<Costmap*>(h)->layers[layer].get();
+  // InflationLayer::reconfigureCB (inflation_layer.cpp:104-107): switching the layer on or off reinflates the whole map
+  if (InflationLayer* il = dynamic_cast<InflationLayer*>(l))
+    if (il->enabled != (enabled != 0)) il->need_reinflation = true;
+  l->enabled = enabled != 0;
+}
 void navo_obstacle_set_observations(void* h, int layer, const navo_observation* obs, int n_obs) {
   ObstacleLayer* ol = static_cast<ObstacleLayer*>(static_cast<Costmap*>(h)->layers[layer].get());
   ol->obs.clear();

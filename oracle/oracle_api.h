@@ -77,7 +77,8 @@ void navo_inflation_set_params(void* h, int layer, double inflation_radius, doub
  * variant 5 bit for bit.  Cells that differ between variants 0-3 form the
  * "tie-variant mask" of a scenario.  Returns 0, or -1 when the library cannot run the variant (libnavref.so: only 0). */
 int navo_inflation_set_variant(void* h, int layer, int variant, uint64_t seed);
-/* rounds (distinct pop levels, incl. repeats after a shorter entry appears) of variant 5's last updateCosts */
+/* rounds (distinct pop levels -- the seeds' level 0 included -- and repeats after a shorter entry appears) of
+ * variant 5's last updateCosts: what navgpu_inflation_last_rounds reports for mode 1 */
 int navo_inflation_last_rounds(void* h, int layer);
 /* LayeredCostmap::updateMap; window_out = {x0, xn, y0, yn} (bx0_, bxn_, by0_, byn_) */
 void navo_costmap_update_map(void* h, double robot_x, double robot_y, double robot_yaw, int32_t window_out[4]);

@@ -23,6 +23,7 @@ pytestmark = pytest.mark.gpu
 RTOL = 1e-5
 RES = 0.05
 CFG = dict(vx_samples=6, vy_samples=1, vth_samples=11, max_vel_y=0.0, min_vel_y=0.0)
+CELL_RADII = {1.575: 32, 2.975: 60, 12.675: 254}  # inflation radius -> the cell radius it was chosen for
 
 
 def single_costmap(api, sx, sy, track_unknown=False, combination_method=1, footprint_clearing=True,
@@ -64,9 +65,17 @@ def edge_scans(robots, i, cycle):
     ((120, 120), dict(combination_method=0)),
     ((120, 120), dict(footprint_clearing=False, track_unknown=True)),
     ((97, 131), dict(combination_method=0)),
+    # cell radii of 32, 60 and 254 (radius (R - 0.5) x resolution): the horizontal seed search reads a second 32-cell
+    # word, and more
+    ((120, 120), dict(inflation_radius=1.575, cost_scaling_factor=1.0)),
+    ((120, 120), dict(inflation_radius=2.975, cost_scaling_factor=3.0, track_unknown=True)),
+    ((120, 120), dict(inflation_radius=12.675, cost_scaling_factor=0.0)),
 ])
 def test_fleet_matches_single_costmaps(cuda, size, opts):
     sx, sy = size
+    radius = opts.get("inflation_radius", 0.55)
+    R = cuda.build_cost_table(RES, 0.0, radius, 1.0)[0]
+    assert R == CELL_RADII.get(radius, R), f"cell radius {R}"
     n, cycles = 6, 6
     robots = [synth.fleet_sensing_robot(40 + i, n=max(sx, sy)) for i in range(n)]
     fleet = cuda.fleet_sensing(n, sx, sy, RES, sc.PENTAGON, **opts, **CFG)
@@ -95,10 +104,10 @@ def test_fleet_matches_single_costmaps(cuda, size, opts):
         assert (fleet.layer(0) == 255).any() and np.isin(fleet.layer(0), [0, 255]).all()
 
 
-def checker_robot(port, sx, sy):
+def checker_robot(port, sx, sy, inflation_radius=0.55, cost_scaling_factor=10.0):
     cm = port.costmap(sx, sy, RES, 0.0, 0.0, rolling=True)
     o = cm.add_obstacle_layer(1, True, 2.0)
-    il = cm.add_inflation_layer(0.55, 10.0)
+    il = cm.add_inflation_layer(inflation_radius, cost_scaling_factor)
     sc.select_inflation(cm, il, "exact")
     cm.set_footprint(sc.PENTAGON)
     return cm, o
@@ -132,11 +141,17 @@ def assert_result(g, e, fleet, d, where):
 
 
 def test_fleet_matches_checker_robot_by_robot(cuda, port):
+    # the defaults, and a cell radius of 60 (2.975 m at 0.05 m)
+    for infl in (dict(), dict(inflation_radius=2.975, cost_scaling_factor=3.0)):
+        fleet_matches_checker(cuda, port, **infl)
+
+
+def fleet_matches_checker(cuda, port, **infl):
     sx = sy = 120
     n, cycles = 8, 5
     robots = [synth.fleet_sensing_robot(200 + i) for i in range(n)]
-    fleet = cuda.fleet_sensing(n, sx, sy, RES, sc.PENTAGON, **CFG)
-    refs = [checker_robot(port, sx, sy) for _ in range(n)]
+    fleet = cuda.fleet_sensing(n, sx, sy, RES, sc.PENTAGON, **infl, **CFG)
+    refs = [checker_robot(port, sx, sy, **infl) for _ in range(n)]
     dwas = [port.dwa(sx, sy, RES, **CFG) for _ in range(n)]
     vels = np.array([r["vel"] for r in robots])
     valid = exact = 0

@@ -55,7 +55,8 @@ def edge_sources(robots, i, cycle):
     ((120, 120), dict(combination_method=0), dict(origin_z=-0.1, z_voxels=4)),
     ((120, 120), dict(footprint_clearing=False), dict()),
     ((97, 131), dict(), dict()),
-], ids=["defaults", "track_unknown", "overwrite_low_column", "no_footprint_clearing", "97x131"])
+    ((120, 120), dict(inflation_radius=2.975, cost_scaling_factor=3.0), dict()),  # a cell radius of 60
+], ids=["defaults", "track_unknown", "overwrite_low_column", "no_footprint_clearing", "97x131", "R60"])
 def test_voxel_fleet_matches_single_costmaps(cuda, size, opts, voxel):
     sx, sy = size
     n, cycles = 6, 6

@@ -2,8 +2,12 @@
 word.  These cases put the map edges, the update window's edges and NO_INFORMATION cells where that shape can get them
 wrong: widths of 4k + 1, 4k + 2 and 4k + 3 cells, so that the last word of a row holds 1-3 cells of the map and the
 rest is row padding; maps narrower or shorter than one tile; window edges inside a tile; NO_INFORMATION next to LETHAL
-in the last columns; and effective reaches that select each of the three instantiations (R <= 12, 20, 31).  The device
-grid must equal the checker's exact nearest-seed variant cell for cell."""
+in the last columns; and effective reaches that select each of the three instantiations (reach <= 12, 20, 31).
+
+launch_sweep picks the instantiation by the effective reach -- the largest distance whose cost is non-zero -- not by
+the cell radius R: with a steep cost scaling the reach is well below R, and k_merge_seed's seed region (R) is wider
+than k_inflate's halo rows (the reach).  The device grid must equal the checker's exact nearest-seed variant cell for
+cell."""
 import numpy as np
 import pytest
 
@@ -12,9 +16,11 @@ import scenarios as sc
 pytestmark = pytest.mark.gpu
 
 RES = 0.05
-# (inflation radius in m, cost scaling): cost 0 is only reached at the radius, so the effective reach is the radius
-# in cells: 11, 19 and 30 -- k_inflate<12>, <20> and <31>
-RADII = [(0.55, 1.0), (0.95, 1.0), (1.5, 1.0)]
+# (inflation radius in m, cost scaling) -> (cell radius R, effective reach).  With scaling 1.0 the cost stays non-zero
+# out to the radius, so the reach is R: k_inflate<12>, <20> and <31>.  Then a reach well below R (12 of 31: <12>;
+# 17 of 25: <20>), the smallest reach that takes <31> (21), and scaling 0 (cost 252 out to R = 31).
+RADII = {(0.55, 1.0): (11, 11), (0.95, 1.0): (19, 19), (1.5, 1.0): (30, 30), (1.525, 20.0): (31, 12),
+         (1.225, 10.0): (25, 17), (1.025, 1.0): (21, 21), (1.525, 0.0): (31, 31)}
 # widths 4k + 1 / 4k + 2 / 4k + 3, narrower than one tile and spanning several; heights not multiples of 64
 SHAPES = [(37, 45), (102, 130), (127, 63), (257, 200), (262, 71), (391, 133)]
 
@@ -49,7 +55,7 @@ def marks(sx, sy, seed):
                  raytrace_range=100.0, marking=True, clearing=False)]
 
 
-@pytest.mark.parametrize("radius,scaling", RADII)
+@pytest.mark.parametrize("radius,scaling", list(RADII))
 @pytest.mark.parametrize("sx,sy", SHAPES)
 def test_tile_edges_exact(cuda, port, sx, sy, radius, scaling):
     static = edge_world(sx, sy, sx * 1000 + sy)
@@ -62,6 +68,11 @@ def test_tile_edges_exact(cuda, port, sx, sy, radius, scaling):
         cm.set_footprint(sc.square_footprint())
         cm.set_grid_layer(s, static)
         sc.select_inflation(cm, il, "exact", 0)
+        R, costs, _ = cm.inflation_tables(il)
+        n = np.arange(R + 2)
+        d2 = n[:, None] ** 2 + n[None, :] ** 2
+        reach = int(np.sqrt(d2[(d2 <= R * R) & (costs > 0)].max() + 0.5))
+        assert (R, reach) == RADII[(radius, scaling)], f"{api.name}: (R, reach) = {(R, reach)}"
         trace = [(cm.update_map(), cm.get())]
         # second cycle: only the marks changed, so the window is their bounds grown by the radius
         cm.set_observations(o, marks(sx, sy, sx + sy))
