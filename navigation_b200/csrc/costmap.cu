@@ -160,7 +160,9 @@ struct Layer {
   // points were seen on the host (navgpu_obstacle_set_observations)
   bool touch_box_valid = false;
   double tbx0 = 0, tby0 = 0, tbx1 = 0, tby1 = 0;
-  std::vector<Pt> transformed_footprint;
+  // this cycle's footprint polygon (footprint_polygon, evaluated before the cycle changes anything) and its mode
+  PolyArgs poly{};
+  int poly_mode = 0;
   // voxel layer (an obstacle layer with columns of 16 voxels, plugins/voxel_layer.cpp)
   bool voxel = false;
   VoxelGeom vg{0.0, 0.2, 10u, 21u, 0u};
@@ -193,6 +195,7 @@ struct navgpu_costmap {
   int cur = 0;
   std::vector<Layer> layers;
   std::vector<Pt> footprint;
+  std::vector<Pt> transformed_footprint;  // this cycle's footprint at the robot's pose (enqueue_update)
   double inscribed = 0, circumscribed = 0;
   DevBox* d_boxes = nullptr;
   InflationBoundsState* d_infl = nullptr;
@@ -263,19 +266,33 @@ int alloc_grid(navgpu_costmap* h, uint8_t** p, uint8_t value) {
   return NAVGPU_OK;
 }
 
-// host mirror of Costmap2D::updateOrigin's scalar part (costmap_2d.cpp:264-275, 301-302); the cell shift runs on the
-// device (k_shift_grid) into the other buffer of the ping-pong pair.
+// Costmap2D::updateOrigin's scalar part (costmap_2d.cpp:264-275, 301-302): the shift in cells and the new origin of
+// a grid at (gox, goy) asked to move to (new_ox, new_oy)
+struct RolledOrigin {
+  int cell_ox, cell_oy;
+  double ox, oy;
+};
+RolledOrigin rolled_origin(const navgpu_costmap* h, double gox, double goy, double new_ox, double new_oy) {
+  RolledOrigin r;
+  r.cell_ox = int((new_ox - gox) / h->res);
+  r.cell_oy = int((new_oy - goy) / h->res);
+  r.ox = gox + r.cell_ox * h->res;
+  r.oy = goy + r.cell_oy * h->res;
+  return r;
+}
+
+// host mirror of Costmap2D::updateOrigin (rolled_origin); the cell shift runs on the device (k_shift_grid) into the
+// other buffer of the ping-pong pair.
 int roll_grid(navgpu_costmap* h, uint8_t* grid[2], int& cur, double& gox, double& goy, uint8_t def, double new_ox,
               double new_oy) {
-  int cell_ox = int((new_ox - gox) / h->res), cell_oy = int((new_oy - goy) / h->res);
-  double new_grid_ox = gox + cell_ox * h->res, new_grid_oy = goy + cell_oy * h->res;
+  const RolledOrigin r = rolled_origin(h, gox, goy, new_ox, new_oy);
   if (!grid[cur ^ 1]) NAVGPU_CUDA(cudaMalloc(&grid[cur ^ 1], h->bytes()));
   dim3 block(256), g((h->pitch + 255) / 256, h->sy);
-  k_shift_grid<<<g, block, 0, h->stream>>>(grid[cur], grid[cur ^ 1], h->sx, h->sy, h->pitch, cell_ox, cell_oy, def);
+  k_shift_grid<<<g, block, 0, h->stream>>>(grid[cur], grid[cur ^ 1], h->sx, h->sy, h->pitch, r.cell_ox, r.cell_oy, def);
   NAVGPU_LAUNCHED(1);
   cur ^= 1;
-  gox = new_grid_ox;
-  goy = new_grid_oy;
+  gox = r.ox;
+  goy = r.oy;
   return NAVGPU_OK;
 }
 
@@ -524,14 +541,16 @@ int launch_update(navgpu_costmap* h, const MergeLayers& ml, int do_reset, int R,
 }
 
 // Host part of ObstacleLayer::updateCosts' footprint clearing (obstacle_layer.cpp:432-435 -> setConvexPolygonCost,
-// costmap_2d.cpp:315-342): vertices to cells; *mode = 0 nothing to clear, 1 fits k_obstacle_update, 2 stand-alone kernel
-int footprint_polygon(navgpu_costmap* h, const Layer& L, PolyArgs& pa, int* mode) {
+// costmap_2d.cpp:315-342) for a layer grid whose origin is (ox, oy): vertices to cells; *mode = 0 nothing to clear,
+// 1 fits k_obstacle_update, 2 stand-alone kernel
+int footprint_polygon(const navgpu_costmap* h, const std::vector<Pt>& footprint, double ox, double oy, PolyArgs& pa,
+                      int* mode) {
   *mode = 0;
   pa.n = 0;
-  if (L.transformed_footprint.size() > 32) return fail(NAVGPU_ERR_UNSUPPORTED, "footprint with more than 32 vertices");
-  for (const Pt& p : L.transformed_footprint) {  // worldToMap, costmap_2d.cpp:208-220; any vertex off the map: no clearing
-    if (p.x < L.ox || p.y < L.oy) return NAVGPU_OK;
-    unsigned mx = (int)((p.x - L.ox) / h->res), my = (int)((p.y - L.oy) / h->res);
+  if (footprint.size() > 32) return fail(NAVGPU_ERR_UNSUPPORTED, "footprint with more than 32 vertices");
+  for (const Pt& p : footprint) {  // worldToMap, costmap_2d.cpp:208-220; any vertex off the map: no clearing
+    if (p.x < ox || p.y < oy) return NAVGPU_OK;
+    unsigned mx = (int)((p.x - ox) / h->res), my = (int)((p.y - oy) / h->res);
     if (!(mx < h->sx && my < h->sy)) return NAVGPU_OK;
     pa.vx[pa.n] = (int)mx;
     pa.vy[pa.n] = (int)my;
@@ -560,9 +579,30 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
   // mirror's bookkeeping untouched -- and the next accepted configuration picks up where it left off.
   for (Layer& L : h->layers)
     if (L.kind == 2 && L.enabled) NAVGPU_TRY(upload_tables(h, L));
+  // The footprint polygons likewise: one the device rasteriser cannot take (too many vertices, too many cells at this
+  // pose, a map too large) is refused before any grid rolls or any obstacle kernel consumes its observations.  Each
+  // layer's polygon is taken on the origin its grid will have once rolled.
+  std::vector<Pt>& footprint = h->transformed_footprint;  // updateFootprint (:415-425) with transformFootprint
+  footprint.clear();                                       // (footprint.cpp:106-120)
+  {
+    const double cos_th = cos(ryaw), sin_th = sin(ryaw);
+    for (const Pt& p : h->footprint)
+      footprint.push_back(Pt{rx + (p.x * cos_th - p.y * sin_th), ry + (p.x * sin_th + p.y * cos_th)});
+  }
+  const double new_ox = rx - h->size_m_x() / 2, new_oy = ry - h->size_m_y() / 2;  // rolling origin (:86-91)
+  for (Layer& L : h->layers) {
+    L.poly_mode = 0;
+    if (L.kind != 1 || !L.enabled || !L.footprint_clearing) continue;
+    double lox = L.ox, loy = L.oy;
+    if (h->rolling) {
+      const RolledOrigin r = rolled_origin(h, L.ox, L.oy, new_ox, new_oy);
+      lox = r.ox;
+      loy = r.oy;
+    }
+    NAVGPU_TRY(footprint_polygon(h, footprint, lox, loy, L.poly, &L.poly_mode));
+  }
   // rolling window: master origin follows the robot (:86-91)
-  if (h->rolling)
-    NAVGPU_TRY(roll_grid(h, h->master, h->cur, h->ox, h->oy, h->def, rx - h->size_m_x() / 2, ry - h->size_m_y() / 2));
+  if (h->rolling) NAVGPU_TRY(roll_grid(h, h->master, h->cur, h->ox, h->oy, h->def, new_ox, new_oy));
   if (h->layers.empty()) return NAVGPU_OK;
 
   // ---- updateBounds of every plugin, in order (:96-115): host-side scalars first
@@ -602,16 +642,15 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
     } else if (L.kind == 1) {  // ObstacleLayer::updateBounds (obstacle_layer.cpp:340-413)
       if (h->rolling) {
         if (L.voxel) {  // VoxelLayer::updateOrigin moves the columns with the 2-D cells (voxel_layer.cpp:371-438)
-          const double new_ox = rx - h->size_m_x() / 2, new_oy = ry - h->size_m_y() / 2;
-          const int cell_ox = int((new_ox - L.ox) / h->res), cell_oy = int((new_oy - L.oy) / h->res);
+          const RolledOrigin r = rolled_origin(h, L.ox, L.oy, new_ox, new_oy);
           if (!L.vox[L.cur ^ 1]) NAVGPU_CUDA(cudaMalloc(&L.vox[L.cur ^ 1], h->bytes() * sizeof(uint32_t)));
           dim3 block(256), g((h->pitch + 255) / 256, h->sy);
-          k_shift_voxels<<<g, block, 0, h->stream>>>(L.vox[L.cur], L.vox[L.cur ^ 1], h->sx, h->sy, h->pitch, cell_ox, cell_oy);
+          k_shift_voxels<<<g, block, 0, h->stream>>>(L.vox[L.cur], L.vox[L.cur ^ 1], h->sx, h->sy, h->pitch, r.cell_ox,
+                                                     r.cell_oy);
           NAVGPU_LAUNCHED(1);
         }
-        NAVGPU_TRY(roll_grid(h, L.grid, L.cur, L.ox, L.oy, L.def, rx - h->size_m_x() / 2, ry - h->size_m_y() / 2));
+        NAVGPU_TRY(roll_grid(h, L.grid, L.cur, L.ox, L.oy, L.def, new_ox, new_oy));
       }
-      L.transformed_footprint.clear();
       if (!L.enabled) continue;
       last_obstacle = (int)li;
       double bx0 = 1e300, by0 = 1e300, bx1 = -1e300, by1 = -1e300;
@@ -625,13 +664,12 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
         bx0 = std::min(o.ox, bx0); by0 = std::min(o.oy, by0);
         bx1 = std::max(o.ox, bx1); by1 = std::max(o.oy, by1);
       }
-      if (L.footprint_clearing) {  // updateFootprint (:415-425) with transformFootprint (footprint.cpp:106-120)
-        double cos_th = cos(ryaw), sin_th = sin(ryaw);
-        for (const Pt& p : h->footprint)
-          L.transformed_footprint.push_back(Pt{rx + (p.x * cos_th - p.y * sin_th), ry + (p.x * sin_th + p.y * cos_th)});
-        for (const Pt& p : L.transformed_footprint) {
+      if (L.footprint_clearing) {  // the transformed footprint (see above)
+        for (const Pt& p : footprint) {
           bx0 = std::min(p.x, bx0); by0 = std::min(p.y, by0);
           bx1 = std::max(p.x, bx1); by1 = std::max(p.y, by1);
+          ebx0 = std::min(ebx0, p.x); eby0 = std::min(eby0, p.y);
+          ebx1 = std::max(ebx1, p.x); eby1 = std::max(eby1, p.y);
         }
       }
       if (bx1 >= bx0) {
@@ -642,10 +680,6 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
       if (L.tbx1 >= L.tbx0 && L.tby1 >= L.tby0) {
         ebx0 = std::min(ebx0, L.tbx0); eby0 = std::min(eby0, L.tby0);
         ebx1 = std::max(ebx1, L.tbx1); eby1 = std::max(eby1, L.tby1);
-      }
-      for (const Pt& p : L.transformed_footprint) {
-        ebx0 = std::min(ebx0, p.x); eby0 = std::min(eby0, p.y);
-        ebx1 = std::max(ebx1, p.x); eby1 = std::max(eby1, p.y);
       }
     } else {  // InflationLayer::updateBounds runs on the device (needs the device-accumulated bounds)
       if (L.need_reinflation) whole_map = true;
@@ -685,8 +719,8 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
       va.box = h->d_boxes + li;
       va.mark_cells = L.d_mark_cells;
       va.ticket = h->d_ticket;
-      int vmode = 0;
-      if (L.footprint_clearing) NAVGPU_TRY(footprint_polygon(h, L, va.poly, &vmode));
+      va.poly = L.poly;
+      const int vmode = L.poly_mode;
       va.do_poly = vmode == 1;
       va.do_finalize = (int)li == last_obstacle;
       if (va.do_finalize) va.ba = ba;
@@ -717,8 +751,8 @@ int enqueue_update(navgpu_costmap* h, double rx, double ry, double ryaw) {
     oa.box = h->d_boxes + li;
     oa.mark_cells = L.d_mark_cells;
     oa.ticket = h->d_ticket;
-    int mode = 0;
-    if (L.footprint_clearing) NAVGPU_TRY(footprint_polygon(h, L, oa.poly, &mode));
+    oa.poly = L.poly;
+    const int mode = L.poly_mode;
     oa.do_poly = mode == 1;
     oa.do_finalize = (int)li == last_obstacle;
     if (oa.do_finalize) oa.ba = ba;

@@ -122,6 +122,9 @@ def cases():
         for radius in (0.55, 1.0):
             out[f"tie_{kind}_{radius}"] = tie_world(kind, radius)
     out["blocked_three_seeds"] = blocked_three_seeds
+    for case in sc.FOOTPRINT_CASES:
+        for host in sc.FOOTPRINT_HOSTS:
+            out[f"footprint_{case}_{host}"] = lambda api, c=case, h=host: sc.run_footprint_case(api, c, h)
     out["plans_11"] = plans(11, 50)
     out["plans_12"] = plans(12, 400)
     return out

@@ -629,3 +629,161 @@ def run_tp_reconfigure_case(api, case):
     else:
         w = dict(tp_open_world(), **world)
     return run_tp_sequence(api, w["grid"], w["origin"], w["pose"], w["plan"], w["vel"], ops, **create)
+
+
+# ---- footprint clearing beyond the square footprint ---------------------------------------------------------------------
+def rectangle(lx, ly, ccw=False):
+    """An lx x ly rectangle about the robot's centre, clockwise like square_footprint (ccw=True: the other way)."""
+    fp = [(lx / 2, ly / 2), (lx / 2, -ly / 2), (-lx / 2, -ly / 2), (-lx / 2, ly / 2)]
+    return fp[::-1] if ccw else fp
+
+
+def regular_polygon(n, r, ccw=True):
+    a = 0.1 + 2 * np.pi * np.arange(n) / n
+    fp = [(float(r * np.cos(t)), float(r * np.sin(t))) for t in a]
+    return fp if ccw else fp[::-1]
+
+
+def star(points, r_out, r_in):
+    a = np.pi * np.arange(2 * points) / points
+    return [(float(r * np.cos(t)), float(r * np.sin(t))) for t, r in zip(a, [r_out, r_in] * points)]
+
+
+L_SHAPE = [(-0.4, -0.4), (0.5, -0.4), (0.5, -0.1), (-0.1, -0.1), (-0.1, 0.5), (-0.4, 0.5)]
+U_SHAPE = [(-0.5, -0.4), (0.5, -0.4), (0.5, 0.5), (0.25, 0.5), (0.25, -0.15), (-0.25, -0.15), (-0.25, 0.5), (-0.5, 0.5)]
+BOWTIE = [(-0.5, -0.4), (0.5, 0.4), (0.5, -0.4), (-0.5, 0.4)]  # self-intersecting
+REPEATED = [(0.4, 0.3), (0.4, 0.3), (0.4, -0.3), (-0.4, -0.3), (-0.4, -0.3), (-0.4, -0.3), (-0.4, 0.3)]
+COLLINEAR = [(0.4, 0.3), (0.4, 0.0), (0.4, -0.3), (-0.4, -0.3), (-0.4, 0.3)]  # the first three on one line
+SLIVER = [(0.0, -0.45), (0.004, 0.0), (0.0, 0.45), (-0.004, 0.0)]  # at yaw 0 or pi every vertex in one 0.05 m column
+PI_16 = np.pi / 16
+# name: footprint, resolution, map size, yaws.  The robot stands at the centre of a cell near the middle of the map.
+FOOTPRINT_CASES = {
+    # 1137 cells at yaw 0 (inside k_obstacle_update), 10121 at pi/8 (k_polygon_clear); 13925 at pi/4 are refused
+    "rect_8x0.2": (rectangle(8.0, 0.2), 0.05, (200, 200), [0.0, PI_16, 2 * PI_16, 8 * PI_16, 10 * PI_16]),
+    "rect_8x0.2_ccw": (rectangle(8.0, 0.2, ccw=True), 0.05, (200, 200), [0.0, 2 * PI_16, 9 * PI_16]),
+    "rect_2x0.5_fine": (rectangle(2.0, 0.5), 0.0125, (240, 240), [0.0, 8 * PI_16, 16 * PI_16, 0.05]),
+    "square_cw": (square_footprint(0.45), 0.05, (90, 80), [0.0, 0.3, 4 * PI_16, 2.5]),
+    "square_ccw": (square_footprint(0.45)[::-1], 0.05, (90, 80), [0.0, 0.3, 4 * PI_16, 2.5]),
+    "triangle_ccw": (regular_polygon(3, 0.6), 0.05, (90, 80), [0.0, 1.0, 3.0]),
+    "triangle_cw": (regular_polygon(3, 0.6, ccw=False), 0.05, (90, 80), [0.0, 1.0, 3.0]),
+    "ngon16": (regular_polygon(16, 0.7), 0.05, (90, 80), [0.0, 0.2, PI_16]),
+    "ngon32": (regular_polygon(32, 0.8), 0.05, (90, 80), [0.0, 0.05, 1.3]),
+    "ngon32_large": (regular_polygon(32, 2.4), 0.05, (140, 130), [0.0, 0.7]),
+    "l_shape": (L_SHAPE, 0.05, (90, 80), [0.0, 2 * PI_16, 4.0]),
+    "u_shape": (U_SHAPE, 0.05, (90, 80), [0.0, 3 * PI_16, 3.3]),
+    "star8": (star(8, 0.7, 0.3), 0.05, (90, 80), [0.0, 0.17, 1.1]),
+    "bowtie": (BOWTIE, 0.05, (90, 80), [0.0, 0.6, 8 * PI_16]),
+    "repeated": (REPEATED, 0.05, (90, 80), [0.0, 0.4]),
+    "collinear": (COLLINEAR, 0.05, (90, 80), [0.0, 0.4, 8 * PI_16]),
+    "one_cell": (square_footprint(0.01), 0.05, (60, 50), [0.0, 0.5]),
+    # every vertex in one column (the reference's column walk, replayed), then in one row at pi/2
+    "sliver": (SLIVER, 0.05, (60, 50), [0.0, np.pi, 8 * PI_16]),
+    # 8 m tall at 0.01 m: 801 rows, past what k_obstacle_update holds, so the walk runs in k_polygon_clear
+    "sliver_tall": ([(0.0, -4.0), (0.002, 0.0), (0.0, 4.0), (-0.002, 0.0)], 0.01, (40, 880), [0.0, np.pi]),
+    "sliver_wide": ([(-4.0, 0.0), (0.0, 0.002), (4.0, 0.0), (0.0, -0.002)], 0.01, (880, 40), [0.0, np.pi]),
+    "no_vertex": ([], 0.05, (60, 50), [0.0, 1.0]),
+    "one_vertex": ([(0.2, 0.1)], 0.05, (60, 50), [0.0, 1.0]),
+    "two_vertices": ([(0.3, 0.2), (-0.3, -0.2)], 0.05, (60, 50), [0.0, 1.0]),
+}
+FOOTPRINT_HOSTS = ["obstacle", "rolling", "voxel", "single"]
+
+
+def footprint_case_pose(case, cycle, host):
+    """Robot pose of a cycle: the centre of a cell near the middle of the map; on a rolling map it drives on."""
+    fp, res, (sx, sy), yaws = FOOTPRINT_CASES[case]
+    cx, cy = sx // 2 + 0.5, sy // 2 + 0.5
+    if host == "rolling":
+        cx, cy = cx + 3.3 * cycle, cy + 1.7 * cycle
+    return cx * res, cy * res, float(yaws[cycle])
+
+
+def transform_footprint(fp, pose):
+    """transformFootprint (footprint.cpp:106-120), as both sides compute it."""
+    x, y, yaw = pose
+    c, s = np.cos(yaw), np.sin(yaw)
+    return [(x + (px * c - py * s), y + (px * s + py * c)) for px, py in fp]
+
+
+def footprint_marks(fp, pose, res, sx, sy, ox, oy, n_rays=2400):
+    """A marking point at every cell centre of the footprint's bounding box grown by three cells (on the map), and
+    n_rays clearing rays from the robot to a ring just outside that box: the obstacle kernel runs n_rays / 8 CTAs,
+    and the footprint's cells hold marks that only the polygon fill, after every mark, turns FREE."""
+    x, y = pose[0], pose[1]
+    w = transform_footprint(fp, pose) or [(x, y)]
+    xs, ys = [p[0] for p in w], [p[1] for p in w]
+    i0 = max(0, int(np.floor((min(xs) - ox) / res)) - 3)
+    i1 = min(sx, int(np.floor((max(xs) - ox) / res)) + 4)
+    j0 = max(0, int(np.floor((min(ys) - oy) / res)) - 3)
+    j1 = min(sy, int(np.floor((max(ys) - oy) / res)) + 4)
+    gx, gy = np.meshgrid(ox + (np.arange(i0, i1) + 0.5) * res, oy + (np.arange(j0, j1) + 0.5) * res)
+    pts = np.stack([gx.ravel(), gy.ravel(), np.full(gx.size, 0.5)], 1).astype(np.float32)
+    reach = float(np.hypot(max(xs) - min(xs), max(ys) - min(ys))) / 2 + 4 * res
+    a = np.linspace(0, 2 * np.pi, n_rays, endpoint=False)
+    ring = np.stack([x + reach * np.cos(a), y + reach * np.sin(a), np.full(n_rays, 0.5)], 1).astype(np.float32)
+    origin = (x, y, 0.5)
+    return [dict(origin=origin, points=ring, obstacle_range=100.0, raytrace_range=100.0, marking=False, clearing=True),
+            dict(origin=origin, points=pts, obstacle_range=100.0, raytrace_range=100.0, marking=True, clearing=False)]
+
+
+def footprint_stack(api, case, host, inflation="exact"):
+    """The stack a host of FOOTPRINT_HOSTS names, on a track_unknown map; returns (costmap, ids).
+    obstacle: static, a bare ObstacleLayer (Overwrite, never observes: its FREE cells are exactly what was cleared),
+              a marked ObstacleLayer (Max), inflation; fixed map.
+    rolling:  the same without the static layer, rolling, the policies swapped.
+    voxel:    obstacle's stack with VoxelLayers.
+    single:   static and one marked ObstacleLayer (Max), no inflation.
+    Footprints of fewer than three vertices get no inflation layer; `inflation` selects its execution
+    (INFLATION_SEMANTICS)."""
+    fp, res, (sx, sy), _ = FOOTPRINT_CASES[case]
+    rolling = host == "rolling"
+    cm = api.costmap(sx, sy, res, 0.0, 0.0, rolling=rolling, track_unknown=True)
+    ids = {}
+    if not rolling:
+        ids["static"] = cm.add_grid_layer(po.TRUE_OVERWRITE)
+    if host == "voxel":
+        ids["bare"] = cm.add_voxel_layer(1, True, 2.0)
+        ids["marked"] = cm.add_voxel_layer(0, True, 2.0)
+    elif host == "single":
+        ids["marked"] = cm.add_obstacle_layer(1, True, 2.0)
+    else:
+        ids["bare"] = cm.add_obstacle_layer(1 if rolling else 0, True, 2.0)
+        ids["marked"] = cm.add_obstacle_layer(0 if rolling else 1, True, 2.0)
+    if host != "single" and len(fp) >= 3:
+        ids["inflation"] = cm.add_inflation_layer(0.3, 3.0)
+        select_inflation(cm, ids["inflation"], inflation)
+    cm.set_footprint(fp)
+    if "static" in ids:
+        g = np.zeros((sy, sx), np.uint8)
+        g[::7, ::5] = 254
+        g[3::11, 2::9] = 128
+        cm.set_grid_layer(ids["static"], g)
+    return cm, ids
+
+
+def footprint_cycle(cm, ids, case, host, cycle):
+    """One cycle: the static layer touched whole, the marks field and its clearing rays on the marked layer."""
+    fp, res, (sx, sy), _ = FOOTPRINT_CASES[case]
+    pose = footprint_case_pose(case, cycle, host)
+    if "static" in ids:
+        cm.touch_grid_layer(ids["static"], 0, 0, sx, sy)
+    ox, oy = cm.origin()
+    if host == "rolling":  # the grids roll to the robot before the marks land
+        ox, oy = pose[0] - (sx - 0.5) * res / 2, pose[1] - (sy - 0.5) * res / 2
+    cm.set_observations(ids["marked"], footprint_marks(fp, pose, res, sx, sy, ox, oy))
+    return pose, cm.update_map(*pose)
+
+
+def run_footprint_case(api, case, host, inflation=None):
+    """Every yaw of a FOOTPRINT_CASES entry on one host, one cycle each; returns the per-cycle records."""
+    cm, ids = footprint_stack(api, case, host, inflation)
+    out = []
+    for cycle in range(len(FOOTPRINT_CASES[case][3])):
+        _, w = footprint_cycle(cm, ids, case, host, cycle)
+        rec = dict(window=w, origin=cm.origin(), master=cm.get())
+        for k in ("bare", "marked"):
+            if k in ids:
+                rec[k] = cm.get_layer(ids[k])
+                if host == "voxel":
+                    rec[k + "_voxels"] = cm.get_voxels(ids[k])
+        out.append(rec)
+    return out
