@@ -392,6 +392,43 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
  * or non-device pointers (NAVGPU_ERR_INVALID), TrajectoryPlanner fleets, use_dwa = 0 and more than 640 per-axis
  * samples by that bound (NAVGPU_ERR_UNSUPPORTED). */
 int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double* vels, navgpu_dwa_result* results);
+/* ---- Plan following on the device (DWAPlanner fleets of every kind) ---------------------------------------------
+ * DWAPlannerROS runs, every control cycle before findBestPath: LocalPlannerUtil::getLocalPlan (transformGlobalPlan to
+ * the stretch of the held global plan within max(size_x, size_y) * resolution / 2 of the robot; with prune_plan,
+ * prunePlan erases the poses the robot has passed from that local plan and as many from the front of the held global
+ * plan), returns without a command when the local plan is empty, else DWAPlanner::updatePlanAndLocalCosts.  The calls
+ * below keep each robot's global plan on the device and run that per cycle for the whole fleet without a host wait.
+ *
+ * navgpu_fleet_set_global_plans: DWAPlannerROS::setPlan for robots[k], k < n_set: the (x, y) poses
+ * plan_xy[offsets[k] .. offsets[k + 1]) (HOST memory, in the frame of the fleet's poses) become the robot's held global
+ * plan, and its oscillation flags are reset (DWAPlanner::setPlan).  Other robots keep their plans and flags; empty plans
+ * are accepted.  It may allocate and wait (a replan, <= 1 Hz); it sizes each robot's device slots so that later updates
+ * never allocate.  Refused, with the fleet unchanged: a robot out of range or given twice, offsets that do not start at
+ * 0 or that decrease, null pointers (NAVGPU_ERR_INVALID), TrajectoryPlanner fleets (NAVGPU_ERR_UNSUPPORTED). */
+int navgpu_fleet_set_global_plans(navgpu_fleet* f, int n_set, const int32_t* robots, const double* plan_xy,
+                                  const int32_t* offsets);
+/* navgpu_fleet_update_plans_device: the per-cycle plan work above for EVERY robot, whatever navgpu_fleet_set_active
+ * says (the wrappers update the plan at the goal too), with the identity transform, enqueued on the fleet's stream;
+ * the call returns without waiting.  poses [n][3] (double) and status [n] (bytes, may be null) are device memory of the
+ * fleet's device.  The kept poses go through the identity with navgpu_plans_transform's arithmetic (-0.0 becomes
+ * +0.0, as tf's multiply does).  status[r] = 1: robot r has a local plan, and its MapGrid plans, alignment scale and
+ * flags are those navgpu_fleet_set_plans would give it for that local plan and pose.  status[r] = 0: it has no global
+ * plan or its local plan came out empty; its planner state is unchanged, and the following steps leave it out as
+ * set_active would (results entry untouched, no wavefronts, no scoring) until an update gives it a local plan again
+ * (navgpu_fleet_set_plans gives every robot one).  Exception by construction: the goal-front point takes atan2 / cos /
+ * sin from CUDA, not the host libm (both within 2 ulp); everything else equals the host computation bit for bit.
+ * An update followed by navgpu_fleet_step_device, repeated with no host call in between, neither waits for the host,
+ * allocates nor copies from pageable memory, so the whole cycle can be captured in a CUDA graph.  Host calls may be
+ * mixed in and see the plans the device computed: navgpu_fleet_step, _check_trajectories, _get_plan, _set_active,
+ * _set_maps, _set_plans and _set_global_plans first wait for the fleet's stream; the update after them uploads the
+ * plans again (waiting once).  navgpu_fleet_set_plans keeps its meaning: it sets every robot's local plan directly and
+ * leaves the global plans alone; the next update replaces its result.  Refused, with the fleet unchanged: null or
+ * non-device pointers (NAVGPU_ERR_INVALID), TrajectoryPlanner fleets (NAVGPU_ERR_UNSUPPORTED). */
+int navgpu_fleet_update_plans_device(navgpu_fleet* f, const double* poses, int prune_plan, uint8_t* status);
+/* robot's held global plan after the prunes (which = 0) or the local plan of the last update (which = 1, empty when it
+ * had none), (x, y) doubles into HOST xy_out; *n_out = the number of poses; NAVGPU_ERR_CAPACITY when more than
+ * capacity (the first capacity are written).  Waits for the fleet's stream first.  For tests and debugging. */
+int navgpu_fleet_get_plan(navgpu_fleet* f, int robot, int which, double* xy_out, int capacity, int32_t* n_out);
 /* inflated local costmap of one robot, HOST size_y x size_x */
 int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out);
 int navgpu_fleet_get_oscillation_mask(navgpu_fleet* f, int robot, int* mask_out);

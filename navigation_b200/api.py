@@ -204,6 +204,9 @@ SIGNATURES = {
     "navgpu_fleet_reset_oscillation": (C.c_int, [C.c_void_p]),
     "navgpu_fleet_step": (C.c_int, [C.c_void_p, _f64p, _f64p, C.POINTER(DwaResult)]),
     "navgpu_fleet_step_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "navgpu_fleet_set_global_plans": (C.c_int, [C.c_void_p, C.c_int, _i32p, _f64p, _i32p]),
+    "navgpu_fleet_update_plans_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "navgpu_fleet_get_plan": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _f64p, C.c_int, _i32p]),
     "navgpu_fleet_get_costmap": (C.c_int, [C.c_void_p, C.c_int, _u8p]),
     "navgpu_fleet_get_oscillation_mask": (C.c_int, [C.c_void_p, C.c_int, _i32p]),
     "navgpu_fleet_create_sensing": (C.c_int, [_vpp, C.c_int, C.POINTER(DwaConfig), C.c_uint32, C.c_uint32, C.c_double,
@@ -923,6 +926,49 @@ class Fleet:
         f64, i32 = out["f64"], out["i32"]
         return dict(cost=f64[:, 0], xv=f64[:, 1], yv=f64[:, 2], thetav=f64[:, 3], best_index=i32[:, 8],
                     n_samples=i32[:, 9], n_scored=i32[:, 10], records=out["records"])
+
+    def set_global_plans(self, plans, robots=None):
+        """DWAPlannerROS::setPlan per robot (navgpu_fleet_set_global_plans): plans[k], a (k_i, 2) array (possibly
+        empty), becomes the held global plan of robots[k] (default: robot k of every robot) and resets its oscillation
+        flags; update_plans_device then follows it."""
+        robots = np.arange(self.n, dtype=np.int32) if robots is None else np.ascontiguousarray(robots, dtype=np.int32)
+        assert len(plans) == len(robots)
+        off = np.zeros(len(plans) + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(q) for q in plans])
+        xy = np.zeros((max(int(off[-1]), 1), 2))
+        if off[-1]:
+            xy[:off[-1]] = np.concatenate([np.asarray(q, dtype=np.float64).reshape(-1, 2) for q in plans])
+        self.api.check(self.lib.navgpu_fleet_set_global_plans(self.h, len(plans), _p(robots, _i32p), _p(xy, _f64p),
+                                                              _p(off, _i32p)))
+
+    def update_plans_device(self, poses, prune_plan=True):
+        """DWAPlannerROS's per-cycle plan work (getLocalPlan, prunePlan, updatePlanAndLocalCosts) for every robot on the
+        device (navgpu_fleet_update_plans_device): poses is a contiguous float64 CUDA tensor [n, 3] on the fleet's
+        device, ordered as in step_device.  Returns a CUDA uint8 tensor [n]: 1 where the robot has a local plan, 0 where
+        it has none (the following steps then leave it out).  Wrong devices, dtypes or shapes raise ValueError."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        if not isinstance(poses, torch.Tensor) or poses.dtype != torch.float64 or tuple(poses.shape) != (self.n, 3) or \
+                not poses.is_cuda or poses.device.index != self.device or not poses.is_contiguous():
+            raise ValueError(f"poses: a contiguous float64 tensor of shape ({self.n}, 3) on cuda:{self.device}")
+        status = torch.empty(self.n, dtype=torch.uint8, device=dev)
+        fleet_stream = torch.cuda.ExternalStream(self.stream(), device=dev)
+        fleet_stream.wait_stream(torch.cuda.current_stream(dev))
+        self.api.check(self.lib.navgpu_fleet_update_plans_device(self.h, poses.data_ptr(), int(bool(prune_plan)),
+                                                                 status.data_ptr()))
+        torch.cuda.current_stream(dev).wait_stream(fleet_stream)
+        return status
+
+    def plan(self, robot, which):
+        """robot's held global plan after the prunes (which = 0) or the local plan of the last update_plans_device
+        (which = 1), as a (k, 2) float64 array (navgpu_fleet_get_plan)."""
+        n = C.c_int32()
+        rc = self.lib.navgpu_fleet_get_plan(self.h, robot, which, None, 0, C.byref(n))
+        if rc != 4:  # NAVGPU_ERR_CAPACITY: the plan has points
+            self.api.check(rc)
+        out = np.zeros((max(n.value, 1), 2))
+        self.api.check(self.lib.navgpu_fleet_get_plan(self.h, robot, which, _p(out, _f64p), out.shape[0], C.byref(n)))
+        return out[:n.value].copy()
 
     def step_tp_device(self, poses, vels, out=None):
         """step() of a TrajectoryPlanner fleet on the device (navgpu_fleet_step_tp_device), as step_device is for

@@ -27,20 +27,16 @@ struct P2 {
 void adjust_plan_resolution(const std::vector<P2>& in, std::vector<P2>& out, double resolution) {
   out.clear();
   if (in.empty()) return;
-  double last_x = in[0].x, last_y = in[0].y;
   out.push_back(in[0]);
-  const double min_sq_resolution = resolution * resolution * 4;
   for (size_t i = 1; i < in.size(); ++i) {
-    const double loop_x = in[i].x, loop_y = in[i].y;
-    const double sqdist = (loop_x - last_x) * (loop_x - last_x) + (loop_y - last_y) * (loop_y - last_y);
-    if (sqdist > min_sq_resolution) {
-      const int steps = ((sqrt(sqdist) - sqrt(min_sq_resolution)) / resolution) - 1;
-      const double deltax = (loop_x - last_x) / steps, deltay = (loop_y - last_y) / steps;
-      for (int j = 1; j < steps; ++j) out.push_back(P2{last_x + j * deltax, last_y + j * deltay});
+    const P2 last = in[i - 1];
+    const int steps = adjust_plan_steps(last.x, last.y, in[i].x, in[i].y, resolution);
+    for (int j = 1; j < steps; ++j) {
+      P2 p;
+      adjust_plan_point(last.x, last.y, in[i].x, in[i].y, steps, j, &p.x, &p.y);
+      out.push_back(p);
     }
     out.push_back(in[i]);
-    last_x = loop_x;
-    last_y = loop_y;
   }
 }
 
@@ -76,13 +72,10 @@ bool update_plan_and_local_costs(DwaPlans& p, const navgpu_dwa_config& c, double
   adjust_plan_resolution(p.plan, p.adjusted[0], res);
   const P2 goal = p.plan.back();
   const float pos[3] = {(float)pose[0], (float)pose[1], (float)pose[2]};
-  const double sq_dist = (pos[0] - goal.x) * (pos[0] - goal.x) + (pos[1] - goal.y) * (pos[1] - goal.y);
   std::vector<P2> front = p.plan;
-  const double angle_to_goal = atan2(goal.y - pos[1], goal.x - pos[0]);
-  front.back().x = front.back().x + c.forward_point_distance * cos(angle_to_goal);
-  front.back().y = front.back().y + c.forward_point_distance * sin(angle_to_goal);
+  goal_front_point(goal.x, goal.y, pos, c.forward_point_distance, &front.back().x, &front.back().y);
   adjust_plan_resolution(front, p.adjusted[1], res);
-  const bool align_replaced = sq_dist > c.forward_point_distance * c.forward_point_distance * c.cheat_factor;
+  const bool align_replaced = alignment_replaced(goal.x, goal.y, pos, c.forward_point_distance, c.cheat_factor);
   if (align_replaced) {
     p.alignment_scale = dwa_scales(c, res).alignment;
     p.adjusted[2] = p.adjusted[0];
@@ -997,7 +990,25 @@ struct navgpu_fleet {
   std::vector<FleetRobot> h_check;
   char* d_check = nullptr;
   size_t check_capacity = 0;
+  // plan following (navgpu_fleet_set_global_plans, navgpu_fleet_update_plans_device).  Per robot: its held global plan
+  // (current from h_slots[r].first unless plans_on_device), the local plan of the last update, and whether that update
+  // gave it one (0: the steps leave it out, as set_active would).  The plan slots live in d_plan_buf; while
+  // plans_on_device, device updates ran since the host last brought the robots' plans back (fleet_plans_to_host) and
+  // the device's MapGrid records and flags are the current ones.
+  std::vector<std::vector<P2>> global_plans;
+  std::vector<int> adjusted_bound;  // adjusted length of the plan as set: no local plan drawn from it adjusts to more
+  std::vector<std::vector<P2>> last_local;
+  std::vector<uint8_t> has_local_plan;
+  std::vector<FleetPlanSlot> h_slots;
+  FleetPlanSlot* d_slots = nullptr;
+  double2* d_plan_buf = nullptr;
+  size_t plan_buf_capacity = 0;  // points
+  bool slots_dirty = true;       // the slots must be laid out and filled again (new global plans, set_plans)
+  bool plans_on_device = false;
 };
+
+// whether the steps plan robot r: set_active's mask, and a local plan from the last plan update
+static bool planned(const navgpu_fleet* f, int r) { return f->active[r] && f->has_local_plan[r]; }
 
 // what every fleet holds for its planner side: the DWAPlanner parameters and critic scales ...
 static void init_planner_scalars(navgpu_fleet* f, int n_robots, const navgpu_dwa_config* cfg, uint32_t size_x,
@@ -1028,6 +1039,11 @@ static int alloc_planner_side(navgpu_fleet* f) {
   f->plans.resize(n_robots);
   f->h_robots.resize(n_robots);
   f->active.assign(n_robots, 1);
+  f->global_plans.resize(n_robots);
+  f->adjusted_bound.assign(n_robots, 0);
+  f->last_local.resize(n_robots);
+  f->has_local_plan.assign(n_robots, 1);
+  f->h_slots.assign(n_robots, FleetPlanSlot{});
   return NAVGPU_OK;
 }
 
@@ -1147,7 +1163,7 @@ static void fleet_dwa_jobs(const navgpu_fleet* f, int r, MapGridJob* job) {
     job[3].dist = dist;
     job[3].skip = 1;
   }
-  if (!f->active[r])  // left out of the search: its grids stay as its last planning step left them
+  if (!planned(f, r))  // left out of the search: its grids stay as its last planning step left them
     for (int k = 0; k < 4; ++k) job[k].skip = 1;
 }
 
@@ -1157,6 +1173,142 @@ static int fleet_dwa_upload_plans(navgpu_fleet* f) {
   auto plan_at = [&](size_t i) -> const std::vector<P2>& { return f->plans[i / 3].adjusted[i % 3]; };
   NAVGPU_TRY(fleet_upload_plans(size_t(3) * f->n, plan_at, f->plan_off, &f->d_plans, &f->plans_capacity, f->stream));
   f->plans_dirty = false;
+  return NAVGPU_OK;
+}
+
+// the per-robot flags of device steps and the pinned staging of the MapGrid records, allocated once
+static int fleet_records_alloc(navgpu_fleet* f) {
+  if (!f->d_flags) NAVGPU_CUDA(cudaMalloc(&f->d_flags, f->n));
+  if (!f->h_records_stage) NAVGPU_CUDA(cudaMallocHost(&f->h_records_stage, (sizeof(FleetRobot) + 1) * f->n));
+  if (!f->ev_records_stage) NAVGPU_CUDA(cudaEventCreateWithFlags(&f->ev_records_stage, cudaEventDisableTiming));
+  return NAVGPU_OK;
+}
+
+// after set_plans, set_active or set_maps: every robot's MapGrid record and flags from the host, through the staging
+static int fleet_dwa_upload_records(navgpu_fleet* f) {
+  if (!f->records_dirty && !f->grids_dirty) return NAVGPU_OK;
+  const int n = f->n;
+  FleetRobot* stage = reinterpret_cast<FleetRobot*>(f->h_records_stage);
+  uint8_t* flags = reinterpret_cast<uint8_t*>(stage + n);
+  NAVGPU_CUDA(cudaEventSynchronize(f->ev_records_stage));  // the previous upload from the staging has been read
+  for (int r = 0; r < n; ++r) {
+    FleetRobot& R = f->h_robots[r];
+    R.grids.g = DwaGeom{f->d_master + size_t(r) * f->stride * f->pitch, f->sx, f->sy, f->pitch, f->res, f->origins[2 * r],
+                        f->origins[2 * r + 1], 1.0 / f->res};
+    fleet_dwa_jobs(f, r, R.grids.job);
+    R.scale_alignment = f->plans[r].alignment_scale;
+    stage[r] = R;
+    flags[r] = (planned(f, r) ? kFleetActive : 0) | (f->active[r] ? kFleetSetActive : 0) |
+               (f->plans[r].align_is_path ? kFleetAligned : 0);
+  }
+  NAVGPU_CUDA(cudaMemcpyAsync(f->d_robots, stage, sizeof(FleetRobot) * n, cudaMemcpyHostToDevice, f->stream));
+  NAVGPU_CUDA(cudaMemcpyAsync(f->d_flags, flags, n, cudaMemcpyHostToDevice, f->stream));
+  NAVGPU_CUDA(cudaEventRecord(f->ev_records_stage, f->stream));
+  f->records_dirty = f->grids_dirty = false;
+  return NAVGPU_OK;
+}
+
+// the local plan poses at .. at + count of robot r's held global plan, through the identity transform
+static std::vector<P2> fleet_local_plan(const navgpu_fleet* f, int r, int at, int count) {
+  std::vector<P2> out(count);
+  for (int k = 0; k < count; ++k) {
+    const P2 p = f->global_plans[r][at + k];
+    identity_transform(p.x, p.y, &out[k].x, &out[k].y);
+  }
+  return out;
+}
+
+// Brings the robots' plans back to the host after device plan updates (a wait, and copies of the plans the updates
+// changed); every host call that reads the plans or rewrites the MapGrid records calls this first.  The host then
+// holds the current plans and rebuilds the records from them; the next device update uploads what it needs.
+static int fleet_plans_to_host(navgpu_fleet* f) {
+  if (!f->plans_on_device) return NAVGPU_OK;
+  NAVGPU_CUDA(cudaSetDevice(f->device));
+  NAVGPU_CUDA(cudaMemcpyAsync(f->h_slots.data(), f->d_slots, sizeof(FleetPlanSlot) * f->n, cudaMemcpyDeviceToHost, f->stream));
+  NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
+  for (int r = 0; r < f->n; ++r) {
+    FleetPlanSlot& S = f->h_slots[r];
+    f->last_local[r] = fleet_local_plan(f, r, S.local_at, S.local_count);
+    f->has_local_plan[r] = S.status;
+    if (!S.updated) continue;
+    DwaPlans& p = f->plans[r];
+    p.plan = fleet_local_plan(f, r, S.plan_at, S.plan_count);
+    const long long at[3] = {S.path_at, S.front_at, S.align_at};
+    const int count[3] = {S.path_count, S.front_count, S.align_count};
+    for (int k = 0; k < 3; ++k) {
+      p.adjusted[k].resize(count[k]);
+      if (k == 2 && S.align_is_path) p.adjusted[2] = p.adjusted[0];
+      else if (count[k])
+        NAVGPU_CUDA(cudaMemcpyAsync(p.adjusted[k].data(), f->d_plan_buf + at[k], sizeof(P2) * count[k],
+                                    cudaMemcpyDeviceToHost, f->stream));
+    }
+    p.alignment_scale = S.alignment_scale;
+    p.align_is_path = S.align_is_path;
+    S.updated = 0;
+  }
+  NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
+  f->plans_on_device = false;
+  f->plans_dirty = f->grids_dirty = f->records_dirty = true;
+  return NAVGPU_OK;
+}
+
+// Before the first device plan update after host calls: the plan slots (laid out again and filled when global plans or
+// set_plans changed them: global slots, then alignment, path and front slots), the slot records, and the host's
+// MapGrid records and flags, which the update then changes robot by robot
+static int fleet_plans_to_device(navgpu_fleet* f) {
+  const int n = f->n;
+  const int front_extra = (int)std::ceil(std::fabs(f->cfg.forward_point_distance) / f->res) + 2;
+  for (int r = 0; r < n && !f->slots_dirty; ++r)
+    if (f->plans[r].adjusted[2].size() > (size_t)f->h_slots[r].align_cap) f->slots_dirty = true;
+  if (f->slots_dirty) {
+    long long total[4] = {0, 0, 0, 0};  // global, alignment, path, front
+    for (int r = 0; r < n; ++r) {
+      FleetPlanSlot& S = f->h_slots[r];
+      std::vector<P2>& g = f->global_plans[r];
+      g.erase(g.begin(), g.begin() + S.first);  // what the prunes left
+      S.first = 0;
+      S.count = (int)g.size();
+      S.global_cap = S.count;
+      S.path_cap = f->adjusted_bound[r];
+      S.front_cap = f->adjusted_bound[r] ? f->adjusted_bound[r] + front_extra : 0;
+      S.align_cap = std::max(f->adjusted_bound[r], (int)f->plans[r].adjusted[2].size());
+      S.align_count = (int)f->plans[r].adjusted[2].size();
+      S.local_at = S.local_count = S.plan_at = S.plan_count = 0;
+      total[0] += S.global_cap; total[1] += S.align_cap; total[2] += S.path_cap; total[3] += S.front_cap;
+    }
+    long long at[4] = {0, total[0], total[0] + total[1], total[0] + total[1] + total[2]};
+    for (int r = 0; r < n; ++r) {
+      FleetPlanSlot& S = f->h_slots[r];
+      S.global_at = at[0]; S.align_at = at[1]; S.path_at = at[2]; S.front_at = at[3];
+      at[0] += S.global_cap; at[1] += S.align_cap; at[2] += S.path_cap; at[3] += S.front_cap;
+    }
+    const size_t need = size_t(at[3]);
+    if (need > f->plan_buf_capacity) {
+      cudaFree(f->d_plan_buf);
+      f->d_plan_buf = nullptr;
+      f->plan_buf_capacity = 0;
+      NAVGPU_CUDA(cudaMalloc(&f->d_plan_buf, std::max<size_t>(need, 1) * sizeof(double2)));
+      f->plan_buf_capacity = need;
+    }
+    // the global and alignment slots are filled; the path and front slots are written by every update before use
+    std::vector<P2> image(size_t(total[0] + total[1]));
+    for (int r = 0; r < n; ++r) {
+      const FleetPlanSlot& S = f->h_slots[r];
+      std::copy(f->global_plans[r].begin(), f->global_plans[r].end(), image.begin() + S.global_at);
+      std::copy(f->plans[r].adjusted[2].begin(), f->plans[r].adjusted[2].end(), image.begin() + S.align_at);
+    }
+    if (!image.empty())
+      NAVGPU_CUDA(cudaMemcpyAsync(f->d_plan_buf, image.data(), image.size() * sizeof(P2), cudaMemcpyHostToDevice, f->stream));
+    NAVGPU_CUDA(cudaStreamSynchronize(f->stream));  // pageable source
+    f->slots_dirty = false;
+  }
+  if (!f->d_slots) NAVGPU_CUDA(cudaMalloc(&f->d_slots, sizeof(FleetPlanSlot) * n));
+  NAVGPU_CUDA(cudaMemcpyAsync(f->d_slots, f->h_slots.data(), sizeof(FleetPlanSlot) * n, cudaMemcpyHostToDevice, f->stream));
+  NAVGPU_TRY(fleet_dwa_upload_plans(f));
+  NAVGPU_TRY(fleet_records_alloc(f));
+  NAVGPU_TRY(fleet_dwa_upload_records(f));
+  NAVGPU_CUDA(cudaStreamSynchronize(f->stream));  // pageable h_slots
+  f->plans_on_device = true;
   return NAVGPU_OK;
 }
 
@@ -1244,6 +1396,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
   cudaFree(f->d_check);
   cudaFreeHost(f->h_results);
   cudaFree(f->d_state); cudaFree(f->d_slot_samples); cudaFree(f->d_flags);
+  cudaFree(f->d_slots); cudaFree(f->d_plan_buf);
   if (f->h_state) cudaFreeHost(f->h_state);
   if (f->h_records_stage) cudaFreeHost(f->h_records_stage);
   if (f->ev_records_stage) cudaEventDestroy(f->ev_records_stage);
@@ -1258,6 +1411,7 @@ int navgpu_fleet_destroy(navgpu_fleet* f) {
 int navgpu_fleet_set_maps(navgpu_fleet* f, const uint8_t* raw_maps, const double* origins_xy) {
   if (!f || !raw_maps || !origins_xy) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   if (f->sensing) return fail(NAVGPU_ERR_INVALID, "a sensing fleet builds its maps from scans (navgpu_fleet_set_scans)");
+  NAVGPU_TRY(fleet_plans_to_host(f));
   NAVGPU_CUDA(cudaSetDevice(f->device));
   f->origins.assign(origins_xy, origins_xy + size_t(2) * f->n);
   f->grids_dirty = true;  // the robots' map origins changed
@@ -1283,6 +1437,7 @@ int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* p
   if (!f || !poses || !plan_xy || !plan_offsets) return fail(NAVGPU_ERR_INVALID, "bad arguments");
   f->started = true;
   if (f->tp) return fleet_tp_set_plans(f, plan_xy, plan_offsets);
+  NAVGPU_TRY(fleet_plans_to_host(f));
   for (int r = 0; r < f->n; ++r) {
     const int b = plan_offsets[r], e = plan_offsets[r + 1];
     if (e <= b) return fail(NAVGPU_ERR_INVALID, "robot %d has an empty plan", r);
@@ -1292,10 +1447,12 @@ int navgpu_fleet_set_plans(navgpu_fleet* f, const double* poses, const double* p
       p.adjusted[2] = p.adjusted[0];
       p.align_is_path = true;
     }
+    f->has_local_plan[r] = 1;
   }
   f->plans_dirty = true;
   f->grids_dirty = true;
   f->records_dirty = true;
+  f->slots_dirty = true;  // the alignment plans changed
   return NAVGPU_OK;
 }
 
@@ -1314,6 +1471,7 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
   if (f->tp) return fail(NAVGPU_ERR_INVALID, "a TrajectoryPlanner fleet steps with navgpu_fleet_step_tp");
   f->started = true;
   NAVGPU_TRY(fleet_state_to_host(f));
+  NAVGPU_TRY(fleet_plans_to_host(f));
   NAVGPU_CUDA(cudaSetDevice(f->device));
   const navgpu_dwa_config& c = f->cfg;
   const int n = f->n;
@@ -1334,7 +1492,7 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
   int max_samples = 0;
   for (int r = 0; r < n; ++r) {
     FleetRobot& R = f->h_robots[r];
-    if (!f->active[r]) {  // no samples: its scoring CTAs exit at once
+    if (!planned(f, r)) {  // no samples: its scoring CTAs exit at once
       R.nx = R.ny = R.nth = 0;
       R.samples_offset = (int)samples.size();
       continue;
@@ -1392,7 +1550,7 @@ int navgpu_fleet_step(navgpu_fleet* f, const double* poses, const double* vels, 
 
   // ---- host epilogue per active robot: result_traj_ bookkeeping + oscillation flags
   for (int r = 0; r < n; ++r) {
-    if (!f->active[r]) continue;
+    if (!planned(f, r)) continue;
     const FleetRobot& R = f->h_robots[r];
     FleetDwaState& S = f->h_state[r];
     apply_dwa_result(f->h_results[r], c, poses + 3 * r, R.nx * R.ny * R.nth, S.res_v, S.osc, &results[r]);
@@ -1423,17 +1581,16 @@ int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double*
   if (slot * n > 0x7fffffffLL || bpr * n > 0x7fffffffLL) return fail(NAVGPU_ERR_UNSUPPORTED, "too many samples in one fleet launch");
   if (f->records_dirty)
     for (int r = 0; r < n; ++r)
-      if (f->plans[r].plan.empty()) return fail(NAVGPU_ERR_INVALID, "robot %d has no plan (navgpu_fleet_set_plans)", r);
+      if (f->has_local_plan[r] && f->plans[r].plan.empty())
+        return fail(NAVGPU_ERR_INVALID, "robot %d has no plan (navgpu_fleet_set_plans)", r);
   NAVGPU_CUDA(cudaSetDevice(f->device));
 
   // buffers of device steps: sized at the first one, so later ones do not allocate
   if (!f->d_state) {
     NAVGPU_CUDA(cudaMalloc(&f->d_state, sizeof(FleetDwaState) * n));
     NAVGPU_CUDA(cudaMalloc(&f->d_slot_samples, sizeof(float) * slot * n));
-    NAVGPU_CUDA(cudaMalloc(&f->d_flags, n));
-    NAVGPU_CUDA(cudaMallocHost(&f->h_records_stage, (sizeof(FleetRobot) + 1) * n));
-    NAVGPU_CUDA(cudaEventCreateWithFlags(&f->ev_records_stage, cudaEventDisableTiming));
   }
+  NAVGPU_TRY(fleet_records_alloc(f));
   const size_t blocks = size_t(bpr) * n;
   if (blocks > f->blocks_capacity) {
     cudaFree(f->d_block_cost);
@@ -1458,24 +1615,9 @@ int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double*
     NAVGPU_CUDA(cudaMemcpyAsync(f->d_state, f->h_state, sizeof(FleetDwaState) * n, cudaMemcpyHostToDevice, f->stream));
     f->state_on_device = true;
   }
-  if (f->records_dirty || f->grids_dirty) {  // set_plans, set_active or set_maps ran: the MapGrid records and flags
-    FleetRobot* stage = reinterpret_cast<FleetRobot*>(f->h_records_stage);
-    uint8_t* flags = reinterpret_cast<uint8_t*>(stage + n);
-    NAVGPU_CUDA(cudaEventSynchronize(f->ev_records_stage));  // the previous upload from the staging has been read
-    for (int r = 0; r < n; ++r) {
-      FleetRobot& R = f->h_robots[r];
-      R.grids.g = DwaGeom{f->d_master + size_t(r) * f->stride * f->pitch, f->sx, f->sy, f->pitch, f->res, f->origins[2 * r],
-                          f->origins[2 * r + 1], 1.0 / f->res};
-      fleet_dwa_jobs(f, r, R.grids.job);
-      R.scale_alignment = f->plans[r].alignment_scale;
-      stage[r] = R;
-      flags[r] = (f->active[r] ? kFleetActive : 0) | (f->plans[r].align_is_path ? kFleetAligned : 0);
-    }
-    NAVGPU_CUDA(cudaMemcpyAsync(f->d_robots, stage, sizeof(FleetRobot) * n, cudaMemcpyHostToDevice, f->stream));
-    NAVGPU_CUDA(cudaMemcpyAsync(f->d_flags, flags, n, cudaMemcpyHostToDevice, f->stream));
-    NAVGPU_CUDA(cudaEventRecord(f->ev_records_stage, f->stream));
-    f->records_dirty = f->grids_dirty = false;
-  }
+  // set_plans, set_active or set_maps ran: the MapGrid records and flags (after device plan updates they are current on
+  // the device, and the host calls that change them bring the plans back first)
+  NAVGPU_TRY(fleet_dwa_upload_records(f));
 
   const unsigned robot_ctas = (unsigned)((n + kFleetRobotThreads - 1) / kFleetRobotThreads);
   FleetPrepareArgs pa;
@@ -1502,6 +1644,89 @@ int navgpu_fleet_step_device(navgpu_fleet* f, const double* poses, const double*
   return NAVGPU_OK;
 }
 
+// DWAPlannerROS::setPlan for robots[k], k < n_set: plan k becomes the robot's held global plan (see navgpu.h)
+int navgpu_fleet_set_global_plans(navgpu_fleet* f, int n_set, const int32_t* robots, const double* plan_xy,
+                                  const int32_t* offsets) {
+  if (!f || n_set < 0 || !robots || !plan_xy || !offsets) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->tp) return fail(NAVGPU_ERR_UNSUPPORTED, "global plans are followed by DWAPlanner fleets only");
+  if (offsets[0] != 0) return fail(NAVGPU_ERR_INVALID, "plan offsets must start at 0");
+  std::vector<uint8_t> seen(f->n, 0);
+  for (int k = 0; k < n_set; ++k) {
+    const int r = robots[k];
+    if (r < 0 || r >= f->n) return fail(NAVGPU_ERR_INVALID, "robot %d out of range", r);
+    if (seen[r]) return fail(NAVGPU_ERR_INVALID, "robot %d given twice", r);
+    seen[r] = 1;
+    if (offsets[k + 1] < offsets[k]) return fail(NAVGPU_ERR_INVALID, "plan offsets must not decrease");
+  }
+  NAVGPU_TRY(fleet_plans_to_host(f));
+  NAVGPU_TRY(fleet_state_to_host(f));
+  for (int k = 0; k < n_set; ++k) {
+    const int r = robots[k];
+    std::vector<P2>& g = f->global_plans[r];
+    g.resize(offsets[k + 1] - offsets[k]);
+    for (size_t i = 0; i < g.size(); ++i) g[i] = P2{plan_xy[2 * (offsets[k] + i)], plan_xy[2 * (offsets[k] + i) + 1]};
+    f->h_slots[r].first = 0;
+    f->h_slots[r].count = (int)g.size();
+    std::vector<P2> adjusted;
+    adjust_plan_resolution(g, adjusted, f->res);
+    f->adjusted_bound[r] = (int)adjusted.size();
+    f->h_state[r].osc.reset();  // DWAPlanner::setPlan, dwa_planner.cpp:204-207
+  }
+  f->slots_dirty = true;
+  f->started = true;
+  return NAVGPU_OK;
+}
+
+// LocalPlannerUtil::getLocalPlan + DWAPlanner::updatePlanAndLocalCosts for every robot, on the fleet's stream
+int navgpu_fleet_update_plans_device(navgpu_fleet* f, const double* poses, int prune_plan, uint8_t* status) {
+  if (!f || !poses) return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->tp) return fail(NAVGPU_ERR_UNSUPPORTED, "global plans are followed by DWAPlanner fleets only");
+  if (!on_device(poses, f->device) || (status && !on_device(status, f->device)))
+    return fail(NAVGPU_ERR_INVALID, "poses and status must be device memory of device %d", f->device);
+  NAVGPU_CUDA(cudaSetDevice(f->device));
+  if (!f->plans_on_device) NAVGPU_TRY(fleet_plans_to_device(f));
+  f->started = true;
+  FleetPlanArgs a;
+  a.slots = f->d_slots;
+  a.buf = f->d_plan_buf;
+  a.poses = poses;
+  a.status = status;
+  a.robots = f->d_robots;
+  a.flags = f->d_flags;
+  a.dist = f->d_dist;
+  a.cells = size_t(f->sx) * f->sy;
+  a.threshold = std::max(f->sx * f->res / 2.0, f->sy * f->res / 2.0);  // goal_functions.cpp:114-115
+  a.res = f->res;
+  a.forward_point_distance = f->cfg.forward_point_distance;
+  a.cheat_factor = f->cfg.cheat_factor;
+  a.scale_alignment = f->scales.alignment;
+  a.prune = prune_plan ? 1 : 0;
+  a.n = f->n;
+  k_fleet_update_plans<<<(f->n + kFleetPlanWarps - 1) / kFleetPlanWarps, kFleetPlanWarps * 32, 0, f->stream>>>(a);
+  NAVGPU_LAUNCHED(1);
+  NAVGPU_CUDA(cudaGetLastError());
+  return NAVGPU_OK;
+}
+
+int navgpu_fleet_get_plan(navgpu_fleet* f, int robot, int which, double* xy_out, int capacity, int32_t* n_out) {
+  if (!f || robot < 0 || robot >= f->n || which < 0 || which > 1 || capacity < 0 || (capacity > 0 && !xy_out) || !n_out)
+    return fail(NAVGPU_ERR_INVALID, "bad arguments");
+  if (f->tp) return fail(NAVGPU_ERR_UNSUPPORTED, "global plans are followed by DWAPlanner fleets only");
+  NAVGPU_CUDA(cudaSetDevice(f->device));
+  FleetPlanSlot S = f->h_slots[robot];
+  if (f->plans_on_device)
+    NAVGPU_CUDA(cudaMemcpyAsync(&S, f->d_slots + robot, sizeof(S), cudaMemcpyDeviceToHost, f->stream));
+  NAVGPU_CUDA(cudaStreamSynchronize(f->stream));
+  const std::vector<P2>& g = f->global_plans[robot];
+  const std::vector<P2> v = which == 0 ? std::vector<P2>(g.begin() + S.first, g.begin() + S.first + S.count)
+                            : f->plans_on_device ? fleet_local_plan(f, robot, S.local_at, S.local_count)
+                                                 : f->last_local[robot];
+  *n_out = (int32_t)v.size();
+  const size_t n = std::min(v.size(), (size_t)capacity);
+  if (n) memcpy(xy_out, v.data(), n * sizeof(P2));
+  return v.size() > (size_t)capacity ? fail(NAVGPU_ERR_CAPACITY, "xy_out holds %d of %zu points", capacity, v.size()) : NAVGPU_OK;
+}
+
 // inflated local costmap of one robot (HOST, size_y x size_x), for parity checks
 int navgpu_fleet_get_costmap(navgpu_fleet* f, int robot, uint8_t* host_out) {
   if (!f || robot < 0 || robot >= f->n || !host_out) return fail(NAVGPU_ERR_INVALID, "bad arguments");
@@ -1522,6 +1747,11 @@ int navgpu_fleet_set_active(navgpu_fleet* f, const uint8_t* active) {
   if (active)
     for (int r = 0; r < f->n; ++r)
       if (active[r] > 1) return fail(NAVGPU_ERR_INVALID, "active[%d] is %d, not 0 or 1", r, (int)active[r]);
+  for (int r = 0; r < f->n; ++r)
+    if ((active ? active[r] : 1) != f->active[r]) {  // the records change: from the current plans
+      NAVGPU_TRY(fleet_plans_to_host(f));
+      break;
+    }
   for (int r = 0; r < f->n; ++r) {
     const uint8_t a = active ? active[r] : 1;
     if (a != f->active[r]) f->grids_dirty = f->records_dirty = true;  // the robot's MapGrid jobs change (skip)
@@ -1542,6 +1772,7 @@ int navgpu_fleet_check_trajectories(navgpu_fleet* f, const double* poses, const 
   for (int r = 0; r < f->n; ++r)
     if (offsets[r + 1] > offsets[r] && !f->h_state[r].planned)
       return fail(NAVGPU_ERR_INVALID, "robot %d has candidates but was never active in a step", r);
+  NAVGPU_TRY(fleet_plans_to_host(f));
   NAVGPU_CUDA(cudaSetDevice(f->device));
   if (f->tp) return fleet_tp_check(f, poses, vels, offsets, vel_samples, costs_out);
   const int n = f->n, total = offsets[n];

@@ -872,6 +872,47 @@ __host__ __device__ inline void apply_dwa_result(const DwaDeviceResult& d, const
   out->n_scored = d.n_scored;
 }
 
+// MapGrid::adjustPlanResolution's arithmetic for one pair of neighbouring plan points (map_grid.cpp:135-171), shared
+// by the host (adjust_plan_resolution) and the device plan update (k_fleet_update_plans): the `steps` of the pair
+// (last -> next; points 1 .. steps - 1 are inserted between them, none when steps < 2) and the j-th inserted point.
+// sqrt(min_sq_resolution) as the reference writes it, int truncation of the step count.
+__host__ __device__ inline int adjust_plan_steps(double last_x, double last_y, double x, double y, double resolution) {
+  const double min_sq_resolution = resolution * resolution * 4;
+  const double sqdist = (x - last_x) * (x - last_x) + (y - last_y) * (y - last_y);
+  if (!(sqdist > min_sq_resolution)) return 0;
+  const int steps = ((sqrt(sqdist) - sqrt(min_sq_resolution)) / resolution) - 1;
+  return steps;
+}
+__host__ __device__ inline void adjust_plan_point(double last_x, double last_y, double x, double y, int steps, int j,
+                                                  double* px, double* py) {
+  const double deltax = (x - last_x) / steps, deltay = (y - last_y) / steps;
+  *px = last_x + j * deltax;
+  *py = last_y + j * deltay;
+}
+
+// plan_to_global_transform * pose for the identity transform, evaluated as navgpu_plans_transform (and tf) evaluate
+// any transform: basis row . (x, y, 0) + origin, left to right.  Not a no-op: -0.0 comes out as +0.0.
+__host__ __device__ inline void identity_transform(double x, double y, double* ox, double* oy) {
+  const double one = 1.0, zero = 0.0;
+  *ox = one * x + zero * y + zero * zero + zero;
+  *oy = zero * x + one * y + zero * zero + zero;
+}
+
+// DWAPlanner::updatePlanAndLocalCosts (dwa_planner.cpp:262-285) at a robot at pos (floats, as Eigen::Vector3f) whose
+// local plan ends at (gx, gy): the goal-front plan's last point, pushed forward_point_distance along the bearing from
+// the robot to the goal, and whether the alignment critic gets the path's poses (else scale 0, poses kept)
+__host__ __device__ inline void goal_front_point(double gx, double gy, const float pos[2], double forward_point_distance,
+                                                 double* fx, double* fy) {
+  const double angle_to_goal = atan2(gy - pos[1], gx - pos[0]);
+  *fx = gx + forward_point_distance * cos(angle_to_goal);
+  *fy = gy + forward_point_distance * sin(angle_to_goal);
+}
+__host__ __device__ inline bool alignment_replaced(double gx, double gy, const float pos[2], double forward_point_distance,
+                                                   double cheat_factor) {
+  const double sq_dist = (pos[0] - gx) * (pos[0] - gx) + (pos[1] - gy) * (pos[1] - gy);
+  return sq_dist > forward_point_distance * forward_point_distance * cheat_factor;
+}
+
 // What a DWAPlanner fleet keeps per robot from one step to the next: the oscillation flags, result_traj_'s
 // velocities, whether a step planned the robot (its distance grids hold that step's wavefronts) and whether its
 // alignment grid was its path grid then, and a sensing fleet's rolled origin.  The fleet holds a host and a device
@@ -1823,6 +1864,200 @@ __global__ void __launch_bounds__(kFleetRobotThreads) k_fleet_apply(navgpu_dwa_c
   S.aliased = (flags[r] & kFleetAligned) ? 1 : 0;
   state[r] = S;
   results[r] = out;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Plan following on the device (navgpu_fleet_update_plans_device): DWAPlannerROS's per-cycle plan work for every
+// robot -- transformGlobalPlan with the identity transform, prunePlan, then DWAPlanner::updatePlanAndLocalCosts -- with
+// the results written straight into the robot's MapGrid record and flags.
+constexpr uint8_t kFleetSetActive = 4;  // per-robot flag: navgpu_fleet_set_active's mask (kFleetActive adds "has a local plan")
+constexpr int kFleetPlanWarps = 8;      // robots (one warp each) per CTA
+
+// A robot's plans in the fleet's plan buffer (double2 points).  The slots are sized by navgpu_fleet_set_global_plans
+// so that no update outgrows them; the held global plan never moves in its slot, a prune advances `first`.
+struct FleetPlanSlot {
+  long long global_at, path_at, front_at, align_at;  // slot starts, in points
+  int global_cap, path_cap, front_cap, align_cap;
+  int first, count;                // the held global plan: global_at + first .. + count
+  int local_at, local_count;       // the last update's local plan: global slot indices (before the transform)
+  int plan_at, plan_count;         // the same for the last update that had a local plan (the planner's plan)
+  int path_count, front_count, align_count;  // the resolution-adjusted plans (DwaPlans::adjusted)
+  double alignment_scale;
+  uint8_t status, align_is_path, updated;  // updated: a local plan was set since the host last read the slot
+};
+
+struct FleetPlanArgs {
+  FleetPlanSlot* slots;
+  double2* buf;
+  const double* poses;  // [n][3], device memory
+  uint8_t* status;      // [n] or null
+  FleetRobot* robots;
+  uint8_t* flags;
+  uint32_t* dist;  // n x 4 x cells
+  size_t cells;
+  double threshold, res, forward_point_distance, cheat_factor, scale_alignment;
+  int prune, n;
+};
+
+// One warp per robot.  The searches of transformGlobalPlan and prunePlan take the first lane whose pose qualifies in
+// each 32-pose chunk (ballot); adjustPlanResolution's output is placed by a warp prefix sum over the per-pair point
+// counts, and each lane writes its pairs' points.  The front plan equals the path plan but for its last pair.
+__global__ void __launch_bounds__(kFleetPlanWarps * 32) k_fleet_update_plans(FleetPlanArgs a) {
+  const int r = blockIdx.x * kFleetPlanWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (r >= a.n) return;
+  constexpr unsigned kAll = 0xffffffffu;
+  FleetPlanSlot S = a.slots[r];
+  const double2* g = a.buf + S.global_at + S.first;  // the held global plan
+  const int first0 = S.first;
+  const double rx = a.poses[3 * r], ry = a.poses[3 * r + 1];
+  auto first_where = [&](int from, int to, auto pred) {  // first i in [from, to) with pred(i), else to
+    for (int base = from; base < to; base += 32) {
+      const int i = base + lane;
+      const unsigned m = __ballot_sync(kAll, i < to && pred(i));
+      if (m) return base + __ffs(m) - 1;
+    }
+    return to;
+  };
+  // transformGlobalPlan (goal_functions.cpp:118-149): distances on the plan's own poses
+  const int n = S.count;
+  const double sq_thr = a.threshold * a.threshold;
+  auto within = [&](int i) {
+    const double2 p = g[i];
+    const double x_diff = rx - p.x, y_diff = ry - p.y;
+    return x_diff * x_diff + y_diff * y_diff <= sq_thr;
+  };
+  const int i0 = first_where(0, n, within);
+  const int i1 = i0 < n ? min(first_where(i0 + 1, n, [&](int i) { return !within(i); }), n - 1) : n - 1;
+  const int L = i0 < n ? i1 - i0 + 1 : 0;
+  auto local = [&](int k) {  // local plan pose k (before the prune), through the identity transform
+    const double2 p = g[i0 + k];
+    double2 q;
+    identity_transform(p.x, p.y, &q.x, &q.y);
+    return q;
+  };
+  // prunePlan (goal_functions.cpp:68-84): erase from the front while the pose is 1 m or more away, from the local plan
+  // and as many from the front of the held global plan
+  int e = 0;
+  if (a.prune)
+    e = first_where(0, L, [&](int k) {
+      const double2 p = local(k);
+      const double x_diff = rx - p.x, y_diff = ry - p.y;
+      return x_diff * x_diff + y_diff * y_diff < 1;
+    });
+  const int lc = L - e, local_at = first0 + i0 + e;
+  S.first += e;
+  S.count -= e;
+  S.local_at = local_at;
+  S.local_count = lc;
+  FleetRobot& R = a.robots[r];
+  const uint8_t set_active = a.flags[r] & kFleetSetActive;
+  if (lc == 0) {  // no local plan: computeVelocityCommands returns before updatePlanAndLocalCosts; the robot sits out
+    if (lane == 0) {
+      S.status = 0;
+      a.slots[r] = S;
+      for (int k = 0; k < 4; ++k) R.grids.job[k].skip = 1;
+      a.flags[r] = set_active | (a.flags[r] & kFleetAligned);
+      if (a.status) a.status[r] = 0;
+    }
+    return;
+  }
+  // updatePlanAndLocalCosts (dwa_planner.cpp:240-286) on local poses e .. L - 1
+  const double2 goal = local(L - 1);
+  const float pos[2] = {(float)a.poses[3 * r], (float)a.poses[3 * r + 1]};
+  double2 front;
+  goal_front_point(goal.x, goal.y, pos, a.forward_point_distance, &front.x, &front.y);
+  const bool replaced = alignment_replaced(goal.x, goal.y, pos, a.forward_point_distance, a.cheat_factor);
+  const bool write_align = replaced || S.align_count == 0;  // (never set before: the path's poses, as set_plans does)
+  double2* path = a.buf + S.path_at;
+  double2* fr = a.buf + S.front_at;
+  double2* al = a.buf + S.align_at;
+  bool differs = false;  // this lane saw an adjusted path point that is not the kept alignment plan's
+  auto put = [&](int idx, double2 p, bool last_pair) {  // path (and alignment) point idx; front too but on the last pair
+    if (idx < S.path_cap) path[idx] = p;
+    if (!last_pair && idx < S.front_cap) fr[idx] = p;
+    if (write_align) {
+      if (idx < S.align_cap) al[idx] = p;
+    } else if (idx >= S.align_count || __double_as_longlong(al[idx].x) != __double_as_longlong(p.x) ||
+               __double_as_longlong(al[idx].y) != __double_as_longlong(p.y)) {
+      differs = true;
+    }
+  };
+  if (lane == 0) {
+    const double2 p0 = local(e);
+    put(0, p0, lc == 1);
+    if (lc == 1 && S.front_cap > 0) fr[0] = front;
+  }
+  int done = 1, front_count = 1;  // points written before the current chunk of pairs
+  for (int base = 1; base < lc; base += 32) {
+    const int i = base + lane;  // pair (i - 1, i) of the local plan
+    int steps = 0, fsteps = 0;
+    double2 p, q;
+    if (i < lc) {
+      p = local(e + i - 1);
+      q = local(e + i);
+      steps = adjust_plan_steps(p.x, p.y, q.x, q.y, a.res);
+      if (i == lc - 1) fsteps = adjust_plan_steps(p.x, p.y, front.x, front.y, a.res);
+    }
+    const int ins = steps > 1 ? steps - 1 : 0;
+    const int cnt = i < lc ? ins + 1 : 0;
+    int incl = cnt;  // inclusive warp prefix sum of the pairs' point counts
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(kAll, incl, o);
+      if (lane >= o) incl += v;
+    }
+    if (i < lc) {
+      const int at = done + incl - cnt;
+      const bool last = i == lc - 1;
+      for (int j = 1; j < steps; ++j) {
+        double2 m;
+        adjust_plan_point(p.x, p.y, q.x, q.y, steps, j, &m.x, &m.y);
+        put(at + j - 1, m, last);
+      }
+      put(at + ins, q, last);
+      if (last) {  // the front plan's own last pair, towards the pushed goal point
+        for (int j = 1; j < fsteps; ++j) {
+          double2 m;
+          adjust_plan_point(p.x, p.y, front.x, front.y, fsteps, j, &m.x, &m.y);
+          if (at + j - 1 < S.front_cap) fr[at + j - 1] = m;
+        }
+        const int fat = at + (fsteps > 1 ? fsteps - 1 : 0);
+        if (fat < S.front_cap) fr[fat] = front;
+        front_count = fat + 1;
+      }
+    }
+    done += __shfl_sync(kAll, incl, 31);
+  }
+  front_count = __reduce_max_sync(kAll, front_count);
+  const bool align_is_path = write_align || (S.align_count == done && !__any_sync(kAll, differs));
+  if (lane != 0) return;
+  const int path_count = min(done, S.path_cap);
+  S.path_count = path_count;
+  S.front_count = min(front_count, S.front_cap);
+  if (write_align) S.align_count = min(done, S.align_cap);
+  S.alignment_scale = replaced ? a.scale_alignment : 0.0;
+  S.align_is_path = align_is_path;
+  S.status = 1;
+  S.plan_at = local_at;
+  S.plan_count = lc;
+  S.updated = 1;
+  a.slots[r] = S;
+  // the robot's record, as fleet_dwa_jobs writes it from the host plans
+  uint32_t* dist = a.dist + (size_t)r * 4 * a.cells;
+  const double* pp = reinterpret_cast<const double*>(path);
+  R.grids.job[0] = MapGridJob{pp, S.path_count, 0, dist};
+  R.grids.job[1] = MapGridJob{pp, S.path_count, 1, dist + a.cells};
+  R.grids.job[2] = MapGridJob{reinterpret_cast<const double*>(fr), S.front_count, 1, dist + 2 * a.cells};
+  R.grids.job[3] = MapGridJob{reinterpret_cast<const double*>(al), S.align_count, 0, dist + 3 * a.cells};
+  if (align_is_path) {
+    R.grids.job[3].dist = dist;
+    R.grids.job[3].skip = 1;
+  }
+  if (!set_active)
+    for (int k = 0; k < 4; ++k) R.grids.job[k].skip = 1;
+  R.scale_alignment = S.alignment_scale;
+  a.flags[r] = set_active | (set_active ? kFleetActive : 0) | (align_is_path ? kFleetAligned : 0);
+  if (a.status) a.status[r] = 1;
 }
 
 }  // namespace navgpu
